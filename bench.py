@@ -2,7 +2,7 @@
 """bench.py -- retrieve queries/sec on B200 for the SVS hot path (BASELINE.json's metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c2] [--configs c1,c5,c3,c4 | --only]
-                    [--impl reference]
+                    [--impl reference] [--dump-outputs DIR]
 
 A "step" is one batch of QUERIES_PER_STEP single-query retrieves (distinct query vectors) against the
 resident matrix: similarity (fp32 GEMV over all rows) + exact top-k, i.e. the body of the reference's
@@ -19,6 +19,11 @@ against MEASURED_PEAKS.json), `e2e` (the same metric through the C ABI with HOST
 from host memory and the k results come back to host memory inside every call), `parity` (a sample of the
 timed queries judged by the oracle's streamed superheavy() over ALL rows read back from the device; a
 mismatch fails the run), `cpu_baseline` (headline only: the reference's NumPy path timed on this host).
+
+--dump-outputs DIR (one process only) writes, after the timed steps of every leg, what that leg's timed path computed in
+its last step: DIR/<config>_scores.npy (float32, one row of k scores per query of the step) and DIR/<config>_ids.npy
+(float64 embeddings.id, exact below 2**53).  A row the path left short (a batched query it routes to the exact path)
+is padded with NaN / -1.  Inputs are seeded, so two builds run with the same arguments can be compared file for file.
 """
 from __future__ import annotations
 
@@ -38,6 +43,7 @@ if "--impl" in sys.argv and sys.argv[sys.argv.index("--impl") + 1:][:1] == ["ref
 
 import numpy as np
 
+sys.dont_write_bytecode = True          # a benchmark run writes nothing into the tree it runs from, which may be read-only
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
@@ -401,6 +407,29 @@ def e2e_pipelined(eng, queries: np.ndarray, k: int, steps: int, in_flight: int =
     return max(rates), first, rates
 
 
+def step_arrays(lists, k: int):
+    """[(score, emb_id), ...] per query -> (scores (nq, k) float32, ids (nq, k) float64), short rows padded NaN / -1."""
+    s = np.full((len(lists), k), np.nan, dtype=np.float32)
+    i = np.full((len(lists), k), -1.0, dtype=np.float64)
+    for j, res in enumerate(lists):
+        s[j, :len(res)] = [a for a, _ in res]
+        i[j, :len(res)] = [b for _, b in res]
+    return s, i
+
+
+def last_step_single(eng, queries: np.ndarray, k: int):
+    """What the device-resident loop (svsb_bench_run) computes in every step: the answers to queries 0 .. QUERIES_PER_STEP-1.
+    The loop keeps only its last query's answer, so each query goes through the same loop once on its own; the uploaded
+    queries are restored afterwards."""
+    res = []
+    for j in range(QUERIES_PER_STEP):
+        eng.bench_set_queries(queries[j % len(queries)][None])
+        eng.bench_run(k, 1)
+        res.append(eng.bench_last_result(k))
+    eng.bench_set_queries(queries)
+    return res
+
+
 def incremental_probe(eng, n: int, d: int, k: int) -> dict:
     """SURVEY.md section 8f rank 4: a one-document add (and a delete) on the resident matrix, then the next retrieve --
     what the reference answers with a full rebuild (src/svs/kb.py:1523, 573-618).  The new row must come back first."""
@@ -429,8 +458,8 @@ def incremental_probe(eng, n: int, d: int, k: int) -> dict:
     return out
 
 
-def leg_single(name: str, steps: int, warmup: int, headline: bool, cpu: bool) -> dict:
-    """Single-query workloads (c1, c2, c4, c5) on one GPU."""
+def leg_single(name: str, steps: int, warmup: int, headline: bool, cpu: bool, outputs: dict | None = None) -> dict:
+    """Single-query workloads (c1, c2, c4, c5) on one GPU.  `outputs`, when given, receives the last step's answers."""
     import svs_b200
     from svs_b200.engine import Engine
     n, d, k, _ = WORKLOADS[name]
@@ -479,6 +508,11 @@ def leg_single(name: str, steps: int, warmup: int, headline: bool, cpu: bool) ->
     parity["device_resident_loop_bits_equal_e2e"] = bool(last_timed == eng.retrieve(queries[(QUERIES_PER_STEP - 1) % len(queries)], k))
     if not parity["device_resident_loop_bits_equal_e2e"]:
         raise AssertionError(f"{name}: the device-resident loop and svsb_query disagree")
+    if outputs is not None:                                      # before the incremental probe changes the matrix
+        step = last_step_single(eng, queries, k)
+        if step[-1] != last_timed:
+            raise AssertionError(f"{name}: a query run alone and the timed loop's last query disagree")
+        outputs[name] = step_arrays(step, k)
     algo_bytes = n * d * 4
     achieved = algo_bytes * nq / (gemv_ms / 1e3) / 1e9
     traffic, traffic_src = replayed_traffic(name)
@@ -510,8 +544,9 @@ def leg_single(name: str, steps: int, warmup: int, headline: bool, cpu: bool) ->
     return line
 
 
-def leg_batch(name: str, steps: int, warmup: int, headline: bool, cpu: bool) -> dict:
-    """c3 on one GPU: one step = one batch of BATCH queries through svsb_query_batch's pipeline."""
+def leg_batch(name: str, steps: int, warmup: int, headline: bool, cpu: bool, outputs: dict | None = None) -> dict:
+    """c3 on one GPU: one step = one batch of BATCH queries through svsb_query_batch's pipeline.  `outputs`, when given,
+    receives the last step's answers."""
     from svs_b200 import pinned_empty
     from svs_b200.engine import Engine
     n, d, k, _ = WORKLOADS[name]
@@ -532,6 +567,8 @@ def leg_batch(name: str, steps: int, warmup: int, headline: bool, cpu: bool) -> 
         r = eng.bench_run_batch(k, 1)
         total_ms += r["total_ms"]; launches += r["launches"]
     clocks = sampler.stop()
+    if outputs is not None:                                      # the last timed batch, still in the pipeline's output buffers
+        outputs[name] = step_arrays([eng.bench_batch_result(qi, k)[0] for qi in range(BATCH)], k)
     for _ in range(steps):                                       # the filter pass's own duration (roofline numerator), bracketed in a
         coarse_ms += eng.bench_run_batch(k, 1, with_coarse=True)["coarse_ms"]   # separate pass: the bracket's host sync idles the GPU ~20 us
     cand, resc, flags = eng.batch_stats(BATCH)
@@ -884,6 +921,20 @@ def summary_of(leg: dict) -> dict:
     return {k: leg[k] for k in keep if k in leg}
 
 
+DUMP_MAX_BYTES = 64 << 20
+
+
+def write_outputs(out_dir: str, outputs: dict) -> None:
+    """--dump-outputs: {config: (scores, ids)} -> out_dir/<config>_scores.npy, out_dir/<config>_ids.npy."""
+    total = sum(a.nbytes for pair in outputs.values() for a in pair)
+    if total > DUMP_MAX_BYTES:
+        raise SystemExit(f"--dump-outputs: {total} bytes, more than {DUMP_MAX_BYTES}")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, (scores, ids) in outputs.items():
+        np.save(os.path.join(out_dir, f"{name}_scores.npy"), scores)
+        np.save(os.path.join(out_dir, f"{name}_ids.npy"), ids)
+
+
 # ---------------------------------------------------------------------------------------------------
 def main():
     ap = argparse.ArgumentParser()
@@ -899,7 +950,13 @@ def main():
     ap.add_argument("--no-inprocess", action="store_true", help="N>1: skip the one-process-all-GPUs leg of the headline workload")
     ap.add_argument("--exchange", default="peer", choices=["peer", "collective"],
                     help="N>1, single queries: fused push over NVLink peer memory (default) or NCCL all-gather + merge")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write every leg's answers of its last timed step to DIR/<config>_{scores,ids}.npy (one process only)")
     args = ap.parse_args()
+    if args.steps < 1 or args.config_steps < 1:
+        ap.error("--steps and --config-steps must be at least 1")
+    if args.dump_outputs is not None and args.impl != "ours":
+        ap.error("--dump-outputs writes what the engine computed: it needs --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     if args.impl == "reference":
@@ -909,6 +966,8 @@ def main():
     world = int(os.environ.get("WORLD_SIZE", "1"))
     if world != args.gpus and world > 1:
         raise SystemExit(f"--gpus {args.gpus} but WORLD_SIZE={world}")
+    if world > 1 and args.dump_outputs is not None:
+        raise SystemExit("--dump-outputs runs in one process (--gpus 1) only")
     import svs_b200                                             # fails loudly if the CUDA library is missing  # noqa: F401
 
     if args.only:
@@ -922,9 +981,11 @@ def main():
             raise SystemExit(f"unknown config {c}")
 
     if world == 1:
+        outputs = {} if args.dump_outputs is not None else None
+
         def run(name, steps, headline):
             fn = leg_batch if name == "c3" else leg_single
-            return fn(name, steps, args.warmup, headline, headline and not args.no_cpu_baseline)
+            return fn(name, steps, args.warmup, headline, headline and not args.no_cpu_baseline, outputs)
         line = run(args.workload, args.steps, True)
         if extra:
             line["configs"] = {}
@@ -935,6 +996,8 @@ def main():
                     raise                                           # a parity failure fails the run
                 except Exception as ex:                             # e.g. not enough free HBM for c4 next to another tenant
                     line["configs"][c] = {"error": f"{type(ex).__name__}: {ex}"}
+        if outputs is not None:
+            write_outputs(args.dump_outputs, outputs)
         print(json.dumps(line), flush=True)
         return
 
