@@ -115,7 +115,7 @@ int svsb_load_synthetic(svsb_t* e, int64_t n, int32_t d, uint64_t seed, int64_t 
  * generation was replaced while the update was being built -- nothing is published and the caller falls back to the full
  * rebuild.  One update at a time (serialised inside); do not run it concurrently with svsb_load_begin .. svsb_load_end.  The result equals a fresh rebuild bit for bit: same ids,
  * same scores (tests/test_gpu_mutate.py).  Generations with tombstones answer batches and large k through the exact
- * kernels; svsb_top_pairs asks for a reload (SVSB_E_INVALID). */
+ * kernels; svsb_top_pairs asks for a reload (SVSB_E_INVALID), on one device or several. */
 int svsb_apply_mutations(svsb_t* e, const int64_t* del_ids, int64_t n_del, const float* add_rows, const int64_t* add_ids,
                          int64_t n_add, int32_t d, uint64_t* generation);
 /* Physical rows of the resident generation (tombstoned ones included) and live rows (== svsb_shape's n). */
@@ -189,7 +189,11 @@ int svsb_batch_threshold_mode(svsb_t* e);
  * np.dot(M, M.T) + get_top_pairs (src/svs/util.py:206-233) without ever materialising the N x N scores: tensor-core
  * coarse pass over the upper triangle, one global threshold, exact fp32 re-score of the survivors.  Outputs have
  * capacity n_pairs; *out_count = min(n_pairs, N(N-1)/2).  Order: score descending, then first row ascending, then
- * second row ascending (the reference orders exact ties by descending flat index).  Single-device engines. */
+ * second row ascending (the reference orders exact ties by descending flat index).  Multi-device engines split the
+ * pairs over the devices (each runs the triangle of its own shard and rectangles against blocks of its peers' rows, with
+ * its own threshold) and merge the per-device lists on device 0: the result equals the single-device engine's bit for
+ * bit.  SVSB_E_INVALID: tombstoned rows, rows far from unit norm, n_pairs above 2^22; SVSB_E_NOMEM: more near-tied pairs
+ * than the candidate lists hold -- refusals the reference's host path still answers. */
 int svsb_top_pairs(svsb_t* e, int64_t n_pairs, float* out_scores, int64_t* out_emb_ids_a, int64_t* out_emb_ids_b,
                    int64_t* out_count);
 int svsb_snapshot_top_pairs(svsb_t* e, svsb_snap_t* s, int64_t n_pairs, float* out_scores, int64_t* out_emb_ids_a,

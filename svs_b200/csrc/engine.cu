@@ -1102,19 +1102,177 @@ extern "C" int svsb_snapshot_query_batch(svsb_t* e, svsb_snap_t* s, const float*
 // pairwise top pairs: document_top_pairwise_scores' compute (reference src/svs/kb.py:1642-1671, 1208-1243;
 // src/svs/util.py:206-233) on the coarse tensor-core pass + exact refine (pairs.cu)
 // ------------------------------------------------------------------------------------------------
-namespace {
-struct DevBufs {                                  // frees everything it handed out
-    int dev; std::vector<void*> ptrs;
-    explicit DevBufs(int d) : dev(d) {}
-    ~DevBufs() { cudaSetDevice(dev); for (void* p : ptrs) cudaFree(p); }
-    template <class T> cudaError_t get(T** out, size_t count) {
-        void* p = nullptr;
-        cudaError_t e = cudaMalloc(&p, std::max<size_t>(count, 1) * sizeof(T));
-        if (e == cudaSuccess) { ptrs.push_back(p); *out = reinterpret_cast<T*>(p); }
-        return e;
+// Static plan of the pass over G row shards: device a runs the upper triangle of its own shard, then the full rectangles
+// (a, a + t mod G) for t = 1 .. ceil(G/2) - 1; for even G the opposite rectangle (a, a + G/2) is split in half between
+// its two devices (a takes all of its rows against the first half of the other shard's, the other device its second
+// half against all of a's).  Invariants:
+//   1. every unordered pair of distinct global rows is covered by exactly one task of one device;
+//   2. with equal shards no device gets more than 1/G of the pair work plus a few percent (the odd half row of a split).
+// Empty tasks are left out.  tests/test_pairs_multi_logic.py restates this function.
+std::vector<std::vector<PairTask>> pairs_plan(const std::vector<int64_t>& shard_rows) {
+    const int G = (int)shard_rows.size();
+    std::vector<std::vector<PairTask>> plan((size_t)G);
+    auto add = [&](int dev, int peer, int64_t m0, int64_t m1, int64_t q0, int64_t q1) {
+        if (m1 > m0 && q1 > q0 && (peer != dev || m1 - m0 >= 2)) plan[(size_t)dev].push_back(PairTask{peer, m0, m1, q0, q1});
+    };
+    for (int a = 0; a < G; ++a) {
+        add(a, a, 0, shard_rows[a], 0, shard_rows[a]);
+        for (int t = 1; t < (G + 1) / 2; ++t) {
+            const int b = (a + t) % G;
+            add(a, b, 0, shard_rows[a], 0, shard_rows[b]);
+        }
     }
-};
-}  // namespace
+    if (G % 2 == 0)
+        for (int a = 0; a < G / 2; ++a) {
+            const int b = a + G / 2;
+            const int64_t h = shard_rows[b] / 2;
+            add(a, b, 0, shard_rows[a], 0, h);
+            add(b, a, h, shard_rows[b], 0, shard_rows[a]);
+        }
+    return plan;
+}
+
+PairRows pair_rows_of(const std::vector<Generation*>& views) {
+    PairRows t;
+    t.n = (int)views.size();
+    const int64_t base = views[0]->shards[0].row0;
+    for (int s = 0; s < t.n; ++s) {
+        const Shard& sh = views[s]->shards[0];
+        t.row0[s] = sh.row0 - base; t.M[s] = sh.M; t.ids[s] = sh.ids;
+    }
+    t.row0[t.n] = t.row0[t.n - 1] + views[t.n - 1]->shards[0].n;
+    return t;
+}
+
+constexpr int PAIRS_BLOCK = 1024;                  // query rows per coarse block
+
+int pairs_dev_prepare(svsb_engine* e, Generation* g, int64_t n, float eps2, PairsDev& r) {
+    r.g = g; r.n = n; r.eps2 = eps2;
+    const int64_t N = g->shards[0].n;
+    if (N == 0 || g->d == 0) return SVSB_OK;       // no rows here: nothing to compute, nothing for a peer to read
+    BatchPlan P;
+    P.n = N; P.d = g->d; P.ld = g->ld; P.ld16 = (g->d + 7) & ~7; P.kk = 1; P.k = 1;
+    P.n_tiles = (int)((N + COARSE_TILE_ROWS - 1) / COARSE_TILE_ROWS);
+    P.cand_cap = env_int("SVSB_BATCH_CAND_CAP", 32768);
+    const int B = PAIRS_BLOCK;
+    // bootstrap sample (only when a first block at threshold -inf would overflow the per-row lists)
+    r.bootstrap = N >= 2048;
+    int64_t want_rows = std::max<int64_t>(std::max<int64_t>(4096, n / 16 + 1),
+                                          (int64_t)((double)N * (double)n / (64.0 * (double)P.cand_cap)) + 1);
+    int64_t st_ = std::max<int64_t>((want_rows + COARSE_TILE_ROWS - 1) / COARSE_TILE_ROWS, 32);
+    st_ = std::min<int64_t>(st_, P.n_tiles);
+    P.s_tiles = (int)st_; P.tile_stride = std::max(1, P.n_tiles / P.s_tiles);
+    P.sample_rows = (int64_t)P.s_tiles * COARSE_TILE_ROWS;
+    r.ld16 = P.ld16; r.cand_cap = P.cand_cap; r.s_tiles = P.s_tiles; r.tile_stride = P.tile_stride; r.sample_rows = P.sample_rows;
+
+    BatchWs* w = nullptr;
+    int rc = batch_ws_get(e, w);
+    if (rc != SVSB_OK) return rc;
+    if ((rc = ensure_m16(g, P, w->st)) != SVSB_OK) return rc;
+    {   // the sample buffer holds 256 x sample_rows floats: size it through the (b_pad x sample_rows) allocation
+        BatchPlan Pa = P;
+        Pa.sample_rows = std::max<int64_t>(1, (256 * P.sample_rows + B - 1) / B);
+        if ((rc = batch_ws_ensure(w, Pa, B)) != SVSB_OK) return rc;
+    }
+    CU(cudaSetDevice(w->dev));
+    r.w = w; r.st = w->st; r.bufs.dev = w->dev;
+    r.LC = std::max<int64_t>(1ll << 22, 16 * n);
+    for (int i = 0; i < 2; ++i) { CU(r.bufs.get(&r.lo[i], (size_t)r.LC)); CU(r.bufs.get(&r.lp[i], (size_t)r.LC)); CU(r.bufs.get(&r.lstate[i], 2)); }
+    CU(r.bufs.get(&r.thr, 1));
+    const uint32_t neg_inf = 0xff800000u;
+    CU(cudaMemcpyAsync(r.thr, &neg_inf, 4, cudaMemcpyHostToDevice, r.st));
+    CU(cudaMemsetAsync(r.lstate[0], 0, 16, r.st));
+    return SVSB_OK;
+}
+
+int pairs_dev_coarse(PairsDev& r, int self, const std::vector<PairTask>& tasks, const std::vector<Generation*>& views, const PairRows& rows) {
+    r.C = 0;
+    if (!r.w) return SVSB_OK;
+    BatchWs* w = r.w;
+    Generation* g = r.g;
+    cudaStream_t st = r.st;
+    const int64_t N = g->shards[0].n;
+    const int B = PAIRS_BLOCK;
+    const int n = (int)r.n;
+    const size_t row16 = (size_t)r.ld16 * 2;
+    const char* m16 = reinterpret_cast<const char*>(g->M16);
+    CU(cudaSetDevice(w->dev));
+    if (r.bootstrap) {
+        CU(launch_coarse_gemm(st, w->dev, 1, g->M16, N, g->M16, 256, r.ld16, r.s_tiles, r.tile_stride, nullptr, nullptr, nullptr, 0,
+                              w->sample, r.sample_rows, /*q_rows=*/std::min<int64_t>(N, 256), /*tri_q0=*/0));
+        CU(launch_pairs_tau(st, nullptr, w->sample, 256 * r.sample_rows, nullptr, 0, n, r.eps2, r.thr));
+    }
+    // bq query rows (q16, q_rows of them readable) against m_rows matrix rows (m16op); global rows of the first of each
+    auto block = [&](const char* m16op, int64_t m_rows, const void* q16, int64_t q_rows, int bq, int64_t tri_q0,
+                     int64_t q_row0, int64_t m_row0) -> int {
+        const int cur = r.cur;
+        const int b_pad = (bq + COARSE_TILE_QUERIES - 1) / COARSE_TILE_QUERIES * COARSE_TILE_QUERIES;
+        const int m_tiles = (int)((m_rows + COARSE_TILE_ROWS - 1) / COARSE_TILE_ROWS);
+        CU(launch_pairs_fill_thr(st, w->thr, b_pad, bq, r.thr));
+        CU(cudaMemsetAsync(w->cand_cnt, 0, (size_t)b_pad * 4, st));
+        CU(launch_coarse_gemm(st, w->dev, 0, m16op, m_rows, q16, b_pad, r.ld16, m_tiles, 1, w->thr,
+                              w->cand, w->cand_cnt, r.cand_cap, nullptr, 0, q_rows, tri_q0));
+        CU(launch_pairs_gather(st, w->cand, w->cand_cnt, r.cand_cap, bq, q_row0, m_row0, r.lo[cur], r.lp[cur], r.LC, r.lstate[cur]));
+        CU(launch_pairs_tau(st, r.lo[cur], nullptr, 0, r.lstate[cur], r.LC, n, r.eps2, r.thr));
+        CU(cudaMemsetAsync(r.lstate[cur ^ 1], 0, 16, st));
+        CU(launch_pairs_compact(st, w->dev, r.lo[cur], r.lp[cur], r.lstate[cur], r.LC, r.lo[cur ^ 1], r.lp[cur ^ 1], r.lstate[cur ^ 1], r.thr));
+        r.cur = cur ^ 1;
+        return SVSB_OK;
+    };
+    const int64_t row0 = rows.row0[self];
+    int rc;
+    for (const PairTask& t : tasks) {
+        if (t.peer == self) {      // upper triangle: the shard itself plays the queries from row q0 on (coarse pairwise mode)
+            for (int64_t q0 = 0; q0 + 1 < N; q0 += B)
+                if ((rc = block(m16, N, m16 + (size_t)q0 * row16, N - q0, (int)std::min<int64_t>(B, N - q0), q0, row0 + q0, row0)) != SVSB_OK)
+                    return rc;
+        } else {                   // rectangle: blocks of the peer's fp16 rows copied next to this shard, no mask
+            const Generation* pv = views[(size_t)t.peer];
+            for (int64_t q0 = t.q0; q0 < t.q1; q0 += B) {
+                const int bq = (int)std::min<int64_t>(B, t.q1 - q0);
+                CU(cudaMemcpyPeerAsync(w->dQ16, w->dev, reinterpret_cast<const char*>(pv->M16) + (size_t)q0 * row16, pv->shards[0].dev,
+                                       (size_t)bq * row16, st));
+                if ((rc = block(m16 + (size_t)t.m0 * row16, t.m1 - t.m0, w->dQ16, bq, bq, -1, rows.row0[t.peer] + q0, row0 + t.m0)) != SVSB_OK)
+                    return rc;
+            }
+        }
+    }
+    unsigned long long hstate[2] = {0, 0};
+    CU(cudaMemcpyAsync(hstate, r.lstate[r.cur], 16, cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    if (hstate[1] != 0)
+        return fail(SVSB_E_NOMEM, hstate[1] & 1 ? "svsb_top_pairs: a row has more than 32768 near-tied partners (raise SVSB_BATCH_CAND_CAP)"
+                                                : "svsb_top_pairs: too many near-tied pairs for the candidate list");
+    r.C = (int64_t)hstate[0];
+    return SVSB_OK;
+}
+
+int pairs_dev_alloc(PairsDev& r) {
+    r.kl = std::min(r.n, r.C);
+    if (r.kl == 0) return SVSB_OK;
+    CU(cudaSetDevice(r.w->dev));
+    const int64_t C = r.C, n = r.kl;
+    r.np2 = next_pow2(C); if (r.np2 < 2048) r.np2 = 2048;
+    r.shift = group_shift_for(C);
+    const int64_t G = (C + ((int64_t)1 << r.shift) - 1) >> r.shift;
+    DevBufs& b = r.bufs;
+    CU(b.get(&r.keys, (size_t)r.np2)); CU(b.get(&r.scores, (size_t)C)); CU(b.get(&r.sortbuf, (size_t)r.np2));
+    CU(b.get(&r.gmax, (size_t)G)); CU(b.get(&r.o_keys, (size_t)n)); CU(b.get(&r.o_scores, (size_t)n)); CU(b.get(&r.o_sel, (size_t)n));
+    CU(b.get(&r.o_cnt, 16)); CU(b.get(&r.o_a, (size_t)n)); CU(b.get(&r.o_b, (size_t)n));
+    return SVSB_OK;
+}
+
+int pairs_dev_finish(PairsDev& r, const PairRows& rows, const int64_t* ids) {
+    if (r.kl == 0) return SVSB_OK;
+    cudaStream_t st = r.st;
+    CU(cudaSetDevice(r.w->dev));
+    CU(launch_pairs_sortkeys(st, r.lp[r.cur], r.C, r.np2, r.keys));
+    CU(launch_sort_keys_desc(st, r.keys, r.np2));                 // ascending (i, j)
+    CU(launch_pairs_rescore(st, r.w->dev, rows, r.g->ld, r.keys, r.C, r.scores));
+    CU(launch_fullsort_topk(st, r.scores, r.C, r.gmax, r.shift, r.kl, nullptr, 0, r.sortbuf, r.o_keys, r.o_scores, r.o_sel, r.o_cnt));
+    CU(launch_pairs_emit(st, r.o_sel, r.kl, r.keys, ids, r.o_a, r.o_b));
+    return SVSB_OK;
+}
 
 static int top_pairs_gen(svsb_engine* e, const std::shared_ptr<Generation>& g, int64_t n_pairs, float* out_scores,
                          int64_t* out_ids_a, int64_t* out_ids_b, int64_t* out_count) {
@@ -1124,7 +1282,6 @@ static int top_pairs_gen(svsb_engine* e, const std::shared_ptr<Generation>& g, i
     const int64_t N = g->n;
     if (n_pairs <= 0 || N < 2 || g->d == 0) return SVSB_OK;       // get_top_k: k <= 0 -> [] (util.py:200-201); no pairs
     if (!out_scores || !out_ids_a || !out_ids_b) return fail(SVSB_E_INVALID, "svsb_top_pairs: NULL buffer");
-    if (e->devs.size() != 1 || g->shards.size() != 1) return fail(SVSB_E_INVALID, "svsb_top_pairs: single-device engines only");
     if (g->has_tombstones()) return fail(SVSB_E_INVALID, "svsb_top_pairs: the resident generation has tombstoned rows (reload to compact it)");
     if (N > 0x7fffff00ll) return fail(SVSB_E_INVALID, "svsb_top_pairs: too many rows");
     const float R = 1.0f + g->max_dev;
@@ -1132,90 +1289,25 @@ static int top_pairs_gen(svsb_engine* e, const std::shared_ptr<Generation>& g, i
     const double total_pairs = 0.5 * (double)N * (double)(N - 1);
     const int64_t n = (double)n_pairs < total_pairs ? n_pairs : (int64_t)total_pairs;       // util.py:198-199
     if (n > (1ll << 22)) return fail(SVSB_E_INVALID, "svsb_top_pairs: at most 2^22 pairs per call");
-    const Shard& s = g->shards[0];
-
-    BatchPlan P;
-    P.n = N; P.d = g->d; P.ld = g->ld; P.ld16 = (g->d + 7) & ~7; P.kk = 1; P.k = 1;
-    P.n_tiles = (int)((N + COARSE_TILE_ROWS - 1) / COARSE_TILE_ROWS);
-    P.cand_cap = env_int("SVSB_BATCH_CAND_CAP", 32768);
-    const int B = 1024;                                            // query rows per block
-    // bootstrap sample (only when a first block at threshold -inf would overflow the per-row lists)
-    const bool bootstrap = N >= 2048;
-    int64_t want_rows = std::max<int64_t>(std::max<int64_t>(4096, n / 16 + 1),
-                                          (int64_t)((double)N * (double)n / (64.0 * (double)P.cand_cap)) + 1);
-    int64_t st_ = std::max<int64_t>((want_rows + COARSE_TILE_ROWS - 1) / COARSE_TILE_ROWS, 32);
-    st_ = std::min<int64_t>(st_, P.n_tiles);
-    P.s_tiles = (int)st_; P.tile_stride = std::max(1, P.n_tiles / P.s_tiles);
-    P.sample_rows = (int64_t)P.s_tiles * COARSE_TILE_ROWS;
     const float eps = (9.765625e-4f + 2.384185791015625e-7f + (float)g->d * (2.384185791015625e-7f + 1.1920928955078125e-7f))
                       * (R * 1.000001f) * (R * 1.000001f) + 1e-8f;
     const float eps2 = 2.0f * eps;
+    if (e->multi) return multi_top_pairs(e, g, n, eps2, out_scores, out_ids_a, out_ids_b, out_count);
 
     std::lock_guard<std::mutex> lk(e->batch_mu);
-    BatchWs* w = nullptr;
-    int rc = batch_ws_get(e, w);
-    if (rc != SVSB_OK) return rc;
-    if ((rc = ensure_m16(g.get(), P, w->st)) != SVSB_OK) return rc;
-    {   // the sample buffer holds 256 x sample_rows floats: size it through the (b_pad x sample_rows) allocation
-        BatchPlan Pa = P;
-        Pa.sample_rows = std::max<int64_t>(1, (256 * P.sample_rows + B - 1) / B);
-        if ((rc = batch_ws_ensure(w, Pa, B)) != SVSB_OK) return rc;
-    }
-    CU(cudaSetDevice(w->dev));
-    cudaStream_t st = w->st;
-    DevBufs bufs(w->dev);
-    const int64_t LC = std::max<int64_t>(1ll << 22, 16 * n);
-    uint32_t* lo[2]; u64* lp[2]; unsigned long long* lstate[2]; float* thr_scalar;
-    for (int i = 0; i < 2; ++i) { CU(bufs.get(&lo[i], (size_t)LC)); CU(bufs.get(&lp[i], (size_t)LC)); CU(bufs.get(&lstate[i], 2)); }
-    CU(bufs.get(&thr_scalar, 1));
-    const uint32_t neg_inf = 0xff800000u;
-    CU(cudaMemcpyAsync(thr_scalar, &neg_inf, 4, cudaMemcpyHostToDevice, st));
-    CU(cudaMemsetAsync(lstate[0], 0, 16, st));
-    const char* m16 = reinterpret_cast<const char*>(g->M16);
-
-    if (bootstrap) {
-        CU(launch_coarse_gemm(st, w->dev, 1, g->M16, N, g->M16, 256, P.ld16, P.s_tiles, P.tile_stride, nullptr, nullptr, nullptr, 0,
-                              w->sample, P.sample_rows, /*q_rows=*/std::min<int64_t>(N, 256), /*tri_q0=*/0));
-        CU(launch_pairs_tau(st, nullptr, w->sample, 256 * P.sample_rows, nullptr, 0, (int)n, eps2, thr_scalar));
-    }
-    int cur = 0;
-    for (int64_t q0 = 0; q0 + 1 < N; q0 += B) {
-        const int bq = (int)std::min<int64_t>(B, N - q0);
-        const int b_pad = (bq + COARSE_TILE_QUERIES - 1) / COARSE_TILE_QUERIES * COARSE_TILE_QUERIES;
-        CU(launch_pairs_fill_thr(st, w->thr, b_pad, bq, thr_scalar));
-        CU(cudaMemsetAsync(w->cand_cnt, 0, (size_t)b_pad * 4, st));
-        CU(launch_coarse_gemm(st, w->dev, 0, g->M16, N, m16 + (size_t)q0 * P.ld16 * 2, b_pad, P.ld16, P.n_tiles, 1, w->thr,
-                              w->cand, w->cand_cnt, P.cand_cap, nullptr, 0, /*q_rows=*/N - q0, /*tri_q0=*/q0));
-        CU(launch_pairs_gather(st, w->cand, w->cand_cnt, P.cand_cap, bq, q0, lo[cur], lp[cur], LC, lstate[cur]));
-        CU(launch_pairs_tau(st, lo[cur], nullptr, 0, lstate[cur], LC, (int)n, eps2, thr_scalar));
-        CU(cudaMemsetAsync(lstate[cur ^ 1], 0, 16, st));
-        CU(launch_pairs_compact(st, w->dev, lo[cur], lp[cur], lstate[cur], LC, lo[cur ^ 1], lp[cur ^ 1], lstate[cur ^ 1], thr_scalar));
-        cur ^= 1;
-    }
-    unsigned long long hstate[2] = {0, 0};
-    CU(cudaMemcpyAsync(hstate, lstate[cur], 16, cudaMemcpyDeviceToHost, st));
-    CU(cudaStreamSynchronize(st));
-    if (hstate[1] != 0)
-        return fail(SVSB_E_NOMEM, hstate[1] & 1 ? "svsb_top_pairs: a row has more than 32768 near-tied partners (raise SVSB_BATCH_CAND_CAP)"
-                                                : "svsb_top_pairs: too many near-tied pairs for the candidate list");
-    const int64_t C = (int64_t)hstate[0];
-    if (C < n) return fail(SVSB_E_CUDA, "internal: pair list shorter than the requested count");
-    int64_t np2 = next_pow2(C); if (np2 < 2048) np2 = 2048;
-    u64* keys; float* scores; u64* sortbuf; u64* gmax; u64* o_keys; float* o_scores; int64_t* o_sel; int32_t* o_cnt; int64_t* o_a; int64_t* o_b;
-    CU(bufs.get(&keys, (size_t)np2)); CU(bufs.get(&scores, (size_t)C)); CU(bufs.get(&sortbuf, (size_t)np2));
-    const int shift = group_shift_for(C);
-    const int64_t G = (C + ((int64_t)1 << shift) - 1) >> shift;
-    CU(bufs.get(&gmax, (size_t)G)); CU(bufs.get(&o_keys, (size_t)n)); CU(bufs.get(&o_scores, (size_t)n)); CU(bufs.get(&o_sel, (size_t)n));
-    CU(bufs.get(&o_cnt, 16)); CU(bufs.get(&o_a, (size_t)n)); CU(bufs.get(&o_b, (size_t)n));
-    CU(launch_pairs_sortkeys(st, lp[cur], C, np2, keys));
-    CU(launch_sort_keys_desc(st, keys, np2));                     // ascending (i, j)
-    CU(launch_pairs_rescore(st, w->dev, s.M, g->ld, keys, C, scores));
-    CU(launch_fullsort_topk(st, scores, C, gmax, shift, n, nullptr, 0, sortbuf, o_keys, o_scores, o_sel, o_cnt));
-    CU(launch_pairs_emit(st, o_sel, n, keys, s.ids, o_a, o_b));
-    CU(cudaMemcpyAsync(out_scores, o_scores, (size_t)n * 4, cudaMemcpyDeviceToHost, st));
-    CU(cudaMemcpyAsync(out_ids_a, o_a, (size_t)n * 8, cudaMemcpyDeviceToHost, st));
-    CU(cudaMemcpyAsync(out_ids_b, o_b, (size_t)n * 8, cudaMemcpyDeviceToHost, st));
-    CU(cudaStreamSynchronize(st));
+    const std::vector<Generation*> views{g.get()};
+    const PairRows rows = pair_rows_of(views);
+    PairsDev r;
+    int rc;
+    if ((rc = pairs_dev_prepare(e, g.get(), n, eps2, r)) != SVSB_OK) return rc;
+    if ((rc = pairs_dev_coarse(r, 0, pairs_plan({N})[0], views, rows)) != SVSB_OK) return rc;
+    if (r.C < n) return fail(SVSB_E_CUDA, "internal: pair list shorter than the requested count");
+    if ((rc = pairs_dev_alloc(r)) != SVSB_OK) return rc;
+    if ((rc = pairs_dev_finish(r, rows, g->shards[0].ids)) != SVSB_OK) return rc;
+    CU(cudaMemcpyAsync(out_scores, r.o_scores, (size_t)n * 4, cudaMemcpyDeviceToHost, r.st));
+    CU(cudaMemcpyAsync(out_ids_a, r.o_a, (size_t)n * 8, cudaMemcpyDeviceToHost, r.st));
+    CU(cudaMemcpyAsync(out_ids_b, r.o_b, (size_t)n * 8, cudaMemcpyDeviceToHost, r.st));
+    CU(cudaStreamSynchronize(r.st));
     *out_count = n;
     return SVSB_OK;
 }

@@ -447,7 +447,59 @@ int publish_generation(svsb_engine* e, const std::shared_ptr<Generation>& g, uin
 int batch_local_records_gen(svsb_engine* e, const std::shared_ptr<Generation>& g, cudaStream_t st, const float* d_Q, int32_t b,
                             int32_t k, int64_t* d_records, int32_t* n_fallback);
 
+// pairwise top pairs (engine.cu): one device's share of the pass, in the phases multi.cu runs on every device in turn
+// so that all allocations happen before any cross-device work is enqueued
+struct DevBufs {                                  // frees everything it handed out
+    int dev = 0; std::vector<void*> ptrs;
+    DevBufs() = default;
+    DevBufs(const DevBufs&) = delete;
+    DevBufs& operator=(const DevBufs&) = delete;
+    ~DevBufs() { if (ptrs.empty()) return; cudaSetDevice(dev); for (void* p : ptrs) cudaFree(p); }
+    template <class T> cudaError_t get(T** out, size_t count) {
+        void* p = nullptr;
+        cudaError_t e = cudaMalloc(&p, std::max<size_t>(count, 1) * sizeof(T));
+        if (e == cudaSuccess) { ptrs.push_back(p); *out = reinterpret_cast<T*>(p); }
+        return e;
+    }
+};
+// A task of device `self`: its own shard's rows [m0, m1) against rows [q0, q1) of shard `peer`, every combination
+// (peer != self); or, with peer == self, the upper triangle of its whole shard.
+struct PairTask { int peer = 0; int64_t m0 = 0, m1 = 0, q0 = 0, q1 = 0; };
+std::vector<std::vector<PairTask>> pairs_plan(const std::vector<int64_t>& shard_rows);
+// The shards of single-shard views (one per device, scan order) as the pair kernels address them; rows are counted
+// from the first view's first row.
+PairRows pair_rows_of(const std::vector<Generation*>& views);
+struct PairsDev {
+    Generation* g = nullptr;                       // this device's single-shard view
+    BatchWs* w = nullptr;                          // its batch workspace (stream, thresholds, candidate lists, Q staging); null: no rows
+    cudaStream_t st = nullptr;
+    DevBufs bufs;
+    int64_t n = 0;                                 // pairs asked for
+    float eps2 = 0.f;
+    int ld16 = 0, cand_cap = 0, s_tiles = 0, tile_stride = 1; int64_t sample_rows = 0; bool bootstrap = false;
+    int64_t LC = 0;                                // pair list capacity
+    uint32_t* lo[2] = {nullptr, nullptr}; u64* lp[2] = {nullptr, nullptr}; unsigned long long* lstate[2] = {nullptr, nullptr};
+    float* thr = nullptr;                          // the device's running threshold
+    int cur = 0;
+    int64_t C = 0;                                 // pairs in the list after the coarse pass
+    int64_t kl = 0;                                // entries of the device's result list: min(n, C)
+    int64_t np2 = 0; int shift = 0;
+    u64* keys = nullptr; float* scores = nullptr; u64* sortbuf = nullptr; u64* gmax = nullptr;
+    u64* o_keys = nullptr; float* o_scores = nullptr; int64_t* o_sel = nullptr; int32_t* o_cnt = nullptr;
+    int64_t* o_a = nullptr; int64_t* o_b = nullptr;
+};
+// workspace, fp16 shadow of the shard, pair lists (sizes fixed by n)
+int pairs_dev_prepare(svsb_engine* e, Generation* g, int64_t n, float eps2, PairsDev& r);
+// coarse filter over the device's tasks with its own running threshold; synchronises the device's stream, sets r.C
+int pairs_dev_coarse(PairsDev& r, int self, const std::vector<PairTask>& tasks, const std::vector<Generation*>& views, const PairRows& rows);
+// buffers sized by r.C
+int pairs_dev_alloc(PairsDev& r);
+// exact re-score of the list, its top r.kl in the final order: r.o_scores, r.o_a / r.o_b (ids[row], or rows if ids is null)
+int pairs_dev_finish(PairsDev& r, const PairRows& rows, const int64_t* ids);
+
 // multi.cu
+int  multi_top_pairs(svsb_engine* e, const std::shared_ptr<Generation>& g, int64_t n, float eps2, float* out_scores,
+                     int64_t* out_ids_a, int64_t* out_ids_b, int64_t* out_count);
 int  multi_create(svsb_engine* e);
 void multi_destroy(svsb_engine* e);
 int  multi_publish(svsb_engine* e, const std::shared_ptr<Generation>& g);

@@ -229,20 +229,35 @@ cudaError_t launch_union_threshold(cudaStream_t st, const float* tops, int64_t l
 constexpr int REFINE_FLAG_THRESHOLD_HIGH = 16;
 
 // ---- pairwise top pairs (pairs.cu): global candidate list on top of the coarse pass's pairwise mode --------
+// The row shards as the pair kernels see them: global rows [row0[s], row0[s + 1]) are M[s] (leading dimension ld) and
+// ids[s], peer pointers where the shard lives on another device.  One entry on a single-device engine.
+struct PairRows {
+    int n = 0;
+    int64_t row0[XCHG_MAX_RANKS + 1];
+    const float* M[XCHG_MAX_RANKS];
+    const int64_t* ids[XCHG_MAX_RANKS];
+    __host__ __device__ int shard_of(int64_t r) const { int s = 0; while (s + 1 < n && r >= row0[s + 1]) ++s; return s; }
+};
 // Sort keys[0..np2) descending; np2 a power of two >= 2048 (pad with 0).
 cudaError_t launch_sort_keys_desc(cudaStream_t st, u64* keys, int64_t np2);
 cudaError_t launch_pairs_fill_thr(cudaStream_t st, float* thr, int b_pad, int b, const float* scalar);
+// query q of the block is global row q_row0 + q, matrix row r global row m_row0 + r; pairs go in as (smaller, larger) row.
 // state[0] = entries in the list, state[1] = error flags (1: a per-query list overflowed, 2: the pair list overflowed)
-cudaError_t launch_pairs_gather(cudaStream_t st, const u64* cand, const int32_t* cand_cnt, int cand_cap, int b, int64_t q0,
-                                uint32_t* list_o, u64* list_pair, int64_t list_cap, unsigned long long* state);
+cudaError_t launch_pairs_gather(cudaStream_t st, const u64* cand, const int32_t* cand_cnt, int cand_cap, int b, int64_t q_row0,
+                                int64_t m_row0, uint32_t* list_o, u64* list_pair, int64_t list_cap, unsigned long long* state);
 // *thr_scalar = max(*thr_scalar, n-th largest coarse score - eps2) over the list (vals == nullptr) or a raw sample
 cudaError_t launch_pairs_tau(cudaStream_t st, const uint32_t* list_o, const void* vals /*fp16 sample*/, int64_t vals_count,
                              const unsigned long long* state, int64_t list_cap, int n, float eps2, float* thr_scalar);
 cudaError_t launch_pairs_compact(cudaStream_t st, int device, const uint32_t* src_o, const u64* src_pair, const unsigned long long* src_state,
                                  int64_t list_cap, uint32_t* dst_o, u64* dst_pair, unsigned long long* dst_state, const float* thr_scalar);
 cudaError_t launch_pairs_sortkeys(cudaStream_t st, const u64* list_pair, int64_t count, int64_t np2, u64* keys);
-cudaError_t launch_pairs_rescore(cudaStream_t st, int device, const float* M, int ld, const u64* keys, int64_t count, float* scores);
+cudaError_t launch_pairs_rescore(cudaStream_t st, int device, const PairRows& rows, int ld, const u64* keys, int64_t count, float* scores);
 cudaError_t launch_pairs_emit(cudaStream_t st, const int64_t* sel, int64_t k, const u64* keys, const int64_t* ids, int64_t* out_a, int64_t* out_b);
+// Merge n_lists pair lists (list l at [l * stride ..), counts[l] valid), each sorted by (score desc, row a asc, row b asc)
+// with no pair in two lists, into the top k under the same order (select.cu); rows become embeddings.ids through rows.ids.
+cudaError_t launch_merge_sorted_pairs(cudaStream_t st, const float* scores, const int64_t* rows_a, const int64_t* rows_b,
+                                      const int32_t* counts, int n_lists, int64_t stride, int64_t k, const PairRows& rows,
+                                      float* out_scores, int64_t* out_a, int64_t* out_b, int32_t* out_count);
 
 int sm_count(int device);
 inline int64_t next_pow2(int64_t v) { int64_t p = 1; while (p < v) p <<= 1; return p; }

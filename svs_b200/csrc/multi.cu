@@ -627,6 +627,75 @@ int multi_query_batch(svsb_engine* e, const std::shared_ptr<Generation>& g, cons
 }
 
 // ------------------------------------------------------------------------------------------------
+// pairwise top pairs: every device runs its share of the static plan (engine.cu: pairs_plan) -- the triangle of its own
+// shard and rectangles against 1024-row blocks of its peers' fp16 rows, copied over -- with its OWN running threshold.
+// That is valid: the n-th largest coarse score over a subset of the pairs is at most the n-th largest over all pairs,
+// so no pair of the exact top n is dropped.  Each device re-scores its survivors exactly (the second row read over the
+// peer mapping; the bits do not depend on the device) and keeps its top min(n, survivors) in the final order; device 0
+// gathers the lists and rank-merges them.  No kernel waits on a flag: devices are ordered by events and stream waits.
+// ------------------------------------------------------------------------------------------------
+int multi_top_pairs(svsb_engine* e, const std::shared_ptr<Generation>& g, int64_t n, float eps2, float* out_scores,
+                    int64_t* out_ids_a, int64_t* out_ids_b, int64_t* out_count) {
+    Multi* m = e->multi;
+    const int nd = (int)m->kids.size();
+    std::unique_lock<std::mutex> lk(m->mu);        // exclusive use of the kids' batch workspaces; fused queries in flight keep running
+    std::vector<Generation*> views;
+    std::vector<int64_t> shard_rows;
+    for (int i = 0; i < nd; ++i) { views.push_back(g->child_gen[i].get()); shard_rows.push_back(g->shards[i].n); }
+    const PairRows rows = pair_rows_of(views);
+    const std::vector<std::vector<PairTask>> plan = pairs_plan(shard_rows);
+    std::vector<PairsDev> r((size_t)nd);
+    // fixed-size buffers and every device's fp16 shadow first: the coarse pass copies blocks of its peers' shadows
+    int rc = m->pool->run_all([&](int i) { return pairs_dev_prepare(m->kids[i], views[i], n, eps2, r[i]); });
+    if (rc != SVSB_OK) return rc;
+    rc = m->pool->run_all([&](int i) { return pairs_dev_coarse(r[i], i, plan[i], views, rows); });   // ends with every device idle
+    if (rc != SVSB_OK) return rc;
+    // every buffer sized by the survivor counts, on every device, before the re-score reads peer rows
+    int64_t stride = 0, total = 0;
+    for (auto& x : r) { stride = std::max(stride, std::min(n, x.C)); total += std::min(n, x.C); }
+    if (total < n) return fail(SVSB_E_CUDA, "internal: pair lists shorter than the requested count");
+    rc = m->pool->run_all([&](int i) { return pairs_dev_alloc(r[i]); });
+    if (rc != SVSB_OK) return rc;
+    const int rd = root_dev(m);
+    CU(cudaSetDevice(rd));
+    DevBufs bufs; bufs.dev = rd;
+    float* l_scores; int64_t* l_a; int64_t* l_b; int32_t* l_cnt; float* o_scores; int64_t* o_a; int64_t* o_b; int32_t* o_cnt;
+    CU(bufs.get(&l_scores, (size_t)(nd * stride))); CU(bufs.get(&l_a, (size_t)(nd * stride))); CU(bufs.get(&l_b, (size_t)(nd * stride)));
+    CU(bufs.get(&l_cnt, (size_t)nd));
+    CU(bufs.get(&o_scores, (size_t)n)); CU(bufs.get(&o_a, (size_t)n)); CU(bufs.get(&o_b, (size_t)n)); CU(bufs.get(&o_cnt, 16));
+    rc = m->pool->run_all([&](int i) -> int {
+        if (r[i].kl == 0) return SVSB_OK;
+        int rc2 = pairs_dev_finish(r[i], rows, nullptr);                      // global rows: device 0 maps them to ids
+        if (rc2 != SVSB_OK) return rc2;
+        CU(cudaEventRecord(m->scratch[i].ev, r[i].st));
+        return SVSB_OK;
+    });
+    if (rc != SVSB_OK) return rc;
+    CU(cudaSetDevice(rd));
+    cudaStream_t rst = m->kids[0]->xchg->st;
+    for (int i = 0; i < nd; ++i) {
+        const int64_t kl = r[i].kl;
+        if (kl == 0) { CU(cudaMemsetAsync(l_cnt + i, 0, 4, rst)); continue; }
+        CU(cudaStreamWaitEvent(rst, m->scratch[i].ev, 0));
+        if ((rc = copy_to_root(m, i, l_scores + i * stride, r[i].o_scores, (size_t)kl * 4, rst)) != SVSB_OK) return rc;
+        if ((rc = copy_to_root(m, i, l_a + i * stride, r[i].o_a, (size_t)kl * 8, rst)) != SVSB_OK) return rc;
+        if ((rc = copy_to_root(m, i, l_b + i * stride, r[i].o_b, (size_t)kl * 8, rst)) != SVSB_OK) return rc;
+        if ((rc = copy_to_root(m, i, l_cnt + i, r[i].o_cnt, 4, rst)) != SVSB_OK) return rc;
+    }
+    CU(launch_merge_sorted_pairs(rst, l_scores, l_a, l_b, l_cnt, nd, stride, n, rows, o_scores, o_a, o_b, o_cnt));
+    int32_t cnt = 0;
+    CU(cudaMemcpyAsync(out_scores, o_scores, (size_t)n * 4, cudaMemcpyDeviceToHost, rst));
+    CU(cudaMemcpyAsync(out_ids_a, o_a, (size_t)n * 8, cudaMemcpyDeviceToHost, rst));
+    CU(cudaMemcpyAsync(out_ids_b, o_b, (size_t)n * 8, cudaMemcpyDeviceToHost, rst));
+    CU(cudaMemcpyAsync(&cnt, o_cnt, 4, cudaMemcpyDeviceToHost, rst));
+    CU(cudaStreamSynchronize(rst));
+    // the copies above read the other devices' lists: their buffers are freed only now
+    if (cnt != (int32_t)n) return fail(SVSB_E_CUDA, "internal: pair merge returned a bad count");
+    *out_count = n;
+    return SVSB_OK;
+}
+
+// ------------------------------------------------------------------------------------------------
 // measurement: `iters` device-resident queries through the fused path, TICKETS in flight
 // ------------------------------------------------------------------------------------------------
 int multi_bench_run(svsb_engine* e, const std::shared_ptr<Generation>& g, int32_t k, int32_t iters, float* total_ms, float* gemv_ms) {

@@ -9,6 +9,9 @@
 // block: it is (the n-th largest coarse score among the pairs seen so far) - 2 eps, a valid lower bound for
 // (final n-th largest coarse) - 2 eps, so every pair that can be in the exact top-n stays in the list (same argument
 // as batch.cu with the global list in place of a query's list).
+// Multi-device engines (multi.cu: multi_top_pairs) run the same pass per device over a share of the pairs -- the
+// triangle of the own shard plus rectangles against blocks of the peers' rows -- with one threshold per device; pairs
+// are kept in global rows and the re-score reads rows through a table of shard pointers (PairRows, peer memory).
 //
 // Order of the result: score descending, then row index of the first document ascending, then of the second
 // (the reference orders exact ties by descending flat index of the upper triangle, src/svs/util.py:203).
@@ -28,10 +31,11 @@ __global__ void pairs_fill_thr_kernel(float* __restrict__ thr, int b_pad, int b,
     if (q < b_pad) thr[q] = q < b ? *scalar : __int_as_float(0x7f800000);
 }
 
-// Append the block's per-query candidate lists to the global pair list.  One CTA per query row.
+// Append the block's per-query candidate lists to the global pair list.  One CTA per query row.  Query q is global
+// row q_row0 + q, matrix row r (the key's row) global row m_row0 + r; the pair goes in as (smaller row, larger row).
 // state[0] = list count, state[1] = error flags (1: a per-query list overflowed, 2: the global list overflowed)
 __global__ void __launch_bounds__(256)
-pairs_gather_kernel(const u64* __restrict__ cand, const int32_t* __restrict__ cand_cnt, int cand_cap, int64_t q0,
+pairs_gather_kernel(const u64* __restrict__ cand, const int32_t* __restrict__ cand_cnt, int cand_cap, int64_t q_row0, int64_t m_row0,
                     uint32_t* __restrict__ list_o, u64* __restrict__ list_pair, int64_t list_cap, unsigned long long* state)
 {
     __shared__ unsigned long long base;
@@ -44,11 +48,12 @@ pairs_gather_kernel(const u64* __restrict__ cand, const int32_t* __restrict__ ca
     const unsigned long long b0 = base;
     if (b0 + (unsigned long long)cnt > (unsigned long long)list_cap) { if (threadIdx.x == 0) atomicOr(&state[1], 2ull); return; }
     const u64* cq = cand + (size_t)q * cand_cap;
-    const u64 i = (u64)(q0 + q);
+    const u64 i = (u64)(q_row0 + q);
     for (int c = threadIdx.x; c < cnt; c += blockDim.x) {
         const u64 key = cq[c];
+        const u64 j = (u64)(m_row0 + (int64_t)key_row(key));
         list_o[b0 + c] = (uint32_t)(key >> 32);
-        list_pair[b0 + c] = (i << 32) | (u64)key_row(key);
+        list_pair[b0 + c] = i < j ? (i << 32) | j : (j << 32) | i;
     }
 }
 
@@ -104,19 +109,21 @@ __global__ void pairs_sortkeys_kernel(const u64* __restrict__ list_pair, int64_t
     for (int64_t c = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; c < np2; c += stride) keys[c] = c < count ? ~list_pair[c] : 0ull;
 }
 
-// exact fp32 score of pair c = (i, j) (keys sorted, ~pair), one warp per pair, the similarity kernel's summation order
-// with row i in the role of the query
+// exact fp32 score of pair c = (i, j) (keys sorted, ~pair; global rows, both rows found through the shard table), one
+// warp per pair, the similarity kernel's summation order with row i in the role of the query.  fma(m, q, acc) ==
+// fma(q, m, acc), so the bits depend neither on the device that scores the pair nor on which shard holds which row.
 __global__ void __launch_bounds__(256)
-pairs_rescore_kernel(const float* __restrict__ M, int d4, const u64* __restrict__ keys, int64_t count, float* __restrict__ scores)
+pairs_rescore_kernel(const __grid_constant__ PairRows rows, int d4, const u64* __restrict__ keys, int64_t count, float* __restrict__ scores)
 {
     const int lane = threadIdx.x & 31;
     const int64_t warp_global = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     const int64_t nwarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
-    const float4* M4 = reinterpret_cast<const float4*>(M);
     for (int64_t c = warp_global; c < count; c += nwarps) {
         const u64 pr = ~keys[c];
-        const float4* pq = M4 + (int64_t)(pr >> 32) * d4;
-        const float4* pm = M4 + (int64_t)(uint32_t)pr * d4;
+        const int64_t ri = (int64_t)(pr >> 32), rj = (int64_t)(uint32_t)pr;
+        const int si = rows.shard_of(ri), sj = rows.shard_of(rj);
+        const float4* pq = reinterpret_cast<const float4*>(rows.M[si]) + (ri - rows.row0[si]) * d4;
+        const float4* pm = reinterpret_cast<const float4*>(rows.M[sj]) + (rj - rows.row0[sj]) * d4;
         float4 a0 = make_float4(0.f, 0.f, 0.f, 0.f), a1 = a0;
         int ch = lane;
         for (; ch + 32 < d4; ch += 64) {
@@ -130,7 +137,7 @@ pairs_rescore_kernel(const float* __restrict__ M, int d4, const u64* __restrict_
     }
 }
 
-// out[r] = (ids[i], ids[j]) of the pair at sorted position sel[r]
+// out[r] = (ids[i], ids[j]) of the pair at sorted position sel[r]; ids == nullptr: the rows themselves
 __global__ void pairs_emit_kernel(const int64_t* __restrict__ sel, int64_t k, const u64* __restrict__ keys, const int64_t* __restrict__ ids,
                                   int64_t* __restrict__ out_a, int64_t* __restrict__ out_b) {
     const int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -149,10 +156,10 @@ cudaError_t launch_pairs_fill_thr(cudaStream_t st, float* thr, int b_pad, int b,
     count_launch();
     return cudaGetLastError();
 }
-cudaError_t launch_pairs_gather(cudaStream_t st, const u64* cand, const int32_t* cand_cnt, int cand_cap, int b, int64_t q0,
-                                uint32_t* list_o, u64* list_pair, int64_t list_cap, unsigned long long* state) {
+cudaError_t launch_pairs_gather(cudaStream_t st, const u64* cand, const int32_t* cand_cnt, int cand_cap, int b, int64_t q_row0,
+                                int64_t m_row0, uint32_t* list_o, u64* list_pair, int64_t list_cap, unsigned long long* state) {
     if (b <= 0) return cudaSuccess;
-    pairs_gather_kernel<<<b, 256, 0, st>>>(cand, cand_cnt, cand_cap, q0, list_o, list_pair, list_cap, state);
+    pairs_gather_kernel<<<b, 256, 0, st>>>(cand, cand_cnt, cand_cap, q_row0, m_row0, list_o, list_pair, list_cap, state);
     count_launch();
     return cudaGetLastError();
 }
@@ -174,12 +181,12 @@ cudaError_t launch_pairs_sortkeys(cudaStream_t st, const u64* list_pair, int64_t
     count_launch();
     return cudaGetLastError();
 }
-cudaError_t launch_pairs_rescore(cudaStream_t st, int device, const float* M, int ld, const u64* keys, int64_t count, float* scores) {
+cudaError_t launch_pairs_rescore(cudaStream_t st, int device, const PairRows& rows, int ld, const u64* keys, int64_t count, float* scores) {
     if (count <= 0) return cudaSuccess;
     int64_t blocks = (count + 7) / 8;
     const int64_t cap = (int64_t)sm_count(device) * 8;
     if (blocks > cap) blocks = cap;
-    pairs_rescore_kernel<<<(unsigned)blocks, 256, 0, st>>>(M, ld / 4, keys, count, scores);
+    pairs_rescore_kernel<<<(unsigned)blocks, 256, 0, st>>>(rows, ld / 4, keys, count, scores);
     count_launch();
     return cudaGetLastError();
 }

@@ -963,6 +963,64 @@ cudaError_t launch_merge_sorted_big(cudaStream_t st, const u64* keys, const int6
     return cudaGetLastError();
 }
 
+// The same rank merge for the per-device lists of the pairwise pass (multi.cu): an entry is (score, row a, row b) and
+// orders by (ordered score desc, then the 64-bit pair a << 32 | b asc) -- a 96-bit key, unique because every pair of
+// rows is scored on exactly one device.  The rows of the top k are mapped to embeddings.ids on the way out.
+__device__ __forceinline__ bool pair_before(uint32_t so, u64 sp, uint32_t to, u64 tp) { return so > to || (so == to && sp < tp); }
+
+__global__ void merge_sorted_pairs_kernel(const float* __restrict__ scores, const int64_t* __restrict__ rows_a,
+                                          const int64_t* __restrict__ rows_b, const int32_t* __restrict__ counts, int n_lists,
+                                          int64_t stride, int64_t k, const __grid_constant__ PairRows rows,
+                                          float* __restrict__ out_scores, int64_t* __restrict__ out_a, int64_t* __restrict__ out_b,
+                                          int32_t* __restrict__ out_count)
+{
+    int64_t total = 0;
+    for (int l = 0; l < n_lists; ++l) total += min((int64_t)max(counts[l], 0), stride);
+    const int64_t kk = k < total ? k : total;
+    const int64_t span = (int64_t)n_lists * stride;
+    const int64_t step = (int64_t)gridDim.x * blockDim.x;
+    for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < span; e += step) {
+        const int l = (int)(e / stride);
+        const int64_t p = e - (int64_t)l * stride;
+        if (p >= min((int64_t)max(counts[l], 0), stride)) continue;
+        const float sc = scores[e];
+        const uint32_t so = f32_to_ordered(sc);
+        const u64 sp = ((u64)rows_a[e] << 32) | (u64)rows_b[e];
+        int64_t rank = p;
+        for (int m = 0; m < n_lists && rank < kk; ++m) {
+            if (m == l) continue;
+            const int64_t base = (int64_t)m * stride;
+            int64_t lo = 0, hi = min((int64_t)max(counts[m], 0), stride);          // first entry of list m not before mine
+            while (lo < hi) {
+                const int64_t mid = (lo + hi) >> 1;
+                const u64 tp = ((u64)rows_a[base + mid] << 32) | (u64)rows_b[base + mid];
+                if (pair_before(f32_to_ordered(scores[base + mid]), tp, so, sp)) lo = mid + 1; else hi = mid;
+            }
+            rank += lo;
+        }
+        if (rank < kk) {
+            const int64_t a = rows_a[e], b = rows_b[e];
+            const int s_a = rows.shard_of(a), s_b = rows.shard_of(b);
+            out_scores[rank] = sc;
+            out_a[rank] = rows.ids[s_a][a - rows.row0[s_a]];
+            out_b[rank] = rows.ids[s_b][b - rows.row0[s_b]];
+        }
+    }
+    if (blockIdx.x == 0 && threadIdx.x == 0) *out_count = (int32_t)kk;
+}
+
+cudaError_t launch_merge_sorted_pairs(cudaStream_t st, const float* scores, const int64_t* rows_a, const int64_t* rows_b,
+                                      const int32_t* counts, int n_lists, int64_t stride, int64_t k, const PairRows& rows,
+                                      float* out_scores, int64_t* out_a, int64_t* out_b, int32_t* out_count)
+{
+    if (n_lists < 1 || n_lists > XCHG_MAX_RANKS || stride < 1 || k < 1) return cudaErrorInvalidValue;
+    const int64_t span = (int64_t)n_lists * stride;
+    const unsigned blocks = (unsigned)std::min<int64_t>((span + 255) / 256, 148 * 8);
+    merge_sorted_pairs_kernel<<<blocks, 256, 0, st>>>(scores, rows_a, rows_b, counts, n_lists, stride, k, rows, out_scores, out_a, out_b, out_count);
+    count_launch();
+    return cudaGetLastError();
+}
+
 cudaError_t launch_merge_window(cudaStream_t st, const u64* slot_base, const u64* flags, unsigned long long seq,
                                 int world, int cap, int k, unsigned long long timeout_ns, u64* scratch_keys, int64_t* scratch_ids,
                                 float* out_scores, int64_t* out_ids, int32_t* out_count, u64* stamps)

@@ -9,14 +9,14 @@ What is replaced -- and nothing else (SURVEY.md section 8b):
   * `svs.kb._EmbeddingsMatrix` (reference src/svs/kb.py:856-893) gains a `.device` member, a
     `DeviceEmbeddingsMatrix`; `invalidate()` drops both caches, so every invalidation site of the
     reference (kb.py:984,1062,1086,1455,1523,1541) keeps working untouched.  The host NumPy cache
-    stays in place (it is only filled if something still asks for it, e.g. the pairwise path of a
-    multi-device install).
+    stays in place (it is only filled if something still asks for it, e.g. the pairwise path of an
+    install with pairwise=False, or a pairwise call the engine declines).
   * `KB.retrieve` (kb.py:1608-1640), `AsyncKB.retrieve` (kb.py:1171-1206): same orchestration --
     cache fetch, query embedding through the magnitude guard, SQL fetch of the n documents -- with the
     `superheavy()` closure (np.dot + get_top_k + emb_id_lookup) replaced by one engine call.
   * `AsyncKB.load` (kb.py:964-967) pre-warms the device cache instead of the host one.
   * `document_top_pairwise_scores` (kb.py:1642-1671, 1208-1243): same orchestration with `superheavy()` =
-    np.dot(M, M.T) + get_top_pairs replaced by `svsb_top_pairs` (single-device engines; SURVEY.md section 8f rank 2).
+    np.dot(M, M.T) + get_top_pairs replaced by `svsb_top_pairs` (one device or several; SURVEY.md section 8f rank 2).
   * additive: `KB.retrieve_many` / `AsyncKB.retrieve_many` (one embedding call, one engine batch).
 
 INTEGRATION.md shows the same change as a source patch to kb.py for a maintainer who prefers that.
@@ -98,8 +98,8 @@ class _Coalescer:
 def install(svs_module: Any = None, devices: Optional[Sequence[int]] = None, normalize: bool = False,
             pairwise: Optional[bool] = None, coalesce: bool = True, prewarm: bool = True, incremental: bool = True) -> None:
     """Patch `svs` in place.  Idempotent.  `devices`: CUDA devices to row-shard the matrix over.
-    `pairwise`: also route document_top_pairwise_scores to the engine (default: yes on a single device; the
-    multi-device engine keeps the reference's host NumPy path for it).
+    `pairwise` (default on): also route document_top_pairwise_scores to the engine, on one device or several (each
+    device runs a share of the pair search); False keeps the reference's host NumPy path for it.
     `coalesce`: batch concurrent AsyncKB.retrieve calls into one engine call (see _Coalescer).
     `prewarm` (default on): create the engine (= the CUDA context, ~2 s once per process on a B200 box,
     profiles/r01_first_query_probe.txt) on a background thread as soon as a KB object exists, instead of inside the
@@ -108,7 +108,7 @@ def install(svs_module: Any = None, devices: Optional[Sequence[int]] = None, nor
     full rebuild the reference does (kb.py:1062, 1086, 1523, 1541): the querier's connection is wrapped so that every
     `INSERT INTO embeddings` / `DELETE FROM embeddings` of a committed transaction is logged (svs_b200.mutations)."""
     if pairwise is None:
-        pairwise = devices is None or len(devices) <= 1
+        pairwise = True
     if svs_module is None:
         import svs as svs_module                         # type: ignore  (the host application)
     kb = svs_module.kb if hasattr(svs_module, "kb") else __import__(svs_module.__name__ + ".kb", fromlist=["kb"])
