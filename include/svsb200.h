@@ -345,6 +345,48 @@ int svsb_enqueue_merge_records(svsb_t* e, void* stream, const int64_t* d_records
 int svsb_enqueue_merge_batch_records(svsb_t* e, void* stream, const int64_t* d_records, int32_t n_lists, int32_t batch,
                                      int32_t rec_cap, int32_t k, int32_t verify_k, float* d_out_scores, int64_t* d_out_ids,
                                      int32_t* d_out_counts);
+/* ---- pairwise top pairs over the ranks' shards (the sharded form of svsb_top_pairs) --------------------------------
+ * The result equals svsb_top_pairs of one single-device engine over the global matrix bit for bit: scores, ids, order.
+ * Rank r runs its share of a static plan over the world's shards (the triangle of its own shard, rectangles against
+ * 1024-row blocks of its peers' fp16 rows, copied over CUDA IPC) with its own threshold, re-scores its survivors
+ * exactly (the peer's row read over the mapping) and keeps its top list; the caller all-gathers the lists and every rank
+ * merges them.  No kernel waits on a flag: a missing peer blocks the caller's collective, never the GPU.  Per call, on
+ * every rank, in this order:
+ *   svsb_pairs_export        pins the resident generation of this single-device engine, builds its fp16 shadow and
+ *                            writes a descriptor of SVSB_PAIRS_DESC_BYTES (CUDA IPC handles of the fp32 rows, the fp16
+ *                            shadow and the ids; n, d, global first row; an empty shard has no handles) for the caller to
+ *                            all-gather.  *max_dev_out = max | ||row|| - 1 | of the shard, *rows_out = its rows.  Refuses
+ *                            as svsb_top_pairs: SVSB_E_NOT_LOADED, tombstoned rows (SVSB_E_INVALID); and an engine over
+ *                            several devices (SVSB_E_INVALID).  Only when disconnected (SVSB_E_STATE otherwise); drops
+ *                            the previously pinned generation.
+ *   svsb_pairs_connect       opens the peers' descriptors (world x SVSB_PAIRS_DESC_BYTES in rank order, own entry
+ *                            ignored; world <= 16); svsb_pairs_connect_local takes the engines of ranks living in THIS
+ *                            process instead (each exported).  Both check that d agrees and that the ranks' rows are
+ *                            contiguous in rank order.  Rows of the protocol are global, counted from rank 0's first.
+ *   (once per load: export, all-gather, connect, barrier; then any number of the calls below)
+ *   svsb_pairs_local         this rank's list: min(n, survivors) pairs in the final order (score desc, first row asc,
+ *                            second row asc), rows in d_rows_a < d_rows_b, into device buffers of capacity n, where n =
+ *                            min(n_pairs, N(N-1)/2) of the GLOBAL N; *out_count (host) = entries.  max_row_norm must be
+ *                            the same on every rank: the max over ranks of 1 + max_dev.  Runs behind the work already on
+ *                            `stream` and returns when its outputs are complete.  SVSB_E_INVALID: rows far from unit norm,
+ *                            n above 2^22; SVSB_E_NOMEM: more near-tied pairs than the candidate lists hold (a rank may
+ *                            refuse alone: the caller must agree on the outcome before the exchange).
+ *   (the caller all-gathers the counts and the lists, padded to stride = max count: list l at [l * stride ..))
+ *   svsb_pairs_merge         merges the world lists on `stream` into the top n, rows mapped to embeddings.id; *d_out_count
+ *                            (device) = n.
+ * Teardown (and before re-exporting after a reload): every rank's last pairs call has returned, every rank calls
+ * svsb_pairs_disconnect (unmaps the peers' shards, releases the pinned generation), the launcher barriers, and only then
+ * are engines destroyed -- no rank frees a shard another rank can still read. */
+#define SVSB_PAIRS_DESC_BYTES 256
+int svsb_pairs_export(svsb_t* e, float* max_dev_out, int64_t* rows_out, void* desc_out);
+int svsb_pairs_connect(svsb_t* e, int32_t world, int32_t rank, const void* descs);
+int svsb_pairs_connect_local(svsb_t* e, int32_t world, int32_t rank, svsb_t* const* engines);
+int svsb_pairs_local(svsb_t* e, void* stream, int64_t n_pairs, float max_row_norm, float* d_scores, int64_t* d_rows_a,
+                     int64_t* d_rows_b, int64_t* out_count);
+int svsb_pairs_merge(svsb_t* e, void* stream, const float* d_scores, const int64_t* d_rows_a, const int64_t* d_rows_b,
+                     const int32_t* d_counts, int32_t world, int64_t stride, int64_t n, float* d_out_scores,
+                     int64_t* d_out_ids_a, int64_t* d_out_ids_b, int32_t* d_out_count);
+int svsb_pairs_disconnect(svsb_t* e);
 /* Sum (ms) of the similarity-kernel durations bracketed by svsb_enqueue_local_topk(time_kernel=1) since the
  * last collect; waits for them to finish. */
 int svsb_kernel_time_collect(svsb_t* e, float* ms);

@@ -1,6 +1,7 @@
 """Pairwise top pairs: svsb_top_pairs vs the reference's np.dot(M, M.T) + get_top_pairs on the host.
 
     python scripts/pairs_bench.py [rows] [dims] [n_pairs] [--devices 0,1,...]... [--calls K] [--normal] [--no-cpu]
+    python -m torch.distributed.run --nproc-per-node G scripts/pairs_bench.py [rows] [dims] [n_pairs] --sharded [--calls K] [--normal]
 Default = the dad-jokes notebook's shape (examples/dad_jokes/Build Dad Jokes KB.ipynb:338-340: 4,875 x 1536, 10,000 pairs,
 0.47 s + 0.03 s on the author's i3-8100).
 
@@ -13,6 +14,12 @@ Rows are uniform in [0, 1) (all pair scores in a narrow band around 0.75) unless
 spread around 0).  On the uniform rows of 200,000 x 768 and up, more pairs lie within the coarse pass's 2 eps margin of
 the n-th best score than a candidate list holds: the engine refuses (SVSB_E_NOMEM) and the drop-in hands the call to
 the reference's host path.
+
+--sharded: the one-process-per-GPU deployment, one rank per GPU (NCCL cannot run two ranks on one GPU).  Every rank
+generates the same seeded matrix and keeps its slice; ShardedRetriever.top_pairs is timed after a warm-up call that
+exports and connects the shards and builds the fp16 shadows: host clock from a barrier to the answer on the host
+followed by a device synchronize, max over ranks, median / best / worst of K calls.  Rank 0 then runs a single-device
+engine over the whole matrix and checks that the answer is bit-identical.
 """
 import os
 import subprocess
@@ -46,17 +53,59 @@ n = int(args[2]) if len(args) > 2 else 10000
 calls = int((_opt_values("--calls") or ["5"])[0])
 dev_lists = [[int(x) for x in v.split(",")] for v in _opt_values("--devices")] or [[0]]
 
+
+def run_sharded(m, ids):
+    import torch
+    import torch.distributed as dist
+    from svs_b200.sharded import ShardedRetriever
+    rank, world = int(os.environ["RANK"]), int(os.environ["WORLD_SIZE"])
+    local = int(os.environ.get("LOCAL_RANK", rank))
+    torch.cuda.set_device(local)
+    dist.init_process_group("nccl", rank=rank, world_size=world, device_id=torch.device("cuda", local))
+    sr = ShardedRetriever(rank, world, local)
+    sr.load_global(m, ids)
+    got = sr.top_pairs(n)                               # export + connect, fp16 shadows
+    ts = []
+    for _ in range(calls):
+        dist.barrier()
+        t0 = time.perf_counter(); got = sr.top_pairs(n); torch.cuda.synchronize(); dt = time.perf_counter() - t0
+        every = [None] * world
+        dist.all_gather_object(every, dt)
+        ts.append(max(every))
+    if rank == 0:
+        with svs_b200.Engine([local]) as e:
+            e.load(m, ids)
+            want = e.top_pairs(n)
+        same = (len(got) == len(want) and
+                np.array_equal(np.array([s for s, _, _ in got], np.float32).view(np.uint32),
+                               np.array([s for s, _, _ in want], np.float32).view(np.uint32)) and
+                [(a, b) for _, a, b in got] == [(a, b) for _, a, b in want])
+        dist_name = "normal" if "--normal" in sys.argv else "uniform"
+        med = float(np.median(ts))
+        print(f"sharded top_pairs: {N} x {d} {dist_name}, n={n}, {world} ranks (one per GPU): median {med * 1e3:.2f} ms, "
+              f"best {min(ts) * 1e3:.2f} ms, worst {max(ts) * 1e3:.2f} ms over {calls} calls (max over ranks; "
+              f"{float(N) * float(N - 1) * d / med / 1e12:.1f} useful TFLOP/s at the median), "
+              f"answer vs one device: {'bit-identical' if same else 'DIFFERENT'}", flush=True)
+    dist.barrier()
+    sr.close()
+    dist.destroy_process_group()
+
+
 try:
     card = subprocess.run(["nvidia-smi", "--query-gpu=index,name,power.limit", "--format=csv,noheader"],
                           capture_output=True, text=True, timeout=60).stdout.strip().replace("\n", "; ")
 except Exception as ex:  # noqa: BLE001
     card = f"nvidia-smi unavailable ({ex})"
-print(f"GPUs: {card}")
+if os.environ.get("RANK", "0") == "0":
+    print(f"GPUs: {card}")
 
 rng = np.random.default_rng(0)
 m = rng.standard_normal((N, d), dtype=np.float32) if "--normal" in sys.argv else rng.random((N, d), dtype=np.float32)
 m /= np.sqrt((m * m).sum(axis=1))[:, None]
 ids = np.arange(1, N + 1, dtype=np.int64)
+if "--sharded" in sys.argv:
+    run_sharded(m, ids)
+    sys.exit(0)
 useful = float(N) * float(N - 1) * d                    # N(N-1)d: the FLOP of the upper triangle's dot products, counted twice
 first = None
 base_t = None

@@ -21,6 +21,7 @@ NORM_CHECK = 0
 NORM_NORMALIZE = 1
 
 K_FAST_MAX = 2048
+PAIRS_DESC_BYTES = 256       # SVSB_PAIRS_DESC_BYTES
 
 c_float_p = C.POINTER(C.c_float)
 c_i64_p = C.POINTER(C.c_int64)
@@ -101,6 +102,13 @@ SIGNATURES = {
     "svsb_enqueue_join": (C.c_int, [C.c_void_p, C.c_void_p]),
     "svsb_enqueue_merge_records": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32,
                                              C.c_void_p, C.c_void_p, C.c_void_p]),
+    "svsb_pairs_export": (C.c_int, [C.c_void_p, c_float_p, c_i64_p, C.c_void_p]),
+    "svsb_pairs_connect": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p]),
+    "svsb_pairs_connect_local": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p]),
+    "svsb_pairs_local": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_float, C.c_void_p, C.c_void_p, C.c_void_p, c_i64_p]),
+    "svsb_pairs_merge": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int64,
+                                   C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "svsb_pairs_disconnect": (C.c_int, [C.c_void_p]),
     "svsb_kernel_time_collect": (C.c_int, [C.c_void_p, c_float_p]),
     "svsb_ws_create": (C.c_int, [C.c_int, C.c_int64, C.c_int32, C.POINTER(C.c_void_p)]),
     "svsb_ws_destroy": (None, [C.c_void_p]),

@@ -158,6 +158,7 @@ static void free_slabs(svsb_engine* e) {
 }
 
 static void bxchg_release(svsb_engine* e);
+static void pairs_release(svsb_engine* e);
 static void xchg_release(svsb_engine* e) {
     Xchg* x = e->xchg.get();
     if (!x) return;
@@ -198,6 +199,7 @@ extern "C" void svsb_destroy(svsb_t* e) {
     for (auto& w : e->shard_ws) if (w) w->release();
     xchg_release(e);
     bxchg_release(e);
+    pairs_release(e);
     if (e->side_st) { cudaSetDevice(e->devs[0]); cudaStreamDestroy(e->side_st); }
     if (e->submit_st) { cudaSetDevice(e->devs[0]); cudaStreamDestroy(e->submit_st); }
     for (auto ev : e->kev) cudaEventDestroy(ev);
@@ -1146,6 +1148,12 @@ PairRows pair_rows_of(const std::vector<Generation*>& views) {
 
 constexpr int PAIRS_BLOCK = 1024;                  // query rows per coarse block
 
+float pairs_eps2(int d, float R) {
+    const float eps = (9.765625e-4f + 2.384185791015625e-7f + (float)d * (2.384185791015625e-7f + 1.1920928955078125e-7f))
+                      * (R * 1.000001f) * (R * 1.000001f) + 1e-8f;
+    return 2.0f * eps;
+}
+
 int pairs_dev_prepare(svsb_engine* e, Generation* g, int64_t n, float eps2, PairsDev& r) {
     r.g = g; r.n = n; r.eps2 = eps2;
     const int64_t N = g->shards[0].n;
@@ -1185,7 +1193,7 @@ int pairs_dev_prepare(svsb_engine* e, Generation* g, int64_t n, float eps2, Pair
     return SVSB_OK;
 }
 
-int pairs_dev_coarse(PairsDev& r, int self, const std::vector<PairTask>& tasks, const std::vector<Generation*>& views, const PairRows& rows) {
+int pairs_dev_coarse(PairsDev& r, int self, const std::vector<PairTask>& tasks, const std::vector<PairShadow>& shadows, const PairRows& rows) {
     r.C = 0;
     if (!r.w) return SVSB_OK;
     BatchWs* w = r.w;
@@ -1227,11 +1235,12 @@ int pairs_dev_coarse(PairsDev& r, int self, const std::vector<PairTask>& tasks, 
                 if ((rc = block(m16, N, m16 + (size_t)q0 * row16, N - q0, (int)std::min<int64_t>(B, N - q0), q0, row0 + q0, row0)) != SVSB_OK)
                     return rc;
         } else {                   // rectangle: blocks of the peer's fp16 rows copied next to this shard, no mask
-            const Generation* pv = views[(size_t)t.peer];
+            const PairShadow& pv = shadows[(size_t)t.peer];
             for (int64_t q0 = t.q0; q0 < t.q1; q0 += B) {
                 const int bq = (int)std::min<int64_t>(B, t.q1 - q0);
-                CU(cudaMemcpyPeerAsync(w->dQ16, w->dev, reinterpret_cast<const char*>(pv->M16) + (size_t)q0 * row16, pv->shards[0].dev,
-                                       (size_t)bq * row16, st));
+                const char* src = reinterpret_cast<const char*>(pv.M16) + (size_t)q0 * row16;
+                if (pv.dev >= 0) CU(cudaMemcpyPeerAsync(w->dQ16, w->dev, src, pv.dev, (size_t)bq * row16, st));
+                else CU(cudaMemcpyAsync(w->dQ16, src, (size_t)bq * row16, cudaMemcpyDefault, st));
                 if ((rc = block(m16 + (size_t)t.m0 * row16, t.m1 - t.m0, w->dQ16, bq, bq, -1, rows.row0[t.peer] + q0, row0 + t.m0)) != SVSB_OK)
                     return rc;
             }
@@ -1289,18 +1298,15 @@ static int top_pairs_gen(svsb_engine* e, const std::shared_ptr<Generation>& g, i
     const double total_pairs = 0.5 * (double)N * (double)(N - 1);
     const int64_t n = (double)n_pairs < total_pairs ? n_pairs : (int64_t)total_pairs;       // util.py:198-199
     if (n > (1ll << 22)) return fail(SVSB_E_INVALID, "svsb_top_pairs: at most 2^22 pairs per call");
-    const float eps = (9.765625e-4f + 2.384185791015625e-7f + (float)g->d * (2.384185791015625e-7f + 1.1920928955078125e-7f))
-                      * (R * 1.000001f) * (R * 1.000001f) + 1e-8f;
-    const float eps2 = 2.0f * eps;
+    const float eps2 = pairs_eps2(g->d, R);
     if (e->multi) return multi_top_pairs(e, g, n, eps2, out_scores, out_ids_a, out_ids_b, out_count);
 
     std::lock_guard<std::mutex> lk(e->batch_mu);
-    const std::vector<Generation*> views{g.get()};
-    const PairRows rows = pair_rows_of(views);
+    const PairRows rows = pair_rows_of({g.get()});
     PairsDev r;
     int rc;
     if ((rc = pairs_dev_prepare(e, g.get(), n, eps2, r)) != SVSB_OK) return rc;
-    if ((rc = pairs_dev_coarse(r, 0, pairs_plan({N})[0], views, rows)) != SVSB_OK) return rc;
+    if ((rc = pairs_dev_coarse(r, 0, pairs_plan({N})[0], {PairShadow{g->M16, g->shards[0].dev}}, rows)) != SVSB_OK) return rc;
     if (r.C < n) return fail(SVSB_E_CUDA, "internal: pair list shorter than the requested count");
     if ((rc = pairs_dev_alloc(r)) != SVSB_OK) return rc;
     if ((rc = pairs_dev_finish(r, rows, g->shards[0].ids)) != SVSB_OK) return rc;
@@ -1321,6 +1327,239 @@ extern "C" int svsb_snapshot_top_pairs(svsb_t* e, svsb_snap_t* s, int64_t n_pair
                                        int64_t* out_ids_b, int64_t* out_count) {
     if (!e || !s) return fail(SVSB_E_INVALID, "svsb_snapshot_top_pairs: NULL argument");
     return top_pairs_gen(e, s->gen, n_pairs, out_scores, out_ids_a, out_ids_b, out_count);
+}
+
+// ---- pairwise top pairs of the one-process-per-GPU deployment (include/svsb200.h svsb_pairs_*) ----------------------
+// Rank r runs pairs_plan(shard rows)[r] -- the same per-device pass as multi_top_pairs -- against its peers' shards opened
+// over CUDA IPC; the caller all-gathers the per-rank lists and every rank merges them.
+constexpr uint32_t PAIRS_DESC_MAGIC = 0x53505231u;
+struct PairsDesc {                                 // svsb_pairs_export's descriptor (SVSB_PAIRS_DESC_BYTES)
+    uint32_t magic = 0; int32_t has_rows = 0;      // has_rows = 0: an empty shard, no handles
+    int64_t n = 0, row0 = 0;
+    uint64_t gen = 0;
+    int32_t d = 0, ld = 0, ld16 = 0, pad = 0;
+    cudaIpcMemHandle_t M, M16, ids;                // fp32 rows, fp16 shadow, embeddings.id
+};
+static_assert(sizeof(PairsDesc) <= SVSB_PAIRS_DESC_BYTES, "pair descriptor does not fit");
+static_assert(sizeof(cudaIpcMemHandle_t) == 64, "cudaIpcMemHandle_t is 64 bytes");
+
+// one rank's shard as connect sees it
+struct PairsPeer { int64_t n = 0, row0 = 0; int d = 0, ld = 0; const float* M = nullptr; const void* M16 = nullptr; const int64_t* ids = nullptr; };
+
+static void pairs_unmap(PairsShard* p) {
+    for (void* q : p->ipc_opened) cudaIpcCloseMemHandle(q);
+    p->ipc_opened.clear();
+    p->connected = false;
+}
+
+static void pairs_release(svsb_engine* e) {
+    PairsShard* p = e->pairs.get();
+    if (!p) return;
+    cudaSetDevice(e->devs[0]);
+    pairs_unmap(p);
+    if (p->ev) cudaEventDestroy(p->ev);
+    e->pairs.reset();
+}
+
+static PairsPeer pairs_peer_of(const Generation* g) {
+    const Shard& s = g->shards[0];
+    PairsPeer q; q.n = s.n; q.row0 = s.row0; q.d = g->d; q.ld = g->ld; q.M = s.M; q.M16 = g->M16; q.ids = s.ids;
+    return q;
+}
+
+extern "C" int svsb_pairs_export(svsb_t* e, float* max_dev_out, int64_t* rows_out, void* desc_out) {
+    if (!e) return fail(SVSB_E_INVALID, "engine is NULL");
+    if (!desc_out) return fail(SVSB_E_INVALID, "svsb_pairs_export: NULL descriptor");
+    if (e->devs.size() != 1) return fail(SVSB_E_INVALID, "svsb_pairs_export: a sharded engine owns exactly one device");
+    auto g = pin(e);
+    if (!g) return fail(SVSB_E_NOT_LOADED, "no matrix resident (call svsb_load_* first)");
+    if (g->has_tombstones()) return fail(SVSB_E_INVALID, "svsb_top_pairs: the resident generation has tombstoned rows (reload to compact it)");
+    std::lock_guard<std::mutex> lk(e->batch_mu);
+    if (e->pairs && e->pairs->connected) return fail(SVSB_E_STATE, "svsb_pairs_export: svsb_pairs_disconnect first");
+    CU(cudaSetDevice(e->devs[0]));
+    if (!e->pairs) {
+        std::unique_ptr<PairsShard> p(new PairsShard());
+        CU(cudaEventCreateWithFlags(&p->ev, cudaEventDisableTiming));
+        e->pairs = std::move(p);
+    }
+    const Shard& s = g->shards[0];
+    PairsDesc D;
+    D.magic = PAIRS_DESC_MAGIC; D.n = s.n; D.row0 = s.row0; D.gen = g->id; D.d = g->d; D.ld = g->ld; D.ld16 = (g->d + 7) & ~7;
+    memset(&D.M, 0, 64); memset(&D.M16, 0, 64); memset(&D.ids, 0, 64);
+    if (s.n > 0 && s.M) {                          // the fp16 shadow the peers' rectangle tasks copy blocks of
+        BatchWs* w = nullptr;
+        int rc = batch_ws_get(e, w);
+        if (rc != SVSB_OK) return rc;
+        BatchPlan P; P.ld16 = D.ld16;
+        if ((rc = ensure_m16(g.get(), P, w->st)) != SVSB_OK) return rc;
+        CU(cudaIpcGetMemHandle(&D.M, s.M));
+        CU(cudaIpcGetMemHandle(&D.M16, g->M16));
+        CU(cudaIpcGetMemHandle(&D.ids, s.ids));
+        D.has_rows = 1;
+    }
+    e->pairs->gen = g;                             // the previous export's generation is released here
+    memset(desc_out, 0, SVSB_PAIRS_DESC_BYTES);
+    memcpy(desc_out, &D, sizeof(D));
+    if (max_dev_out) *max_dev_out = g->max_dev;
+    if (rows_out) *rows_out = s.n;
+    return SVSB_OK;
+}
+
+// Check the ranks' shards (peers[rank] is this rank's own) and build the tables of the pass and the merge.
+static int pairs_finish_connect(PairsShard* p, int world, int rank, const std::vector<PairsPeer>& peers, const char* who) {
+    int d = -1, ld = -1;
+    for (int r = 0; r < world; ++r) {
+        const PairsPeer& q = peers[(size_t)r];
+        if (r + 1 < world && peers[(size_t)r + 1].row0 != q.row0 + q.n)
+            return fail(SVSB_E_INVALID, std::string(who) + ": the ranks' row ranges are not contiguous in rank order");
+        if (q.n == 0 || q.d == 0) continue;
+        if (!q.M || !q.M16 || !q.ids) return fail(SVSB_E_INVALID, std::string(who) + ": a rank exported rows without buffers");
+        if (d < 0) { d = q.d; ld = q.ld; }
+        else if (q.d != d || q.ld != ld) return fail(SVSB_E_INVALID, std::string(who) + ": the ranks' row widths (d, ld) differ");
+    }
+    PairRows t;
+    t.n = world;
+    for (int r = 0; r < world; ++r) {
+        t.row0[r] = peers[(size_t)r].row0 - peers[0].row0; t.M[r] = peers[(size_t)r].M; t.ids[r] = peers[(size_t)r].ids;
+    }
+    t.row0[world] = t.row0[world - 1] + peers[(size_t)world - 1].n;
+    p->rows = t;
+    p->world = world; p->rank = rank; p->d = d < 0 ? 0 : d;
+    p->shard_rows.clear(); p->shadows.clear();
+    for (const PairsPeer& q : peers) { p->shard_rows.push_back(q.n); p->shadows.push_back(PairShadow{q.M16, -1}); }
+    p->connected = true;
+    return SVSB_OK;
+}
+
+static int pairs_connect_check(svsb_engine* e, int32_t world, int32_t rank, const void* arg, const char* who) {
+    if (!e) return fail(SVSB_E_INVALID, "engine is NULL");
+    if (!arg) return fail(SVSB_E_INVALID, std::string(who) + ": NULL argument");
+    if (!e->pairs || !e->pairs->gen) return fail(SVSB_E_STATE, std::string(who) + ": svsb_pairs_export first");
+    if (e->pairs->connected) return fail(SVSB_E_STATE, std::string(who) + ": already connected (svsb_pairs_disconnect first)");
+    if (world < 1 || world > XCHG_MAX_RANKS || rank < 0 || rank >= world)
+        return fail(SVSB_E_INVALID, std::string(who) + ": bad world / rank (<= 16 ranks)");
+    return SVSB_OK;
+}
+
+extern "C" int svsb_pairs_connect(svsb_t* e, int32_t world, int32_t rank, const void* descs) {
+    int rc = pairs_connect_check(e, world, rank, descs, "svsb_pairs_connect");
+    if (rc != SVSB_OK) return rc;
+    std::lock_guard<std::mutex> lk(e->batch_mu);
+    PairsShard* p = e->pairs.get();
+    CU(cudaSetDevice(e->devs[0]));
+    std::vector<PairsPeer> peers((size_t)world);
+    for (int r = 0; r < world; ++r) {
+        if (r == rank) { peers[(size_t)r] = pairs_peer_of(p->gen.get()); continue; }
+        PairsDesc D;
+        memcpy(&D, static_cast<const unsigned char*>(descs) + (size_t)r * SVSB_PAIRS_DESC_BYTES, sizeof(D));
+        if (D.magic != PAIRS_DESC_MAGIC) { pairs_unmap(p); return fail(SVSB_E_INVALID, "svsb_pairs_connect: not a svsb_pairs_export descriptor"); }
+        PairsPeer& q = peers[(size_t)r];
+        q.n = D.n; q.row0 = D.row0; q.d = D.d; q.ld = D.ld;
+        if (!D.has_rows) continue;
+        void* ptr[3] = {nullptr, nullptr, nullptr};
+        const cudaIpcMemHandle_t* h[3] = {&D.M, &D.M16, &D.ids};
+        for (int i = 0; i < 3; ++i) {
+            cudaError_t ce = cudaIpcOpenMemHandle(&ptr[i], *h[i], cudaIpcMemLazyEnablePeerAccess);
+            if (ce != cudaSuccess) {
+                (void)cudaGetLastError();
+                pairs_unmap(p);
+                return fail(SVSB_E_CUDA, std::string("svsb_pairs_connect: cudaIpcOpenMemHandle: ") + cudaGetErrorString(ce));
+            }
+            p->ipc_opened.push_back(ptr[i]);
+        }
+        q.M = static_cast<const float*>(ptr[0]); q.M16 = ptr[1]; q.ids = static_cast<const int64_t*>(ptr[2]);
+    }
+    if ((rc = pairs_finish_connect(p, world, rank, peers, "svsb_pairs_connect")) != SVSB_OK) pairs_unmap(p);
+    return rc;
+}
+
+extern "C" int svsb_pairs_connect_local(svsb_t* e, int32_t world, int32_t rank, svsb_t* const* engines) {
+    int rc = pairs_connect_check(e, world, rank, engines, "svsb_pairs_connect_local");
+    if (rc != SVSB_OK) return rc;
+    std::lock_guard<std::mutex> lk(e->batch_mu);
+    PairsShard* p = e->pairs.get();
+    CU(cudaSetDevice(e->devs[0]));
+    std::vector<PairsPeer> peers((size_t)world);
+    for (int r = 0; r < world; ++r) {
+        svsb_engine* o = r == rank ? e : engines[r];
+        if (!o || !o->pairs || !o->pairs->gen)
+            return fail(SVSB_E_INVALID, "svsb_pairs_connect_local: a peer engine has not exported (svsb_pairs_export)");
+        if (o->devs[0] != e->devs[0]) {            // the re-score and the merge read the peer's rows and ids directly
+            int can = 0;
+            CU(cudaDeviceCanAccessPeer(&can, e->devs[0], o->devs[0]));
+            if (!can) return fail(SVSB_E_CUDA, "svsb_pairs_connect_local: no peer access between the devices");
+            cudaError_t pe = cudaDeviceEnablePeerAccess(o->devs[0], 0);
+            if (pe != cudaSuccess && pe != cudaErrorPeerAccessAlreadyEnabled) CU(pe);
+            (void)cudaGetLastError();
+        }
+        peers[(size_t)r] = pairs_peer_of(o->pairs->gen.get());
+    }
+    return pairs_finish_connect(p, world, rank, peers, "svsb_pairs_connect_local");
+}
+
+extern "C" int svsb_pairs_local(svsb_t* e, void* stream, int64_t n_pairs, float max_row_norm, float* d_scores, int64_t* d_rows_a,
+                                int64_t* d_rows_b, int64_t* out_count) {
+    if (!e) return fail(SVSB_E_INVALID, "engine is NULL");
+    if (!out_count) return fail(SVSB_E_INVALID, "svsb_pairs_local: out_count is NULL");
+    *out_count = 0;
+    PairsShard* p = e->pairs.get();
+    if (!p || !p->connected) return fail(SVSB_E_STATE, "svsb_pairs_local: svsb_pairs_connect first");
+    const int64_t N = p->rows.row0[p->world];
+    if (n_pairs <= 0 || N < 2 || p->d == 0) return SVSB_OK;
+    if (!d_scores || !d_rows_a || !d_rows_b) return fail(SVSB_E_INVALID, "svsb_pairs_local: NULL buffer");
+    if (N > 0x7fffff00ll) return fail(SVSB_E_INVALID, "svsb_top_pairs: too many rows");
+    const float R = max_row_norm;
+    if (!(R <= 8.0f)) return fail(SVSB_E_INVALID, "svsb_top_pairs: rows are too far from unit norm for the fp16 coarse pass");
+    const double total_pairs = 0.5 * (double)N * (double)(N - 1);
+    const int64_t n = (double)n_pairs < total_pairs ? n_pairs : (int64_t)total_pairs;
+    if (n > (1ll << 22)) return fail(SVSB_E_INVALID, "svsb_top_pairs: at most 2^22 pairs per call");
+    const float eps2 = pairs_eps2(p->d, R);
+
+    std::lock_guard<std::mutex> lk(e->batch_mu);
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    PairsDev r;
+    int rc;
+    if ((rc = pairs_dev_prepare(e, p->gen.get(), n, eps2, r)) != SVSB_OK) return rc;
+    if (!r.w) return SVSB_OK;                      // no rows on this rank: its share of the plan is empty
+    CU(cudaEventRecord(p->ev, st));                // the caller's outputs are written behind what its stream already holds
+    CU(cudaStreamWaitEvent(r.st, p->ev, 0));
+    if ((rc = pairs_dev_coarse(r, p->rank, pairs_plan(p->shard_rows)[(size_t)p->rank], p->shadows, p->rows)) != SVSB_OK) return rc;
+    if ((rc = pairs_dev_alloc(r)) != SVSB_OK) return rc;
+    if (r.kl == 0) return SVSB_OK;
+    if ((rc = pairs_dev_finish(r, p->rows, nullptr)) != SVSB_OK) return rc;          // global rows: the merge maps them to ids
+    CU(cudaMemcpyAsync(d_scores, r.o_scores, (size_t)r.kl * 4, cudaMemcpyDeviceToDevice, r.st));
+    CU(cudaMemcpyAsync(d_rows_a, r.o_a, (size_t)r.kl * 8, cudaMemcpyDeviceToDevice, r.st));
+    CU(cudaMemcpyAsync(d_rows_b, r.o_b, (size_t)r.kl * 8, cudaMemcpyDeviceToDevice, r.st));
+    CU(cudaStreamSynchronize(r.st));
+    *out_count = r.kl;
+    return SVSB_OK;
+}
+
+extern "C" int svsb_pairs_merge(svsb_t* e, void* stream, const float* d_scores, const int64_t* d_rows_a, const int64_t* d_rows_b,
+                                const int32_t* d_counts, int32_t world, int64_t stride, int64_t n, float* d_out_scores,
+                                int64_t* d_out_ids_a, int64_t* d_out_ids_b, int32_t* d_out_count) {
+    if (!e) return fail(SVSB_E_INVALID, "engine is NULL");
+    PairsShard* p = e->pairs.get();
+    if (!p || !p->connected) return fail(SVSB_E_STATE, "svsb_pairs_merge: svsb_pairs_connect first");
+    if (world != p->world) return fail(SVSB_E_INVALID, "svsb_pairs_merge: world differs from the connected one");
+    if (stride < 1 || n < 1 || n > (1ll << 22)) return fail(SVSB_E_INVALID, "svsb_pairs_merge: stride >= 1, 1 <= n <= 2^22");
+    if (!d_scores || !d_rows_a || !d_rows_b || !d_counts || !d_out_scores || !d_out_ids_a || !d_out_ids_b || !d_out_count)
+        return fail(SVSB_E_INVALID, "svsb_pairs_merge: NULL buffer");
+    CU(cudaSetDevice(e->devs[0]));
+    CU(launch_merge_sorted_pairs(static_cast<cudaStream_t>(stream), d_scores, d_rows_a, d_rows_b, d_counts, world, stride, n, p->rows,
+                                 d_out_scores, d_out_ids_a, d_out_ids_b, d_out_count));
+    return SVSB_OK;
+}
+
+extern "C" int svsb_pairs_disconnect(svsb_t* e) {
+    if (!e) return fail(SVSB_E_INVALID, "engine is NULL");
+    PairsShard* p = e->pairs.get();
+    if (!p) return SVSB_OK;
+    std::lock_guard<std::mutex> lk(e->batch_mu);
+    CU(cudaSetDevice(e->devs[0]));
+    pairs_unmap(p);
+    p->gen.reset();
+    return SVSB_OK;
 }
 
 // Diagnostics of the last svsb_query_batch / svsb_bench_run_batch chunk: per query the number of coarse candidates,

@@ -389,6 +389,25 @@ struct Xchg {
     }
 };
 
+// The fp16 shadow of one shard as a rectangle task of the pair search copies blocks of it.  dev >= 0: memory of that
+// device of this process (cudaMemcpyPeerAsync names it by ordinal).  dev < 0: a pointer the copying device's context
+// addresses directly -- a CUDA IPC mapping of another process's shard, or a peer engine's memory in this process; it
+// is copied with cudaMemcpyAsync (device ordinals are per process, so they cannot name another process's device).
+struct PairShadow { const void* M16 = nullptr; int dev = -1; };
+
+// Pair search of the one-process-per-GPU deployment (svsb_pairs_*): the generation this rank exported (pinned: the peers
+// map its buffers) and, once connected, every rank's shard as the pair kernels address it.
+struct PairsShard {
+    std::shared_ptr<Generation> gen;
+    int world = 0, rank = 0, d = 0;
+    bool connected = false;
+    std::vector<int64_t> shard_rows;                     // per rank
+    std::vector<PairShadow> shadows;                     // per rank
+    PairRows rows;                                       // global rows, counted from rank 0's first row
+    std::vector<void*> ipc_opened;
+    cudaEvent_t ev = nullptr;                            // the caller's stream -> the pass's stream
+};
+
 struct svsb_engine {
     std::vector<int> devs;
     std::mutex mu;                          // guards current, loading, pool bookkeeping
@@ -421,6 +440,7 @@ struct svsb_engine {
     std::vector<char> sel_pending;                       // per slot: a selection is (or was) in flight on side_st
     std::unique_ptr<Xchg> xchg;
     std::unique_ptr<BXchg> bxchg;
+    std::unique_ptr<PairsShard> pairs;
     // several devices in ONE process (svsb_create with n_dev > 1, multi.cu): one shard engine per device, driven by one
     // worker thread each, candidate records pushed into device 0's gather window by the selection kernels
     struct Multi* multi = nullptr;
@@ -488,10 +508,13 @@ struct PairsDev {
     u64* o_keys = nullptr; float* o_scores = nullptr; int64_t* o_sel = nullptr; int32_t* o_cnt = nullptr;
     int64_t* o_a = nullptr; int64_t* o_b = nullptr;
 };
+// threshold margin (2 eps) of the fp16 coarse pair score for d components and rows of norm at most R
+float pairs_eps2(int d, float R);
 // workspace, fp16 shadow of the shard, pair lists (sizes fixed by n)
 int pairs_dev_prepare(svsb_engine* e, Generation* g, int64_t n, float eps2, PairsDev& r);
-// coarse filter over the device's tasks with its own running threshold; synchronises the device's stream, sets r.C
-int pairs_dev_coarse(PairsDev& r, int self, const std::vector<PairTask>& tasks, const std::vector<Generation*>& views, const PairRows& rows);
+// coarse filter over the device's tasks with its own running threshold; synchronises the device's stream, sets r.C.
+// shadows[s]: shard s's fp16 rows (read only by rectangle tasks against shard s)
+int pairs_dev_coarse(PairsDev& r, int self, const std::vector<PairTask>& tasks, const std::vector<PairShadow>& shadows, const PairRows& rows);
 // buffers sized by r.C
 int pairs_dev_alloc(PairsDev& r);
 // exact re-score of the list, its top r.kl in the final order: r.o_scores, r.o_a / r.o_b (ids[row], or rows if ids is null)

@@ -648,7 +648,9 @@ int multi_top_pairs(svsb_engine* e, const std::shared_ptr<Generation>& g, int64_
     // fixed-size buffers and every device's fp16 shadow first: the coarse pass copies blocks of its peers' shadows
     int rc = m->pool->run_all([&](int i) { return pairs_dev_prepare(m->kids[i], views[i], n, eps2, r[i]); });
     if (rc != SVSB_OK) return rc;
-    rc = m->pool->run_all([&](int i) { return pairs_dev_coarse(r[i], i, plan[i], views, rows); });   // ends with every device idle
+    std::vector<PairShadow> shadows;
+    for (const Generation* v : views) shadows.push_back(PairShadow{v->M16, v->shards[0].dev});
+    rc = m->pool->run_all([&](int i) { return pairs_dev_coarse(r[i], i, plan[i], shadows, rows); });   // ends with every device idle
     if (rc != SVSB_OK) return rc;
     // every buffer sized by the survivor counts, on every device, before the re-score reads peer rows
     int64_t stride = 0, total = 0;

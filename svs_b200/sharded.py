@@ -18,8 +18,16 @@ its own window (include/svsb200.h "peer exchange").  The windows are exchanged o
 torch.distributed.  `exchange="collective"` keeps the NCCL all-gather (the baseline the fused path is measured
 against; also what batches use: one all-gather per batch is already amortised).
 
+Pairwise top pairs (`top_pairs`, document_top_pairwise_scores) run over the same shards: once per load every rank
+exports its shard (CUDA IPC handles of its fp32 rows, fp16 shadow and ids) and opens its peers'; per call every rank
+runs its share of a static plan over the shard pairs -- the triangle of its own shard and rectangles against blocks of
+its peers' rows -- with its own threshold, re-scores its survivors exactly and keeps its top n; one all-gather of the
+lists (at most 20 bytes x n per rank) and a rank merge on every rank give every rank the single-device answer, bit for
+bit (include/svsb200.h svsb_pairs_*).
+
 The collective / packing / batching logic is backend-agnostic so that it can be exercised on CPU with
-`gloo` (tests/test_sharded_gloo.py injects a NumPy backend); the product backend is `CudaShardBackend`.
+`gloo` (tests/test_sharded_gloo.py and tests/test_sharded_pairs_gloo.py inject NumPy backends); the product backend is
+`CudaShardBackend`.
 """
 from __future__ import annotations
 
@@ -27,6 +35,8 @@ import ctypes as C
 from typing import List, Optional, Tuple
 
 import numpy as np
+
+from ._lib import SVSB_E_CUDA, EngineError
 
 MICRO_BATCH = 16
 TIME_EVERY = 8        # bracket one similarity launch in 8 with timing events (two records cost ~5 us of stream time)
@@ -49,6 +59,8 @@ class CudaShardBackend:
         self.torch = torch
         self._lib = _lib.load()
         self._check = _lib.check
+        self._last_error = _lib.last_error
+        self._desc_bytes = _lib.PAIRS_DESC_BYTES
         self.device = torch.device("cuda", device_index)
         self.engine = Engine([device_index])
         self.d = 0
@@ -238,6 +250,54 @@ class CudaShardBackend:
                                                          n_lists, batch, k, C.c_void_p(out_scores.data_ptr()),
                                                          C.c_void_p(out_ids.data_ptr()), C.c_void_p(out_counts.data_ptr())))
 
+    # -- pairwise top pairs over the ranks' shards (include/svsb200.h svsb_pairs_*) ---------------------------------
+    def pairs_export(self) -> Tuple[bytes, int, str, float]:
+        """Pin the resident generation and describe it for the peers: (descriptor, status, message, max_dev).  A refusal
+        comes back as its SVSB_E_* status instead of raising, so that every rank can learn it."""
+        buf = C.create_string_buffer(self._desc_bytes)
+        max_dev, rows = C.c_float(), C.c_int64()
+        rc = self._lib.svsb_pairs_export(self.engine._h, C.byref(max_dev), C.byref(rows), buf)
+        return buf.raw, rc, self._last_error() if rc else "", float(max_dev.value)
+
+    def pairs_connect(self, world: int, rank: int, descs: List[bytes]) -> None:
+        self._check(self._lib.svsb_pairs_connect(self.engine._h, world, rank, C.c_char_p(b"".join(descs))))
+
+    def pairs_connect_local(self, world: int, rank: int, backends: List["CudaShardBackend"]) -> None:
+        """All ranks live in this process (tests; one process driving several GPUs): plain pointers, no IPC."""
+        arr = (C.c_void_p * len(backends))(*[b.engine._h for b in backends])
+        self._check(self._lib.svsb_pairs_connect_local(self.engine._h, world, rank, arr))
+
+    def pairs_disconnect(self) -> None:
+        self._check(self._lib.svsb_pairs_disconnect(self.engine._h))
+
+    def new_pair_lists(self, count: int, lists: int = 1):
+        """(scores float32, first rows int64, second rows int64), each (lists, count), on the device."""
+        t = self.torch
+        return (t.zeros((lists, count), dtype=t.float32, device=self.device), t.zeros((lists, count), dtype=t.int64, device=self.device),
+                t.zeros((lists, count), dtype=t.int64, device=self.device))
+
+    def pairs_local(self, n: int, max_row_norm: float, out) -> Tuple[int, str, int]:
+        """This rank's top list into row 0 of `out` (new_pair_lists(n)): (status, message, entries)."""
+        st = self.torch.cuda.current_stream(self.device).cuda_stream
+        cnt = C.c_int64()
+        rc = self._lib.svsb_pairs_local(self.engine._h, C.c_void_p(st), n, C.c_float(max_row_norm), C.c_void_p(out[0].data_ptr()),
+                                        C.c_void_p(out[1].data_ptr()), C.c_void_p(out[2].data_ptr()), C.byref(cnt))
+        return rc, self._last_error() if rc else "", cnt.value
+
+    def pairs_merge(self, lists, counts: List[int], n: int, out) -> int:
+        """Merge the all-gathered lists (new_pair_lists(stride, world), counts[l] valid in list l) into row 0 of `out`
+        (new_pair_lists(n)), rows mapped to embeddings.id.  Returns the merged count (synchronises)."""
+        t = self.torch
+        world, stride = lists[0].shape
+        d_counts = t.tensor(counts, dtype=t.int32).to(self.device)
+        d_out = t.zeros(1, dtype=t.int32, device=self.device)
+        st = t.cuda.current_stream(self.device).cuda_stream
+        self._check(self._lib.svsb_pairs_merge(self.engine._h, C.c_void_p(st), C.c_void_p(lists[0].data_ptr()), C.c_void_p(lists[1].data_ptr()),
+                                               C.c_void_p(lists[2].data_ptr()), C.c_void_p(d_counts.data_ptr()), world, stride, n,
+                                               C.c_void_p(out[0].data_ptr()), C.c_void_p(out[1].data_ptr()), C.c_void_p(out[2].data_ptr()),
+                                               C.c_void_p(d_out.data_ptr())))
+        return int(d_out.item())
+
     def collect_kernel_ms(self) -> float:
         ms = C.c_float()
         self._check(self._lib.svsb_kernel_time_collect(self.engine._h, C.byref(ms)))
@@ -274,6 +334,8 @@ class ShardedRetriever:
         self._epoch = 0
         self.last_fallbacks = 0
         self._last_counts = None
+        self._pairs_epoch = None         # load epoch of the connected pair export (None: not connected)
+        self._pairs_norm = 1.0
 
     # -- load ------------------------------------------------------------------------------------
     def load_synthetic(self, n: int, d: int, seed: int = 0, id0: int = 0, id_step: int = 1) -> None:
@@ -572,8 +634,72 @@ class ShardedRetriever:
         s, i = self.retrieve_arrays(query_vec, n)
         return [(float(a), int(b)) for a, b in zip(s, i)]
 
+    # -- pairwise top pairs ---------------------------------------------------------------------------
+    def _all_gather_object(self, obj) -> list:
+        if self.world == 1:
+            return [obj]
+        out: list = [None] * self.world
+        self.dist.all_gather_object(out, obj, group=self.group)
+        return out
+
+    @staticmethod
+    def _agree(outcomes) -> None:
+        """Every rank raises the first refusal any rank reported: ranks never disagree about answering."""
+        for status, message in outcomes:
+            if status != 0:
+                raise EngineError(status, message)
+
+    def _pairs_disconnect(self) -> None:
+        """Every rank's last pair call has returned before any rank unmaps its peers and releases its export."""
+        if self.world > 1:
+            self.dist.barrier(group=self.group)
+        self.backend.pairs_disconnect()
+        self._pairs_epoch = None
+
+    def _ensure_pairs(self) -> None:
+        """Export, all-gather, connect: once per load (a reload re-exports)."""
+        if self._pairs_epoch == self._epoch:
+            return
+        if self._pairs_epoch is not None:
+            self._pairs_disconnect()
+        desc, status, message, max_dev = self.backend.pairs_export()
+        got = self._all_gather_object((desc, status, message, max_dev))
+        self._agree([(g[1], g[2]) for g in got])
+        self.backend.pairs_connect(self.world, self.rank, [g[0] for g in got])
+        if self.world > 1:
+            self.dist.barrier(group=self.group)                    # every rank has opened its peers' shards
+        self._pairs_norm = max(1.0 + g[3] for g in got)            # one coarse error bound for every rank
+        self._pairs_epoch = self._epoch
+
+    def top_pairs(self, n: int) -> List[Tuple[float, int, int]]:
+        """document_top_pairwise_scores' superheavy() over the global matrix, on every rank: [(score, emb_id_1,
+        emb_id_2)] of the n best pairs of distinct rows, equal to Engine.top_pairs on one device bit for bit."""
+        n = min(int(n), self.n * (self.n - 1) // 2)
+        if n <= 0 or self.d == 0:
+            return []
+        self._ensure_pairs()
+        be = self.backend
+        own = be.new_pair_lists(n)
+        outcomes = self._all_gather_object(be.pairs_local(n, self._pairs_norm, own))
+        self._agree([(s, m) for s, m, _ in outcomes])
+        counts = [c for _, _, c in outcomes]
+        stride = max(1, max(counts))
+        lists = be.new_pair_lists(stride, self.world)
+        for whole, mine in zip(lists, own):
+            self.dist.all_gather_into_tensor(whole.view(-1), mine[0, :stride].contiguous(), group=self.group)
+        out = be.new_pair_lists(n)
+        c = be.pairs_merge(lists, counts, n, out)
+        if c != n:
+            raise EngineError(SVSB_E_CUDA, f"sharded top_pairs: the merge returned {c} of {n} pairs")
+        s, a, b = (x[0, :c].cpu().numpy() for x in out)
+        return [(float(x), int(y), int(z)) for x, y, z in zip(s, a, b)]
+
     def close(self) -> None:
-        """Collective when the peer exchange is up: unmap the peers' windows everywhere before any rank frees its own."""
+        """Collective when an exchange is up: unmap the peers' memory everywhere before any rank frees its own."""
+        if self._pairs_epoch is not None:
+            self._pairs_disconnect()
+            if self.world > 1:
+                self.dist.barrier(group=self.group)
         if self._peer_ready or self._batch_peer_ready:
             if self._peer_ready and hasattr(self.backend, "exchange_disconnect"):
                 self.backend.exchange_disconnect()
