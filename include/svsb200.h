@@ -179,6 +179,10 @@ int svsb_host_free(void* p);
 /* Diagnostics of the last batch chunk (<= 2048 queries): coarse candidates per query, rows re-scored exactly per
  * query, flag word per query (0 = answered by the coarse path; otherwise it took the single-query kernels). */
 int svsb_batch_stats(svsb_t* e, int32_t b, int32_t* candidates, int32_t* rescored, int32_t* flags);
+/* Diagnostics of the last svsb_bench_run: *filter = 1 when its queries took the fp16 filter (a pass over the fp16
+ * shadow, then an exact fp32 re-score of the candidate rows), 0 for the fp32 similarity kernel; *rescored = rows the
+ * last query re-scored exactly (0 without the filter). */
+int svsb_bench_filter_stats(svsb_t* e, int32_t* filter, int64_t* rescored);
 /* How the resident generation picks the coarse pass's filter thresholds: 0 = an order statistic of a row sample that
  * bounds the true cut-off with overwhelming probability and is VERIFIED per query after the pass (default; several
  * times fewer candidates), 1 = a proven bound (the engine switches a generation to it when verification fails for

@@ -470,9 +470,13 @@ extern "C" int svsb_is_loaded(svsb_t* e) {
     return e->current ? 1 : 0;
 }
 
+static int filter_attach(svsb_engine* e, Generation* g);
+
 int publish_generation(svsb_engine* e, const std::shared_ptr<Generation>& g, uint64_t* generation) {
+    int rc = filter_attach(e, g.get());
+    if (rc != SVSB_OK) return rc;
     { std::lock_guard<std::mutex> lk(e->mu); g->id = e->next_gen++; }
-    if (e->multi) { int rc = multi_publish(e, g); if (rc != SVSB_OK) return rc; }   // per-device views + workspaces first
+    if (e->multi && (rc = multi_publish(e, g)) != SVSB_OK) return rc;   // per-device views + workspaces first
     std::lock_guard<std::mutex> lk(e->mu);
     e->current = g;
     if (generation) *generation = g->id;
@@ -557,6 +561,78 @@ extern "C" int svsb_read_rows(svsb_t* e, int64_t row0, int64_t count, float* row
 // ------------------------------------------------------------------------------------------------
 // the hot path
 // ------------------------------------------------------------------------------------------------
+int shadow_sync(const Shard& s, int ld, int64_t fresh_from, int create, cudaStream_t st, void** out) {
+    *out = nullptr;
+    ShardBuf* b = s.buf.get();
+    if (!b || s.n == 0 || ld == 0) return create == 2 ? fail(SVSB_E_STATE, "fp16 shadow of an empty shard") : SVSB_OK;
+    const int ld16 = (ld + 7) & ~7;
+    std::lock_guard<std::mutex> lk(b->m16_mu);
+    CU(cudaSetDevice(s.dev));
+    if (!b->M16) {
+        if (create == 0) return SVSB_OK;
+        const size_t bytes = (size_t)b->cap_rows * ld16 * 2;
+        if (create == 1) {                               // +50 % of the matrix: only with an eighth of the device still free
+            size_t fr = 0, tot = 0;
+            if (cudaMemGetInfo(&fr, &tot) != cudaSuccess || fr < bytes + tot / 8) { (void)cudaGetLastError(); return SVSB_OK; }
+        }
+        void* p = nullptr;
+        const cudaError_t ce = cudaMalloc(&p, bytes);
+        if (ce != cudaSuccess) {
+            (void)cudaGetLastError();
+            return create == 1 ? SVSB_OK : fail(SVSB_E_NOMEM, std::string("fp16 shadow: ") + cudaGetErrorString(ce));
+        }
+        b->M16 = p; b->ld16 = ld16; b->m16_rows = 0;
+    }
+    if (fresh_from < b->m16_rows) b->m16_rows = fresh_from;
+    if (b->m16_rows < s.n) {
+        const int64_t r0 = b->m16_rows;
+        cudaError_t ce = launch_rows_to_f16(st, s.dev, s.M + r0 * ld, s.n - r0, ld, static_cast<char*>(b->M16) + (size_t)r0 * ld16 * 2, ld16);
+        if (ce == cudaSuccess) ce = cudaStreamSynchronize(st);
+        if (ce != cudaSuccess) { (void)cudaGetLastError(); return fail(SVSB_E_CUDA, std::string("fp16 shadow: ") + cudaGetErrorString(ce)); }
+        b->m16_rows = s.n;
+    }
+    *out = b->M16;
+    return SVSB_OK;
+}
+
+// Single queries of a single-device engine take the fp16 filter (DESIGN.md section 4, K1f) when the view has a shadow:
+// rows of norm <= 8 (fp16 range of the scaled operands), d <= FILTER_MAX_LD, and a matrix large enough to gain:
+// SVSB_FILTER_MIN_MB, default 512 MB of fp32 rows.  Measured on a B200 (profiles/r05_filter_ab.txt, 1536-d rows): at
+// 246 MB K1's pass is still faster than filter + threshold + re-score, at 492 MB the filter takes 25 % less time.
+static int filter_attach(svsb_engine* e, Generation* g) {
+    for (auto& s : g->shards) s.M16 = nullptr;
+    if (e->devs.size() != 1 || e->is_kid || g->shards.size() != 1) return SVSB_OK;
+    Shard& s = g->shards[0];
+    if (s.n == 0 || g->ld > FILTER_MAX_LD || !(1.0f + g->max_dev <= 8.0f)) return SVSB_OK;
+    if ((double)s.n * g->ld * 4 < (double)env_int("SVSB_FILTER_MIN_MB", 512) * 1048576.0) return SVSB_OK;
+    void* p = nullptr;
+    int rc = shadow_sync(s, g->ld, INT64_MAX, 1, e->copy_st[0], &p);
+    if (rc != SVSB_OK) return rc;
+    s.M16 = p;
+    return SVSB_OK;
+}
+
+// SVSB_FILTER=0 forces K1 (read per call).  The LDG variant of K1 (SVSB_GEMV_VARIANT=1) sums in another order than the
+// re-score, which reproduces the TMA kernel's bits.
+static bool use_filter(const Shard& s, int64_t kk) {
+    if (!s.M16 || kk > K_FAST_MAX || env_int("SVSB_FILTER", 1) == 0) return false;
+    const char* v = getenv("SVSB_GEMV_VARIANT");
+    return !(v && atoi(v) == 1);
+}
+
+// The similarity pass of one query: K1, or the fp16 filter (then filter_finish before the selection).
+static cudaError_t similarity_pass(cudaStream_t st, const DevWs& w, const Generation* g, const Shard& s, const float* q,
+                                   int shift, int reserve_sms, bool filter) {
+    if (filter) return launch_filter(st, w.dev, s.M16, s.n, g->ld, (g->ld + 7) & ~7, q, w.scores, w.gmax, shift, reserve_sms, s.live);
+    return launch_gemv(st, w.dev, s.M, s.n, g->d, g->ld, q, w.scores, w.gmax, shift, 0, 0, 0, reserve_sms, s.live);
+}
+// Threshold + exact re-score: afterwards scores / gmax give launch_select K1's top-kk.
+static cudaError_t filter_finish(cudaStream_t st, const DevWs& w, const Generation* g, const Shard& s, const float* q,
+                                 int shift, int64_t kk) {
+    return launch_filter_refine(st, w.dev, s.M, s.n, g->ld, q, w.scores, w.gmax, shift, (int)kk, coarse_eps_coef(g->d),
+                                (1.0f + g->max_dev) * 1.000001f, s.live, w.fstate);
+}
+
 int prepare_ws(DevWs& w, const Generation* g, const Shard& s, int64_t kk) {
     int rc;
     if ((rc = w.ensure_rows(s.n)) != SVSB_OK) return rc;
@@ -612,15 +688,17 @@ static int enqueue_single(QueryCtx* c, const Generation* g, const float* q, int3
         }
         CU(launch_stage_query(gst, c->h_q, w.d_q, g->ld));
         w.gmax_dirty = true;
+        const bool filter = use_filter(s, kk);
         {   // programmatic dependent launch: the similarity kernel streams its first tiles under the staging kernel
             PdlScope pdl(env_int("SVSB_PDL", 1) != 0);
-            CU(launch_gemv(gst, w.dev, s.M, s.n, g->d, g->ld, w.d_q, w.scores, w.gmax, shift, 0, 0, 0, reserve_sm ? 1 : 0, s.live));
+            CU(similarity_pass(gst, w, g, s, w.d_q, shift, reserve_sm ? 1 : 0, filter));
         }
         if (chain) {
             CU(cudaEventRecord(c->ev_gemv, gst));
             chain_lk.unlock();
             CU(cudaStreamWaitEvent(w.st, c->ev_gemv, 0));
         }
+        if (filter) CU(filter_finish(w.st, w, g, s, w.d_q, shift, kk));
         CU(launch_select(w.st, w.scores, s.n, w.gmax, shift, (int)kk, s.ids, s.row0, w.cand, w.cand_cap,
                          w.out_keys, c->h_scores, c->h_ids, c->h_count));
         w.gmax_dirty = false;
@@ -807,7 +885,7 @@ static bool batch_plan(svsb_engine* e, const Generation* g, int32_t k, BatchPlan
     }
     // |coarse - exact| <= eps_coef * ||q|| * max||row|| + 1e-8: two fp16 roundings per product (2u + u^2, u = 2^-11),
     // fp32 accumulation inside the tensor core (d * 2^-22, generous) and the exact kernel's own rounding (d * 2^-23)
-    P.eps_coef = 9.765625e-4f + 2.384185791015625e-7f + (float)g->d * (2.384185791015625e-7f + 1.1920928955078125e-7f);
+    P.eps_coef = coarse_eps_coef(g->d);
     P.max_row_norm = R * 1.000001f;
     return true;
 }
@@ -854,17 +932,13 @@ static int batch_ws_ensure(BatchWs* w, const BatchPlan& P, int b_pad) {
     return SVSB_OK;
 }
 
-// fp16 shadow of the matrix, built once per generation
+// fp16 shadow of the matrix: the shard buffer's (shared by the generations of one lineage), covering this view's rows
 static int ensure_m16(Generation* g, const BatchPlan& P, cudaStream_t st) {
     std::lock_guard<std::mutex> lk(g->m16_mu);
     if (g->M16) return SVSB_OK;
-    const Shard& s = g->shards[0];
-    CU(cudaSetDevice(s.dev));
     void* p = nullptr;
-    CU(cudaMalloc(&p, (size_t)s.n * P.ld16 * 2));
-    cudaError_t ce = launch_rows_to_f16(st, s.dev, s.M, s.n, g->ld, p, P.ld16);
-    if (ce == cudaSuccess) ce = cudaStreamSynchronize(st);
-    if (ce != cudaSuccess) { cudaFree(p); (void)cudaGetLastError(); return fail(SVSB_E_CUDA, std::string("fp16 shadow: ") + cudaGetErrorString(ce)); }
+    int rc = shadow_sync(g->shards[0], g->ld, INT64_MAX, 2, st, &p);
+    if (rc != SVSB_OK) return rc;
     g->M16 = p; g->ld16 = P.ld16;
     return SVSB_OK;
 }
@@ -1680,6 +1754,8 @@ extern "C" int svsb_bench_run(svsb_t* e, int32_t k, int32_t iters, float* total_
     // k <= 2048: software pipeline.  The similarity kernel of query i+1 (stream A, all SMs but one) runs while the
     // one-CTA selection kernel of query i (stream B) finishes on the SM left free; two buffer sets.
     const bool pipelined = kk <= K_FAST_MAX && env_int("SVSB_PIPELINE", 1) != 0 && sm_count(w0.dev) > 8;
+    const bool filter = use_filter(s, kk);
+    e->bench_filter = filter;
     if (pipelined) {
         if (!c->alt) {
             c->alt.reset(new DevWs());
@@ -1708,10 +1784,11 @@ extern "C" int svsb_bench_run(svsb_t* e, int32_t k, int32_t iters, float* total_
             if (it >= 2) CU(cudaStreamWaitEvent(sa, W.ev_sel, 0));           // selection of query it-2 is done with W
             if (timed_it(it)) CU(cudaEventRecord(kev[2 * it], sa));
             W.gmax_dirty = true;
-            CU(launch_gemv(sa, W.dev, s.M, s.n, g->d, g->ld, e->bench_q[0] + qoff, W.scores, W.gmax, shift, 0, 0, 0, /*reserve_sms=*/1, s.live));
+            CU(similarity_pass(sa, W, g.get(), s, e->bench_q[0] + qoff, shift, /*reserve_sms=*/1, filter));
             if (timed_it(it)) CU(cudaEventRecord(kev[2 * it + 1], sa));
             CU(cudaEventRecord(W.ev, sa));
             CU(cudaStreamWaitEvent(sb, W.ev, 0));
+            if (filter) CU(filter_finish(sb, W, g.get(), s, e->bench_q[0] + qoff, shift, kk));
             CU(launch_select(sb, W.scores, s.n, W.gmax, shift, (int)kk, s.ids, s.row0, W.cand, W.cand_cap,
                              W.out_keys, W.out_scores, W.out_ids, W.out_count));
             W.gmax_dirty = false;
@@ -1725,8 +1802,9 @@ extern "C" int svsb_bench_run(svsb_t* e, int32_t k, int32_t iters, float* total_
             const int64_t qoff = (int64_t)(it % e->bench_nq) * e->bench_ld;
             if (timed_it(it)) CU(cudaEventRecord(kev[2 * it], w0.st));
             w0.gmax_dirty = true;
-            CU(launch_gemv(w0.st, w0.dev, s.M, s.n, g->d, g->ld, e->bench_q[0] + qoff, w0.scores, w0.gmax, shift, 0, 0, 0, 0, s.live));
+            CU(similarity_pass(w0.st, w0, g.get(), s, e->bench_q[0] + qoff, shift, 0, filter));
             if (timed_it(it)) CU(cudaEventRecord(kev[2 * it + 1], w0.st));
+            if (filter) CU(filter_finish(w0.st, w0, g.get(), s, e->bench_q[0] + qoff, shift, kk));
             if (kk <= K_FAST_MAX)
                 CU(launch_select(w0.st, w0.scores, s.n, w0.gmax, shift, (int)kk, s.ids, s.row0, w0.cand, w0.cand_cap,
                                  w0.out_keys, w0.out_scores, w0.out_ids, w0.out_count));
@@ -1748,6 +1826,20 @@ extern "C" int svsb_bench_run(svsb_t* e, int32_t k, int32_t iters, float* total_
             if (timed_it(it)) { float t = 0.f; CU(cudaEventElapsedTime(&t, kev[2 * it], kev[2 * it + 1])); sum += t; ++cnt; }
         *gemv_ms = sum * (float)iters / (float)cnt;            // mean bracketed launch x launches
     } else if (gemv_ms) *gemv_ms = 0.f;
+    return SVSB_OK;
+}
+
+extern "C" int svsb_bench_filter_stats(svsb_t* e, int32_t* filter, int64_t* rescored) {
+    if (!e || !filter || !rescored) return fail(SVSB_E_INVALID, "svsb_bench_filter_stats: NULL argument");
+    *filter = 0; *rescored = 0;
+    if (e->multi || !e->bench_ctx || !e->bench_ctx->last) return SVSB_OK;
+    if (!e->bench_filter) return SVSB_OK;
+    const DevWs& w = *e->bench_ctx->last;
+    uint32_t st[2] = {0, 0};
+    CU(cudaSetDevice(w.dev));
+    CU(cudaStreamSynchronize(w.st));
+    CU(cudaMemcpy(st, w.fstate, 8, cudaMemcpyDeviceToHost));
+    *filter = 1; *rescored = st[1];
     return SVSB_OK;
 }
 

@@ -46,10 +46,16 @@ struct ShardBuf {
     float* M = nullptr;          // cap_rows x ld floats
     int64_t* ids = nullptr;      // cap_rows
     int64_t cap_rows = 0;
+    // fp16 shadow M16 = fp16(M * 2^12), cap_rows x ld16 halfs (DESIGN.md section 6): rows [0, m16_rows) are converted.
+    // Built at load for the single-query filter when it fits, else lazily by the first batch; appended rows are
+    // converted by the update that writes them (shadow_sync).
+    std::mutex m16_mu;
+    void* M16 = nullptr; int ld16 = 0; int64_t m16_rows = 0;
     ~ShardBuf() {
-        if (M || ids) cudaSetDevice(dev);
+        if (M || ids || M16) cudaSetDevice(dev);
         if (M) cudaFree(M);
         if (ids) cudaFree(ids);
+        if (M16) cudaFree(M16);
     }
 };
 
@@ -63,6 +69,9 @@ struct Shard {
     // generation (a delete must not disturb queries still running on the previous generation).
     uint8_t* live = nullptr;
     int64_t n_live = 0;
+    // == buf->M16 when this view's single queries take the fp16 filter (set before the generation is published, never
+    // changed after; null: K1 -- see filter_shadow in engine.cu)
+    const void* M16 = nullptr;
 };
 
 struct Generation {
@@ -77,7 +86,7 @@ struct Generation {
     int64_t n_out_of_tol = 0;
     // multi-device engines: one single-shard view per device, what that device's shard engine queries
     std::vector<std::shared_ptr<Generation>> child_gen;
-    // fp16 shadow of shard 0 for the batched coarse contraction (built lazily by the first batch, DESIGN.md section 6)
+    // fp16 shadow of shard 0 for the batched coarse contraction (shard 0's buf->M16 once ensure_m16 has covered its rows)
     std::mutex m16_mu;
     void* M16 = nullptr; int ld16 = 0;
     // set once a batch saw its statistical filter thresholds fail verification (rows not in random order w.r.t. the
@@ -88,7 +97,6 @@ struct Generation {
         child_gen.clear();
         if (owns_live)
             for (auto& s : shards) if (s.live) { cudaSetDevice(s.dev); cudaFree(s.live); }
-        if (M16 && !shards.empty()) { cudaSetDevice(shards[0].dev); cudaFree(M16); }
     }
 };
 
@@ -104,6 +112,7 @@ struct svsb_workspace {
     u64* sortbuf = nullptr;  int64_t sort_cap = 0;
     u64* out_keys = nullptr; float* out_scores = nullptr; int64_t* out_ids = nullptr; int64_t out_cap = 0;
     int32_t* out_count = nullptr;
+    uint32_t* fstate = nullptr;      // fp16 filter: candidate threshold + rows re-scored (launch_filter_refine)
     u64* mscr_keys = nullptr; int64_t* mscr_ids = nullptr; int64_t mscr_cap = 0;   // merge scratch
     cudaEvent_t ev = nullptr, ev0 = nullptr, ev1 = nullptr, ev_sel = nullptr;
     // The similarity kernel leaves group maxima in gmax and only a SUCCESSFUL selection kernel re-zeroes them
@@ -144,6 +153,7 @@ struct svsb_workspace {
     int ensure_out(int64_t k) {
         cudaSetDevice(dev);
         if (!out_count) CU(cudaMalloc(&out_count, 64));
+        if (!fstate) CU(cudaMalloc(&fstate, 8));
         if (k > out_cap) {
             if (out_keys) cudaFree(out_keys); if (out_scores) cudaFree(out_scores); if (out_ids) cudaFree(out_ids);
             out_keys = nullptr; out_scores = nullptr; out_ids = nullptr; out_cap = 0;
@@ -173,7 +183,7 @@ struct svsb_workspace {
     }
     void release() {
         cudaSetDevice(dev);
-        void* ptrs[] = {d_q, scores, gmax, cand, sortbuf, out_keys, out_scores, out_ids, out_count, mscr_keys, mscr_ids};
+        void* ptrs[] = {d_q, scores, gmax, cand, sortbuf, out_keys, out_scores, out_ids, out_count, fstate, mscr_keys, mscr_ids};
         for (void* p : ptrs) if (p) cudaFree(p);
         if (ev) cudaEventDestroy(ev); if (ev0) cudaEventDestroy(ev0); if (ev1) cudaEventDestroy(ev1);
         if (ev_sel) cudaEventDestroy(ev_sel);
@@ -432,6 +442,7 @@ struct svsb_engine {
     std::vector<float*> bench_q; int bench_nq = 0, bench_d = 0, bench_ld = 0;
     std::unique_ptr<QueryCtx> bench_ctx;
     std::vector<cudaEvent_t> bench_kev;                  // similarity-kernel timing events of svsb_bench_run (device 0)
+    bool bench_filter = false;                           // the last svsb_bench_run took the fp16 filter
     // sharded deployment (one process per GPU)
     int64_t shard_row0 = 0;                              // global row of this engine's first row
     std::vector<std::unique_ptr<DevWs>> shard_ws;        // workspaces for svsb_enqueue_local_topk (by slot)
@@ -458,6 +469,10 @@ struct svsb_snapshot { std::shared_ptr<Generation> gen; };
 // ------------------------------------------------------------------------------------------------
 std::shared_ptr<Generation> pin(svsb_engine* e);
 int prepare_ws(DevWs& w, const Generation* g, const Shard& s, int64_t kk);
+// Convert rows [buf->m16_rows, s.n) of the shard's fp16 shadow (rows from `fresh_from` on were (re)written: they are
+// converted again).  No shadow yet: create = 0 leaves it so (*out = null), 1 allocates it when the device keeps ample
+// room after it (else *out = null, not an error), 2 allocates it or fails.
+int shadow_sync(const Shard& s, int ld, int64_t fresh_from, int create, cudaStream_t st, void** out);
 int engine_create(const int* device_ids, int n_dev, bool as_kid, svsb_engine** out);
 int alloc_generation(svsb_engine* e, int64_t n, int d, std::shared_ptr<Generation>& out);
 int finish_generation(svsb_engine* e, Generation* g, int norm_mode);

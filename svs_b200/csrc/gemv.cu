@@ -14,6 +14,7 @@
 //                      on mbarriers; consumer warps read the tile and the query from shared memory.
 // Which one runs by default is decided by measurement (profiles/), not by taste.
 #include "kernels.cuh"
+#include <cuda_fp16.h>
 #include <cstdlib>
 
 namespace svsb {
@@ -378,6 +379,243 @@ gemv_tma_mq_kernel(const float* __restrict__ M, int64_t n, int d4, int tile_rows
 }
 
 // =============================================================================================
+// variant 3: the fp16 filter -- the same ring over the fp16 shadow, then an exact re-score of the few candidates
+// =============================================================================================
+// A single query reads n*d*4 bytes with K1 at the HBM rate; the filter reads the shadow M16 = fp16(M * 2^12) instead
+// (n*d*2 bytes) and writes K1's outputs -- scores[n], group maxima -- as COARSE values.  filter_threshold_kernel turns
+// them into a threshold T <= tau~ - 2 eps (tau~ = the kk-th largest coarse score), filter_rescore_kernel gives every
+// row with coarse >= T its exact score (K1's arithmetic, bit for bit) and every other row of the groups it rescans the
+// tombstone score, and rewrites the group maxima so that the unchanged selection kernel sees only exact scores.
+// Exactness (DESIGN.md section 4, "K1f"): |coarse - exact| <= eps, kk rows have coarse >= tau~, so every row of the exact
+// top-kk has coarse >= tau~ - 2 eps >= T.
+
+// NC: 16-byte chunks (8 halfs) of the shadow row per lane, c16 = ld16 / 8 <= 32 * NC.  The query stays fp32 (its
+// 8 floats per chunk in registers); the row is widened exactly to fp32 and accumulated with fp32 FMAs.
+template <int CW, int NC>
+__global__ void __launch_bounds__((CW + 1) * 32, 1)
+gemv16_tma_kernel(const __half* __restrict__ M16, int64_t n, int c16, int tile_rows, int stages,
+                  const float* __restrict__ q, int ld, float* __restrict__ scores, u64* __restrict__ gmax, int group_shift,
+                  const uint8_t* __restrict__ live)
+{
+    extern __shared__ __align__(128) unsigned char smem_raw[];
+    const uint32_t row_bytes = (uint32_t)c16 * 16u;
+    const uint32_t stage_bytes = (uint32_t)tile_rows * row_bytes;
+    uint64_t* full = reinterpret_cast<uint64_t*>(smem_raw + (size_t)stages * stage_bytes);
+    uint64_t* empty = full + stages;
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    if (threadIdx.x == 0) {
+        pdl_trigger();
+        for (int s = 0; s < stages; ++s) { mbar_init(&full[s], 1); mbar_init(&empty[s], CW); }
+        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    }
+    __syncthreads();
+
+    const int64_t ntiles = (n + tile_rows - 1) / tile_rows;
+    if (warp == CW) {
+        if (lane == 0) {
+            u64 policy;
+            asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(policy));
+            int s = 0; uint32_t phase = 0;
+            for (int64_t t = blockIdx.x; t < ntiles; t += gridDim.x) {
+                mbar_wait(&empty[s], phase ^ 1u);
+                const int64_t r0 = t * tile_rows;
+                const int64_t left = n - r0;
+                const uint32_t rows = left < tile_rows ? (uint32_t)left : (uint32_t)tile_rows;
+                const uint32_t bytes = rows * row_bytes;
+                mbar_arrive_expect_tx(&full[s], bytes);
+                bulk_g2s(smem_raw + (size_t)s * stage_bytes, reinterpret_cast<const unsigned char*>(M16) + (size_t)r0 * row_bytes,
+                         bytes, &full[s], policy);
+                if (++s == stages) { s = 0; phase ^= 1u; }
+            }
+        }
+    } else {
+        pdl_wait();                                   // the query is written by the previous kernel (see gemv_tma_kernel)
+        float4 qr[NC][2];
+        const int ld4 = ld >> 2;
+#pragma unroll
+        for (int j = 0; j < NC; ++j) {
+            const int c = lane + 32 * j;
+            qr[j][0] = 2 * c < ld4 ? __ldcg(reinterpret_cast<const float4*>(q) + 2 * c) : make_float4(0.f, 0.f, 0.f, 0.f);
+            qr[j][1] = 2 * c + 1 < ld4 ? __ldcg(reinterpret_cast<const float4*>(q) + 2 * c + 1) : make_float4(0.f, 0.f, 0.f, 0.f);
+        }
+        int s = 0; uint32_t phase = 0;
+        for (int64_t t = blockIdx.x; t < ntiles; t += gridDim.x) {
+            const int64_t r0 = t * tile_rows;
+            const int64_t left = n - r0;
+            const int rows = left < tile_rows ? (int)left : tile_rows;
+            mbar_wait(&full[s], phase);
+            const uint4* tile = reinterpret_cast<const uint4*>(smem_raw + (size_t)s * stage_bytes);
+            u64 kmax = 0;
+            for (int r = warp; r < rows; r += CW) {
+                const uint4* p = tile + (size_t)r * c16;
+                const uint8_t alive = live ? __ldg(live + r0 + r) : (uint8_t)1;
+                uint4 m[NC];
+#pragma unroll
+                for (int j = 0; j < NC; ++j) { const int c = lane + 32 * j; m[j] = c < c16 ? p[c] : make_uint4(0u, 0u, 0u, 0u); }
+                float4 a0 = make_float4(0.f, 0.f, 0.f, 0.f), a1 = a0;
+#pragma unroll
+                for (int j = 0; j < NC; ++j) {
+                    const float2 h0 = __half22float2(*reinterpret_cast<const __half2*>(&m[j].x));
+                    const float2 h1 = __half22float2(*reinterpret_cast<const __half2*>(&m[j].y));
+                    const float2 h2 = __half22float2(*reinterpret_cast<const __half2*>(&m[j].z));
+                    const float2 h3 = __half22float2(*reinterpret_cast<const __half2*>(&m[j].w));
+                    fma4(a0, make_float4(h0.x, h0.y, h1.x, h1.y), qr[j][0]);
+                    fma4(a1, make_float4(h2.x, h2.y, h3.x, h3.y), qr[j][1]);
+                }
+                // x 2^-12 undoes the operand scale exactly
+                float sc = warp_sum(((a0.x + a1.x) + (a0.y + a1.y)) + ((a0.z + a1.z) + (a0.w + a1.w))) * (1.0f / COARSE_OPERAND_SCALE);
+                if (!alive) sc = dead_score();
+                if (lane == 0) {
+                    scores[r0 + r] = sc;
+                    const u64 k0 = make_key(sc, (uint32_t)(r0 + r));
+                    kmax = k0 > kmax ? k0 : kmax;
+                }
+            }
+            __syncwarp();
+            if (lane == 0) {
+                mbar_arrive(&empty[s]);
+                if (kmax) atomicMax(&gmax[r0 >> group_shift], kmax);
+            }
+            if (++s == stages) { s = 0; phase ^= 1u; }
+        }
+    }
+}
+
+// One CTA.  state[0] = T as an ordered key word (f32_to_ordered): the rows with f32_to_ordered(coarse) >= T are the
+// candidates; T = 0 takes every row (no usable threshold: at most kk groups, a non-finite query or group maximum).
+// state[1] = 0 (the re-score kernel counts its rows there).
+// T = (kk-th largest group maximum) - 2 eps, rounded down: that maximum comes from kk distinct rows, so it is <= tau~.
+constexpr int FT_THREADS = 1024;
+constexpr int FT_PER_THREAD = (int)(GROUPS_TARGET / FT_THREADS);
+__global__ void __launch_bounds__(FT_THREADS, 1)
+filter_threshold_kernel(const u64* __restrict__ gmax, int G, int kk, const float* __restrict__ q, int ld,
+                        float eps_coef, float max_row_norm, uint32_t* __restrict__ state)
+{
+    __shared__ uint32_t hist[256];
+    __shared__ float red[FT_THREADS / 32];
+    __shared__ uint32_t sh_prefix, sh_want;
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    float ss = 0.f;
+    for (int i = tid; i < ld; i += FT_THREADS) { const float v = __ldcg(q + i); ss = fmaf(v, v, ss); }
+    ss = warp_sum(ss);
+    if (lane == 0) red[warp] = ss;
+    uint32_t v[FT_PER_THREAD];                         // high words of the group maxima (ordered coarse scores)
+#pragma unroll
+    for (int j = 0; j < FT_PER_THREAD; ++j) { const int i = tid + j * FT_THREADS; v[j] = i < G ? (uint32_t)(__ldcg(gmax + i) >> 32) : 0u; }
+    if (tid == 0) { sh_prefix = 0u; sh_want = (uint32_t)kk; }
+    __syncthreads();
+    // kk-th largest of the G words: radix select, 8 bits per round from the top
+    uint32_t mask = 0u;
+    for (int shift = 24; shift >= 0; shift -= 8) {
+        if (tid < 256) hist[tid] = 0u;
+        __syncthreads();
+        const uint32_t prefix = sh_prefix;
+#pragma unroll
+        for (int j = 0; j < FT_PER_THREAD; ++j)
+            if (tid + j * FT_THREADS < G && (v[j] & mask) == prefix) atomicAdd(&hist[(v[j] >> shift) & 255u], 1u);
+        __syncthreads();
+        if (warp == 0) {
+            // lane l owns bins [8l, 8l + 8); suffix[l] = entries in bins >= 8l
+            uint32_t c = 0;
+#pragma unroll
+            for (int b = 0; b < 8; ++b) c += hist[8 * lane + b];
+            uint32_t suf = c;
+#pragma unroll
+            for (int o = 1; o < 32; o <<= 1) { const uint32_t t = __shfl_down_sync(0xffffffffu, suf, o); if (lane + o < 32) suf += t; }
+            const uint32_t want = sh_want;
+            const unsigned ball = __ballot_sync(0xffffffffu, suf >= want);
+            const int top = 31 - __clz(ball);              // the highest lane whose bins reach the kk-th entry
+            if (lane == top) {
+                uint32_t cum = suf - c;
+                for (int b = 7; b >= 0; --b) {
+                    const uint32_t h = hist[8 * lane + b];
+                    if (cum + h >= want) { sh_prefix = prefix | ((uint32_t)(8 * lane + b) << shift); sh_want = want - cum; break; }
+                    cum += h;
+                }
+            }
+        }
+        mask |= 255u << shift;
+        __syncthreads();
+    }
+    if (tid == 0) {
+        float qq = 0.f;
+        for (int w = 0; w < FT_THREADS / 32; ++w) qq += red[w];
+        const float qn = sqrtf(qq);
+        const float tau = ordered_to_f32(sh_prefix);
+        uint32_t T = 0u;
+        if (G > kk && isfinite(tau) && isfinite(qn)) {
+            const double eps = (double)eps_coef * (double)qn * (double)max_row_norm + 1e-8;
+            float t = __double2float_rd((double)tau - 2.0 * eps);
+            if (t == 0.f) t = -0.f;                         // f32_to_ordered(-0) < f32_to_ordered(+0): keep both zeros
+            T = f32_to_ordered(t);
+        }
+        state[0] = T;
+        state[1] = 0u;
+    }
+}
+
+// One warp per row group (grid-stride).  A group whose coarse maximum reaches T: every candidate row (live, coarse >= T)
+// is re-scored by the warp with gemv_tma_kernel's arithmetic (lane l owns float4 chunks l, l+32, ...; even chunks into
+// a0, odd ones into a1; same combine, same xor tree) -- the bits K1 would have written; the group's other rows get the
+// tombstone score; its maximum becomes the largest key over both.  Any other group's maximum becomes 0, so the
+// selection kernel (which rescans only groups whose maximum reaches its kk-th largest, a candidate's key: at least kk
+// groups hold a candidate) never reads its coarse scores.
+template <int NQ>
+__global__ void __launch_bounds__(256)
+filter_rescore_kernel(const float* __restrict__ M, int64_t n, int d4, const float* __restrict__ q, float* __restrict__ scores,
+                      u64* __restrict__ gmax, int group_shift, const uint8_t* __restrict__ live, uint32_t* __restrict__ state)
+{
+    __shared__ float4 sq[32 * NQ];
+    for (int c = threadIdx.x; c < 32 * NQ; c += blockDim.x) sq[c] = c < d4 ? __ldcg(reinterpret_cast<const float4*>(q) + c) : make_float4(0.f, 0.f, 0.f, 0.f);
+    __syncthreads();
+    const uint32_t T = __ldcg(state);
+    const int lane = threadIdx.x & 31;
+    const int64_t G = (n + ((int64_t)1 << group_shift) - 1) >> group_shift;
+    const int64_t nwarps = (int64_t)gridDim.x * (blockDim.x >> 5);
+    for (int64_t g = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); g < G; g += nwarps) {
+        const u64 gm = gmax[g];
+        u64 kmax = 0;
+        if ((uint32_t)(gm >> 32) >= T) {
+            const int64_t r_beg = g << group_shift;
+            const int64_t r_end = min(n, r_beg + ((int64_t)1 << group_shift));
+            int found = 0;
+            for (int64_t rb = r_beg; rb < r_end; rb += 32) {
+                const int64_t r = rb + lane;
+                const bool in = r < r_end;
+                const bool alive = in && (!live || live[r]);
+                const bool cand = alive && f32_to_ordered(scores[r]) >= T;
+                if (in && !cand) {
+                    scores[r] = dead_score();
+                    const u64 k0 = make_key(dead_score(), (uint32_t)r);
+                    kmax = k0 > kmax ? k0 : kmax;
+                }
+                unsigned ball = __ballot_sync(0xffffffffu, cand);
+                found += __popc(ball);
+                while (ball) {
+                    const int b = __ffs(ball) - 1;
+                    ball &= ball - 1;
+                    const int64_t rr = rb + b;
+                    const float4* p = reinterpret_cast<const float4*>(M) + rr * (int64_t)d4;
+                    float4 m[NQ];
+#pragma unroll
+                    for (int j = 0; j < NQ; ++j) { const int c = lane + 32 * j; m[j] = c < d4 ? ldg_stream(p + c) : make_float4(0.f, 0.f, 0.f, 0.f); }
+                    float4 a0 = make_float4(0.f, 0.f, 0.f, 0.f), a1 = a0;
+#pragma unroll
+                    for (int j = 0; j < NQ; ++j) { if (j & 1) fma4(a1, m[j], sq[lane + 32 * j]); else fma4(a0, m[j], sq[lane + 32 * j]); }
+                    const float sc = warp_sum(((a0.x + a1.x) + (a0.y + a1.y)) + ((a0.z + a1.z) + (a0.w + a1.w)));
+                    if (lane == b) scores[rr] = sc;
+                    const u64 k0 = make_key(sc, (uint32_t)rr);
+                    kmax = k0 > kmax ? k0 : kmax;
+                }
+            }
+            kmax = warp_max_u64(kmax);
+            if (lane == 0 && found) atomicAdd(state + 1, (uint32_t)found);
+        }
+        if (lane == 0) gmax[g] = kmax;
+    }
+}
+
+// =============================================================================================
 // host side
 // =============================================================================================
 int sm_count(int device) {
@@ -483,6 +721,11 @@ cudaError_t preload_gemv_kernels()
     SVSB_PRE((gemv_tma_kernel<16, 2>)); SVSB_PRE((gemv_tma_kernel<16, 6>)); SVSB_PRE((gemv_tma_kernel<16, 12>));
     SVSB_PRE((gemv_tma_kernel<16, 24>)); SVSB_PRE((gemv_tma_kernel<16, 0>));
     SVSB_PRE((gemv_ldg_kernel<4, 3, 256>));
+    SVSB_PRE((gemv16_tma_kernel<8, 1>)); SVSB_PRE((gemv16_tma_kernel<8, 2>)); SVSB_PRE((gemv16_tma_kernel<8, 4>));
+    SVSB_PRE((gemv16_tma_kernel<8, 6>)); SVSB_PRE((gemv16_tma_kernel<8, 8>)); SVSB_PRE((gemv16_tma_kernel<8, 12>));
+    SVSB_PRE(filter_threshold_kernel);
+    SVSB_PRE((filter_rescore_kernel<2>)); SVSB_PRE((filter_rescore_kernel<6>)); SVSB_PRE((filter_rescore_kernel<12>));
+    SVSB_PRE((filter_rescore_kernel<24>));
 #undef SVSB_PRE
     return e;
 }
@@ -522,6 +765,79 @@ cudaError_t launch_gemv(cudaStream_t st, int device, const float* M, int64_t n, 
         case 9:  return run_ldg<8, 3, 128>(st, device, M, n, d4, q, scores, gmax, group_shift, live, tune_b);
         default: return run_ldg<4, 3, 256>(st, device, M, n, d4, q, scores, gmax, group_shift, live, tune_b);
     }
+}
+
+// ---- fp16 filter launchers --------------------------------------------------------------------
+template <int CW, int NC>
+static cudaError_t run_filter_inst(cudaStream_t st, int64_t grid, size_t smem, const void* M16, int64_t n, int c16, int tile_rows,
+                                   int stages, const float* q, int ld, float* scores, u64* gmax, int group_shift, const uint8_t* live)
+{
+    auto kern = gemv16_tma_kernel<CW, NC>;
+    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return e;
+    e = launch_kernel(kern, dim3((unsigned)grid), dim3((CW + 1) * 32), smem, st, reinterpret_cast<const __half*>(M16), n, c16,
+                      tile_rows, stages, q, ld, scores, gmax, group_shift, live);
+    count_launch();
+    return e != cudaSuccess ? e : cudaGetLastError();
+}
+
+cudaError_t launch_filter(cudaStream_t st, int device, const void* M16, int64_t n, int ld, int ld16, const float* q,
+                          float* scores, u64* gmax, int group_shift, int reserve_sms, const uint8_t* live)
+{
+    if (n <= 0) return cudaSuccess;
+    if (ld > FILTER_MAX_LD || ld16 < ld || (ld16 & 7)) return cudaErrorInvalidValue;
+    const int c16 = ld16 / 8;
+    const size_t row_bytes = (size_t)ld16 * 2;
+    // K1's ring: ~48 KB tiles x 3 stages (profiles/r01_tune_gemv.md)
+    int tile_rows = 64;
+    while (tile_rows > 1 && (size_t)tile_rows * row_bytes > 48 * 1024) tile_rows >>= 1;
+    const int stages = 3;
+    const size_t smem = (size_t)stages * tile_rows * row_bytes + (size_t)stages * 16 + 64;
+    const int64_t ntiles = (n + tile_rows - 1) / tile_rows;
+    int64_t grid = sm_count(device) - reserve_sms;
+    if (grid > ntiles) grid = ntiles;
+    if (grid < 1) grid = 1;
+#define SVSB_F16_CASE(NCV) \
+    return run_filter_inst<8, NCV>(st, grid, smem, M16, n, c16, tile_rows, stages, q, ld, scores, gmax, group_shift, live)
+    if (c16 <= 32) SVSB_F16_CASE(1);
+    if (c16 <= 64) SVSB_F16_CASE(2);
+    if (c16 <= 128) SVSB_F16_CASE(4);
+    if (c16 <= 192) SVSB_F16_CASE(6);
+    if (c16 <= 256) SVSB_F16_CASE(8);
+    SVSB_F16_CASE(12);
+#undef SVSB_F16_CASE
+}
+
+template <int NQ>
+static cudaError_t run_rescore_inst(cudaStream_t st, int device, const float* M, int64_t n, int d4, const float* q, float* scores,
+                                    u64* gmax, int group_shift, const uint8_t* live, uint32_t* state)
+{
+    const int64_t G = (n + ((int64_t)1 << group_shift) - 1) >> group_shift;
+    int64_t blocks = (G + 7) / 8;
+    const int64_t cap = (int64_t)sm_count(device) * 4;
+    if (blocks > cap) blocks = cap;
+    filter_rescore_kernel<NQ><<<(unsigned)blocks, 256, 0, st>>>(M, n, d4, q, scores, gmax, group_shift, live, state);
+    count_launch();
+    return cudaGetLastError();
+}
+
+cudaError_t launch_filter_refine(cudaStream_t st, int device, const float* M, int64_t n, int ld, const float* q, float* scores,
+                                 u64* gmax, int group_shift, int kk, float eps_coef, float max_row_norm, const uint8_t* live,
+                                 uint32_t* state)
+{
+    if (n <= 0) return cudaSuccess;
+    if (ld > FILTER_MAX_LD) return cudaErrorInvalidValue;
+    const int64_t G = (n + ((int64_t)1 << group_shift) - 1) >> group_shift;
+    if (G > GROUPS_TARGET) return cudaErrorInvalidValue;
+    filter_threshold_kernel<<<1, FT_THREADS, 0, st>>>(gmax, (int)G, kk, q, ld, eps_coef, max_row_norm, state);
+    count_launch();
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return e;
+    const int d4 = ld / 4;
+    if (d4 <= 64) return run_rescore_inst<2>(st, device, M, n, d4, q, scores, gmax, group_shift, live, state);
+    if (d4 <= 192) return run_rescore_inst<6>(st, device, M, n, d4, q, scores, gmax, group_shift, live, state);
+    if (d4 <= 384) return run_rescore_inst<12>(st, device, M, n, d4, q, scores, gmax, group_shift, live, state);
+    return run_rescore_inst<24>(st, device, M, n, d4, q, scores, gmax, group_shift, live, state);
 }
 
 // ---- multi-query launcher ---------------------------------------------------------------------

@@ -48,6 +48,23 @@ cudaError_t launch_gemv(cudaStream_t st, int device, const float* M, int64_t n, 
                         int variant = 0, int tune_a = 0, int tune_b = 0, int reserve_sms = 0,
                         const uint8_t* live = nullptr);
 
+// K1f, the fp16 filter (gemv.cu, DESIGN.md section 4): launch_filter writes launch_gemv's outputs as COARSE values from
+// the shadow M16[n][ld16] = fp16(M * 2^12) (launch_rows_to_f16) and the fp32 query q[ld]; launch_filter_refine then
+// (1 CTA) sets the candidate threshold state[0] from the group maxima and the bound
+// eps = eps_coef * ||q|| * max_row_norm + 1e-8 on |coarse - exact|, and (many CTAs) re-scores every candidate exactly --
+// the bits launch_gemv writes -- leaving scores / gmax such that launch_select returns launch_gemv's top-kk.
+// state: 2 device words, state[1] = rows re-scored.  ld <= FILTER_MAX_LD.
+constexpr int FILTER_MAX_LD = 3072;
+cudaError_t launch_filter(cudaStream_t st, int device, const void* M16, int64_t n, int ld, int ld16, const float* q,
+                          float* scores, u64* gmax, int group_shift, int reserve_sms = 0, const uint8_t* live = nullptr);
+cudaError_t launch_filter_refine(cudaStream_t st, int device, const float* M, int64_t n, int ld, const float* q, float* scores,
+                                 u64* gmax, int group_shift, int kk, float eps_coef, float max_row_norm, const uint8_t* live,
+                                 uint32_t* state);
+// the bound's coefficient for d components (fp16 operands, fp32 accumulation; DESIGN.md section 6, step 4)
+inline float coarse_eps_coef(int d) {
+    return 9.765625e-4f + 2.384185791015625e-7f + (float)d * (2.384185791015625e-7f + 1.1920928955078125e-7f);
+}
+
 // b queries Q[b][ld] in ONE pass over the matrix: scores[q * n_stride + r], gmax[q * g_stride + (r >> shift)] (zero on
 // entry), bit-identical to b launch_gemv calls.  cudaErrorInvalidConfiguration: rows too long (ld > 3072) or b larger
 // than 8 warps' worth of queries (8 * gemv_mq_queries_per_warp(ld)); the caller chunks / falls back.

@@ -195,6 +195,9 @@ extern "C" int svsb_apply_mutations(svsb_t* e, const int64_t* del_ids, int64_t n
         }
         s.n = new_n;
         s.n_live += n_add;
+        void* m16 = nullptr;                                     // a shadow of this buffer: convert the new rows only
+        int rc = shadow_sync(s, ng->ld, os.n, 0, st, &m16);
+        if (rc != SVSB_OK) return rc;
     }
     ng->n = 0; ng->n_live = 0;
     for (auto& s : ng->shards) { ng->n += s.n; ng->n_live += s.n_live; }

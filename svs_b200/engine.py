@@ -305,6 +305,12 @@ class Engine:
         check(self._lib.svsb_batch_stats(self._h, b, cand.ctypes.data, resc.ctypes.data, flags.ctypes.data))
         return cand, resc, flags
 
+    def bench_filter_stats(self) -> Tuple[bool, int]:
+        """(took the fp16 filter, rows the last query re-scored exactly) of the last bench_run."""
+        f, r = C.c_int32(), C.c_int64()
+        check(self._lib.svsb_bench_filter_stats(self._h, C.byref(f), C.byref(r)))
+        return bool(f.value), int(r.value)
+
     def batch_threshold_mode(self) -> int:
         """0 = verified statistical filter thresholds (default), 1 = proven-bound thresholds (see svsb200.h)."""
         rc = self._lib.svsb_batch_threshold_mode(self._h)
