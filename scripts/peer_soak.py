@@ -38,7 +38,7 @@ def main():
     sr = ShardedRetriever(rank, world, local, exchange="peer")
     sr.load_global(m, ids)
     sr.set_queries(qs)
-    sr._ensure_peer()
+    sr._ensure_window()
     ks = (1, 10, 100, 1000, 2048, 7, 100, 100)
     mult = torch.arange(1, 2049, device="cuda", dtype=torch.int64)
     h = torch.zeros((), device="cuda", dtype=torch.int64)

@@ -164,7 +164,7 @@ static void xchg_release(svsb_engine* e) {
     if (!x) return;
     cudaSetDevice(e->devs[0]);
     if (x->st) cudaStreamSynchronize(x->st);
-    for (void* p : x->ipc_opened) cudaIpcCloseMemHandle(p);
+    x->maps.close();
     if (x->block) cudaFree(x->block);
     if (x->stamps) cudaFree(x->stamps);
     x->ws.release();
@@ -1403,6 +1403,91 @@ extern "C" int svsb_snapshot_top_pairs(svsb_t* e, svsb_snap_t* s, int64_t n_pair
     return top_pairs_gen(e, s->gen, n_pairs, out_scores, out_ids_a, out_ids_b, out_count);
 }
 
+// ---- peer memory of the one-process-per-GPU deployment: what a rank maps of its peers, and when it lets go -----------
+// The query exchange (Xchg), the batch window (BXchg) and the pair search (PairsShard) read or write other ranks' device
+// memory.  A connect that fails part-way closes what it opened; an unmap leaves the state create left.
+static_assert(sizeof(cudaIpcMemHandle_t) == 64, "cudaIpcMemHandle_t is 64 bytes");
+
+int PeerMaps::open(const void* handle, void** out, const char* who) {
+    cudaIpcMemHandle_t h;
+    memcpy(&h, handle, 64);
+    const cudaError_t ce = cudaIpcOpenMemHandle(out, h, cudaIpcMemLazyEnablePeerAccess);
+    (void)cudaGetLastError();
+    if (ce != cudaSuccess) return fail(SVSB_E_CUDA, std::string(who) + ": cudaIpcOpenMemHandle: " + cudaGetErrorString(ce));
+    opened.push_back(*out);
+    return SVSB_OK;
+}
+
+int PeerMaps::reach(int self, int dev, const char* who) {
+    if (dev == self) return SVSB_OK;
+    int can = 0;
+    CU(cudaDeviceCanAccessPeer(&can, self, dev));
+    if (!can) return fail(SVSB_E_CUDA, std::string(who) + ": no peer access between the devices");
+    const cudaError_t pe = cudaDeviceEnablePeerAccess(dev, 0);
+    (void)cudaGetLastError();
+    if (pe == cudaSuccess || pe == cudaErrorPeerAccessAlreadyEnabled) return SVSB_OK;    // another connect enabled it before
+    return fail(SVSB_E_CUDA, std::string(who) + ": enabling peer access: " + cudaGetErrorString(pe));
+}
+
+void PeerMaps::close() {
+    for (void* p : opened) cudaIpcCloseMemHandle(p);
+    opened.clear();
+}
+
+int PeerWindow::publish(void* handle_out) {
+    peer_block.assign(world, nullptr);
+    peer_block[rank] = block;
+    if (const char* v = getenv("SVSB_XCHG_TIMEOUT_MS")) { const long long ms = atoll(v); if (ms > 0) timeout_ns = (unsigned long long)ms * 1000000ull; }
+    if (handle_out) {
+        cudaIpcMemHandle_t h;
+        CU(cudaIpcGetMemHandle(&h, block));
+        memcpy(handle_out, &h, 64);
+    }
+    connected = world == 1;
+    return SVSB_OK;
+}
+
+int PeerWindow::connect(const void* handles, const char* who) {
+    for (int r = 0; r < world; ++r) {
+        if (r == rank) continue;
+        void* p = nullptr;
+        const int rc = maps.open(static_cast<const unsigned char*>(handles) + (size_t)r * 64, &p, who);
+        if (rc != SVSB_OK) { unmap(); return rc; }
+        peer_block[r] = static_cast<unsigned char*>(p);
+    }
+    connected = true;
+    return SVSB_OK;
+}
+
+int PeerWindow::connect_local(int dev, svsb_engine* const* engines, PeerWindow* (*window_of)(svsb_engine*, const PeerWindow*),
+                              const char* who) {
+    for (int r = 0; r < world; ++r) {
+        if (r == rank) continue;
+        svsb_engine* o = engines[r];
+        const PeerWindow* w = o ? window_of(o, this) : nullptr;
+        if (!w || w->world != world || w->rank != r) { unmap(); return fail(SVSB_E_INVALID, std::string(who) + ": peer engine has no matching window"); }
+        const int rc = maps.reach(dev, o->devs[0], who);
+        if (rc != SVSB_OK) { unmap(); return rc; }
+        peer_block[r] = w->block;
+    }
+    connected = true;
+    return SVSB_OK;
+}
+
+void PeerWindow::unmap() {
+    maps.close();
+    for (size_t r = 0; r < peer_block.size(); ++r) if ((int)r != rank) peer_block[r] = nullptr;
+    connected = world == 1;
+}
+
+// world / rank of a protocol of the one-process-per-GPU deployment, on an engine of one device
+static int check_world_rank(const svsb_engine* e, int32_t world, int32_t rank, const char* who) {
+    if (e->devs.size() != 1) return fail(SVSB_E_INVALID, std::string(who) + ": a sharded engine owns exactly one device");
+    if (world < 1 || world > XCHG_MAX_RANKS || rank < 0 || rank >= world)
+        return fail(SVSB_E_INVALID, std::string(who) + ": bad world / rank (<= 16 ranks)");
+    return SVSB_OK;
+}
+
 // ---- pairwise top pairs of the one-process-per-GPU deployment (include/svsb200.h svsb_pairs_*) ----------------------
 // Rank r runs pairs_plan(shard rows)[r] -- the same per-device pass as multi_top_pairs -- against its peers' shards opened
 // over CUDA IPC; the caller all-gathers the per-rank lists and every rank merges them.
@@ -1415,14 +1500,12 @@ struct PairsDesc {                                 // svsb_pairs_export's descri
     cudaIpcMemHandle_t M, M16, ids;                // fp32 rows, fp16 shadow, embeddings.id
 };
 static_assert(sizeof(PairsDesc) <= SVSB_PAIRS_DESC_BYTES, "pair descriptor does not fit");
-static_assert(sizeof(cudaIpcMemHandle_t) == 64, "cudaIpcMemHandle_t is 64 bytes");
 
 // one rank's shard as connect sees it
 struct PairsPeer { int64_t n = 0, row0 = 0; int d = 0, ld = 0; const float* M = nullptr; const void* M16 = nullptr; const int64_t* ids = nullptr; };
 
 static void pairs_unmap(PairsShard* p) {
-    for (void* q : p->ipc_opened) cudaIpcCloseMemHandle(q);
-    p->ipc_opened.clear();
+    p->maps.close();
     p->connected = false;
 }
 
@@ -1510,9 +1593,7 @@ static int pairs_connect_check(svsb_engine* e, int32_t world, int32_t rank, cons
     if (!arg) return fail(SVSB_E_INVALID, std::string(who) + ": NULL argument");
     if (!e->pairs || !e->pairs->gen) return fail(SVSB_E_STATE, std::string(who) + ": svsb_pairs_export first");
     if (e->pairs->connected) return fail(SVSB_E_STATE, std::string(who) + ": already connected (svsb_pairs_disconnect first)");
-    if (world < 1 || world > XCHG_MAX_RANKS || rank < 0 || rank >= world)
-        return fail(SVSB_E_INVALID, std::string(who) + ": bad world / rank (<= 16 ranks)");
-    return SVSB_OK;
+    return check_world_rank(e, world, rank, who);
 }
 
 extern "C" int svsb_pairs_connect(svsb_t* e, int32_t world, int32_t rank, const void* descs) {
@@ -1532,15 +1613,8 @@ extern "C" int svsb_pairs_connect(svsb_t* e, int32_t world, int32_t rank, const 
         if (!D.has_rows) continue;
         void* ptr[3] = {nullptr, nullptr, nullptr};
         const cudaIpcMemHandle_t* h[3] = {&D.M, &D.M16, &D.ids};
-        for (int i = 0; i < 3; ++i) {
-            cudaError_t ce = cudaIpcOpenMemHandle(&ptr[i], *h[i], cudaIpcMemLazyEnablePeerAccess);
-            if (ce != cudaSuccess) {
-                (void)cudaGetLastError();
-                pairs_unmap(p);
-                return fail(SVSB_E_CUDA, std::string("svsb_pairs_connect: cudaIpcOpenMemHandle: ") + cudaGetErrorString(ce));
-            }
-            p->ipc_opened.push_back(ptr[i]);
-        }
+        for (int i = 0; i < 3; ++i)
+            if ((rc = p->maps.open(h[i], &ptr[i], "svsb_pairs_connect")) != SVSB_OK) { pairs_unmap(p); return rc; }
         q.M = static_cast<const float*>(ptr[0]); q.M16 = ptr[1]; q.ids = static_cast<const int64_t*>(ptr[2]);
     }
     if ((rc = pairs_finish_connect(p, world, rank, peers, "svsb_pairs_connect")) != SVSB_OK) pairs_unmap(p);
@@ -1558,14 +1632,8 @@ extern "C" int svsb_pairs_connect_local(svsb_t* e, int32_t world, int32_t rank, 
         svsb_engine* o = r == rank ? e : engines[r];
         if (!o || !o->pairs || !o->pairs->gen)
             return fail(SVSB_E_INVALID, "svsb_pairs_connect_local: a peer engine has not exported (svsb_pairs_export)");
-        if (o->devs[0] != e->devs[0]) {            // the re-score and the merge read the peer's rows and ids directly
-            int can = 0;
-            CU(cudaDeviceCanAccessPeer(&can, e->devs[0], o->devs[0]));
-            if (!can) return fail(SVSB_E_CUDA, "svsb_pairs_connect_local: no peer access between the devices");
-            cudaError_t pe = cudaDeviceEnablePeerAccess(o->devs[0], 0);
-            if (pe != cudaSuccess && pe != cudaErrorPeerAccessAlreadyEnabled) CU(pe);
-            (void)cudaGetLastError();
-        }
+        // the re-score and the merge read the peer's rows and ids directly
+        if ((rc = p->maps.reach(e->devs[0], o->devs[0], "svsb_pairs_connect_local")) != SVSB_OK) return rc;
         peers[(size_t)r] = pairs_peer_of(o->pairs->gen.get());
     }
     return pairs_finish_connect(p, world, rank, peers, "svsb_pairs_connect_local");
@@ -2214,7 +2282,7 @@ static void bxchg_release(svsb_engine* e) {
     if (!x) return;
     cudaSetDevice(e->devs[0]);
     cudaDeviceSynchronize();
-    for (void* p : x->ipc_opened) cudaIpcCloseMemHandle(p);
+    x->maps.close();
     if (x->block) cudaFree(x->block);
     if (x->done) cudaFree(x->done);
     if (x->status) cudaFree(x->status);
@@ -2224,8 +2292,8 @@ static void bxchg_release(svsb_engine* e) {
 
 extern "C" int svsb_bxchg_create(svsb_t* e, int32_t world, int32_t rank, int32_t rec_cap, void* handle_out) {
     if (!e) return fail(SVSB_E_INVALID, "engine is NULL");
-    if (e->devs.size() != 1) return fail(SVSB_E_INVALID, "svsb_bxchg_create: a sharded engine owns exactly one device");
-    if (world < 1 || world > XCHG_MAX_RANKS || rank < 0 || rank >= world) return fail(SVSB_E_INVALID, "svsb_bxchg_create: bad world / rank (<= 16 ranks)");
+    int rc = check_world_rank(e, world, rank, "svsb_bxchg_create");
+    if (rc != SVSB_OK) return rc;
     if (rec_cap < 1 || rec_cap > 1024) return fail(SVSB_E_INVALID, "svsb_bxchg_create: 1 <= rec_cap <= 1024");
     bxchg_release(e);
     e->bxchg.reset(new BXchg());
@@ -2243,58 +2311,23 @@ extern "C" int svsb_bxchg_create(svsb_t* e, int32_t world, int32_t rank, int32_t
     CU(cudaMalloc(&x->done, 64)); CU(cudaMemset(x->done, 0, 64));
     CU(cudaMalloc(&x->status, 64)); CU(cudaMemset(x->status, 0, 64));
     CU(cudaDeviceSynchronize());
-    if (const char* v = getenv("SVSB_XCHG_TIMEOUT_MS")) { const long long ms = atoll(v); if (ms > 0) x->timeout_ns = (unsigned long long)ms * 1000000ull; }
-    x->peer_block.assign(world, nullptr);
-    x->peer_block[rank] = x->block;
-    if (handle_out) {
-        cudaIpcMemHandle_t h;
-        CU(cudaIpcGetMemHandle(&h, x->block));
-        memcpy(handle_out, &h, 64);
-    }
-    x->connected = world == 1;
-    return SVSB_OK;
+    return x->publish(handle_out);
 }
 
 extern "C" int svsb_bxchg_connect(svsb_t* e, const void* handles) {
     if (!e || !e->bxchg) return fail(SVSB_E_STATE, "svsb_bxchg_connect: svsb_bxchg_create first");
     if (!handles) return fail(SVSB_E_INVALID, "svsb_bxchg_connect: NULL handles");
-    BXchg* x = e->bxchg.get();
     CU(cudaSetDevice(e->devs[0]));
-    for (int r = 0; r < x->world; ++r) {
-        if (r == x->rank) continue;
-        cudaIpcMemHandle_t h;
-        memcpy(&h, static_cast<const unsigned char*>(handles) + (size_t)r * 64, 64);
-        void* p = nullptr;
-        CU(cudaIpcOpenMemHandle(&p, h, cudaIpcMemLazyEnablePeerAccess));
-        x->ipc_opened.push_back(p);
-        x->peer_block[r] = static_cast<unsigned char*>(p);
-    }
-    x->connected = true;
-    return SVSB_OK;
+    return e->bxchg->connect(handles, "svsb_bxchg_connect");
 }
 
 extern "C" int svsb_bxchg_connect_local(svsb_t* e, svsb_t* const* engines) {
     if (!e || !e->bxchg) return fail(SVSB_E_STATE, "svsb_bxchg_connect_local: svsb_bxchg_create first");
     if (!engines) return fail(SVSB_E_INVALID, "svsb_bxchg_connect_local: NULL engines");
-    BXchg* x = e->bxchg.get();
     CU(cudaSetDevice(e->devs[0]));
-    for (int r = 0; r < x->world; ++r) {
-        if (r == x->rank) continue;
-        svsb_engine* o = engines[r];
-        if (!o || !o->bxchg || o->bxchg->world != x->world || o->bxchg->rank != r || o->bxchg->rec_cap != x->rec_cap)
-            return fail(SVSB_E_INVALID, "svsb_bxchg_connect_local: peer engine has no matching batch window");
-        if (o->devs[0] != e->devs[0]) {
-            int can = 0;
-            CU(cudaDeviceCanAccessPeer(&can, e->devs[0], o->devs[0]));
-            if (!can) return fail(SVSB_E_CUDA, "svsb_bxchg_connect_local: no peer access between the devices");
-            cudaError_t pe = cudaDeviceEnablePeerAccess(o->devs[0], 0);
-            if (pe != cudaSuccess && pe != cudaErrorPeerAccessAlreadyEnabled) CU(pe);
-            (void)cudaGetLastError();
-        }
-        x->peer_block[r] = o->bxchg->block;
-    }
-    x->connected = true;
-    return SVSB_OK;
+    return e->bxchg->connect_local(e->devs[0], engines, [](svsb_engine* o, const PeerWindow* self) -> PeerWindow* {
+        return o->bxchg && o->bxchg->rec_cap == static_cast<const BXchg*>(self)->rec_cap ? o->bxchg.get() : nullptr;
+    }, "svsb_bxchg_connect_local");
 }
 
 // Stop pushing into the peers' windows (they may be freed next); the own window stays until svsb_destroy / the next create.
@@ -2304,10 +2337,7 @@ extern "C" int svsb_bxchg_disconnect(svsb_t* e) {
     if (!x) return SVSB_OK;
     CU(cudaSetDevice(e->devs[0]));
     CU(cudaDeviceSynchronize());
-    for (void* p : x->ipc_opened) cudaIpcCloseMemHandle(p);
-    x->ipc_opened.clear();
-    for (int r = 0; r < x->world; ++r) if (r != x->rank) x->peer_block[r] = nullptr;
-    x->connected = x->world == 1;
+    x->unmap();
     x->deferred.pending = false;             // a merge nobody flushed dies with the connection
     return SVSB_OK;
 }
@@ -2434,8 +2464,8 @@ static int xchg_prepare(svsb_engine* e, const Generation* g);
 static int xchg_flush_merge(svsb_engine* e, cudaStream_t st_sel);
 extern "C" int svsb_xchg_create(svsb_t* e, int32_t world, int32_t rank, int32_t k_max, void* handle_out) {
     if (!e) return fail(SVSB_E_INVALID, "engine is NULL");
-    if (e->devs.size() != 1) return fail(SVSB_E_INVALID, "svsb_xchg_create: a sharded engine owns exactly one device");
-    if (world < 1 || world > XCHG_MAX_RANKS || rank < 0 || rank >= world) return fail(SVSB_E_INVALID, "svsb_xchg_create: bad world / rank (<= 16 ranks)");
+    int rc = check_world_rank(e, world, rank, "svsb_xchg_create");
+    if (rc != SVSB_OK) return rc;
     if (k_max < 1 || k_max > K_FAST_MAX) return fail(SVSB_E_INVALID, "svsb_xchg_create: 1 <= k_max <= 2048");
     xchg_release(e);
     e->xchg.reset(new Xchg());                 // owned by the engine from the start: a failure below leaves a window that
@@ -2451,7 +2481,6 @@ extern "C" int svsb_xchg_create(svsb_t* e, int32_t world, int32_t rank, int32_t 
     CU(cudaDeviceSynchronize());
     CU(cudaStreamCreateWithFlags(&x->st, cudaStreamNonBlocking));
     x->ws.dev = e->devs[0]; x->ws.st = x->st;
-    if (const char* v = getenv("SVSB_XCHG_TIMEOUT_MS")) { const long long ms = atoll(v); if (ms > 0) x->timeout_ns = (unsigned long long)ms * 1000000ull; }
     CU(cudaMallocHost(&x->h_scores, (size_t)k_max * 4));
     CU(cudaMallocHost(&x->h_ids, (size_t)k_max * 8));
     CU(cudaMallocHost(&x->h_count, 64));
@@ -2461,16 +2490,7 @@ extern "C" int svsb_xchg_create(svsb_t* e, int32_t world, int32_t rank, int32_t 
         CU(cudaMemset(x->stamps, 0, (size_t)Xchg::STAMP_RING * Xchg::STAMP_WORDS * 8));
         CU(cudaDeviceSynchronize());
     }
-    x->peer_block.assign(world, nullptr);
-    x->peer_block[rank] = x->block;
-    if (handle_out) {
-        cudaIpcMemHandle_t h;
-        CU(cudaIpcGetMemHandle(&h, x->block));
-        static_assert(sizeof(h) == 64, "cudaIpcMemHandle_t is 64 bytes");
-        memcpy(handle_out, &h, 64);
-    }
-    x->connected = world == 1;
-    return SVSB_OK;
+    return x->publish(handle_out);
 }
 
 // Close the peers' windows (this rank stops pushing) but keep the own one alive: peers may still have it mapped.
@@ -2483,54 +2503,29 @@ extern "C" int svsb_xchg_disconnect(svsb_t* e) {
     if (x->deferred.pending && e->side_st) { int rc = xchg_flush_merge(e, e->side_st); if (rc != SVSB_OK) return rc; }
     if (x->st) CU(cudaStreamSynchronize(x->st));
     if (e->side_st) CU(cudaStreamSynchronize(e->side_st));
-    for (void* p : x->ipc_opened) cudaIpcCloseMemHandle(p);
-    x->ipc_opened.clear();
-    for (int r = 0; r < x->world; ++r) if (r != x->rank) x->peer_block[r] = nullptr;
-    x->connected = false;
+    x->unmap();
     return SVSB_OK;
 }
 
 extern "C" int svsb_xchg_connect(svsb_t* e, const void* handles) {
     if (!e || !e->xchg) return fail(SVSB_E_STATE, "svsb_xchg_connect: svsb_xchg_create first");
     if (!handles) return fail(SVSB_E_INVALID, "svsb_xchg_connect: NULL handles");
-    Xchg* x = e->xchg.get();
     CU(cudaSetDevice(e->devs[0]));
-    for (int r = 0; r < x->world; ++r) {
-        if (r == x->rank) continue;
-        cudaIpcMemHandle_t h;
-        memcpy(&h, static_cast<const unsigned char*>(handles) + (size_t)r * 64, 64);
-        void* p = nullptr;
-        CU(cudaIpcOpenMemHandle(&p, h, cudaIpcMemLazyEnablePeerAccess));
-        x->ipc_opened.push_back(p);
-        x->peer_block[r] = static_cast<unsigned char*>(p);
-    }
-    x->connected = true;
-    if (auto g = pin(e)) { int rc = xchg_prepare(e, g.get()); if (rc != SVSB_OK) return rc; }
+    int rc = e->xchg->connect(handles, "svsb_xchg_connect");
+    if (rc != SVSB_OK) return rc;
+    if (auto g = pin(e)) return xchg_prepare(e, g.get());
     return SVSB_OK;
 }
 
 extern "C" int svsb_xchg_connect_local(svsb_t* e, svsb_t* const* engines) {
     if (!e || !e->xchg) return fail(SVSB_E_STATE, "svsb_xchg_connect_local: svsb_xchg_create first");
     if (!engines) return fail(SVSB_E_INVALID, "svsb_xchg_connect_local: NULL engines");
-    Xchg* x = e->xchg.get();
     CU(cudaSetDevice(e->devs[0]));
-    for (int r = 0; r < x->world; ++r) {
-        if (r == x->rank) continue;
-        svsb_engine* o = engines[r];
-        if (!o || !o->xchg || o->xchg->world != x->world || o->xchg->rank != r || o->xchg->cap != x->cap)
-            return fail(SVSB_E_INVALID, "svsb_xchg_connect_local: peer engine has no matching exchange window");
-        if (o->devs[0] != e->devs[0]) {
-            int can = 0;
-            CU(cudaDeviceCanAccessPeer(&can, e->devs[0], o->devs[0]));
-            if (!can) return fail(SVSB_E_CUDA, "svsb_xchg_connect_local: no peer access between the devices");
-            cudaError_t pe = cudaDeviceEnablePeerAccess(o->devs[0], 0);
-            if (pe != cudaSuccess && pe != cudaErrorPeerAccessAlreadyEnabled) CU(pe);
-            (void)cudaGetLastError();
-        }
-        x->peer_block[r] = o->xchg->block;
-    }
-    x->connected = true;
-    if (auto g = pin(e)) { int rc = xchg_prepare(e, g.get()); if (rc != SVSB_OK) return rc; }
+    int rc = e->xchg->connect_local(e->devs[0], engines, [](svsb_engine* o, const PeerWindow* self) -> PeerWindow* {
+        return o->xchg && o->xchg->cap == static_cast<const Xchg*>(self)->cap ? o->xchg.get() : nullptr;
+    }, "svsb_xchg_connect_local");
+    if (rc != SVSB_OK) return rc;
+    if (auto g = pin(e)) return xchg_prepare(e, g.get());
     return SVSB_OK;
 }
 

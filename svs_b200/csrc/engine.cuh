@@ -321,19 +321,38 @@ struct MqWs {
     }
 };
 
+// Other ranks' memory as the one-process-per-GPU deployment reaches it (engine.cu "peer memory"): the CUDA IPC mappings
+// a rank opened, and peer access to the devices of this process.
+struct PeerMaps {
+    std::vector<void*> opened;
+    int open(const void* handle, void** out, const char* who);   // a peer's 64-byte cudaIpcMemHandle_t
+    int reach(int self, int dev, const char* who);                // device self (the current one) -> device dev's memory
+    void close();
+};
+
+// What the gather window (Xchg) and the batch window (BXchg) share.
+struct PeerWindow {
+    int world = 0, rank = 0;
+    unsigned char* block = nullptr;
+    std::vector<unsigned char*> peer_block;              // per rank (own entry = block)
+    PeerMaps maps;
+    bool connected = false;
+    unsigned long long seq = 0;
+    unsigned long long timeout_ns = 30ull * 1000000000ull;   // a wait kernel gives up on a peer (SVSB_XCHG_TIMEOUT_MS)
+    int publish(void* handle_out);                       // the end of a create; handle_out: this window's IPC handle
+    int connect(const void* handles, const char* who);   // world x 64-byte IPC handles in rank order
+    // windows of engines in this process; window_of(peer, this) = the peer's window if it matches this one, else null
+    int connect_local(int dev, svsb_engine* const* engines, PeerWindow* (*window_of)(svsb_engine*, const PeerWindow*), const char* who);
+    void unmap();                                        // back to the state publish left
+};
+
 // Batch window of the one-process-per-GPU deployment (svsb_bxchg_*, svsb_batch_peer): per slot and source rank a region
 // for the rank's sample maxima and one for its candidate records, written by the peers' kernels over NVLink peer memory.
 //   [flags: 2 phases x slots x world u64, padded to 256 B][tops: slots x world x B_MAX x 32 f32][records: slots x world x B_MAX x (2 rec_cap + 1) i64]
-struct BXchg {
+struct BXchg : PeerWindow {
     static constexpr int SLOTS = 2, B_MAX = COARSE_MAX_BATCH;
-    int world = 0, rank = 0, rec_cap = 0;
-    unsigned char* block = nullptr;
+    int rec_cap = 0;
     size_t flags_bytes = 0, tops_bytes = 0, bytes = 0;
-    std::vector<unsigned char*> peer_block;
-    std::vector<void*> ipc_opened;
-    bool connected = false;
-    unsigned long long seq = 0;
-    unsigned long long timeout_ns = 30ull * 1000000000ull;
     unsigned int* done = nullptr;            // two last-block tickets (sample maxima, records)
     int* status = nullptr;                   // device word: 1 = a wait timed out
     // svsb_batch_peer with flag bit 0: the verifying merge of batch j is enqueued behind the FIRST phase of batch j+1 (or by
@@ -352,16 +371,11 @@ struct BXchg {
 
 // Peer exchange of the one-process-per-GPU deployment (kernels.cuh "peer exchange"): this rank's gather window,
 // the peers' windows opened over CUDA IPC (or plain pointers inside one process), and a synchronous query context.
-struct Xchg {
-    int world = 0, rank = 0, cap = 0, slots = 4;
+// block = [flags: slots*world u64, padded to 256 B][window]
+struct Xchg : PeerWindow {
+    int cap = 0, slots = 4;
     int64_t rec_words = 0;
-    unsigned char* block = nullptr;                      // [flags: slots*world u64, padded to 256 B][window]
     size_t flags_bytes = 0;
-    std::vector<unsigned char*> peer_block;              // per rank (own entry = block)
-    std::vector<void*> ipc_opened;
-    bool connected = false;
-    unsigned long long seq = 0;
-    unsigned long long timeout_ns = 30ull * 1000000000ull;   // merge kernel gives up waiting for a peer (SVSB_XCHG_TIMEOUT_MS)
     // Pipelined path: the merge of query j is enqueued on the side stream BEHIND the selection of query j+1, so a
     // peer has a whole query time to deliver its record before this rank's side stream would wait for it.
     struct DeferredMerge {
@@ -414,7 +428,7 @@ struct PairsShard {
     std::vector<int64_t> shard_rows;                     // per rank
     std::vector<PairShadow> shadows;                     // per rank
     PairRows rows;                                       // global rows, counted from rank 0's first row
-    std::vector<void*> ipc_opened;
+    PeerMaps maps;
     cudaEvent_t ev = nullptr;                            // the caller's stream -> the pass's stream
 };
 

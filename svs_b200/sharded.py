@@ -165,8 +165,7 @@ class CudaShardBackend:
         self._check(self._lib.svsb_bxchg_connect(self.engine._h, C.c_char_p(b"".join(handles))))
 
     def batch_exchange_connect_local(self, backends: List["CudaShardBackend"]) -> None:
-        arr = (C.c_void_p * len(backends))(*[b.engine._h for b in backends])
-        self._check(self._lib.svsb_bxchg_connect_local(self.engine._h, arr))
+        self._check(self._lib.svsb_bxchg_connect_local(self.engine._h, self._engines(backends)))
 
     def batch_exchange_disconnect(self) -> None:
         self._check(self._lib.svsb_bxchg_disconnect(self.engine._h))
@@ -200,8 +199,7 @@ class CudaShardBackend:
 
     def exchange_connect_local(self, backends: List["CudaShardBackend"]) -> None:
         """All ranks live in this process (tests; one process driving several GPUs): plain pointers, no IPC."""
-        arr = (C.c_void_p * len(backends))(*[b.engine._h for b in backends])
-        self._check(self._lib.svsb_xchg_connect_local(self.engine._h, arr))
+        self._check(self._lib.svsb_xchg_connect_local(self.engine._h, self._engines(backends)))
 
     def exchange_disconnect(self) -> None:
         self._check(self._lib.svsb_xchg_disconnect(self.engine._h))
@@ -264,8 +262,7 @@ class CudaShardBackend:
 
     def pairs_connect_local(self, world: int, rank: int, backends: List["CudaShardBackend"]) -> None:
         """All ranks live in this process (tests; one process driving several GPUs): plain pointers, no IPC."""
-        arr = (C.c_void_p * len(backends))(*[b.engine._h for b in backends])
-        self._check(self._lib.svsb_pairs_connect_local(self.engine._h, world, rank, arr))
+        self._check(self._lib.svsb_pairs_connect_local(self.engine._h, world, rank, self._engines(backends)))
 
     def pairs_disconnect(self) -> None:
         self._check(self._lib.svsb_pairs_disconnect(self.engine._h))
@@ -302,6 +299,11 @@ class CudaShardBackend:
         ms = C.c_float()
         self._check(self._lib.svsb_kernel_time_collect(self.engine._h, C.byref(ms)))
         return ms.value
+
+    @staticmethod
+    def _engines(backends: List["CudaShardBackend"]):
+        """The backends' engine handles as the C array the *_connect_local entry points take."""
+        return (C.c_void_p * len(backends))(*[b.engine._h for b in backends])
 
     def synchronize(self) -> None:
         self.torch.cuda.current_stream(self.device).synchronize()
@@ -354,31 +356,27 @@ class ShardedRetriever:
         sl = slice(self.row0, self.row0 + self.local_rows)
         self.backend.load_rows(np.ascontiguousarray(rows[sl]), np.ascontiguousarray(emb_ids[sl]))
 
-    def _ensure_peer(self) -> None:
-        """One-time window exchange: every rank allocates its gather window and all-gathers the IPC handles."""
-        if self._peer_ready:
+    def _all_gather_object(self, obj) -> list:
+        if self.world == 1:
+            return [obj]
+        out: list = [None] * self.world
+        self.dist.all_gather_object(out, obj, group=self.group)
+        return out
+
+    def _ensure_window(self, batch: bool = False) -> None:
+        """One-time window exchange: every rank allocates its gather window (`batch`: its batch window), all-gathers the
+        IPC handles and opens its peers' windows."""
+        if self._batch_peer_ready if batch else self._peer_ready:
             return
-        handle = self.backend.exchange_handle(self.world, self.rank)
-        handles: List[Optional[bytes]] = [None] * self.world
-        if self.world > 1:
-            self.dist.all_gather_object(handles, handle, group=self.group)
-        else:
-            handles[0] = handle
-        self.backend.exchange_connect(handles)
+        be = self.backend
+        create, connect = (be.batch_exchange_handle, be.batch_exchange_connect) if batch else (be.exchange_handle, be.exchange_connect)
+        connect(self._all_gather_object(create(self.world, self.rank)))
         if self.world > 1:
             self.dist.barrier(group=self.group)                    # every window is open before the first push
-        self._peer_ready = True
-
-    def _ensure_batch_peer(self) -> None:
-        """One-time batch-window exchange (the batched counterpart of _ensure_peer)."""
-        if self._batch_peer_ready:
-            return
-        handle = self.backend.batch_exchange_handle(self.world, self.rank)
-        handles: List[Optional[bytes]] = [None] * self.world
-        self.dist.all_gather_object(handles, handle, group=self.group)
-        self.backend.batch_exchange_connect(handles)
-        self.dist.barrier(group=self.group)                        # every window is open before the first push
-        self._batch_peer_ready = True
+        if batch:
+            self._batch_peer_ready = True
+        else:
+            self._peer_ready = True
 
     # -- queries ---------------------------------------------------------------------------------
     def set_queries(self, Q: np.ndarray) -> None:
@@ -397,7 +395,7 @@ class ShardedRetriever:
         rec, gath, (o_s, o_i, o_c) = self._buffers(k)
         nb = len(qrows)
         if self.exchange == "peer":
-            self._ensure_peer()
+            self._ensure_window()
             for j, q in enumerate(qrows):                          # no collective, no separate merge launch per batch
                 self.backend.enqueue_query_peer(q, k, o_s[j], o_i[j], o_c[j], time_gemv and j % TIME_EVERY == 0, pipelined=True)
             self.backend.join()
@@ -419,7 +417,7 @@ class ShardedRetriever:
         if self.exchange == "peer":
             # no collective and nothing consumed on the host: enqueue every query back to back (outputs cycle through the
             # micro-batch buffers in stream order) and join once -- ranks couple only through the window flags
-            self._ensure_peer()
+            self._ensure_window()
             _rec, _gath, (o_s, o_i, o_c) = self._buffers(k)
             for done in range(count):
                 j = done % MICRO_BATCH
@@ -486,7 +484,7 @@ class ShardedRetriever:
         self.last_fallbacks = 0
         if self.exchange == "peer" and hasattr(self.backend, "batch_peer") and cap <= self.backend.BATCH_WINDOW_CAP:
             # both exchanges fused into the kernels over NVLink peer memory: no collective call at all
-            self._ensure_batch_peer()
+            self._ensure_window(batch=True)
             for c0 in range(0, b, 2048):                           # chunks pipeline: merge of chunk c behind the first phase of c+1
                 bc = min(2048, b - c0)
                 self.backend.batch_peer(dq[c0:c0 + bc], k, max_row_norm, sample_rank, cap, o_s[c0:c0 + bc], o_i[c0:c0 + bc], o_c[c0:c0 + bc],
@@ -602,7 +600,7 @@ class ShardedRetriever:
         if n > 2048 and self.n > 2048:
             raise NotImplementedError("n > 2048 is not supported by the sharded path")
         if self.exchange == "peer":
-            self._ensure_peer()
+            self._ensure_window()
             return self.backend.query_peer(q, k)                   # one synchronous C call, result written to host
         dq = self.backend.device_queries(q[None, :])
         o_s, o_i, o_c = self._micro_batch([dq[0]], k, False)
@@ -620,7 +618,7 @@ class ShardedRetriever:
         k = min(int(n), 2048, self.n)
         if k <= 0 or self.exchange != "peer":
             return ("done", self.retrieve_arrays(q, n))           # nothing to overlap: answered synchronously
-        self._ensure_peer()
+        self._ensure_window()
         return ("ticket", self.backend.query_peer_submit(q, k), k)
 
     def wait(self, handle) -> Tuple[np.ndarray, np.ndarray]:
@@ -635,13 +633,6 @@ class ShardedRetriever:
         return [(float(a), int(b)) for a, b in zip(s, i)]
 
     # -- pairwise top pairs ---------------------------------------------------------------------------
-    def _all_gather_object(self, obj) -> list:
-        if self.world == 1:
-            return [obj]
-        out: list = [None] * self.world
-        self.dist.all_gather_object(out, obj, group=self.group)
-        return out
-
     @staticmethod
     def _agree(outcomes) -> None:
         """Every rank raises the first refusal any rank reported: ranks never disagree about answering."""

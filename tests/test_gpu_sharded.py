@@ -1,7 +1,10 @@
 """GPU: the one-process-per-GPU shard path (svsb_set_shard / svsb_enqueue_local_topk /
 svsb_enqueue_merge_records) on ONE device: two shard engines stand in for two ranks and the all-gather is
 a concatenation.  The collective itself is covered on CPU with gloo (tests/test_sharded_gloo.py) and on
-N GPUs by bench.py under torchrun."""
+N GPUs by bench.py under torchrun; the peer windows over CUDA IPC by two processes on two GPUs."""
+import os
+import socket
+
 import numpy as np
 import pytest
 
@@ -550,3 +553,53 @@ def test_world_size_one_process_group_runs_the_real_collective(exchange):
         sr.close()
     finally:
         dist.destroy_process_group()
+
+
+def _peer_worker(rank, world, port, mats, ids, qs, k, ret):
+    import torch
+    import torch.distributed as dist
+    from svs_b200.sharded import ShardedRetriever
+    os.environ["MASTER_ADDR"] = "127.0.0.1"
+    os.environ["MASTER_PORT"] = str(port)
+    os.environ["SVSB_XCHG_TIMEOUT_MS"] = "10000"               # a protocol bug must fail the test, not hang the GPU
+    torch.cuda.set_device(rank)
+    dist.init_process_group("nccl", rank=rank, world_size=world, device_id=torch.device("cuda", rank))
+    try:
+        sr = ShardedRetriever(rank, world, rank, exchange="peer")
+        out = []
+        for m in mats:                                          # the second matrix is a reload over the same windows
+            sr.load_global(m, ids)
+            single = [sr.retrieve(q, k) for q in qs[:3]]
+            s, i = sr.wait(sr.submit(qs[3], k))
+            many = sr.retrieve_many(qs, k)
+            out.append((single, [(float(a), int(b)) for a, b in zip(s, i)], many, sr._batch_peer_ready))
+        sr.close()
+        ret[rank] = out
+    finally:
+        dist.destroy_process_group()
+
+
+def test_peer_windows_over_cuda_ipc_in_two_processes():
+    """Both peer windows opened over real CUDA IPC: two processes, one GPU each, the query exchange for retrieve and
+    submit / wait, the batch window for retrieve_many.  Every rank must hold the oracle's answer, before and after a
+    reload."""
+    torch = pytest.importorskip("torch")
+    import torch.multiprocessing as mp
+    if torch.cuda.device_count() < 2:
+        pytest.skip("needs two GPUs (NCCL runs one rank per GPU)")
+    n, d, k = 60_000, 128, 100
+    mats = [oracle.synth_matrix_uniform(n, d, seed) for seed in (71, 72)]
+    ids = np.cumsum(np.random.default_rng(73).integers(1, 4, size=n)).astype(np.int64)
+    qs = oracle.synth_queries(64, d, 74)
+    s = socket.socket(); s.bind(("127.0.0.1", 0)); port = s.getsockname()[1]; s.close()
+    ret = mp.Manager().dict()
+    mp.spawn(_peer_worker, args=(2, port, mats, ids, qs, k, ret), nprocs=2, join=True)
+    assert ret[0] == ret[1]                                     # every rank holds the same answers
+    for m, (single, waited, many, batch_peer) in zip(mats, ret[0]):
+        assert batch_peer                                       # the batch went through the batch window
+        for q, got in zip(qs[:3], single):
+            oracle.compare_retrieval(got, oracle.superheavy(m, ids, q, k), oracle.scores_of(m, q), ids)
+        oracle.compare_retrieval(waited, oracle.superheavy(m, ids, qs[3], k), oracle.scores_of(m, qs[3]), ids)
+        assert len(many) == len(qs)
+        for q, got in zip(qs, many):
+            oracle.compare_retrieval(got, oracle.superheavy(m, ids, q, k), oracle.scores_of(m, q), ids)
