@@ -840,6 +840,9 @@ struct BatchPlan {
     float eps_coef = 0.f, max_row_norm = 1.f;
 };
 
+// b queries padded to whole query tiles of the coarse pass
+static inline int batch_pad(int b) { return (b + COARSE_TILE_QUERIES - 1) / COARSE_TILE_QUERIES * COARSE_TILE_QUERIES; }
+
 // Can this generation / k take the coarse path at all?  (Purely a performance gate: both paths return the same bits.)
 // guaranteed: thresholds are a proven bound (the kk-th largest of the sample); else an order statistic of the sample
 // that is a bound except with probability ~1e-9 per query for a random sample, verified per query by the refine
@@ -943,34 +946,56 @@ static int ensure_m16(Generation* g, const BatchPlan& P, cudaStream_t st) {
     return SVSB_OK;
 }
 
-// Enqueue the whole pipeline for b (<= COARSE_MAX_BATCH) device-resident fp32 queries dQ[b][ld] on w->st.
-// Results: w->o_scores / o_ids [b][k], w->o_counts[b], w->flags[b] (!= 0: the query needs the exact path).
-// time_coarse: bracket the filter pass with w->ev[2], w->ev[3].
-// st: the stream everything is enqueued on (the workspace's own, or the caller's in the sharded path).
-// out == nullptr: results go to w->o_scores / o_ids [b][k], w->o_counts[b].
-static int batch_enqueue(BatchWs* w, const Generation* g, const BatchPlan& P, const float* dQ, int b, bool time_coarse,
-                         cudaStream_t st, const RefineOut* out = nullptr) {
-    const Shard& s = g->shards[0];
-    const int b_pad = (b + COARSE_TILE_QUERIES - 1) / COARSE_TILE_QUERIES * COARSE_TILE_QUERIES;
+// The batch workspace, sized for b queries of plan P, over the generation's fp16 shadow (converted on st, the stream the
+// batch's kernels run on; null: the workspace's own).  The caller holds batch_mu.
+static int batch_acquire(svsb_engine* e, Generation* g, const BatchPlan& P, int b, cudaStream_t st, BatchWs*& w) {
+    int rc = batch_ws_get(e, w);
+    if (rc != SVSB_OK) return rc;
+    if ((rc = ensure_m16(g, P, st ? st : w->st)) != SVSB_OK) return rc;
+    return batch_ws_ensure(w, P, batch_pad(b));
+}
+
+// The two phases of the pipeline for b (<= COARSE_MAX_BATCH) device-resident fp32 queries dQ[b][ld], enqueued on st
+// (the workspace's own stream, or the caller's in the sharded path).  Between them a threshold kernel fills w->thr.
+// Sample phase: the queries -> fp16 (with their error bounds, flags and candidate counts reset), then the sample pass.
+static int batch_sample(BatchWs* w, const Generation* g, const BatchPlan& P, const float* dQ, int b, cudaStream_t st) {
+    const int b_pad = batch_pad(b);
     CU(cudaSetDevice(w->dev));
     CU(launch_queries_to_f16(st, dQ, b, b_pad, P.d, P.ld, w->dQ16, P.ld16, P.eps_coef, P.max_row_norm, w->eps, w->thr, w->flags, w->cand_cnt));
     CU(launch_coarse_gemm(st, w->dev, 1, g->M16, P.n, w->dQ16, b_pad, P.ld16, P.s_tiles, P.tile_stride,
                           nullptr, nullptr, nullptr, 0, w->sample, P.sample_rows));
-    CU(launch_sample_threshold(st, w->sample, P.sample_rows, b, P.sample_rank, w->eps, w->thr));
-    if (env_int("SVSB_DEBUG_NO_SURVIVORS", 0)) {          // measurement aid: thresholds +inf -> the filter pass keeps nothing
-        std::vector<uint32_t> inf((size_t)b_pad, 0x7f800000u);
-        CU(cudaMemcpyAsync(w->thr, inf.data(), (size_t)b_pad * 4, cudaMemcpyHostToDevice, st));
-        CU(cudaStreamSynchronize(st));
-    }
+    return SVSB_OK;
+}
+
+// Filter + refine phase: the filter pass keeps every row whose coarse score reaches w->thr, the refine re-scores them
+// exactly into `out` (mode: REFINE_* flags; push: records into the peers' windows).  w->flags[q] != 0: query q needs
+// the exact path.  time_coarse: bracket the filter pass with w->ev[2], w->ev[3].
+static int batch_filter_refine(BatchWs* w, const Generation* g, const BatchPlan& P, const float* dQ, int b, cudaStream_t st,
+                               const RefineOut& out, int mode = 0, const BatchPush* push = nullptr, bool time_coarse = false) {
+    const Shard& s = g->shards[0];
     if (time_coarse) CU(cudaEventRecord(w->ev[2], st));
-    CU(launch_coarse_gemm(st, w->dev, 0, g->M16, P.n, w->dQ16, b_pad, P.ld16, P.n_tiles, 1,
+    CU(launch_coarse_gemm(st, w->dev, 0, g->M16, P.n, w->dQ16, batch_pad(b), P.ld16, P.n_tiles, 1,
                           w->thr, w->cand, w->cand_cnt, P.cand_cap, nullptr, 0));
     if (time_coarse) CU(cudaEventRecord(w->ev[3], st));
-    RefineOut o{w->o_scores, nullptr, w->o_ids, (int64_t)P.k, w->o_counts, 1};
-    if (out) o = *out;
     CU(launch_refine(st, s.M, P.n, P.ld, s.ids, s.row0, dQ, b, P.ld, P.k, w->cand, w->cand_cnt, P.cand_cap, w->eps, w->thr, w->flags,
-                     o, w->stats, &w->rs, 0));
+                     out, w->stats, &w->rs, mode, push));
     return SVSB_OK;
+}
+
+// The whole pipeline with this shard's own thresholds.  out == nullptr: results go to w->o_scores / o_ids [b][k],
+// w->o_counts[b].
+static int batch_enqueue(BatchWs* w, const Generation* g, const BatchPlan& P, const float* dQ, int b, bool time_coarse,
+                         cudaStream_t st, const RefineOut* out = nullptr) {
+    int rc = batch_sample(w, g, P, dQ, b, st);
+    if (rc != SVSB_OK) return rc;
+    CU(launch_sample_threshold(st, w->sample, P.sample_rows, b, P.sample_rank, w->eps, w->thr));
+    if (env_int("SVSB_DEBUG_NO_SURVIVORS", 0)) {          // measurement aid: thresholds +inf -> the filter pass keeps nothing
+        std::vector<uint32_t> inf((size_t)batch_pad(b), 0x7f800000u);
+        CU(cudaMemcpyAsync(w->thr, inf.data(), inf.size() * 4, cudaMemcpyHostToDevice, st));
+        CU(cudaStreamSynchronize(st));
+    }
+    const RefineOut own{w->o_scores, nullptr, w->o_ids, (int64_t)P.k, w->o_counts, 1};
+    return batch_filter_refine(w, g, P, dQ, b, st, out ? *out : own, 0, nullptr, time_coarse);
 }
 
 // Did enough statistical thresholds fail verification (flag 16) that the chunk should be redone with guaranteed ones?
@@ -983,6 +1008,23 @@ static bool batch_thresholds_failed(Generation* g, const BatchPlan& P, const int
     if (bad <= std::max(2, b / 256)) return false;
     g->batch_guaranteed.store(true, std::memory_order_relaxed);
     return true;
+}
+
+// Run bc device-resident queries dQ[bc][ld] (one chunk of at most COARSE_MAX_BATCH) through the pipeline on st and bring
+// their flags to w->h_flags, with ONE synchronisation of st: fetch() enqueues the caller's result copies before it.
+// If too many statistical thresholds failed, P is re-planned with guaranteed ones and the chunk redone in place.
+template <class Fetch>
+static int batch_run_chunk(svsb_engine* e, Generation* g, BatchPlan& P, BatchWs* w, cudaStream_t st, const float* dQ, int bc,
+                           const RefineOut* out, Fetch fetch) {
+    for (int attempt = 0; attempt < 2; ++attempt) {
+        int rc = batch_enqueue(w, g, P, dQ, bc, false, st, out);
+        if (rc != SVSB_OK || (rc = fetch()) != SVSB_OK) return rc;
+        CU(cudaMemcpyAsync(w->h_flags, w->flags, (size_t)bc * 4, cudaMemcpyDeviceToHost, st));
+        CU(cudaStreamSynchronize(st));
+        if (!batch_thresholds_failed(g, P, w->h_flags, bc)) break;
+        batch_plan(e, g, P.k, P, true);
+    }
+    return SVSB_OK;
 }
 
 static bool is_pinned_host(const void* p) {
@@ -1033,48 +1075,59 @@ static int mq_ws_get(svsb_engine* e, MqWs*& out) {
     return SVSB_OK;
 }
 
-// enqueue gemv + selection for b (<= chunk) device-resident queries dQ[b][ld] on st; outputs through `os` strides
-static int mq_enqueue(MqWs* w, const Generation* g, cudaStream_t st, const float* dQ, int b, int64_t kk, const SelectStrides& os,
-                      u64* out_keys, float* out_scores, int64_t* out_ids, int32_t* out_count) {
+// Multi-query passes over b queries, P.chunk at a time: each query's top-kk list goes to the records `recs` or, with
+// recs.base null, to the workspace's dense [chunk][kk] outputs.  Per chunk the workspace is sized and its own stream
+// drained (its zeroing is done, its staging buffer free), stage(w, c0, bc, dQ) points dQ at the chunk's device-resident
+// queries [bc][ld], gemv + selection run on st (null: the workspace's stream) and drain(w, c0, bc) takes the results.
+// The caller holds batch_mu.
+template <class Stage, class Drain>
+static int mq_run(svsb_engine* e, const Generation* g, const MqPlan& P, int32_t b, int64_t kk, cudaStream_t st, const RecordView& recs,
+                  Stage stage, Drain drain) {
+    MqWs* w = nullptr;
+    int rc = mq_ws_get(e, w);
+    if (rc != SVSB_OK) return rc;
     const Shard& s = g->shards[0];
-    const int shift = group_shift_for(w->cap_n);                 // group layout of the workspace (>= this shard's rows)
-    CU(cudaSetDevice(w->dev));
-    w->gmax_dirty = true;
-    CU(launch_gemv_mq(st, w->dev, s.M, s.n, g->d, g->ld, dQ, b, w->scores, w->cap_n, w->gmax, w->G, shift, s.live, 0));
-    SelectStrides ss = os;
-    ss.scores = w->cap_n; ss.gmax = w->G; ss.cand = w->cand_cap;
-    CU(launch_select_batch(st, b, ss, w->scores, s.n, w->gmax, shift, (int)std::min<int64_t>(kk, s.n_live), s.ids, s.row0, w->cand, w->cand_cap,
-                           out_keys, out_scores, out_ids, out_count));
-    w->gmax_dirty = false;
+    for (int32_t c0 = 0; c0 < b; c0 += P.chunk) {
+        const int bc = std::min<int32_t>(P.chunk, b - c0);
+        if ((rc = w->ensure(std::min<int32_t>(P.chunk, b), s.n, g->ld, kk)) != SVSB_OK) return rc;
+        CU(cudaStreamSynchronize(w->st));
+        const float* dQ = nullptr;
+        if ((rc = stage(w, c0, bc, dQ)) != SVSB_OK) return rc;
+        cudaStream_t run = st ? st : w->st;
+        SelectStrides ss; ss.keys = kk; ss.oscores = kk; ss.ids = kk; ss.count = 1;
+        u64* keys = w->o_keys; int64_t* ids = w->o_ids; int32_t* counts = w->o_counts;
+        if (recs.base) { ss = recs.select_strides(kk); keys = recs.keys(c0); ids = recs.ids(c0); counts = recs.count(c0); }
+        ss.scores = w->cap_n; ss.gmax = w->G; ss.cand = w->cand_cap;
+        const int shift = group_shift_for(w->cap_n);             // group layout of the workspace (>= this shard's rows)
+        CU(cudaSetDevice(w->dev));
+        w->gmax_dirty = true;
+        CU(launch_gemv_mq(run, w->dev, s.M, s.n, g->d, g->ld, dQ, bc, w->scores, w->cap_n, w->gmax, w->G, shift, s.live, 0));
+        CU(launch_select_batch(run, bc, ss, w->scores, s.n, w->gmax, shift, (int)std::min<int64_t>(kk, s.n_live), s.ids, s.row0, w->cand,
+                               w->cand_cap, keys, w->o_scores, ids, counts));
+        w->gmax_dirty = false;
+        if ((rc = drain(w, c0, bc)) != SVSB_OK) return rc;
+    }
     return SVSB_OK;
 }
 
 static int query_batch_mq(svsb_engine* e, const std::shared_ptr<Generation>& g, const MqPlan& P, const float* Q, int32_t b, int32_t d,
                           int32_t k, int64_t kk, float* out_scores, int64_t* out_emb_ids, int32_t* out_counts) {
     std::lock_guard<std::mutex> lk(e->batch_mu);
-    MqWs* w = nullptr;
-    int rc = mq_ws_get(e, w);
-    if (rc != SVSB_OK) return rc;
-    const Shard& s = g->shards[0];
     const int ld = g->ld;
-    for (int32_t c0 = 0; c0 < b; c0 += P.chunk) {
-        const int bc = std::min<int32_t>(P.chunk, b - c0);
-        if ((rc = w->ensure(std::min<int32_t>(P.chunk, b), s.n, ld, kk)) != SVSB_OK) return rc;
-        CU(cudaStreamSynchronize(w->st));                        // h_Q is free again
-        for (int i = 0; i < bc; ++i) {
-            float* dst = w->h_Q + (size_t)i * ld;
-            memcpy(dst, Q + (size_t)(c0 + i) * d, (size_t)d * 4);
-            for (int c = d; c < ld; ++c) dst[c] = 0.f;
-        }
+    auto stage = [&](MqWs* w, int c0, int bc, const float*& dQ) -> int {
+        stage_queries(w->h_Q, Q + (size_t)c0 * d, bc, d, ld);
         CU(cudaMemcpyAsync(w->dQ, w->h_Q, (size_t)bc * ld * 4, cudaMemcpyHostToDevice, w->st));
-        SelectStrides os; os.keys = kk; os.oscores = kk; os.ids = kk; os.count = 1;
-        if ((rc = mq_enqueue(w, g.get(), w->st, w->dQ, bc, kk, os, w->o_keys, w->o_scores, w->o_ids, w->o_counts)) != SVSB_OK) return rc;
+        dQ = w->dQ;
+        return SVSB_OK;
+    };
+    auto drain = [&](MqWs* w, int c0, int bc) -> int {
         CU(cudaMemcpy2DAsync(out_scores + (int64_t)c0 * k, (size_t)k * 4, w->o_scores, (size_t)kk * 4, (size_t)kk * 4, (size_t)bc, cudaMemcpyDeviceToHost, w->st));
         CU(cudaMemcpy2DAsync(out_emb_ids + (int64_t)c0 * k, (size_t)k * 8, w->o_ids, (size_t)kk * 8, (size_t)kk * 8, (size_t)bc, cudaMemcpyDeviceToHost, w->st));
         CU(cudaMemcpyAsync(out_counts + c0, w->o_counts, (size_t)bc * 4, cudaMemcpyDeviceToHost, w->st));
         CU(cudaStreamSynchronize(w->st));
-    }
-    return SVSB_OK;
+        return SVSB_OK;
+    };
+    return mq_run(e, g.get(), P, b, kk, nullptr, RecordView{}, stage, drain);
 }
 
 static int query_batch_loop(svsb_engine* e, const std::shared_ptr<Generation>& g, const float* Q, int32_t b, int32_t d, int32_t k,
@@ -1109,43 +1162,31 @@ static int query_batch_gen(svsb_engine* e, const std::shared_ptr<Generation>& g,
 
     std::lock_guard<std::mutex> lk(e->batch_mu);
     BatchWs* w = nullptr;
-    int rc = batch_ws_get(e, w);
+    int rc = batch_acquire(e, g.get(), P, std::min<int32_t>(b, COARSE_MAX_BATCH), nullptr, w);
+    if (rc == SVSB_E_NOMEM) return query_batch_loop(e, g, Q, b, d, k, out_scores, out_emb_ids, out_counts);
     if (rc != SVSB_OK) return rc;
-    if ((rc = ensure_m16(g.get(), P, w->st)) != SVSB_OK) {
-        if (rc == SVSB_E_NOMEM) return query_batch_loop(e, g, Q, b, d, k, out_scores, out_emb_ids, out_counts);
-        return rc;
-    }
     // Page-locked caller buffers (svsb_host_alloc, cudaHostRegister, torch pin_memory) are DMA'd from / into directly;
     // pageable ones are staged through the workspace's pinned buffers.
     const bool q_direct = is_pinned_host(Q) && d == P.ld;
     const bool out_direct = is_pinned_host(out_scores) && is_pinned_host(out_emb_ids);
     for (int32_t c0 = 0; c0 < b; c0 += COARSE_MAX_BATCH) {
         const int bc = std::min<int32_t>(COARSE_MAX_BATCH, b - c0);
-        const int b_pad = (bc + COARSE_TILE_QUERIES - 1) / COARSE_TILE_QUERIES * COARSE_TILE_QUERIES;
-        if ((rc = batch_ws_ensure(w, P, b_pad)) != SVSB_OK) return rc;
         const float* src = Q + (size_t)c0 * d;
         if (!q_direct) {
-            for (int i = 0; i < bc; ++i) {
-                float* dst = w->h_Q + (size_t)i * P.ld;
-                memcpy(dst, Q + (size_t)(c0 + i) * d, (size_t)d * 4);
-                for (int c = d; c < P.ld; ++c) dst[c] = 0.f;
-            }
+            stage_queries(w->h_Q, src, bc, d, P.ld);
             src = w->h_Q;
         }
         float* dst_scores = out_direct ? out_scores + (int64_t)c0 * k : w->h_scores;
         int64_t* dst_ids = out_direct ? out_emb_ids + (int64_t)c0 * k : w->h_ids;
         CU(cudaSetDevice(w->dev));
         CU(cudaMemcpyAsync(w->dQ, src, (size_t)bc * P.ld * 4, cudaMemcpyHostToDevice, w->st));
-        for (int attempt = 0; attempt < 2; ++attempt) {
-            if ((rc = batch_enqueue(w, g.get(), P, w->dQ, bc, false, w->st)) != SVSB_OK) return rc;
+        rc = batch_run_chunk(e, g.get(), P, w, w->st, w->dQ, bc, nullptr, [&]() -> int {
             CU(cudaMemcpyAsync(dst_scores, w->o_scores, (size_t)bc * k * 4, cudaMemcpyDeviceToHost, w->st));
             CU(cudaMemcpyAsync(dst_ids, w->o_ids, (size_t)bc * k * 8, cudaMemcpyDeviceToHost, w->st));
             CU(cudaMemcpyAsync(w->h_counts, w->o_counts, (size_t)bc * 4, cudaMemcpyDeviceToHost, w->st));
-            CU(cudaMemcpyAsync(w->h_flags, w->flags, (size_t)bc * 4, cudaMemcpyDeviceToHost, w->st));
-            CU(cudaStreamSynchronize(w->st));
-            if (!batch_thresholds_failed(g.get(), P, w->h_flags, bc)) break;
-            batch_plan(e, g.get(), k, P, true);       // redo the chunk with guaranteed thresholds (same buffers)
-        }
+            return SVSB_OK;
+        });
+        if (rc != SVSB_OK) return rc;
         for (int i = 0; i < bc; ++i) {
             const int64_t o = (int64_t)(c0 + i) * k;
             if (w->h_flags[i] == 0 && w->h_counts[i] == P.kk) {
@@ -1288,7 +1329,7 @@ int pairs_dev_coarse(PairsDev& r, int self, const std::vector<PairTask>& tasks, 
     auto block = [&](const char* m16op, int64_t m_rows, const void* q16, int64_t q_rows, int bq, int64_t tri_q0,
                      int64_t q_row0, int64_t m_row0) -> int {
         const int cur = r.cur;
-        const int b_pad = (bq + COARSE_TILE_QUERIES - 1) / COARSE_TILE_QUERIES * COARSE_TILE_QUERIES;
+        const int b_pad = batch_pad(bq);
         const int m_tiles = (int)((m_rows + COARSE_TILE_ROWS - 1) / COARSE_TILE_ROWS);
         CU(launch_pairs_fill_thr(st, w->thr, b_pad, bq, r.thr));
         CU(cudaMemsetAsync(w->cand_cnt, 0, (size_t)b_pad * 4, st));
@@ -1949,14 +1990,11 @@ extern "C" int svsb_bench_run_batch(svsb_t* e, int32_t k, int32_t iters, float* 
     if (e->bench_nq > COARSE_MAX_BATCH) return fail(SVSB_E_INVALID, "svsb_bench_run_batch: at most 2048 uploaded queries");
     BatchPlan P;
     if (!batch_plan(e, g.get(), k, P)) return fail(SVSB_E_INVALID, "svsb_bench_run_batch: this matrix / k does not take the coarse path");
+    const int b = e->bench_nq;
     std::lock_guard<std::mutex> lk(e->batch_mu);
     BatchWs* w = nullptr;
-    int rc = batch_ws_get(e, w);
+    int rc = batch_acquire(e, g.get(), P, b, nullptr, w);
     if (rc != SVSB_OK) return rc;
-    if ((rc = ensure_m16(g.get(), P, w->st)) != SVSB_OK) return rc;
-    const int b = e->bench_nq;
-    const int b_pad = (b + COARSE_TILE_QUERIES - 1) / COARSE_TILE_QUERIES * COARSE_TILE_QUERIES;
-    if ((rc = batch_ws_ensure(w, P, b_pad)) != SVSB_OK) return rc;
     CU(cudaSetDevice(w->dev));
     const int64_t l0 = g_launches.load();
     CU(cudaStreamSynchronize(w->st));
@@ -2028,6 +2066,20 @@ extern "C" int svsb_set_shard(svsb_t* e, int64_t global_row0) {
     return SVSB_OK;
 }
 
+// merge_records with the engine's merge scratch (slot 0's workspace holds it; only n_lists * cap > K_FAST_MAX needs it)
+static int engine_merge_records(svsb_engine* e, cudaStream_t st, const RecordView& recs, int n_lists, int64_t list_words, int batch,
+                                int k, float* out_scores, int64_t* out_ids, int32_t* out_counts, int verify_k, const int* status = nullptr) {
+    u64* sk = nullptr; int64_t* sp = nullptr;
+    if ((int64_t)n_lists * recs.cap > K_FAST_MAX) {
+        if (e->shard_ws.empty()) e->shard_ws.resize(1);
+        if (!e->shard_ws[0]) { e->shard_ws[0].reset(new DevWs()); e->shard_ws[0]->dev = e->devs[0]; }
+        int rc = e->shard_ws[0]->ensure_merge_scratch((int64_t)batch * n_lists * recs.cap);
+        if (rc != SVSB_OK) return rc;
+        sk = e->shard_ws[0]->mscr_keys; sp = e->shard_ws[0]->mscr_ids;
+    }
+    return merge_records(st, recs, n_lists, list_words, batch, k, sk, sp, out_scores, out_ids, out_counts, verify_k, status);
+}
+
 static int enqueue_local_topk_gen(svsb_engine* e, const std::shared_ptr<Generation>& g, void* stream, int32_t slot, const float* d_query,
                                   int32_t k, int64_t* d_record, int32_t flags);
 extern "C" int svsb_enqueue_local_topk(svsb_t* e, void* stream, int32_t slot, const float* d_query, int32_t k,
@@ -2047,8 +2099,8 @@ static int enqueue_local_topk_gen(svsb_engine* e, const std::shared_ptr<Generati
     const Shard& s = g->shards[0];
     cudaStream_t st = (cudaStream_t)stream;
     CU(cudaSetDevice(s.dev));
-    int32_t* d_count = reinterpret_cast<int32_t*>(d_record + 2 * (int64_t)k);
-    if (s.n_live == 0) { CU(cudaMemsetAsync(d_count, 0, 8, st)); return SVSB_OK; }
+    const RecordView r{d_record, k};
+    if (s.n_live == 0) { CU(cudaMemsetAsync(r.count(0), 0, 8, st)); return SVSB_OK; }
     if ((size_t)slot >= e->shard_ws.size()) e->shard_ws.resize(slot + 1);
     if (e->sel_pending.size() < e->shard_ws.size()) e->sel_pending.resize(e->shard_ws.size(), 0);
     if (!e->shard_ws[slot]) { e->shard_ws[slot].reset(new DevWs()); e->shard_ws[slot]->dev = s.dev; }
@@ -2081,7 +2133,7 @@ static int enqueue_local_topk_gen(svsb_engine* e, const std::shared_ptr<Generati
         sel_st = e->side_st;
     }
     CU(launch_select(sel_st, w.scores, s.n, w.gmax, shift, (int)std::min<int64_t>(k, s.n_live), s.ids, s.row0, w.cand, w.cand_cap,
-                     reinterpret_cast<u64*>(d_record), w.out_scores, d_record + k, d_count));
+                     r.keys(0), w.out_scores, r.ids(0), r.count(0)));
     w.gmax_dirty = false;
     if (pipelined) { CU(cudaEventRecord(w.ev_sel, e->side_st)); e->sel_pending[slot] = 1; }
     return SVSB_OK;
@@ -2105,7 +2157,7 @@ int batch_local_records_gen(svsb_engine* e, const std::shared_ptr<Generation>& g
     if (b == 0) return SVSB_OK;
     if (!d_Q || !d_records) return fail(SVSB_E_INVALID, "svsb_batch_local_records: NULL pointer");
     cudaStream_t st = stream;
-    const int64_t rec = 2 * (int64_t)k + 1;
+    const RecordView recs{d_records, k};
     int fallbacks = 0;
     BatchPlan P;
     bool coarse = g->n_live > 0 && b >= env_int("SVSB_BATCH_MIN", 4) && batch_plan(e, g.get(), k, P);
@@ -2113,20 +2165,13 @@ int batch_local_records_gen(svsb_engine* e, const std::shared_ptr<Generation>& g
     if (b >= 2 && mq_plan(g.get(), std::min<int64_t>(k, g->n_live), MP) && (b <= MP.max_b || !coarse)) {
         // small batch (or no tensor-core path for this shard): multi-query passes straight into the records
         std::lock_guard<std::mutex> lk(e->batch_mu);
-        MqWs* w = nullptr;
-        int rc = mq_ws_get(e, w);
-        if (rc != SVSB_OK) return rc;
-        const Shard& s = g->shards[0];
-        for (int32_t c0 = 0; c0 < b; c0 += MP.chunk) {
-            const int bc = std::min<int32_t>(MP.chunk, b - c0);
-            if ((rc = w->ensure(std::min<int32_t>(MP.chunk, b), s.n, g->ld, k)) != SVSB_OK) return rc;
-            CU(cudaStreamSynchronize(w->st));                    // the workspace's own (zeroing) work is done before `st` uses it
-            int64_t* r0 = d_records + (int64_t)c0 * rec;
-            SelectStrides os; os.keys = rec; os.oscores = k; os.ids = rec; os.count = 2 * rec;
-            if ((rc = mq_enqueue(w, g.get(), st, d_Q + (int64_t)c0 * g->ld, bc, k, os, reinterpret_cast<u64*>(r0), w->o_scores, r0 + k,
-                                 reinterpret_cast<int32_t*>(r0 + 2 * (int64_t)k))) != SVSB_OK) return rc;
+        auto stage = [&](MqWs*, int c0, int, const float*& dQ) -> int { dQ = d_Q + (int64_t)c0 * g->ld; return SVSB_OK; };
+        auto drain = [&](MqWs*, int c0, int) -> int {
             if (c0 + MP.chunk < b) CU(cudaStreamSynchronize(st));   // the next chunk reuses the score vectors
-        }
+            return SVSB_OK;
+        };
+        int rc = mq_run(e, g.get(), MP, b, k, st, recs, stage, drain);
+        if (rc != SVSB_OK) return rc;
         if (n_fallback) *n_fallback = 0;
         return SVSB_OK;
     }
@@ -2134,31 +2179,21 @@ int batch_local_records_gen(svsb_engine* e, const std::shared_ptr<Generation>& g
     if (coarse) {
         std::lock_guard<std::mutex> lk(e->batch_mu);
         BatchWs* w = nullptr;
-        int rc = batch_ws_get(e, w);
-        if (rc != SVSB_OK) return rc;
-        rc = ensure_m16(g.get(), P, st);
-        if (rc == SVSB_E_NOMEM) std::fill(todo.begin(), todo.end(), 1);    // no room for the fp16 shadow (+50 % of the shard):
-        else if (rc != SVSB_OK) return rc;                                 // the exact kernels answer, as in svsb_query_batch
+        int rc = batch_acquire(e, g.get(), P, std::min<int32_t>(b, COARSE_MAX_BATCH), st, w);
+        if (rc == SVSB_E_NOMEM) std::fill(todo.begin(), todo.end(), 1);    // no room for the fp16 shadow (+50 % of the shard)
+        else if (rc != SVSB_OK) return rc;                                 // or the workspace: the exact kernels answer, as in svsb_query_batch
         for (int32_t c0 = 0; rc == SVSB_OK && c0 < b; c0 += COARSE_MAX_BATCH) {
             const int bc = std::min<int32_t>(COARSE_MAX_BATCH, b - c0);
-            const int b_pad = (bc + COARSE_TILE_QUERIES - 1) / COARSE_TILE_QUERIES * COARSE_TILE_QUERIES;
-            if ((rc = batch_ws_ensure(w, P, b_pad)) != SVSB_OK) return rc;
-            int64_t* r0 = d_records + (int64_t)c0 * rec;
-            RefineOut o{nullptr, reinterpret_cast<u64*>(r0), r0 + k, rec, reinterpret_cast<int32_t*>(r0 + 2 * (int64_t)k), 2 * rec};
-            for (int attempt = 0; attempt < 2; ++attempt) {
-                if ((rc = batch_enqueue(w, g.get(), P, d_Q + (int64_t)c0 * P.ld, bc, false, st, &o)) != SVSB_OK) return rc;
-                CU(cudaMemcpyAsync(w->h_flags, w->flags, (size_t)bc * 4, cudaMemcpyDeviceToHost, st));
-                CU(cudaStreamSynchronize(st));
-                if (!batch_thresholds_failed(g.get(), P, w->h_flags, bc)) break;
-                batch_plan(e, g.get(), k, P, true);   // redo the chunk with guaranteed thresholds
-            }
+            const RefineOut o = recs.from(c0).refine_out();
+            rc = batch_run_chunk(e, g.get(), P, w, st, d_Q + (int64_t)c0 * P.ld, bc, &o, [] { return SVSB_OK; });
+            if (rc != SVSB_OK) return rc;
             for (int i = 0; i < bc; ++i) if (w->h_flags[i] != 0) todo[c0 + i] = 1;
         }
     }
     for (int32_t i = 0; i < b; ++i) {
         if (!todo[i]) continue;
         ++fallbacks;
-        int rc = enqueue_local_topk_gen(e, g, stream, 0, d_Q + (int64_t)i * g->ld, k, d_records + (int64_t)i * rec, 0);
+        int rc = enqueue_local_topk_gen(e, g, stream, 0, d_Q + (int64_t)i * g->ld, k, recs.rec(i), 0);
         if (rc != SVSB_OK) return rc;
     }
     if (n_fallback) *n_fallback = fallbacks;
@@ -2205,6 +2240,18 @@ extern "C" int svsb_batch_global_probe(svsb_t* e, int32_t k, int32_t* eligible, 
     return SVSB_OK;
 }
 
+// The arguments the caller chose for ALL ranks must cover this shard: max_row_norm at least its own (and safe for fp16
+// operands), sample_rank at least its own statistical bound (or SAMPLE_TOPX, all a rank ships).  svsb_batch_sample_tops
+// has no sample_rank yet and passes SAMPLE_TOPX; svsb_batch_global_records takes the norm svsb_batch_sample_tops checked.
+static int batch_global_check(const BatchPlan& P, float max_row_norm, int32_t sample_rank, const char* who) {
+    if (!(max_row_norm >= P.max_row_norm) || !(max_row_norm <= 8.1f))
+        return fail(SVSB_E_INVALID, std::string(who) + ": max_row_norm below this shard's own, or unsafe for fp16 operands");
+    const double lam = (double)P.kk * std::min(1.0, (double)P.sample_rows / (double)P.n);
+    if ((double)sample_rank < std::ceil(lam + 6.0 * std::sqrt(lam) + 4.0) && sample_rank < SAMPLE_TOPX && env_int("SVSB_BATCH_GLOBAL_ANY_RANK", 0) == 0)
+        return fail(SVSB_E_INVALID, std::string(who) + ": sample_rank below this shard's own bound");
+    return SVSB_OK;
+}
+
 extern "C" int svsb_batch_sample_tops(svsb_t* e, void* stream, const float* d_Q, int32_t b, int32_t k, float max_row_norm, float* d_tops) {
     if (!e) return fail(SVSB_E_INVALID, "engine is NULL");
     auto g = pin(e);
@@ -2212,20 +2259,14 @@ extern "C" int svsb_batch_sample_tops(svsb_t* e, void* stream, const float* d_Q,
     if (b < 1 || b > COARSE_MAX_BATCH || !d_Q || !d_tops) return fail(SVSB_E_INVALID, "svsb_batch_sample_tops: 1 <= b <= 2048, non-NULL buffers");
     BatchPlan P;
     if (!batch_plan_global(e, g.get(), k, P)) return fail(SVSB_E_STATE, "svsb_batch_sample_tops: this shard / k is not eligible (svsb_batch_global_probe)");
-    if (!(max_row_norm >= P.max_row_norm) || !(max_row_norm <= 8.1f)) return fail(SVSB_E_INVALID, "svsb_batch_sample_tops: max_row_norm below this shard's own, or unsafe for fp16 operands");
+    int rc = batch_global_check(P, max_row_norm, SAMPLE_TOPX, "svsb_batch_sample_tops");
+    if (rc != SVSB_OK) return rc;
     P.max_row_norm = max_row_norm;
     cudaStream_t st = (cudaStream_t)stream;
     std::lock_guard<std::mutex> lk(e->batch_mu);
     BatchWs* w = nullptr;
-    int rc = batch_ws_get(e, w);
-    if (rc != SVSB_OK) return rc;
-    if ((rc = ensure_m16(g.get(), P, st)) != SVSB_OK) return rc;
-    const int b_pad = (b + COARSE_TILE_QUERIES - 1) / COARSE_TILE_QUERIES * COARSE_TILE_QUERIES;
-    if ((rc = batch_ws_ensure(w, P, b_pad)) != SVSB_OK) return rc;
-    CU(cudaSetDevice(w->dev));
-    CU(launch_queries_to_f16(st, d_Q, b, b_pad, P.d, P.ld, w->dQ16, P.ld16, P.eps_coef, P.max_row_norm, w->eps, w->thr, w->flags, w->cand_cnt));
-    CU(launch_coarse_gemm(st, w->dev, 1, g->M16, P.n, w->dQ16, b_pad, P.ld16, P.s_tiles, P.tile_stride,
-                          nullptr, nullptr, nullptr, 0, w->sample, P.sample_rows));
+    if ((rc = batch_acquire(e, g.get(), P, b, st, w)) != SVSB_OK) return rc;
+    if ((rc = batch_sample(w, g.get(), P, d_Q, b, st)) != SVSB_OK) return rc;
     CU(launch_sample_top(st, w->sample, P.sample_rows, b, d_tops));
     w->global_gen = g->id; w->global_b = b; w->global_k = k;
     return SVSB_OK;
@@ -2248,22 +2289,11 @@ extern "C" int svsb_batch_global_records(svsb_t* e, void* stream, const float* d
     if (!w || w->global_gen != g->id || w->global_b != b || w->global_k != k)
         return fail(SVSB_E_STATE, "svsb_batch_global_records: no matching svsb_batch_sample_tops call precedes it");
     w->global_gen = 0;
-    {   // this rank's own statistical requirement must be covered by the caller's rank (it maximises over the ranks)
-        const double lam = (double)P.kk * std::min(1.0, (double)P.sample_rows / (double)P.n);
-        if ((double)sample_rank < std::ceil(lam + 6.0 * std::sqrt(lam) + 4.0) && sample_rank < SAMPLE_TOPX && env_int("SVSB_BATCH_GLOBAL_ANY_RANK", 0) == 0)
-            return fail(SVSB_E_INVALID, "svsb_batch_global_records: sample_rank below this shard's own bound");
-    }
-    const Shard& s = g->shards[0];
+    int rc = batch_global_check(P, P.max_row_norm, sample_rank, "svsb_batch_global_records");
+    if (rc != SVSB_OK) return rc;
     CU(cudaSetDevice(w->dev));
-    const int b_pad = (b + COARSE_TILE_QUERIES - 1) / COARSE_TILE_QUERIES * COARSE_TILE_QUERIES;
     CU(launch_union_threshold(st, d_tops_all, (int64_t)b * SAMPLE_TOPX, world, b, sample_rank, w->eps, w->thr));
-    CU(launch_coarse_gemm(st, w->dev, 0, g->M16, P.n, w->dQ16, b_pad, P.ld16, P.n_tiles, 1,
-                          w->thr, w->cand, w->cand_cnt, P.cand_cap, nullptr, 0));
-    const int64_t rec = 2 * (int64_t)rec_cap + 1;
-    RefineOut o{nullptr, reinterpret_cast<u64*>(d_records), d_records + rec_cap, rec, reinterpret_cast<int32_t*>(d_records + 2 * (int64_t)rec_cap), 2 * rec, rec_cap};
-    CU(launch_refine(st, s.M, P.n, P.ld, s.ids, s.row0, d_Q, b, P.ld, P.k, w->cand, w->cand_cnt, P.cand_cap, w->eps, w->thr, w->flags,
-                     o, w->stats, &w->rs, REFINE_PARTIAL | REFINE_DEFER));
-    return SVSB_OK;
+    return batch_filter_refine(w, g.get(), P, d_Q, b, st, RecordView{d_records, rec_cap}.refine_out(true), REFINE_PARTIAL | REFINE_DEFER);
 }
 
 // ---- the same batch protocol with BOTH exchanges fused into the kernels over NVLink peer memory (no collective) -------
@@ -2353,11 +2383,8 @@ extern "C" int svsb_batch_peer_prepare(svsb_t* e, int32_t b, int32_t k) {
     if (!batch_plan_global(e, g.get(), k, P)) return fail(SVSB_E_STATE, "svsb_batch_peer_prepare: this shard / k is not eligible (svsb_batch_global_probe)");
     std::lock_guard<std::mutex> lk(e->batch_mu);
     BatchWs* w = nullptr;
-    int rc = batch_ws_get(e, w);
+    int rc = batch_acquire(e, g.get(), P, b, nullptr, w);
     if (rc != SVSB_OK) return rc;
-    if ((rc = ensure_m16(g.get(), P, w->st)) != SVSB_OK) return rc;
-    const int b_pad = (b + COARSE_TILE_QUERIES - 1) / COARSE_TILE_QUERIES * COARSE_TILE_QUERIES;
-    if ((rc = batch_ws_ensure(w, P, b_pad)) != SVSB_OK) return rc;
     CU(cudaSetDevice(w->dev));
     CU(cudaDeviceSynchronize());
     return SVSB_OK;
@@ -2367,19 +2394,8 @@ extern "C" int svsb_batch_peer_prepare(svsb_t* e, int32_t b, int32_t k) {
 static int bxchg_enqueue_merge(svsb_engine* e, cudaStream_t st, const BXchg::Deferred& d) {
     BXchg* x = e->bxchg.get();
     CU(launch_wait_flags(st, x->flag(x->block, 1, d.slot, 0), x->world, d.seq, x->timeout_ns, x->status));
-    const int64_t rec = 2 * (int64_t)d.rec_cap + 1;
-    const int64_t* r0 = x->recs(x->block, d.slot, 0);
-    u64* sk = nullptr; int64_t* sp = nullptr;
-    if ((int64_t)x->world * d.rec_cap > K_FAST_MAX) {
-        if (e->shard_ws.empty() || !e->shard_ws[0]) { e->shard_ws.resize(std::max<size_t>(1, e->shard_ws.size())); e->shard_ws[0].reset(new DevWs()); e->shard_ws[0]->dev = e->devs[0]; }
-        int rc = e->shard_ws[0]->ensure_merge_scratch((int64_t)d.b * x->world * d.rec_cap);
-        if (rc != SVSB_OK) return rc;
-        sk = e->shard_ws[0]->mscr_keys; sp = e->shard_ws[0]->mscr_ids;
-    }
-    CU(launch_merge_ex(st, reinterpret_cast<const u64*>(r0), r0 + d.rec_cap, reinterpret_cast<const int32_t*>(r0 + 2 * (int64_t)d.rec_cap),
-                       x->world, d.rec_cap, d.k, d.b, x->rec_region(), rec, x->rec_region() * 2, rec * 2, sk, sp,
-                       d.out_scores, d.out_ids, d.out_counts, d.k, x->status));
-    return SVSB_OK;
+    return engine_merge_records(e, st, RecordView{x->recs(x->block, d.slot, 0), d.rec_cap}, x->world, x->rec_region(), d.b, d.k,
+                                d.out_scores, d.out_ids, d.out_counts, d.k, x->status);
 }
 
 extern "C" int svsb_batch_peer_flush(svsb_t* e, void* stream) {
@@ -2407,23 +2423,13 @@ extern "C" int svsb_batch_peer(svsb_t* e, void* stream, const float* d_Q, int32_
     if (rec_cap < k && (int64_t)x->world * rec_cap > K_FAST_MAX) return fail(SVSB_E_INVALID, "svsb_batch_peer: truncated records need world * rec_cap <= 2048");
     BatchPlan P;
     if (!batch_plan_global(e, g.get(), k, P)) return fail(SVSB_E_STATE, "svsb_batch_peer: this shard / k is not eligible (svsb_batch_global_probe)");
-    if (!(max_row_norm >= P.max_row_norm) || !(max_row_norm <= 8.1f)) return fail(SVSB_E_INVALID, "svsb_batch_peer: max_row_norm below this shard's own, or unsafe for fp16 operands");
-    {
-        const double lam = (double)P.kk * std::min(1.0, (double)P.sample_rows / (double)P.n);
-        if ((double)sample_rank < std::ceil(lam + 6.0 * std::sqrt(lam) + 4.0) && sample_rank < SAMPLE_TOPX && env_int("SVSB_BATCH_GLOBAL_ANY_RANK", 0) == 0)
-            return fail(SVSB_E_INVALID, "svsb_batch_peer: sample_rank below this shard's own bound");
-    }
+    int rc = batch_global_check(P, max_row_norm, sample_rank, "svsb_batch_peer");
+    if (rc != SVSB_OK) return rc;
     P.max_row_norm = max_row_norm;
     cudaStream_t st = (cudaStream_t)stream;
     std::lock_guard<std::mutex> lk(e->batch_mu);
     BatchWs* w = nullptr;
-    int rc = batch_ws_get(e, w);
-    if (rc != SVSB_OK) return rc;
-    if ((rc = ensure_m16(g.get(), P, st)) != SVSB_OK) return rc;
-    const int b_pad = (b + COARSE_TILE_QUERIES - 1) / COARSE_TILE_QUERIES * COARSE_TILE_QUERIES;
-    if ((rc = batch_ws_ensure(w, P, b_pad)) != SVSB_OK) return rc;
-    const Shard& s = g->shards[0];
-    CU(cudaSetDevice(w->dev));
+    if ((rc = batch_acquire(e, g.get(), P, b, st, w)) != SVSB_OK) return rc;
     const unsigned long long seq = ++x->seq;
     const int slot = (int)(seq % BXchg::SLOTS);
     BatchPush pa, pb;
@@ -2432,11 +2438,8 @@ extern "C" int svsb_batch_peer(svsb_t* e, void* stream, const float* d_Q, int32_
         pa.dst[p] = x->tops(x->peer_block[p], slot, x->rank); pa.flag[p] = x->flag(x->peer_block[p], 0, slot, x->rank);
         pb.dst[p] = x->recs(x->peer_block[p], slot, x->rank); pb.flag[p] = x->flag(x->peer_block[p], 1, slot, x->rank);
     }
-    const int64_t rec = 2 * (int64_t)rec_cap + 1;
     // 1. this rank's sample maxima -> every rank's window
-    CU(launch_queries_to_f16(st, d_Q, b, b_pad, P.d, P.ld, w->dQ16, P.ld16, P.eps_coef, P.max_row_norm, w->eps, w->thr, w->flags, w->cand_cnt));
-    CU(launch_coarse_gemm(st, w->dev, 1, g->M16, P.n, w->dQ16, b_pad, P.ld16, P.s_tiles, P.tile_stride,
-                          nullptr, nullptr, nullptr, 0, w->sample, P.sample_rows));
+    if ((rc = batch_sample(w, g.get(), P, d_Q, b, st)) != SVSB_OK) return rc;
     CU(launch_sample_top(st, w->sample, P.sample_rows, b, nullptr, &pa));
     if (x->deferred.pending) {                 // the previous batch's merge: its peers had this phase's time to deliver
         rc = bxchg_enqueue_merge(e, st, x->deferred);
@@ -2446,11 +2449,8 @@ extern "C" int svsb_batch_peer(svsb_t* e, void* stream, const float* d_Q, int32_
     // 2. all ranks' maxima are here -> ONE threshold per query; filter; exact re-score; records -> every rank's window
     CU(launch_wait_flags(st, x->flag(x->block, 0, slot, 0), x->world, seq, x->timeout_ns, x->status));
     CU(launch_union_threshold(st, x->tops(x->block, slot, 0), x->tops_region(), x->world, b, sample_rank, w->eps, w->thr));
-    CU(launch_coarse_gemm(st, w->dev, 0, g->M16, P.n, w->dQ16, b_pad, P.ld16, P.n_tiles, 1,
-                          w->thr, w->cand, w->cand_cnt, P.cand_cap, nullptr, 0));
-    RefineOut o{nullptr, nullptr, nullptr, rec, nullptr, 2 * rec, rec_cap};
-    CU(launch_refine(st, s.M, P.n, P.ld, s.ids, s.row0, d_Q, b, P.ld, P.k, w->cand, w->cand_cnt, P.cand_cap, w->eps, w->thr, w->flags,
-                     o, w->stats, &w->rs, REFINE_PARTIAL | REFINE_DEFER, &pb));
+    if ((rc = batch_filter_refine(w, g.get(), P, d_Q, b, st, RecordView{nullptr, rec_cap}.refine_out(true), REFINE_PARTIAL | REFINE_DEFER, &pb)) != SVSB_OK)
+        return rc;
     // 3. all ranks' records are here -> verifying merge (now, or behind the first phase of the next batch)
     BXchg::Deferred d;
     d.pending = true; d.slot = slot; d.rec_cap = rec_cap; d.k = k; d.b = b; d.seq = seq;
@@ -2841,19 +2841,9 @@ static int enqueue_merge_records(svsb_t* e, void* stream, const int64_t* d_recor
     if (cap < k && ((int64_t)n_lists * cap > K_FAST_MAX || n_lists > 16)) return fail(SVSB_E_INVALID, std::string(who) + ": truncated records need n_lists <= 16 and n_lists * rec_cap <= 2048");
     if (!d_records || !d_out_scores || !d_out_ids || !d_out_counts) return fail(SVSB_E_INVALID, std::string(who) + ": NULL pointer");
     CU(cudaSetDevice(e->devs[0]));
-    const int64_t rec = 2 * (int64_t)cap + 1;
-    u64* sk = nullptr; int64_t* sp = nullptr;
-    if ((int64_t)n_lists * cap > K_FAST_MAX) {
-        if (e->shard_ws.empty() || !e->shard_ws[0]) { e->shard_ws.resize(std::max<size_t>(1, e->shard_ws.size())); e->shard_ws[0].reset(new DevWs()); e->shard_ws[0]->dev = e->devs[0]; }
-        int rc = e->shard_ws[0]->ensure_merge_scratch((int64_t)batch * n_lists * k);
-        if (rc != SVSB_OK) return rc;
-        sk = e->shard_ws[0]->mscr_keys; sp = e->shard_ws[0]->mscr_ids;
-    }
-    CU(launch_merge_ex((cudaStream_t)stream, reinterpret_cast<const u64*>(d_records), d_records + cap,
-                       reinterpret_cast<const int32_t*>(d_records + 2 * (int64_t)cap), n_lists, cap, k, batch,
-                       (int64_t)batch * rec, rec, (int64_t)batch * rec * 2, rec * 2, sk, sp,
-                       d_out_scores, d_out_ids, d_out_counts, verify_k));
-    return SVSB_OK;
+    const RecordView recs{const_cast<int64_t*>(d_records), cap};           // read only
+    return engine_merge_records(e, (cudaStream_t)stream, recs, n_lists, (int64_t)batch * recs.words(), batch, k,
+                                d_out_scores, d_out_ids, d_out_counts, verify_k);
 }
 extern "C" int svsb_enqueue_merge_records(svsb_t* e, void* stream, const int64_t* d_records, int32_t n_lists, int32_t batch,
                                           int32_t k, float* d_out_scores, int64_t* d_out_ids, int32_t* d_out_counts) {

@@ -10,6 +10,7 @@
 #include <condition_variable>
 #include <cstdio>
 #include <cstdlib>
+#include <cstring>
 #include <memory>
 #include <mutex>
 #include <string>
@@ -220,6 +221,43 @@ struct Loading {
     int cur = 0;
     bool borrowed = false;
 };
+
+// A block of packed candidate records, one per query (include/svsb200.h, sharded deployment):
+// Record layout: 2*cap+1 int64 words = [ keys (cap, uint64: ordered score << 32 | ~global_row) |
+//                                        embeddings.id (cap) | count (int32 in the low half of the last word) ].
+// The batch records of the global threshold (REFINE_PARTIAL) carry [count, ver] in the last word.
+struct RecordView {
+    int64_t* base = nullptr;                 // record 0
+    int cap = 0;                             // entries per record
+    int64_t words() const { return 2 * (int64_t)cap + 1; }
+    int64_t* rec(int64_t q) const { return base + q * words(); }
+    u64* keys(int64_t q) const { return reinterpret_cast<u64*>(rec(q)); }
+    int64_t* ids(int64_t q) const { return rec(q) + cap; }
+    int32_t* count(int64_t q) const { return reinterpret_cast<int32_t*>(rec(q) + 2 * (int64_t)cap); }
+    RecordView from(int64_t q) const { return {rec(q), cap}; }
+    // the refine kernel writing records 0, 1, ...; partial: REFINE_PARTIAL records of at most cap entries.
+    // base == null: a BatchPush stores the records into the peers' windows, only the layout is used.
+    RefineOut refine_out(bool partial = false) const {
+        if (!base) return {nullptr, nullptr, nullptr, words(), nullptr, 2 * words(), partial ? cap : 0};
+        return {nullptr, keys(0), ids(0), words(), count(0), 2 * words(), partial ? cap : 0};
+    }
+    // the multi-query selection writing records 0, 1, ... (its scores go to a separate buffer, score_stride apart)
+    SelectStrides select_strides(int64_t score_stride) const {
+        SelectStrides s; s.keys = words(); s.oscores = score_stride; s.ids = words(); s.count = 2 * words();
+        return s;
+    }
+};
+
+// Merge [n_lists][batch] records (list l + 1's block starts list_words words after list l's) into [batch][k] outputs.
+// sk / sp: merge scratch of batch * n_lists * recs.cap entries, needed only when n_lists * recs.cap > K_FAST_MAX.
+// verify_k >= 0: the records carry [count, ver] (REFINE_PARTIAL); status: a batch window's timeout word (or null).
+static inline int merge_records(cudaStream_t st, const RecordView& recs, int n_lists, int64_t list_words, int batch, int k, u64* sk,
+                                int64_t* sp, float* out_scores, int64_t* out_ids, int32_t* out_counts, int verify_k = -1,
+                                const int* status = nullptr) {
+    CU(launch_merge_ex(st, recs.keys(0), recs.ids(0), recs.count(0), n_lists, recs.cap, k, batch, list_words, recs.words(),
+                       2 * list_words, 2 * recs.words(), sk, sp, out_scores, out_ids, out_counts, verify_k, status));
+    return SVSB_OK;
+}
 
 // workspace of the batched path: coarse operands, thresholds, candidate lists, outputs (device) + pinned staging
 struct BatchWs {
@@ -474,6 +512,14 @@ struct svsb_engine {
 };
 
 static inline int round_up4(int d) { return (d + 3) & ~3; }
+
+// host queries Q[b][d] -> dst[b][ld], zero padded to the rows' leading dimension (staging of the batched paths)
+static inline void stage_queries(float* dst, const float* Q, int b, int d, int ld) {
+    for (int i = 0; i < b; ++i) {
+        memcpy(dst + (size_t)i * ld, Q + (size_t)i * d, (size_t)d * 4);
+        std::fill(dst + (size_t)i * ld + d, dst + (size_t)(i + 1) * ld, 0.f);
+    }
+}
 
 // a query handle that keeps "the arrays it fetched" alive across an invalidate (svsb_snapshot_*)
 struct svsb_snapshot { std::shared_ptr<Generation> gen; };

@@ -545,7 +545,7 @@ int multi_query_batch(svsb_engine* e, const std::shared_ptr<Generation>& g, cons
     }
     std::unique_lock<std::mutex> lk(m->mu);        // exclusive use of the gather scratch; fused queries in flight keep running
     const int kr = (int)kk;                         // entries per record
-    const int64_t rec = 2 * (int64_t)kr + 1;
+    const int64_t rec = RecordView{nullptr, kr}.words();
     const int ld = g->ld;
     CU(cudaSetDevice(root_dev(m)));
     if ((int64_t)b * ld > m->h_Q_cap) {
@@ -554,11 +554,7 @@ int multi_query_batch(svsb_engine* e, const std::shared_ptr<Generation>& g, cons
         CU(cudaHostAlloc(&m->h_Q, (size_t)b * ld * 4, cudaHostAllocPortable));
         m->h_Q_cap = (int64_t)b * ld;
     }
-    for (int32_t i = 0; i < b; ++i) {
-        float* dst = m->h_Q + (size_t)i * ld;
-        memcpy(dst, Q + (size_t)i * d, (size_t)d * 4);
-        for (int c = d; c < ld; ++c) dst[c] = 0.f;
-    }
+    stage_queries(m->h_Q, Q, b, d, ld);
     if ((int64_t)nd * b * rec > m->g_rec_cap) {
         if (m->g_rec) cudaFree(m->g_rec);
         m->g_rec = nullptr; m->g_rec_cap = 0;
@@ -616,8 +612,8 @@ int multi_query_batch(svsb_engine* e, const std::shared_ptr<Generation>& g, cons
     }
     u64* sk = nullptr; int64_t* sp = nullptr;
     if ((int64_t)nd * kr > K_FAST_MAX) { sk = m->b_sk; sp = m->b_sp; }
-    CU(launch_merge_ex(rst, reinterpret_cast<const u64*>(m->g_rec), m->g_rec + kr, reinterpret_cast<const int32_t*>(m->g_rec + 2 * (int64_t)kr),
-                       nd, kr, kr, b, (int64_t)b * rec, rec, (int64_t)b * rec * 2, rec * 2, sk, sp, m->b_scores, m->b_ids, m->b_counts));
+    if ((rc = merge_records(rst, RecordView{m->g_rec, kr}, nd, (int64_t)b * rec, b, kr, sk, sp, m->b_scores, m->b_ids, m->b_counts)) != SVSB_OK)
+        return rc;
     // results: (b, kr) on the device, (b, k) at the caller
     CU(cudaMemcpy2DAsync(out_scores, (size_t)k * 4, m->b_scores, (size_t)kr * 4, (size_t)kr * 4, (size_t)b, cudaMemcpyDeviceToHost, rst));
     CU(cudaMemcpy2DAsync(out_ids, (size_t)k * 8, m->b_ids, (size_t)kr * 8, (size_t)kr * 8, (size_t)b, cudaMemcpyDeviceToHost, rst));
