@@ -183,6 +183,9 @@ int svsb_batch_stats(svsb_t* e, int32_t b, int32_t* candidates, int32_t* rescore
  * shadow, then an exact fp32 re-score of the candidate rows), 0 for the fp32 similarity kernel; *rescored = rows the
  * last query re-scored exactly (0 without the filter). */
 int svsb_bench_filter_stats(svsb_t* e, int32_t* filter, int64_t* rescored);
+/* The route the last svsb_bench_run's queries took: *route = 0 for the fp32 similarity kernel, 16 for the filter over the
+ * fp16 shadow, 8 for the filter over the int8 shadow (one scale per row; +25 % of the matrix in device memory). */
+int svsb_bench_filter_route(svsb_t* e, int32_t* route);
 /* How the resident generation picks the coarse pass's filter thresholds: 0 = an order statistic of a row sample that
  * bounds the true cut-off with overwhelming probability and is VERIFIED per query after the pass (default; several
  * times fewer candidates), 1 = a proven bound (the engine switches a generation to it when verification fails for

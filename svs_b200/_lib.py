@@ -69,6 +69,7 @@ SIGNATURES = {
     "svsb_bench_batch_result": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, c_i32_p, c_i32_p]),
     "svsb_batch_stats": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p]),
     "svsb_bench_filter_stats": (C.c_int, [C.c_void_p, c_i32_p, c_i64_p]),
+    "svsb_bench_filter_route": (C.c_int, [C.c_void_p, c_i32_p]),
     "svsb_host_alloc": (C.c_int, [C.c_size_t, C.POINTER(C.c_void_p)]),
     "svsb_host_free": (C.c_int, [C.c_void_p]),
     "svsb_batch_threshold_mode": (C.c_int, [C.c_void_p]),

@@ -592,6 +592,28 @@ int shadow_sync(const Shard& s, int ld, int64_t fresh_from, int create, cudaStre
         b->m16_rows = s.n;
     }
     *out = b->M16;
+    if (ld > FILTER_MAX_LD || (!b->M8 && create != 1)) return SVSB_OK;
+    const int ld8 = (ld + 15) & ~15;
+    if (!b->M8) {                                        // +25 % of the matrix: only with an eighth of the device still free
+        const size_t rows8 = (size_t)b->cap_rows * ld8, bytes = rows8 + (size_t)b->cap_rows * 4 + 16;
+        size_t fr = 0, tot = 0;
+        if (cudaMemGetInfo(&fr, &tot) != cudaSuccess || fr < bytes + tot / 8) { (void)cudaGetLastError(); return SVSB_OK; }
+        void* p = nullptr;
+        if (cudaMalloc(&p, bytes) != cudaSuccess) { (void)cudaGetLastError(); return SVSB_OK; }   // no int8 route, not an error
+        float* e8 = reinterpret_cast<float*>(static_cast<char*>(p) + rows8 + (size_t)b->cap_rows * 4);
+        if (cudaMemset(e8, 0, 4) != cudaSuccess) { (void)cudaGetLastError(); cudaFree(p); return SVSB_OK; }
+        b->M8 = p; b->ld8 = ld8; b->m8_rows = 0;
+        b->s8 = reinterpret_cast<float*>(static_cast<char*>(p) + rows8); b->e8 = e8;
+    }
+    if (fresh_from < b->m8_rows) b->m8_rows = fresh_from;
+    if (b->m8_rows < s.n) {
+        const int64_t r0 = b->m8_rows;
+        cudaError_t ce = launch_rows_to_i8(st, s.dev, s.M + r0 * ld, s.n - r0, ld, static_cast<char*>(b->M8) + (size_t)r0 * ld8, ld8,
+                                           b->s8 + r0, b->e8);
+        if (ce == cudaSuccess) ce = cudaStreamSynchronize(st);
+        if (ce != cudaSuccess) { (void)cudaGetLastError(); return fail(SVSB_E_CUDA, std::string("int8 shadow: ") + cudaGetErrorString(ce)); }
+        b->m8_rows = s.n;
+    }
     return SVSB_OK;
 }
 
@@ -599,8 +621,9 @@ int shadow_sync(const Shard& s, int ld, int64_t fresh_from, int create, cudaStre
 // rows of norm <= 8 (fp16 range of the scaled operands), d <= FILTER_MAX_LD, and a matrix large enough to gain:
 // SVSB_FILTER_MIN_MB, default 512 MB of fp32 rows.  Measured on a B200 (profiles/r05_filter_ab.txt, 1536-d rows): at
 // 246 MB K1's pass is still faster than filter + threshold + re-score, at 492 MB the filter takes 25 % less time.
+// The int8 shadow is built with it when it fits as well (shadow_sync).
 static int filter_attach(svsb_engine* e, Generation* g) {
-    for (auto& s : g->shards) s.M16 = nullptr;
+    for (auto& s : g->shards) { s.M16 = nullptr; s.M8 = nullptr; }
     if (e->devs.size() != 1 || e->is_kid || g->shards.size() != 1) return SVSB_OK;
     Shard& s = g->shards[0];
     if (s.n == 0 || g->ld > FILTER_MAX_LD || !(1.0f + g->max_dev <= 8.0f)) return SVSB_OK;
@@ -609,28 +632,38 @@ static int filter_attach(svsb_engine* e, Generation* g) {
     int rc = shadow_sync(s, g->ld, INT64_MAX, 1, e->copy_st[0], &p);
     if (rc != SVSB_OK) return rc;
     s.M16 = p;
+    if (p) s.M8 = s.buf->M8;
     return SVSB_OK;
 }
 
-// SVSB_FILTER=0 forces K1 (read per call).  The LDG variant of K1 (SVSB_GEMV_VARIANT=1) sums in another order than the
-// re-score, which reproduces the TMA kernel's bits.
-static bool use_filter(const Shard& s, int64_t kk) {
-    if (!s.M16 || kk > K_FAST_MAX || env_int("SVSB_FILTER", 1) == 0) return false;
+// The route of one single query: 0 = K1, 16 = the fp16 filter, 8 = the int8 filter (DESIGN.md section 4, K1f8).
+// SVSB_FILTER (read per call): 0 forces K1, 16 or 8 force that filter where the view has its shadow, 1 or unset choose:
+// int8 wherever its shadow exists.  Measured on a B200 (profiles/r06_filter8_ab.txt), int8 against fp16 per query: C2
+// (1M x 1536, k = 100) 254 against 426 us, C4 (10M x 1536) 2.76 against 4.30 ms, and C5 (1M x 3072, k = 1000: ~99 000 rows
+// re-scored, 1.2 GB) still 741 against 936 us -- no shape the filters serve favours fp16.
+// The LDG variant of K1 (SVSB_GEMV_VARIANT=1) sums in another order than the re-score, which reproduces the TMA kernel's
+// bits: it turns the filters off.
+static int filter_route(const Shard& s, int64_t kk) {
+    const int f = env_int("SVSB_FILTER", 1);
+    if (!s.M16 || kk > K_FAST_MAX || f == 0) return 0;
     const char* v = getenv("SVSB_GEMV_VARIANT");
-    return !(v && atoi(v) == 1);
+    if (v && atoi(v) == 1) return 0;
+    return s.M8 && f != 16 ? 8 : 16;
 }
 
-// The similarity pass of one query: K1, or the fp16 filter (then filter_finish before the selection).
+// The similarity pass of one query: K1, or a filter (then filter_finish before the selection).
 static cudaError_t similarity_pass(cudaStream_t st, const DevWs& w, const Generation* g, const Shard& s, const float* q,
-                                   int shift, int reserve_sms, bool filter) {
-    if (filter) return launch_filter(st, w.dev, s.M16, s.n, g->ld, (g->ld + 7) & ~7, q, w.scores, w.gmax, shift, reserve_sms, s.live);
+                                   int shift, int reserve_sms, int route) {
+    if (route == 8)
+        return launch_filter8(st, w.dev, s.M8, s.buf->s8, s.n, g->ld, s.buf->ld8, q, w.scores, w.gmax, shift, reserve_sms, s.live);
+    if (route == 16) return launch_filter(st, w.dev, s.M16, s.n, g->ld, (g->ld + 7) & ~7, q, w.scores, w.gmax, shift, reserve_sms, s.live);
     return launch_gemv(st, w.dev, s.M, s.n, g->d, g->ld, q, w.scores, w.gmax, shift, 0, 0, 0, reserve_sms, s.live);
 }
 // Threshold + exact re-score: afterwards scores / gmax give launch_select K1's top-kk.
 static cudaError_t filter_finish(cudaStream_t st, const DevWs& w, const Generation* g, const Shard& s, const float* q,
-                                 int shift, int64_t kk) {
+                                 int shift, int64_t kk, int route) {
     return launch_filter_refine(st, w.dev, s.M, s.n, g->ld, q, w.scores, w.gmax, shift, (int)kk, coarse_eps_coef(g->d),
-                                (1.0f + g->max_dev) * 1.000001f, s.live, w.fstate);
+                                (1.0f + g->max_dev) * 1.000001f, route == 8 ? s.buf->e8 : nullptr, s.live, w.fstate);
 }
 
 int prepare_ws(DevWs& w, const Generation* g, const Shard& s, int64_t kk) {
@@ -688,17 +721,17 @@ static int enqueue_single(QueryCtx* c, const Generation* g, const float* q, int3
         }
         CU(launch_stage_query(gst, c->h_q, w.d_q, g->ld));
         w.gmax_dirty = true;
-        const bool filter = use_filter(s, kk);
+        const int route = filter_route(s, kk);
         {   // programmatic dependent launch: the similarity kernel streams its first tiles under the staging kernel
             PdlScope pdl(env_int("SVSB_PDL", 1) != 0);
-            CU(similarity_pass(gst, w, g, s, w.d_q, shift, reserve_sm ? 1 : 0, filter));
+            CU(similarity_pass(gst, w, g, s, w.d_q, shift, reserve_sm ? 1 : 0, route));
         }
         if (chain) {
             CU(cudaEventRecord(c->ev_gemv, gst));
             chain_lk.unlock();
             CU(cudaStreamWaitEvent(w.st, c->ev_gemv, 0));
         }
-        if (filter) CU(filter_finish(w.st, w, g, s, w.d_q, shift, kk));
+        if (route) CU(filter_finish(w.st, w, g, s, w.d_q, shift, kk, route));
         CU(launch_select(w.st, w.scores, s.n, w.gmax, shift, (int)kk, s.ids, s.row0, w.cand, w.cand_cap,
                          w.out_keys, c->h_scores, c->h_ids, c->h_count));
         w.gmax_dirty = false;
@@ -1863,8 +1896,8 @@ extern "C" int svsb_bench_run(svsb_t* e, int32_t k, int32_t iters, float* total_
     // k <= 2048: software pipeline.  The similarity kernel of query i+1 (stream A, all SMs but one) runs while the
     // one-CTA selection kernel of query i (stream B) finishes on the SM left free; two buffer sets.
     const bool pipelined = kk <= K_FAST_MAX && env_int("SVSB_PIPELINE", 1) != 0 && sm_count(w0.dev) > 8;
-    const bool filter = use_filter(s, kk);
-    e->bench_filter = filter;
+    const int route = filter_route(s, kk);
+    e->bench_route = route;
     if (pipelined) {
         if (!c->alt) {
             c->alt.reset(new DevWs());
@@ -1893,11 +1926,11 @@ extern "C" int svsb_bench_run(svsb_t* e, int32_t k, int32_t iters, float* total_
             if (it >= 2) CU(cudaStreamWaitEvent(sa, W.ev_sel, 0));           // selection of query it-2 is done with W
             if (timed_it(it)) CU(cudaEventRecord(kev[2 * it], sa));
             W.gmax_dirty = true;
-            CU(similarity_pass(sa, W, g.get(), s, e->bench_q[0] + qoff, shift, /*reserve_sms=*/1, filter));
+            CU(similarity_pass(sa, W, g.get(), s, e->bench_q[0] + qoff, shift, /*reserve_sms=*/1, route));
             if (timed_it(it)) CU(cudaEventRecord(kev[2 * it + 1], sa));
             CU(cudaEventRecord(W.ev, sa));
             CU(cudaStreamWaitEvent(sb, W.ev, 0));
-            if (filter) CU(filter_finish(sb, W, g.get(), s, e->bench_q[0] + qoff, shift, kk));
+            if (route) CU(filter_finish(sb, W, g.get(), s, e->bench_q[0] + qoff, shift, kk, route));
             CU(launch_select(sb, W.scores, s.n, W.gmax, shift, (int)kk, s.ids, s.row0, W.cand, W.cand_cap,
                              W.out_keys, W.out_scores, W.out_ids, W.out_count));
             W.gmax_dirty = false;
@@ -1911,9 +1944,9 @@ extern "C" int svsb_bench_run(svsb_t* e, int32_t k, int32_t iters, float* total_
             const int64_t qoff = (int64_t)(it % e->bench_nq) * e->bench_ld;
             if (timed_it(it)) CU(cudaEventRecord(kev[2 * it], w0.st));
             w0.gmax_dirty = true;
-            CU(similarity_pass(w0.st, w0, g.get(), s, e->bench_q[0] + qoff, shift, 0, filter));
+            CU(similarity_pass(w0.st, w0, g.get(), s, e->bench_q[0] + qoff, shift, 0, route));
             if (timed_it(it)) CU(cudaEventRecord(kev[2 * it + 1], w0.st));
-            if (filter) CU(filter_finish(w0.st, w0, g.get(), s, e->bench_q[0] + qoff, shift, kk));
+            if (route) CU(filter_finish(w0.st, w0, g.get(), s, e->bench_q[0] + qoff, shift, kk, route));
             if (kk <= K_FAST_MAX)
                 CU(launch_select(w0.st, w0.scores, s.n, w0.gmax, shift, (int)kk, s.ids, s.row0, w0.cand, w0.cand_cap,
                                  w0.out_keys, w0.out_scores, w0.out_ids, w0.out_count));
@@ -1942,13 +1975,19 @@ extern "C" int svsb_bench_filter_stats(svsb_t* e, int32_t* filter, int64_t* resc
     if (!e || !filter || !rescored) return fail(SVSB_E_INVALID, "svsb_bench_filter_stats: NULL argument");
     *filter = 0; *rescored = 0;
     if (e->multi || !e->bench_ctx || !e->bench_ctx->last) return SVSB_OK;
-    if (!e->bench_filter) return SVSB_OK;
+    if (!e->bench_route) return SVSB_OK;
     const DevWs& w = *e->bench_ctx->last;
     uint32_t st[2] = {0, 0};
     CU(cudaSetDevice(w.dev));
     CU(cudaStreamSynchronize(w.st));
     CU(cudaMemcpy(st, w.fstate, 8, cudaMemcpyDeviceToHost));
     *filter = 1; *rescored = st[1];
+    return SVSB_OK;
+}
+
+extern "C" int svsb_bench_filter_route(svsb_t* e, int32_t* route) {
+    if (!e || !route) return fail(SVSB_E_INVALID, "svsb_bench_filter_route: NULL argument");
+    *route = e->multi || !e->bench_ctx || !e->bench_ctx->last ? 0 : e->bench_route;
     return SVSB_OK;
 }
 

@@ -52,11 +52,16 @@ struct ShardBuf {
     // converted by the update that writes them (shadow_sync).
     std::mutex m16_mu;
     void* M16 = nullptr; int ld16 = 0; int64_t m16_rows = 0;
+    // int8 shadow for the single-query int8 filter (DESIGN.md section 4, K1f8), one allocation: M8 = cap_rows x ld8 bytes,
+    // then s8 = cap_rows scales, then e8 = the error word E (only raised).  Built next to M16 by filter_attach when it fits,
+    // rows [0, m8_rows) converted; guarded by m16_mu.
+    void* M8 = nullptr; float* s8 = nullptr; float* e8 = nullptr; int ld8 = 0; int64_t m8_rows = 0;
     ~ShardBuf() {
-        if (M || ids || M16) cudaSetDevice(dev);
+        if (M || ids || M16 || M8) cudaSetDevice(dev);
         if (M) cudaFree(M);
         if (ids) cudaFree(ids);
         if (M16) cudaFree(M16);
+        if (M8) cudaFree(M8);
     }
 };
 
@@ -73,6 +78,8 @@ struct Shard {
     // == buf->M16 when this view's single queries take the fp16 filter (set before the generation is published, never
     // changed after; null: K1 -- see filter_shadow in engine.cu)
     const void* M16 = nullptr;
+    // == buf->M8 when the int8 filter is available to this view as well (set with M16)
+    const void* M8 = nullptr;
 };
 
 struct Generation {
@@ -494,7 +501,7 @@ struct svsb_engine {
     std::vector<float*> bench_q; int bench_nq = 0, bench_d = 0, bench_ld = 0;
     std::unique_ptr<QueryCtx> bench_ctx;
     std::vector<cudaEvent_t> bench_kev;                  // similarity-kernel timing events of svsb_bench_run (device 0)
-    bool bench_filter = false;                           // the last svsb_bench_run took the fp16 filter
+    int bench_route = 0;                                 // the last svsb_bench_run's route: 0 K1, 16 / 8 the fp16 / int8 filter
     // sharded deployment (one process per GPU)
     int64_t shard_row0 = 0;                              // global row of this engine's first row
     std::vector<std::unique_ptr<DevWs>> shard_ws;        // workspaces for svsb_enqueue_local_topk (by slot)
@@ -531,7 +538,8 @@ std::shared_ptr<Generation> pin(svsb_engine* e);
 int prepare_ws(DevWs& w, const Generation* g, const Shard& s, int64_t kk);
 // Convert rows [buf->m16_rows, s.n) of the shard's fp16 shadow (rows from `fresh_from` on were (re)written: they are
 // converted again).  No shadow yet: create = 0 leaves it so (*out = null), 1 allocates it when the device keeps ample
-// room after it (else *out = null, not an error), 2 allocates it or fails.
+// room after it (else *out = null, not an error), 2 allocates it or fails.  The int8 shadow (ShardBuf::M8) is kept the
+// same way when it exists; create = 1 also allocates it, under the same room rule, for rows of ld <= FILTER_MAX_LD.
 int shadow_sync(const Shard& s, int ld, int64_t fresh_from, int create, cudaStream_t st, void** out);
 int engine_create(const int* device_ids, int n_dev, bool as_kid, svsb_engine** out);
 int alloc_generation(svsb_engine* e, int64_t n, int d, std::shared_ptr<Generation>& out);

@@ -481,29 +481,237 @@ gemv16_tma_kernel(const __half* __restrict__ M16, int64_t n, int c16, int tile_r
     }
 }
 
+// =============================================================================================
+// variant 4: the int8 filter -- the same ring over the int8 shadow (DESIGN.md section 4, "K1f8")
+// =============================================================================================
+// Row r of the shadow is Q_r[ld8] (int8, zero padded) with one fp32 scale s_r = max|r_j| / 127: r^ = s_r * Q_r.  The
+// device word E >= max_r ||r - r^|| bounds the quantisation error of every row converted so far (it only grows).  The
+// query is split into two int8 terms q^ = s1 * q_hi + s2 * q_lo (s1 = max|q_j| / 127, s2 = s1 / 254) by q8_split, the
+// same function in the pass and in the threshold kernel, so both see the same bits; each row is two exact int32 dp4a
+// sums and one fp32 combine, coarse = s_r * (s1 * D_hi + s2 * D_lo).  The bound is in filter_threshold_kernel.
+__device__ __forceinline__ int q8_round(float x) { return max(-127, min(127, __float2int_rn(x))); }
+// |x| as bits: unsigned order is the order of non-negative floats, NaN above +inf (the same maximum in any order)
+__device__ __forceinline__ uint32_t abs_bits(float x) { return __float_as_uint(x) & 0x7fffffffu; }
+__device__ __forceinline__ void q8_scales(uint32_t amax_bits, float& s1, float& s2) {
+    s1 = __fdiv_rn(__uint_as_float(amax_bits), 127.f);
+    s2 = __fdiv_rn(s1, 254.f);
+}
+// s1 == 0 (a zero query) divides by nothing; a non-finite query gives some q_hi / q_lo and its threshold takes every row
+__device__ __forceinline__ void q8_split(float v, float s1, float s2, int& hi, int& lo) {
+    hi = s1 > 0.f ? q8_round(__fdiv_rn(v, s1)) : 0;
+    const float res = fmaf(-s1, (float)hi, v);
+    lo = s2 > 0.f ? q8_round(__fdiv_rn(res, s2)) : 0;
+}
+
+// One warp per row: scale8[r], M8[r][0..ld8), and E raised to this row's ||r - r^|| (computed in double, rounded up).
+__global__ void __launch_bounds__(256)
+rows_to_i8_kernel(const float* __restrict__ M, int64_t n, int ld, int8_t* __restrict__ M8, int ld8, float* __restrict__ scale8,
+                  uint32_t* __restrict__ emax)
+{
+    const int lane = threadIdx.x & 31;
+    const int64_t nwarps = (int64_t)gridDim.x * (blockDim.x >> 5);
+    for (int64_t r = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); r < n; r += nwarps) {
+        const float4* row = reinterpret_cast<const float4*>(M + r * (int64_t)ld);
+        uint32_t mb = 0u;
+        for (int c = lane; c < ld / 4; c += 32) {
+            const float4 v = __ldg(row + c);
+            mb = max(max(mb, abs_bits(v.x)), max(abs_bits(v.y), max(abs_bits(v.z), abs_bits(v.w))));
+        }
+        mb = __reduce_max_sync(0xffffffffu, mb);
+        const float s = __fdiv_rn(__uint_as_float(mb), 127.f);
+        double e2 = 0.0;
+        for (int c = lane; c < ld8 / 4; c += 32) {
+            const float4 v = 4 * c < ld ? __ldg(row + c) : make_float4(0.f, 0.f, 0.f, 0.f);
+            const float x[4] = {v.x, v.y, v.z, v.w};
+            uint32_t packed = 0u;
+#pragma unroll
+            for (int t = 0; t < 4; ++t) {
+                const int qv = s > 0.f ? q8_round(__fdiv_rn(x[t], s)) : 0;
+                const double err = (double)x[t] - (double)s * (double)qv;          // s * qv is exact in double
+                e2 = fma(err, err, e2);
+                packed |= (uint32_t)(qv & 0xff) << (8 * t);
+            }
+            reinterpret_cast<uint32_t*>(M8 + r * (int64_t)ld8)[c] = packed;
+        }
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) e2 += __shfl_xor_sync(0xffffffffu, e2, o);
+        if (lane == 0) {
+            scale8[r] = s;
+            atomicMax(emax, __float_as_uint(__double2float_ru(sqrt(e2) * (1.0 + 1.0 / 1048576.0))));
+        }
+    }
+}
+
+// NC: 16-byte chunks (16 int8) of the shadow row per lane, c8 = ld8 / 16 <= 32 * NC.  The query's two int8 terms stay in
+// registers (2 * NC uint4).  No element is widened to fp32: per row 8 * NC dp4a per lane, two warp reductions, one combine.
+template <int CW, int NC>
+__global__ void __launch_bounds__((CW + 1) * 32, 1)
+gemv8_tma_kernel(const int8_t* __restrict__ M8, const float* __restrict__ scale8, int64_t n, int c8, int tile_rows, int stages,
+                 const float* __restrict__ q, int ld, float* __restrict__ scores, u64* __restrict__ gmax, int group_shift,
+                 const uint8_t* __restrict__ live)
+{
+    extern __shared__ __align__(128) unsigned char smem_raw[];
+    const uint32_t row_bytes = (uint32_t)c8 * 16u;
+    const uint32_t stage_bytes = (uint32_t)tile_rows * row_bytes;
+    uint64_t* full = reinterpret_cast<uint64_t*>(smem_raw + (size_t)stages * stage_bytes);
+    uint64_t* empty = full + stages;
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    if (threadIdx.x == 0) {
+        pdl_trigger();
+        for (int s = 0; s < stages; ++s) { mbar_init(&full[s], 1); mbar_init(&empty[s], CW); }
+        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    }
+    __syncthreads();
+
+    const int64_t ntiles = (n + tile_rows - 1) / tile_rows;
+    if (warp == CW) {
+        if (lane == 0) {
+            u64 policy;
+            asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(policy));
+            int s = 0; uint32_t phase = 0;
+            for (int64_t t = blockIdx.x; t < ntiles; t += gridDim.x) {
+                mbar_wait(&empty[s], phase ^ 1u);
+                const int64_t r0 = t * tile_rows;
+                const int64_t left = n - r0;
+                const uint32_t rows = left < tile_rows ? (uint32_t)left : (uint32_t)tile_rows;
+                const uint32_t bytes = rows * row_bytes;
+                mbar_arrive_expect_tx(&full[s], bytes);
+                bulk_g2s(smem_raw + (size_t)s * stage_bytes, reinterpret_cast<const unsigned char*>(M8) + (size_t)r0 * row_bytes,
+                         bytes, &full[s], policy);
+                if (++s == stages) { s = 0; phase ^= 1u; }
+            }
+        }
+    } else {
+        pdl_wait();                                   // the query is written by the previous kernel (see gemv_tma_kernel)
+        // lane l's chunks l, l + 32, ... hold query components [16c, 16c + 16): together the lanes read q once, so the
+        // warp's maximum of |q_j| needs no second pass
+        float qv[NC][16];
+        uint32_t mb = 0u;
+        const int ld4 = ld >> 2;
+#pragma unroll
+        for (int j = 0; j < NC; ++j)
+#pragma unroll
+            for (int t = 0; t < 4; ++t) {
+                const int c4 = 4 * (lane + 32 * j) + t;
+                const float4 v = c4 < ld4 ? __ldcg(reinterpret_cast<const float4*>(q) + c4) : make_float4(0.f, 0.f, 0.f, 0.f);
+                qv[j][4 * t] = v.x; qv[j][4 * t + 1] = v.y; qv[j][4 * t + 2] = v.z; qv[j][4 * t + 3] = v.w;
+                mb = max(max(mb, abs_bits(v.x)), max(abs_bits(v.y), max(abs_bits(v.z), abs_bits(v.w))));
+            }
+        float s1, s2;
+        q8_scales(__reduce_max_sync(0xffffffffu, mb), s1, s2);
+        uint32_t qh[NC][4], ql[NC][4];
+#pragma unroll
+        for (int j = 0; j < NC; ++j)
+#pragma unroll
+            for (int w = 0; w < 4; ++w) {
+                qh[j][w] = 0u; ql[j][w] = 0u;
+#pragma unroll
+                for (int b = 0; b < 4; ++b) {
+                    int hi, lo;
+                    q8_split(qv[j][4 * w + b], s1, s2, hi, lo);
+                    qh[j][w] |= (uint32_t)(hi & 0xff) << (8 * b);
+                    ql[j][w] |= (uint32_t)(lo & 0xff) << (8 * b);
+                }
+            }
+        int s = 0; uint32_t phase = 0;
+        for (int64_t t = blockIdx.x; t < ntiles; t += gridDim.x) {
+            const int64_t r0 = t * tile_rows;
+            const int64_t left = n - r0;
+            const int rows = left < tile_rows ? (int)left : tile_rows;
+            // scale and tombstone byte of the warp's rows of this tile (<= 64 / CW of them): lane i loads those of its
+            // i-th row before the wait, so a row costs no global-memory round trip of its own
+            const int ri = warp + CW * lane;
+            float sr_l = 0.f; uint32_t alive_l = 1u;
+            if (ri < rows) { sr_l = __ldg(scale8 + r0 + ri); if (live) alive_l = __ldg(live + r0 + ri); }
+            mbar_wait(&full[s], phase);
+            const uint4* tile = reinterpret_cast<const uint4*>(smem_raw + (size_t)s * stage_bytes);
+            u64 kmax = 0;
+            for (int r = warp, i = 0; r < rows; r += CW, ++i) {
+                const uint4* p = tile + (size_t)r * c8;
+                const uint32_t alive = __shfl_sync(0xffffffffu, alive_l, i);
+                const float sr = __shfl_sync(0xffffffffu, sr_l, i);
+                uint4 m[NC];
+#pragma unroll
+                for (int j = 0; j < NC; ++j) { const int c = lane + 32 * j; m[j] = c < c8 ? p[c] : make_uint4(0u, 0u, 0u, 0u); }
+                int dh = 0, dl = 0;                  // |sum| <= 3072 * 127^2 < 2^31: exact
+#pragma unroll
+                for (int j = 0; j < NC; ++j) {
+                    dh = __dp4a((int)m[j].x, (int)qh[j][0], dh); dl = __dp4a((int)m[j].x, (int)ql[j][0], dl);
+                    dh = __dp4a((int)m[j].y, (int)qh[j][1], dh); dl = __dp4a((int)m[j].y, (int)ql[j][1], dl);
+                    dh = __dp4a((int)m[j].z, (int)qh[j][2], dh); dl = __dp4a((int)m[j].z, (int)ql[j][2], dl);
+                    dh = __dp4a((int)m[j].w, (int)qh[j][3], dh); dl = __dp4a((int)m[j].w, (int)ql[j][3], dl);
+                }
+                dh = __reduce_add_sync(0xffffffffu, dh);
+                dl = __reduce_add_sync(0xffffffffu, dl);
+                float sc = sr * fmaf(s2, (float)dl, s1 * (float)dh);
+                if (!alive) sc = dead_score();
+                if (lane == 0) {
+                    scores[r0 + r] = sc;
+                    const u64 k0 = make_key(sc, (uint32_t)(r0 + r));
+                    kmax = k0 > kmax ? k0 : kmax;
+                }
+            }
+            __syncwarp();
+            if (lane == 0) {
+                mbar_arrive(&empty[s]);
+                if (kmax) atomicMax(&gmax[r0 >> group_shift], kmax);
+            }
+            if (++s == stages) { s = 0; phase ^= 1u; }
+        }
+    }
+}
+
 // One CTA.  state[0] = T as an ordered key word (f32_to_ordered): the rows with f32_to_ordered(coarse) >= T are the
-// candidates; T = 0 takes every row (no usable threshold: at most kk groups, a non-finite query or group maximum).
+// candidates; T = 0 takes every row (no usable threshold: at most kk groups, a non-finite query, bound or group maximum).
 // state[1] = 0 (the re-score kernel counts its rows there).
 // T = (kk-th largest group maximum) - 2 eps, rounded down: that maximum comes from kk distinct rows, so it is <= tau~.
+// e8 == null: the fp16 filter's bound, eps = eps_coef * ||q|| * max_row_norm + 1e-8.  e8 = the int8 shadow's E: the int8
+// filter's bound (DESIGN.md section 4, "K1f8"), with R = max_row_norm, R^ = R + E >= max ||r^||, q^ from q8_split,
+// eps = ||q|| E + ||q - q^|| R^ + ld 2^-23 ||q|| R (K1's fp32 sum) + 2^-21 (||s1 q_hi|| + ||s2 q_lo||) R^ (the combine's
+// five roundings) + 1e-8, times 1 + 2^-10 for the fp32 norms.
 constexpr int FT_THREADS = 1024;
 constexpr int FT_PER_THREAD = (int)(GROUPS_TARGET / FT_THREADS);
 __global__ void __launch_bounds__(FT_THREADS, 1)
 filter_threshold_kernel(const u64* __restrict__ gmax, int G, int kk, const float* __restrict__ q, int ld,
-                        float eps_coef, float max_row_norm, uint32_t* __restrict__ state)
+                        float eps_coef, float max_row_norm, const float* __restrict__ e8, uint32_t* __restrict__ state)
 {
     __shared__ uint32_t hist[256];
     __shared__ float red[FT_THREADS / 32];
+    __shared__ uint32_t amx[FT_THREADS / 32];
+    __shared__ double red8[3][FT_THREADS / 32];
     __shared__ uint32_t sh_prefix, sh_want;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     float ss = 0.f;
-    for (int i = tid; i < ld; i += FT_THREADS) { const float v = __ldcg(q + i); ss = fmaf(v, v, ss); }
+    uint32_t mb = 0u;
+    for (int i = tid; i < ld; i += FT_THREADS) { const float v = __ldcg(q + i); ss = fmaf(v, v, ss); mb = max(mb, abs_bits(v)); }
     ss = warp_sum(ss);
     if (lane == 0) red[warp] = ss;
+    mb = __reduce_max_sync(0xffffffffu, mb);
+    if (lane == 0) amx[warp] = mb;
     uint32_t v[FT_PER_THREAD];                         // high words of the group maxima (ordered coarse scores)
 #pragma unroll
     for (int j = 0; j < FT_PER_THREAD; ++j) { const int i = tid + j * FT_THREADS; v[j] = i < G ? (uint32_t)(__ldcg(gmax + i) >> 32) : 0u; }
     if (tid == 0) { sh_prefix = 0u; sh_want = (uint32_t)kk; }
     __syncthreads();
+    if (e8) {                                          // ||q - q^||^2, ||s1 q_hi||^2, ||s2 q_lo||^2 (double: exact enough)
+        for (int w = 0; w < FT_THREADS / 32; ++w) mb = max(mb, amx[w]);
+        float s1, s2;
+        q8_scales(mb, s1, s2);
+        double a[3] = {0.0, 0.0, 0.0};
+        for (int i = tid; i < ld; i += FT_THREADS) {
+            const float x = __ldcg(q + i);
+            int hi, lo;
+            q8_split(x, s1, s2, hi, lo);
+            const double th = (double)s1 * hi, tl = (double)s2 * lo, r = (double)x - th - tl;
+            a[0] = fma(r, r, a[0]); a[1] = fma(th, th, a[1]); a[2] = fma(tl, tl, a[2]);
+        }
+#pragma unroll
+        for (int c = 0; c < 3; ++c) {
+#pragma unroll
+            for (int o = 16; o > 0; o >>= 1) a[c] += __shfl_xor_sync(0xffffffffu, a[c], o);
+            if (lane == 0) red8[c][warp] = a[c];
+        }
+    }
     // kk-th largest of the G words: radix select, 8 bits per round from the top
     uint32_t mask = 0u;
     for (int shift = 24; shift >= 0; shift -= 8) {
@@ -543,8 +751,15 @@ filter_threshold_kernel(const u64* __restrict__ gmax, int G, int kk, const float
         const float qn = sqrtf(qq);
         const float tau = ordered_to_f32(sh_prefix);
         uint32_t T = 0u;
-        if (G > kk && isfinite(tau) && isfinite(qn)) {
-            const double eps = (double)eps_coef * (double)qn * (double)max_row_norm + 1e-8;
+        double eps = (double)eps_coef * (double)qn * (double)max_row_norm + 1e-8;
+        if (e8) {
+            double a[3] = {0.0, 0.0, 0.0};
+            for (int w = 0; w < FT_THREADS / 32; ++w) for (int c = 0; c < 3; ++c) a[c] += red8[c][w];
+            const double E = (double)__ldcg(e8), R = (double)max_row_norm, Rh = R + E;
+            eps = ((double)qn * E + sqrt(a[0]) * Rh + (double)ld * 0x1p-23 * (double)qn * R + 0x1p-21 * (sqrt(a[1]) + sqrt(a[2])) * Rh)
+                  * (1.0 + 0x1p-10) + 1e-8;
+        }
+        if (G > kk && isfinite(tau) && isfinite(qn) && isfinite(eps)) {
             float t = __double2float_rd((double)tau - 2.0 * eps);
             if (t == 0.f) t = -0.f;                         // f32_to_ordered(-0) < f32_to_ordered(+0): keep both zeros
             T = f32_to_ordered(t);
@@ -723,6 +938,8 @@ cudaError_t preload_gemv_kernels()
     SVSB_PRE((gemv_ldg_kernel<4, 3, 256>));
     SVSB_PRE((gemv16_tma_kernel<8, 1>)); SVSB_PRE((gemv16_tma_kernel<8, 2>)); SVSB_PRE((gemv16_tma_kernel<8, 4>));
     SVSB_PRE((gemv16_tma_kernel<8, 6>)); SVSB_PRE((gemv16_tma_kernel<8, 8>)); SVSB_PRE((gemv16_tma_kernel<8, 12>));
+    SVSB_PRE((gemv8_tma_kernel<8, 1>)); SVSB_PRE((gemv8_tma_kernel<8, 2>)); SVSB_PRE((gemv8_tma_kernel<8, 3>));
+    SVSB_PRE((gemv8_tma_kernel<8, 4>)); SVSB_PRE((gemv8_tma_kernel<8, 6>));
     SVSB_PRE(filter_threshold_kernel);
     SVSB_PRE((filter_rescore_kernel<2>)); SVSB_PRE((filter_rescore_kernel<6>)); SVSB_PRE((filter_rescore_kernel<12>));
     SVSB_PRE((filter_rescore_kernel<24>));
@@ -808,6 +1025,59 @@ cudaError_t launch_filter(cudaStream_t st, int device, const void* M16, int64_t 
 #undef SVSB_F16_CASE
 }
 
+cudaError_t launch_rows_to_i8(cudaStream_t st, int device, const float* M, int64_t n, int ld, void* M8, int ld8, float* scale8,
+                              float* emax)
+{
+    if (n <= 0) return cudaSuccess;
+    if (ld8 < ld || (ld8 & 15) || (ld & 3)) return cudaErrorInvalidValue;
+    int64_t blocks = (n + 7) / 8;
+    const int64_t cap = (int64_t)sm_count(device) * 16;
+    if (blocks > cap) blocks = cap;
+    rows_to_i8_kernel<<<(unsigned)blocks, 256, 0, st>>>(M, n, ld, static_cast<int8_t*>(M8), ld8, scale8, reinterpret_cast<uint32_t*>(emax));
+    count_launch();
+    return cudaGetLastError();
+}
+
+template <int CW, int NC>
+static cudaError_t run_filter8_inst(cudaStream_t st, int64_t grid, size_t smem, const void* M8, const float* scale8, int64_t n, int c8,
+                                    int tile_rows, int stages, const float* q, int ld, float* scores, u64* gmax, int group_shift,
+                                    const uint8_t* live)
+{
+    auto kern = gemv8_tma_kernel<CW, NC>;
+    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return e;
+    e = launch_kernel(kern, dim3((unsigned)grid), dim3((CW + 1) * 32), smem, st, static_cast<const int8_t*>(M8), scale8, n, c8,
+                      tile_rows, stages, q, ld, scores, gmax, group_shift, live);
+    count_launch();
+    return e != cudaSuccess ? e : cudaGetLastError();
+}
+
+cudaError_t launch_filter8(cudaStream_t st, int device, const void* M8, const float* scale8, int64_t n, int ld, int ld8,
+                           const float* q, float* scores, u64* gmax, int group_shift, int reserve_sms, const uint8_t* live)
+{
+    if (n <= 0) return cudaSuccess;
+    if (ld > FILTER_MAX_LD || ld8 < ld || (ld8 & 15)) return cudaErrorInvalidValue;
+    const int c8 = ld8 / 16;
+    const size_t row_bytes = (size_t)ld8;
+    // K1's ring: ~48 KB tiles x 3 stages (profiles/r01_tune_gemv.md)
+    int tile_rows = 64;
+    while (tile_rows > 1 && (size_t)tile_rows * row_bytes > 48 * 1024) tile_rows >>= 1;
+    const int stages = 3;
+    const size_t smem = (size_t)stages * tile_rows * row_bytes + (size_t)stages * 16 + 64;
+    const int64_t ntiles = (n + tile_rows - 1) / tile_rows;
+    int64_t grid = sm_count(device) - reserve_sms;
+    if (grid > ntiles) grid = ntiles;
+    if (grid < 1) grid = 1;
+#define SVSB_F8_CASE(NCV) \
+    return run_filter8_inst<8, NCV>(st, grid, smem, M8, scale8, n, c8, tile_rows, stages, q, ld, scores, gmax, group_shift, live)
+    if (c8 <= 32) SVSB_F8_CASE(1);
+    if (c8 <= 64) SVSB_F8_CASE(2);
+    if (c8 <= 96) SVSB_F8_CASE(3);
+    if (c8 <= 128) SVSB_F8_CASE(4);
+    SVSB_F8_CASE(6);
+#undef SVSB_F8_CASE
+}
+
 template <int NQ>
 static cudaError_t run_rescore_inst(cudaStream_t st, int device, const float* M, int64_t n, int d4, const float* q, float* scores,
                                     u64* gmax, int group_shift, const uint8_t* live, uint32_t* state)
@@ -822,14 +1092,14 @@ static cudaError_t run_rescore_inst(cudaStream_t st, int device, const float* M,
 }
 
 cudaError_t launch_filter_refine(cudaStream_t st, int device, const float* M, int64_t n, int ld, const float* q, float* scores,
-                                 u64* gmax, int group_shift, int kk, float eps_coef, float max_row_norm, const uint8_t* live,
-                                 uint32_t* state)
+                                 u64* gmax, int group_shift, int kk, float eps_coef, float max_row_norm, const float* e8,
+                                 const uint8_t* live, uint32_t* state)
 {
     if (n <= 0) return cudaSuccess;
     if (ld > FILTER_MAX_LD) return cudaErrorInvalidValue;
     const int64_t G = (n + ((int64_t)1 << group_shift) - 1) >> group_shift;
     if (G > GROUPS_TARGET) return cudaErrorInvalidValue;
-    filter_threshold_kernel<<<1, FT_THREADS, 0, st>>>(gmax, (int)G, kk, q, ld, eps_coef, max_row_norm, state);
+    filter_threshold_kernel<<<1, FT_THREADS, 0, st>>>(gmax, (int)G, kk, q, ld, eps_coef, max_row_norm, e8, state);
     count_launch();
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return e;

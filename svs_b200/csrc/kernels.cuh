@@ -57,9 +57,20 @@ cudaError_t launch_gemv(cudaStream_t st, int device, const float* M, int64_t n, 
 constexpr int FILTER_MAX_LD = 3072;
 cudaError_t launch_filter(cudaStream_t st, int device, const void* M16, int64_t n, int ld, int ld16, const float* q,
                           float* scores, u64* gmax, int group_shift, int reserve_sms = 0, const uint8_t* live = nullptr);
+// e8: null for the fp16 filter; the int8 shadow's error word E for launch_filter8's coarse scores (then the threshold
+// uses the int8 bound, gemv.cu filter_threshold_kernel).
 cudaError_t launch_filter_refine(cudaStream_t st, int device, const float* M, int64_t n, int ld, const float* q, float* scores,
-                                 u64* gmax, int group_shift, int kk, float eps_coef, float max_row_norm, const uint8_t* live,
-                                 uint32_t* state);
+                                 u64* gmax, int group_shift, int kk, float eps_coef, float max_row_norm, const float* e8,
+                                 const uint8_t* live, uint32_t* state);
+// K1f8, the int8 filter (gemv.cu, DESIGN.md section 4): launch_filter's contract over the int8 shadow M8[n][ld8] with
+// one scale per row (launch_rows_to_i8).  ld8 % 16 == 0, ld <= FILTER_MAX_LD.
+cudaError_t launch_filter8(cudaStream_t st, int device, const void* M8, const float* scale8, int64_t n, int ld, int ld8,
+                           const float* q, float* scores, u64* gmax, int group_shift, int reserve_sms = 0,
+                           const uint8_t* live = nullptr);
+// M8[r] = round(M[r] / scale8[r]) with scale8[r] = max|M[r][.]| / 127, zero padded; *emax (a float, only raised) >= every
+// converted row's ||M[r] - scale8[r] * M8[r]||.  ld % 4 == 0, ld8 % 16 == 0, ld8 >= ld.
+cudaError_t launch_rows_to_i8(cudaStream_t st, int device, const float* M, int64_t n, int ld, void* M8, int ld8, float* scale8,
+                              float* emax);
 // the bound's coefficient for d components (fp16 operands, fp32 accumulation; DESIGN.md section 6, step 4)
 inline float coarse_eps_coef(int d) {
     return 9.765625e-4f + 2.384185791015625e-7f + (float)d * (2.384185791015625e-7f + 1.1920928955078125e-7f);

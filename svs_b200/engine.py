@@ -311,6 +311,12 @@ class Engine:
         check(self._lib.svsb_bench_filter_stats(self._h, C.byref(f), C.byref(r)))
         return bool(f.value), int(r.value)
 
+    def bench_filter_route(self) -> int:
+        """Route of the last bench_run: 0 = fp32 similarity kernel, 16 = fp16 filter, 8 = int8 filter."""
+        r = C.c_int32()
+        check(self._lib.svsb_bench_filter_route(self._h, C.byref(r)))
+        return int(r.value)
+
     def batch_threshold_mode(self) -> int:
         """0 = verified statistical filter thresholds (default), 1 = proven-bound thresholds (see svsb200.h)."""
         rc = self._lib.svsb_batch_threshold_mode(self._h)
