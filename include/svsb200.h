@@ -235,7 +235,7 @@ int svsb_bench_last_result(svsb_t* e, int32_t k, float* out_scores, int64_t* out
  * Each process owns ONE device and the rows [global_row0, global_row0 + n) of the matrix, in scan order.
  * Two ways to do the one exchange step.  (1) Collective: the library does the compute on the caller's stream and
  * the caller (torch.distributed / NCCL) all-gathers one packed record per query per rank, then
- * svsb_enqueue_merge_records.  (2) Fused ("peer exchange", below): the kernels themselves move the records over
+ * svsb_enqueue_merge_records (k > 2048: svsb_enqueue_merge_sorted_records).  (2) Fused ("peer exchange", below): the kernels themselves move the records over
  * NVLink peer memory; the caller only exchanges 64-byte IPC handles once.  None of the svsb_enqueue_* / svsb_xchg_* /
  * svsb_*_peer entry points is re-entrant: one host thread drives a shard engine.
  * Record layout: 2*k+1 int64 words = [ keys (k, uint64: ordered score << 32 | ~global_row) |
@@ -244,7 +244,11 @@ int svsb_set_shard(svsb_t* e, int64_t global_row0);           /* call before svs
 /* flags: bit 0 = bracket the similarity kernel with timing events (svsb_kernel_time_collect); bit 1 = pipelined:
  * the similarity kernel runs on `stream` leaving one SM free and the one-CTA selection kernel runs on an engine-owned
  * side stream, so the selection of query i overlaps the similarity pass of query i+1 when consecutive calls
- * alternate `slot`.  With bit 1 the record is complete only after svsb_enqueue_join(e, stream). */
+ * alternate `slot`.  With bit 1 the record is complete only after svsb_enqueue_join(e, stream).
+ * Any k >= 1; the record has room for k entries and holds min(k, rows of this shard), sorted descending.  k > 2048
+ * (full rankings) sorts all of the shard's keys after the similarity pass; it always runs unpipelined on `stream`
+ * (bit 1 is ignored) and needs sort scratch of next_pow2(rows) keys in the slot's workspace (SVSB_E_NOMEM if that
+ * cannot be allocated; nothing is enqueued then).  Merge such records with svsb_enqueue_merge_sorted_records. */
 int svsb_enqueue_local_topk(svsb_t* e, void* stream, int32_t slot, const float* d_query, int32_t k,
                             int64_t* d_record, int32_t flags);
 /* Batched form: local top-k records of b device-resident queries d_Q[b][ld] (ld = d rounded up to 4, zero padded)
@@ -352,6 +356,14 @@ int svsb_enqueue_merge_records(svsb_t* e, void* stream, const int64_t* d_records
 int svsb_enqueue_merge_batch_records(svsb_t* e, void* stream, const int64_t* d_records, int32_t n_lists, int32_t batch,
                                      int32_t rec_cap, int32_t k, int32_t verify_k, float* d_out_scores, int64_t* d_out_ids,
                                      int32_t* d_out_counts);
+/* Any k: merge `n_lists` records of `cap` entries each, [n_lists][2*cap+1] words, every one sorted descending (what
+ * svsb_enqueue_local_topk writes; keys carry the global row, so keys are unique across ranks and ties break by ascending
+ * row).  Outputs: the top min(k, sum of counts) entries in d_out_scores[k] / d_out_ids[k] and that number in
+ * *d_out_count.  Each rank's record must hold everything of its shard that can reach the top k: cap >= min(k, rows of
+ * the largest shard).  A record whose count is negative or above cap (e.g. RECORD_TRUNCATED, bit 30, of the batch
+ * records) cannot be merged exactly: *d_out_count = -1 and nothing else is written.  Nothing is verified beyond that. */
+int svsb_enqueue_merge_sorted_records(svsb_t* e, void* stream, const int64_t* d_records, int32_t n_lists, int32_t cap, int32_t k,
+                                      float* d_out_scores, int64_t* d_out_ids, int32_t* d_out_count);
 /* ---- pairwise top pairs over the ranks' shards (the sharded form of svsb_top_pairs) --------------------------------
  * The result equals svsb_top_pairs of one single-device engine over the global matrix bit for bit: scores, ids, order.
  * Rank r runs its share of a static plan over the world's shards (the triangle of its own shard, rectangles against

@@ -104,6 +104,8 @@ SIGNATURES = {
     "svsb_enqueue_join": (C.c_int, [C.c_void_p, C.c_void_p]),
     "svsb_enqueue_merge_records": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32,
                                              C.c_void_p, C.c_void_p, C.c_void_p]),
+    "svsb_enqueue_merge_sorted_records": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32,
+                                                    C.c_void_p, C.c_void_p, C.c_void_p]),
     "svsb_pairs_export": (C.c_int, [C.c_void_p, c_float_p, c_i64_p, C.c_void_p]),
     "svsb_pairs_connect": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p]),
     "svsb_pairs_connect_local": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p]),
@@ -133,6 +135,7 @@ class EngineError(RuntimeError):
     def __init__(self, code: int, message: str):
         super().__init__(f"svs_b200 error {code}: {message}")
         self.code = code
+        self.message = message
 
 
 def load() -> C.CDLL:

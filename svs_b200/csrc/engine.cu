@@ -2132,9 +2132,10 @@ static int enqueue_local_topk_gen(svsb_engine* e, const std::shared_ptr<Generati
     if (!g) return fail(SVSB_E_NOT_LOADED, "no matrix resident");
     if (e->devs.size() != 1) return fail(SVSB_E_INVALID, "svsb_enqueue_local_topk: single-device engines only");
     if (slot < 0 || slot >= 8) return fail(SVSB_E_INVALID, "svsb_enqueue_local_topk: slot out of range (0..7)");
-    if (k < 1 || k > K_FAST_MAX) return fail(SVSB_E_INVALID, "svsb_enqueue_local_topk: 1 <= k <= 2048");
+    if (k < 1) return fail(SVSB_E_INVALID, "svsb_enqueue_local_topk: k must be positive");
     if (!d_query || !d_record) return fail(SVSB_E_INVALID, "svsb_enqueue_local_topk: NULL pointer");
-    const bool time_kernel = (flags & 1) != 0, pipelined = (flags & 2) != 0;
+    const bool big = k > K_FAST_MAX;                        // full sort of the shard's keys, unpipelined (bit 1 ignored)
+    const bool time_kernel = (flags & 1) != 0, pipelined = (flags & 2) != 0 && !big;
     const Shard& s = g->shards[0];
     cudaStream_t st = (cudaStream_t)stream;
     CU(cudaSetDevice(s.dev));
@@ -2145,8 +2146,10 @@ static int enqueue_local_topk_gen(svsb_engine* e, const std::shared_ptr<Generati
     if (!e->shard_ws[slot]) { e->shard_ws[slot].reset(new DevWs()); e->shard_ws[slot]->dev = s.dev; }
     DevWs& w = *e->shard_ws[slot];
     int rc;
+    const int64_t kl = std::min<int64_t>(k, s.n_live);
     if ((rc = w.ensure_rows(s.n)) != SVSB_OK) return rc;
-    if ((rc = w.ensure_out(K_FAST_MAX)) != SVSB_OK) return rc;
+    if ((rc = w.ensure_out(std::max<int64_t>(kl, K_FAST_MAX))) != SVSB_OK) return rc;
+    if (big && (rc = w.ensure_sort(s.n)) != SVSB_OK) return rc;
     if (pipelined) {
         if (!e->side_st) CU(cudaStreamCreateWithFlags(&e->side_st, cudaStreamNonBlocking));
         if (!w.ev) CU(cudaEventCreateWithFlags(&w.ev, cudaEventDisableTiming));
@@ -2171,8 +2174,12 @@ static int enqueue_local_topk_gen(svsb_engine* e, const std::shared_ptr<Generati
         CU(cudaStreamWaitEvent(e->side_st, w.ev, 0));
         sel_st = e->side_st;
     }
-    CU(launch_select(sel_st, w.scores, s.n, w.gmax, shift, (int)std::min<int64_t>(k, s.n_live), s.ids, s.row0, w.cand, w.cand_cap,
-                     r.keys(0), w.out_scores, r.ids(0), r.count(0)));
+    if (big)
+        CU(launch_fullsort_topk(st, w.scores, s.n, w.gmax, shift, kl, s.ids, s.row0, w.sortbuf, r.keys(0), w.out_scores, r.ids(0),
+                                r.count(0)));
+    else
+        CU(launch_select(sel_st, w.scores, s.n, w.gmax, shift, (int)kl, s.ids, s.row0, w.cand, w.cand_cap,
+                         r.keys(0), w.out_scores, r.ids(0), r.count(0)));
     w.gmax_dirty = false;
     if (pipelined) { CU(cudaEventRecord(w.ev_sel, e->side_st)); e->sel_pending[slot] = 1; }
     return SVSB_OK;
@@ -2887,6 +2894,18 @@ static int enqueue_merge_records(svsb_t* e, void* stream, const int64_t* d_recor
 extern "C" int svsb_enqueue_merge_records(svsb_t* e, void* stream, const int64_t* d_records, int32_t n_lists, int32_t batch,
                                           int32_t k, float* d_out_scores, int64_t* d_out_ids, int32_t* d_out_counts) {
     return enqueue_merge_records(e, stream, d_records, n_lists, batch, k, k, d_out_scores, d_out_ids, d_out_counts, -1, "svsb_enqueue_merge_records");
+}
+extern "C" int svsb_enqueue_merge_sorted_records(svsb_t* e, void* stream, const int64_t* d_records, int32_t n_lists, int32_t cap,
+                                                 int32_t k, float* d_out_scores, int64_t* d_out_ids, int32_t* d_out_count) {
+    if (!e) return fail(SVSB_E_INVALID, "engine is NULL");
+    if (n_lists < 1 || cap < 1 || k < 1) return fail(SVSB_E_INVALID, "svsb_enqueue_merge_sorted_records: n_lists, cap and k must be positive");
+    if (!d_records || !d_out_scores || !d_out_ids || !d_out_count)
+        return fail(SVSB_E_INVALID, "svsb_enqueue_merge_sorted_records: NULL pointer");
+    CU(cudaSetDevice(e->devs[0]));
+    const RecordView recs{const_cast<int64_t*>(d_records), cap};           // read only
+    CU(launch_merge_sorted_big((cudaStream_t)stream, recs.keys(0), recs.ids(0), recs.count(0), n_lists, cap, recs.words(),
+                               2 * recs.words(), k, d_out_scores, d_out_ids, d_out_count));
+    return SVSB_OK;
 }
 extern "C" int svsb_enqueue_merge_batch_records(svsb_t* e, void* stream, const int64_t* d_records, int32_t n_lists, int32_t batch,
                                                 int32_t rec_cap, int32_t k, int32_t verify_k, float* d_out_scores, int64_t* d_out_ids,

@@ -175,7 +175,12 @@ struct svsb_workspace {
     int ensure_sort(int64_t n) {
         cudaSetDevice(dev);
         int64_t need = next_pow2(n); if (need < 2048) need = 2048;
-        if (need > sort_cap) { if (sortbuf) cudaFree(sortbuf); sortbuf = nullptr; CU(cudaMalloc(&sortbuf, (size_t)need * 8)); sort_cap = need; }
+        if (need > sort_cap) {
+            if (sortbuf) cudaFree(sortbuf);
+            sortbuf = nullptr; sort_cap = 0;                // a failed allocation leaves no capacity behind
+            CU(cudaMalloc(&sortbuf, (size_t)need * 8));
+            sort_cap = need;
+        }
         return SVSB_OK;
     }
     int ensure_merge_scratch(int64_t entries) {

@@ -131,9 +131,12 @@ cudaError_t launch_merge_ex(cudaStream_t st, const u64* keys, const int64_t* ids
                             int verify_k = -1,    // >= 0: count words are [count, ver] pairs, see MergeLayout (select.cu)
                             const int* abort_flag = nullptr);   // device word; non-zero: every out_count = MERGE_WINDOW_TIMED_OUT
 
-// Any k: merge n_lists lists, each SORTED descending with unique keys (list l at keys / ids [l * stride ..), counts[l] valid).
+// Any k: merge n_lists lists, each SORTED descending with unique keys.  List l holds counts[l * count_stride] <= cap
+// entries at keys / ids [l * list_stride ..) (strides in elements of the respective array).  out_count = min(k, sum of
+// counts), or -1 when a count is negative or above cap (a truncated list: the answer is unknown, nothing is written).
 cudaError_t launch_merge_sorted_big(cudaStream_t st, const u64* keys, const int64_t* ids, const int32_t* counts, int n_lists,
-                                    int64_t stride, int64_t k, float* out_scores, int64_t* out_ids, int32_t* out_count);
+                                    int64_t cap, int64_t list_stride, int64_t count_stride, int64_t k, float* out_scores,
+                                    int64_t* out_ids, int32_t* out_count);
 
 // ---- peer exchange (select.cu): candidate records pushed into every rank's window, merged after a flag wait ----
 // A window holds `slots` x `world` records of rec_words = 2*cap + 2 u64 words: [keys(cap) | ids(cap) | count | pad],

@@ -512,7 +512,7 @@ static int multi_query_big(svsb_engine* e, const std::shared_ptr<Generation>& g,
         if ((rc = copy_to_root(m, i, m->g_ids + (int64_t)i * kk, w.out_ids, (size_t)kl * 8, rst)) != SVSB_OK) return rc;
         if ((rc = copy_to_root(m, i, m->g_counts + i, w.out_count, 4, rst)) != SVSB_OK) return rc;
     }
-    CU(launch_merge_sorted_big(rst, m->g_keys, m->g_ids, m->g_counts, nd, kk, kk, m->m_scores, m->m_ids, m->m_count));
+    CU(launch_merge_sorted_big(rst, m->g_keys, m->g_ids, m->g_counts, nd, kk, kk, 1, kk, m->m_scores, m->m_ids, m->m_count));
     CU(cudaMemcpyAsync(m->h_big_scores, m->m_scores, (size_t)kk * 4, cudaMemcpyDeviceToHost, rst));
     CU(cudaMemcpyAsync(m->h_big_ids, m->m_ids, (size_t)kk * 8, cudaMemcpyDeviceToHost, rst));
     CU(cudaMemcpyAsync(m->h_big_count, m->m_count, 4, cudaMemcpyDeviceToHost, rst));

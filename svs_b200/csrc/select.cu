@@ -924,41 +924,54 @@ merge_window_kernel(const u64* slot_base, const u64* flags, u64 seq, int world, 
 // matrix): every list is sorted descending and keys are unique, so an element's global rank is its index in its own
 // list plus, per other list, the number of greater keys (one binary search each, lists are L2-resident).  Elements of
 // rank < k go straight to the output; no sort, any k.
+// List l holds at most cap entries at keys / ids [l * list_stride ..); its count is counts[l * count_stride].  A count
+// outside [0, cap] (negative, or RECORD_TRUNCATED set: the list lost entries) makes the whole merge unanswerable: the
+// kernel writes nothing but out_count = -1, since a missing entry could belong anywhere in the top k.
 // ---------------------------------------------------------------------------------------------
 __global__ void merge_sorted_big_kernel(const u64* __restrict__ keys, const int64_t* __restrict__ ids, const int32_t* __restrict__ counts,
-                                        int n_lists, int64_t stride, int64_t k, float* __restrict__ out_scores,
-                                        int64_t* __restrict__ out_ids, int32_t* __restrict__ out_count)
+                                        int n_lists, int64_t cap, int64_t list_stride, int64_t count_stride, int64_t k,
+                                        float* __restrict__ out_scores, int64_t* __restrict__ out_ids, int32_t* __restrict__ out_count)
 {
     int64_t total = 0;
-    for (int l = 0; l < n_lists; ++l) total += min((int64_t)max(counts[l], 0), stride);
+    for (int l = 0; l < n_lists; ++l) {
+        const int32_t c = counts[l * count_stride];
+        if (c < 0 || c > cap) {
+            if (blockIdx.x == 0 && threadIdx.x == 0) *out_count = -1;
+            return;
+        }
+        total += c;
+    }
     const int64_t kk = k < total ? k : total;
-    const int64_t span = (int64_t)n_lists * stride;
+    const int64_t span = (int64_t)n_lists * cap;
     const int64_t step = (int64_t)gridDim.x * blockDim.x;
     for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < span; e += step) {
-        const int l = (int)(e / stride);
-        const int64_t p = e - (int64_t)l * stride;
-        if (p >= min((int64_t)max(counts[l], 0), stride)) continue;
-        const u64 key = keys[e];
+        const int l = (int)(e / cap);
+        const int64_t p = e - (int64_t)l * cap;
+        if (p >= counts[l * count_stride]) continue;
+        const int64_t at = (int64_t)l * list_stride + p;
+        const u64 key = keys[at];
         int64_t rank = p;
         for (int m = 0; m < n_lists && rank < kk; ++m) {
             if (m == l) continue;
-            const u64* lm = keys + (int64_t)m * stride;
-            int64_t lo = 0, hi = min((int64_t)max(counts[m], 0), stride);          // first position whose key is < mine
+            const u64* lm = keys + (int64_t)m * list_stride;
+            int64_t lo = 0, hi = counts[m * count_stride];                          // first position whose key is < mine
             while (lo < hi) { const int64_t mid = (lo + hi) >> 1; if (lm[mid] > key) lo = mid + 1; else hi = mid; }
             rank += lo;
         }
-        if (rank < kk) { out_scores[rank] = key_score(key); out_ids[rank] = ids[e]; }
+        if (rank < kk) { out_scores[rank] = key_score(key); out_ids[rank] = ids[at]; }
     }
     if (blockIdx.x == 0 && threadIdx.x == 0) *out_count = (int32_t)kk;
 }
 
 cudaError_t launch_merge_sorted_big(cudaStream_t st, const u64* keys, const int64_t* ids, const int32_t* counts, int n_lists,
-                                    int64_t stride, int64_t k, float* out_scores, int64_t* out_ids, int32_t* out_count)
+                                    int64_t cap, int64_t list_stride, int64_t count_stride, int64_t k, float* out_scores,
+                                    int64_t* out_ids, int32_t* out_count)
 {
-    if (n_lists < 1 || stride < 1 || k < 1) return cudaErrorInvalidValue;
-    const int64_t span = (int64_t)n_lists * stride;
+    if (n_lists < 1 || cap < 1 || list_stride < cap || count_stride < 1 || k < 1) return cudaErrorInvalidValue;
+    const int64_t span = (int64_t)n_lists * cap;
     const unsigned blocks = (unsigned)std::min<int64_t>((span + 255) / 256, 148 * 8);
-    merge_sorted_big_kernel<<<blocks, 256, 0, st>>>(keys, ids, counts, n_lists, stride, k, out_scores, out_ids, out_count);
+    merge_sorted_big_kernel<<<blocks, 256, 0, st>>>(keys, ids, counts, n_lists, cap, list_stride, count_stride, k, out_scores,
+                                                    out_ids, out_count);
     count_launch();
     return cudaGetLastError();
 }

@@ -11,6 +11,11 @@ their embeddings.ids.  A query is answered by
 No reduction over scores is needed: rows are independent (splitting D instead would need an all-reduce
 of N floats).
 
+k > 2048 (up to the full ranking n = N) takes its own path under either exchange: every rank fully sorts its shard's
+keys into one record of cap = min(k, ceil(N / world)) entries -- no shard holds more rows, so every record is complete
+--, the ranks agree on the outcome of that local phase, all-gather the records and rank-merge the sorted lists on every
+rank (include/svsb200.h svsb_enqueue_merge_sorted_records).
+
 Single queries do not call a collective at all by default (`exchange="peer"`): steps 2 and 3 are fused into the
 kernels over NVLink / NVSwitch peer memory -- the selection kernel's epilogue stores its record into every rank's
 gather window and publishes it with a release store, and each rank's merge kernel waits for the `world` flags of
@@ -36,7 +41,7 @@ from typing import List, Optional, Tuple
 
 import numpy as np
 
-from ._lib import SVSB_E_CUDA, EngineError
+from ._lib import K_FAST_MAX, SVSB_E_CUDA, SVSB_E_NOMEM, EngineError
 
 MICRO_BATCH = 16
 TIME_EVERY = 8        # bracket one similarity launch in 8 with timing events (two records cost ~5 us of stream time)
@@ -110,7 +115,7 @@ class CudaShardBackend:
     def enqueue_local(self, query_row, k: int, record_row, time_kernel: bool = False, seq: int = 0) -> None:
         """Similarity on the current stream, selection pipelined on the engine's side stream (slots alternate with
         `seq`, so the selection of one query overlaps the similarity pass of the next).  Call join() before the
-        records are consumed."""
+        records are consumed.  k > 2048: the shard's keys are fully sorted, unpipelined, on the current stream."""
         st = self.torch.cuda.current_stream(self.device).cuda_stream
         self._check(self._lib.svsb_enqueue_local_topk(self.engine._h, C.c_void_p(st), seq & 1, C.c_void_p(query_row.data_ptr()),
                                                       k, C.c_void_p(record_row.data_ptr()), (1 if time_kernel else 0) | 2))
@@ -248,6 +253,14 @@ class CudaShardBackend:
                                                          n_lists, batch, k, C.c_void_p(out_scores.data_ptr()),
                                                          C.c_void_p(out_ids.data_ptr()), C.c_void_p(out_counts.data_ptr())))
 
+    def enqueue_merge_sorted(self, gathered, n_lists: int, cap: int, k: int, out_scores, out_ids, out_count) -> None:
+        """Any k: rank-merge n_lists sorted records of cap entries (gathered: [n_lists][2 * cap + 1]) into out_scores[k],
+        out_ids[k], out_count[1] (-1: a record was truncated)."""
+        st = self.torch.cuda.current_stream(self.device).cuda_stream
+        self._check(self._lib.svsb_enqueue_merge_sorted_records(self.engine._h, C.c_void_p(st), C.c_void_p(gathered.data_ptr()),
+                                                                n_lists, cap, k, C.c_void_p(out_scores.data_ptr()),
+                                                                C.c_void_p(out_ids.data_ptr()), C.c_void_p(out_count.data_ptr())))
+
     # -- pairwise top pairs over the ranks' shards (include/svsb200.h svsb_pairs_*) ---------------------------------
     def pairs_export(self) -> Tuple[bytes, int, str, float]:
         """Pin the resident generation and describe it for the peers: (descriptor, status, message, max_dev).  A refusal
@@ -332,6 +345,7 @@ class ShardedRetriever:
         self.local_rows = 0
         self._queries = None
         self._bufs = {}
+        self._big = None                 # (cap, record, gathered records, outputs) of the large-k path: one set at a time
         self._plans = {}
         self._epoch = 0
         self.last_fallbacks = 0
@@ -343,6 +357,7 @@ class ShardedRetriever:
     def load_synthetic(self, n: int, d: int, seed: int = 0, id0: int = 0, id_step: int = 1) -> None:
         self.n, self.d = n, d
         self._epoch += 1
+        self._big = None
         self.row0, self.local_rows = partition(n, self.world, self.rank)
         self.backend.set_shard(self.row0)
         self.backend.load_synthetic(self.local_rows, d, seed, id0, id_step)
@@ -351,6 +366,7 @@ class ShardedRetriever:
         """Every rank passes the same global (n, d) matrix / ids and keeps only its slice (tests, small KBs)."""
         self.n, self.d = rows.shape
         self._epoch += 1
+        self._big = None
         self.row0, self.local_rows = partition(self.n, self.world, self.rank)
         self.backend.set_shard(self.row0)
         sl = slice(self.row0, self.row0 + self.local_rows)
@@ -530,9 +546,9 @@ class ShardedRetriever:
             raise ValueError(f"shapes ({self.n},{self.d if self.n else 0}) and {Q.shape} not aligned")
         if n <= 0 or Q.shape[0] == 0:
             return (np.zeros((Q.shape[0], 0), np.float32), np.zeros((Q.shape[0], 0), np.int64), np.zeros(Q.shape[0], np.int32))
-        if n > 2048 and self.n > 2048:
-            raise NotImplementedError("n > 2048 is not supported by the sharded path")
-        k = min(int(n), 2048, self.n)                               # get_top_k clips n to the row count (util.py:198-199)
+        k = min(int(n), self.n)                                     # get_top_k clips n to the row count (util.py:198-199)
+        if k > K_FAST_MAX:
+            return self._retrieve_many_big(Q, k)
         o_s, o_i, o_c = self._batch(self.backend.device_queries(Q), k)
         cnt = o_c.cpu().numpy()                                     # synchronises the stream
         s, i = o_s.cpu().numpy(), o_i.cpu().numpy()
@@ -548,7 +564,8 @@ class ShardedRetriever:
     def retrieve_many_pinned(self, queries, n: int) -> Tuple[np.ndarray, np.ndarray, np.ndarray]:
         """retrieve_many_arrays without pageable staging: `queries` is a PINNED torch tensor (b, d) float32 (torch
         `pin_memory()`), DMA'd to the device as is; the results come back into page-locked buffers owned by this object and
-        are returned as NumPy views of them -- valid until the next call.  Same answers as retrieve_many_arrays."""
+        are returned as NumPy views of them -- valid until the next call.  Same answers as retrieve_many_arrays.  Above
+        2048 results per query the answers come back in new arrays instead, one query at a time."""
         t = self.backend.torch
         if not (isinstance(queries, t.Tensor) and queries.is_pinned() and queries.dtype == t.float32 and queries.dim() == 2
                 and queries.is_contiguous()):
@@ -558,9 +575,9 @@ class ShardedRetriever:
         b = queries.shape[0]
         if n <= 0 or b == 0:
             return (np.zeros((b, 0), np.float32), np.zeros((b, 0), np.int64), np.zeros(b, np.int32))
-        if n > 2048 and self.n > 2048:
-            raise NotImplementedError("n > 2048 is not supported by the sharded path")
-        k = min(int(n), 2048, self.n)
+        k = min(int(n), self.n)
+        if k > K_FAST_MAX:
+            return self._retrieve_many_big(queries.numpy(), k)
         ld = (self.d + 3) & ~3
         dq = queries.to(self.backend.device, non_blocking=True)
         if ld != self.d:
@@ -596,9 +613,9 @@ class ShardedRetriever:
             raise ValueError(f"shapes ({self.n},{self.d if self.n else 0}) and ({q.shape[0]},) not aligned")
         if n <= 0:
             return np.zeros(0, np.float32), np.zeros(0, np.int64)
-        k = min(int(n), 2048, self.n)                               # get_top_k clips n to the row count (util.py:198-199)
-        if n > 2048 and self.n > 2048:
-            raise NotImplementedError("n > 2048 is not supported by the sharded path")
+        k = min(int(n), self.n)                                     # get_top_k clips n to the row count (util.py:198-199)
+        if k > K_FAST_MAX:
+            return self._retrieve_big(q, k)
         if self.exchange == "peer":
             self._ensure_window()
             return self.backend.query_peer(q, k)                   # one synchronous C call, result written to host
@@ -613,10 +630,8 @@ class ShardedRetriever:
         q = np.ascontiguousarray(query_vec, dtype=np.float32)
         if q.ndim != 1 or q.shape[0] != self.d or self.n == 0:
             raise ValueError(f"shapes ({self.n},{self.d if self.n else 0}) and ({q.shape[0]},) not aligned")
-        if n > 2048 and self.n > 2048:
-            raise NotImplementedError("n > 2048 is not supported by the sharded path")
-        k = min(int(n), 2048, self.n)
-        if k <= 0 or self.exchange != "peer":
+        k = min(int(n), self.n)
+        if k <= 0 or k > K_FAST_MAX or self.exchange != "peer":
             return ("done", self.retrieve_arrays(q, n))           # nothing to overlap: answered synchronously
         self._ensure_window()
         return ("ticket", self.backend.query_peer_submit(q, k), k)
@@ -631,6 +646,48 @@ class ShardedRetriever:
         """The reference's superheavy() result, on every rank: host query in, host list out."""
         s, i = self.retrieve_arrays(query_vec, n)
         return [(float(a), int(b)) for a, b in zip(s, i)]
+
+    # -- k > 2048: full sort per shard, one all-gather of the sorted records, rank merge on every rank ----------------
+    def _big_buffers(self, cap: int):
+        """The large-k path's one buffer set, replaced when cap changes: this rank's record, the gathered records and
+        outputs of world * cap >= k entries.  A full ranking of 10M rows on 8 ranks gathers ~160 MB per rank: it is
+        not kept once for every k ever asked."""
+        if self._big is None or self._big[0] != cap:
+            self._big = None                                       # the old set goes before the new one is allocated
+            be = self.backend
+            self._big = (cap, be.new_records(1, cap), be.new_records(self.world, cap), be.new_outputs(1, self.world * cap))
+        return self._big[1:]
+
+    def _retrieve_big(self, q: np.ndarray, k: int) -> Tuple[np.ndarray, np.ndarray]:
+        """superheavy() for 2048 < k <= N, on every rank, through the collective under either exchange (the peer
+        windows are sized for k <= 2048)."""
+        cap = min(k, -(-self.n // self.world))                     # rows of the largest shard (partition) bound every record
+        try:
+            rec, gath, (o_s, o_i, o_c) = self._big_buffers(cap)
+            self.backend.enqueue_local(self.backend.device_queries(q[None, :])[0], cap, rec[0])
+            self.backend.join()
+            outcome = (0, "")
+        except EngineError as ex:
+            outcome = (ex.code, ex.message)
+        except (MemoryError, RuntimeError) as ex:                  # a buffer the framework could not allocate
+            outcome = (SVSB_E_NOMEM, f"sharded retrieve, n = {k}: {ex}")
+        # every rank learns every rank's outcome before the collective: one refusal raises the same error everywhere
+        # instead of leaving the others blocked in the all-gather
+        self._agree(self._all_gather_object(outcome))
+        self.dist.all_gather_into_tensor(gath.view(-1), rec.view(-1), group=self.group)
+        self.backend.enqueue_merge_sorted(gath, self.world, cap, k, o_s[0], o_i[0], o_c[0])
+        cnt = int(o_c[0].item())                                   # synchronises the stream
+        if cnt != k:
+            raise EngineError(SVSB_E_CUDA, f"sharded retrieve: the large-k merge returned {cnt} of {k} entries")
+        return o_s[0, :cnt].cpu().numpy(), o_i[0, :cnt].cpu().numpy()
+
+    def _retrieve_many_big(self, Q: np.ndarray, k: int) -> Tuple[np.ndarray, np.ndarray, np.ndarray]:
+        """retrieve_many_arrays for k > 2048: one large-k retrieve per query into (b, k) outputs."""
+        s, i = np.zeros((Q.shape[0], k), np.float32), np.zeros((Q.shape[0], k), np.int64)
+        for j in range(Q.shape[0]):
+            s[j], i[j] = self._retrieve_big(np.ascontiguousarray(Q[j]), k)
+        self.last_fallbacks, self._last_counts = 0, None
+        return s, i, np.full(Q.shape[0], k, np.int32)
 
     # -- pairwise top pairs ---------------------------------------------------------------------------
     @staticmethod
@@ -699,4 +756,5 @@ class ShardedRetriever:
             if self.world > 1:
                 self.dist.barrier(group=self.group)
             self._peer_ready = self._batch_peer_ready = False
+        self._big = None
         self.backend.close()
