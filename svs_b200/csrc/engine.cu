@@ -595,6 +595,8 @@ int shadow_sync(const Shard& s, int ld, int64_t fresh_from, int create, cudaStre
     if (ld > FILTER_MAX_LD || (!b->M8 && create != 1)) return SVSB_OK;
     const int ld8 = (ld + 15) & ~15;
     if (!b->M8) {                                        // +25 % of the matrix: only with an eighth of the device still free
+        // [int8 rows | f32 scales | 16-byte E word]: the int8 filter copies a partial last tile's scales in 16-byte units,
+        // up to 12 bytes past scale cap_rows - 1, which the E word keeps inside this allocation (gemv8_tma_kernel)
         const size_t rows8 = (size_t)b->cap_rows * ld8, bytes = rows8 + (size_t)b->cap_rows * 4 + 16;
         size_t fr = 0, tot = 0;
         if (cudaMemGetInfo(&fr, &tot) != cudaSuccess || fr < bytes + tot / 8) { (void)cudaGetLastError(); return SVSB_OK; }

@@ -542,8 +542,34 @@ rows_to_i8_kernel(const float* __restrict__ M, int64_t n, int ld, int8_t* __rest
     }
 }
 
+// One row's two dp4a sums over the lane's NC chunks, each split into two partial accumulators (x, y words and z, w
+// words): integer sums are exact in any order, so the split halves the dependent chain without changing a bit.
+template <int NC>
+__device__ __forceinline__ void dot8(const uint4 (&m)[NC], const uint32_t (&qh)[NC][4], const uint32_t (&ql)[NC][4], int& dh, int& dl) {
+    int h0 = 0, h1 = 0, l0 = 0, l1 = 0;                      // |sum| <= 3072 * 127^2 < 2^31: exact
+#pragma unroll
+    for (int j = 0; j < NC; ++j) {
+        h0 = __dp4a((int)m[j].x, (int)qh[j][0], h0); l0 = __dp4a((int)m[j].x, (int)ql[j][0], l0);
+        h1 = __dp4a((int)m[j].z, (int)qh[j][2], h1); l1 = __dp4a((int)m[j].z, (int)ql[j][2], l1);
+        h0 = __dp4a((int)m[j].y, (int)qh[j][1], h0); l0 = __dp4a((int)m[j].y, (int)ql[j][1], l0);
+        h1 = __dp4a((int)m[j].w, (int)qh[j][3], h1); l1 = __dp4a((int)m[j].w, (int)ql[j][3], l1);
+    }
+    dh = h0 + h1; dl = l0 + l1;
+}
+
+// Shared memory of gemv8_tma_kernel behind the ring of `stages` tiles: per stage a side slot (the tile's row scales,
+// then its tombstone bytes), then the query's two int8 terms, the consumer warps' maxima of |q_j| and the barriers.
+// tile_rows % 16 == 0 keeps every part 16-byte aligned.
+__host__ __device__ constexpr size_t filter8_side_bytes(int tile_rows) { return (size_t)tile_rows * 5; }
+__host__ __device__ constexpr size_t filter8_smem_bytes(int tile_rows, int stages, int ld8) {
+    return (size_t)stages * ((size_t)tile_rows * ld8 + filter8_side_bytes(tile_rows)) + 2 * (size_t)ld8 + 64 + (size_t)stages * 16;
+}
+
 // NC: 16-byte chunks (16 int8) of the shadow row per lane, c8 = ld8 / 16 <= 32 * NC.  The query's two int8 terms stay in
 // registers (2 * NC uint4).  No element is widened to fp32: per row 8 * NC dp4a per lane, two warp reductions, one combine.
+// The producer stages each tile's row scales (and tombstone bytes) through the ring with the rows, so the consumers'
+// tile loop reads shared memory only; a consumer warp works on two rows of a tile at once (w and w + CW) to overlap
+// their shared-memory loads, dp4a chains and reductions.
 template <int CW, int NC>
 __global__ void __launch_bounds__((CW + 1) * 32, 1)
 gemv8_tma_kernel(const int8_t* __restrict__ M8, const float* __restrict__ scale8, int64_t n, int c8, int tile_rows, int stages,
@@ -553,7 +579,12 @@ gemv8_tma_kernel(const int8_t* __restrict__ M8, const float* __restrict__ scale8
     extern __shared__ __align__(128) unsigned char smem_raw[];
     const uint32_t row_bytes = (uint32_t)c8 * 16u;
     const uint32_t stage_bytes = (uint32_t)tile_rows * row_bytes;
-    uint64_t* full = reinterpret_cast<uint64_t*>(smem_raw + (size_t)stages * stage_bytes);
+    const uint32_t side_bytes = (uint32_t)filter8_side_bytes(tile_rows);
+    unsigned char* side = smem_raw + (size_t)stages * stage_bytes;
+    uint32_t* sqh = reinterpret_cast<uint32_t*>(side + (size_t)stages * side_bytes);   // c8 * 4 words each
+    uint32_t* sql = sqh + 4 * c8;
+    uint32_t* samax = sql + 4 * c8;                                                      // CW <= 16 words
+    uint64_t* full = reinterpret_cast<uint64_t*>(samax + 16);
     uint64_t* empty = full + stages;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     if (threadIdx.x == 0) {
@@ -575,80 +606,112 @@ gemv8_tma_kernel(const int8_t* __restrict__ M8, const float* __restrict__ scale8
                 const int64_t left = n - r0;
                 const uint32_t rows = left < tile_rows ? (uint32_t)left : (uint32_t)tile_rows;
                 const uint32_t bytes = rows * row_bytes;
-                mbar_arrive_expect_tx(&full[s], bytes);
+                // bulk copies move multiples of 16 bytes: the scales are read up to round_up(n, 4) (inside the shadow's
+                // allocation: its E word follows them), the tombstone bytes up to round_up(n, 16) (svsb_apply_mutations
+                // allocates that much); the rounded tails land in the side slot and are never read
+                const uint32_t sbytes = ((rows + 3u) & ~3u) * 4u, lbytes = live ? (rows + 15u) & ~15u : 0u;
+                unsigned char* sd = side + (size_t)s * side_bytes;
+                mbar_arrive_expect_tx(&full[s], bytes + sbytes + lbytes);
                 bulk_g2s(smem_raw + (size_t)s * stage_bytes, reinterpret_cast<const unsigned char*>(M8) + (size_t)r0 * row_bytes,
                          bytes, &full[s], policy);
+                bulk_g2s(sd, scale8 + r0, sbytes, &full[s], policy);
+                if (live) bulk_g2s(sd + 4 * tile_rows, live + r0, lbytes, &full[s], policy);
                 if (++s == stages) { s = 0; phase ^= 1u; }
             }
         }
     } else {
+        // The query's split, once per CTA: consumer thread i converts words i, i + 32 CW, ... (4 components each) of
+        // the c8 * 4; the maximum of |q_j| is reduced over the consumer warps first (a named barrier: the producer
+        // does not join).  q8_scales / q8_split are the threshold kernel's, so both see the same bits.
         pdl_wait();                                   // the query is written by the previous kernel (see gemv_tma_kernel)
-        // lane l's chunks l, l + 32, ... hold query components [16c, 16c + 16): together the lanes read q once, so the
-        // warp's maximum of |q_j| needs no second pass
-        float qv[NC][16];
+        constexpr int QW = (128 * NC + 32 * CW - 1) / (32 * CW);      // words per consumer thread
+        const int ct = threadIdx.x, nw = 4 * c8, ld4 = ld >> 2;
+        float4 qv[QW];
         uint32_t mb = 0u;
-        const int ld4 = ld >> 2;
 #pragma unroll
-        for (int j = 0; j < NC; ++j)
+        for (int i = 0; i < QW; ++i) {
+            const int w = ct + 32 * CW * i;
+            qv[i] = w < ld4 ? __ldcg(reinterpret_cast<const float4*>(q) + w) : make_float4(0.f, 0.f, 0.f, 0.f);
+            mb = max(max(mb, abs_bits(qv[i].x)), max(abs_bits(qv[i].y), max(abs_bits(qv[i].z), abs_bits(qv[i].w))));
+        }
+        mb = __reduce_max_sync(0xffffffffu, mb);
+        if (lane == 0) samax[warp] = mb;
+        asm volatile("bar.sync 1, %0;" :: "n"(CW * 32) : "memory");
 #pragma unroll
-            for (int t = 0; t < 4; ++t) {
-                const int c4 = 4 * (lane + 32 * j) + t;
-                const float4 v = c4 < ld4 ? __ldcg(reinterpret_cast<const float4*>(q) + c4) : make_float4(0.f, 0.f, 0.f, 0.f);
-                qv[j][4 * t] = v.x; qv[j][4 * t + 1] = v.y; qv[j][4 * t + 2] = v.z; qv[j][4 * t + 3] = v.w;
-                mb = max(max(mb, abs_bits(v.x)), max(abs_bits(v.y), max(abs_bits(v.z), abs_bits(v.w))));
-            }
+        for (int w = 0; w < CW; ++w) mb = max(mb, samax[w]);
         float s1, s2;
-        q8_scales(__reduce_max_sync(0xffffffffu, mb), s1, s2);
-        uint32_t qh[NC][4], ql[NC][4];
+        q8_scales(mb, s1, s2);
 #pragma unroll
-        for (int j = 0; j < NC; ++j)
-#pragma unroll
-            for (int w = 0; w < 4; ++w) {
-                qh[j][w] = 0u; ql[j][w] = 0u;
+        for (int i = 0; i < QW; ++i) {
+            const int w = ct + 32 * CW * i;
+            if (w < nw) {
+                const float x[4] = {qv[i].x, qv[i].y, qv[i].z, qv[i].w};
+                uint32_t h = 0u, l = 0u;
 #pragma unroll
                 for (int b = 0; b < 4; ++b) {
                     int hi, lo;
-                    q8_split(qv[j][4 * w + b], s1, s2, hi, lo);
-                    qh[j][w] |= (uint32_t)(hi & 0xff) << (8 * b);
-                    ql[j][w] |= (uint32_t)(lo & 0xff) << (8 * b);
+                    q8_split(x[b], s1, s2, hi, lo);
+                    h |= (uint32_t)(hi & 0xff) << (8 * b);
+                    l |= (uint32_t)(lo & 0xff) << (8 * b);
                 }
+                sqh[w] = h; sql[w] = l;
             }
+        }
+        asm volatile("bar.sync 1, %0;" :: "n"(CW * 32) : "memory");
+        // lane l's chunks l, l + 32, ... are query components [16c, 16c + 16)
+        uint32_t qh[NC][4], ql[NC][4];
+#pragma unroll
+        for (int j = 0; j < NC; ++j) {
+            const int c = lane + 32 * j;
+            const uint4 h = c < c8 ? reinterpret_cast<const uint4*>(sqh)[c] : make_uint4(0u, 0u, 0u, 0u);
+            const uint4 l = c < c8 ? reinterpret_cast<const uint4*>(sql)[c] : make_uint4(0u, 0u, 0u, 0u);
+            qh[j][0] = h.x; qh[j][1] = h.y; qh[j][2] = h.z; qh[j][3] = h.w;
+            ql[j][0] = l.x; ql[j][1] = l.y; ql[j][2] = l.z; ql[j][3] = l.w;
+        }
         int s = 0; uint32_t phase = 0;
         for (int64_t t = blockIdx.x; t < ntiles; t += gridDim.x) {
             const int64_t r0 = t * tile_rows;
             const int64_t left = n - r0;
             const int rows = left < tile_rows ? (int)left : tile_rows;
-            // scale and tombstone byte of the warp's rows of this tile (<= 64 / CW of them): lane i loads those of its
-            // i-th row before the wait, so a row costs no global-memory round trip of its own
-            const int ri = warp + CW * lane;
-            float sr_l = 0.f; uint32_t alive_l = 1u;
-            if (ri < rows) { sr_l = __ldg(scale8 + r0 + ri); if (live) alive_l = __ldg(live + r0 + ri); }
             mbar_wait(&full[s], phase);
             const uint4* tile = reinterpret_cast<const uint4*>(smem_raw + (size_t)s * stage_bytes);
+            const float* ssc = reinterpret_cast<const float*>(side + (size_t)s * side_bytes);
+            const uint8_t* slive = side + (size_t)s * side_bytes + 4 * tile_rows;
             u64 kmax = 0;
-            for (int r = warp, i = 0; r < rows; r += CW, ++i) {
-                const uint4* p = tile + (size_t)r * c8;
-                const uint32_t alive = __shfl_sync(0xffffffffu, alive_l, i);
-                const float sr = __shfl_sync(0xffffffffu, sr_l, i);
-                uint4 m[NC];
-#pragma unroll
-                for (int j = 0; j < NC; ++j) { const int c = lane + 32 * j; m[j] = c < c8 ? p[c] : make_uint4(0u, 0u, 0u, 0u); }
-                int dh = 0, dl = 0;                  // |sum| <= 3072 * 127^2 < 2^31: exact
+            for (int ra = warp; ra < rows; ra += 2 * CW) {
+                // rows ra and rb = ra + CW together; a missing rb (odd count, partial tile) repeats ra and is not stored
+                const int rb = ra + CW < rows ? ra + CW : ra;
+                const uint4* pa = tile + (size_t)ra * c8;
+                const uint4* pb = tile + (size_t)rb * c8;
+                uint4 ma[NC], mbv[NC];
 #pragma unroll
                 for (int j = 0; j < NC; ++j) {
-                    dh = __dp4a((int)m[j].x, (int)qh[j][0], dh); dl = __dp4a((int)m[j].x, (int)ql[j][0], dl);
-                    dh = __dp4a((int)m[j].y, (int)qh[j][1], dh); dl = __dp4a((int)m[j].y, (int)ql[j][1], dl);
-                    dh = __dp4a((int)m[j].z, (int)qh[j][2], dh); dl = __dp4a((int)m[j].z, (int)ql[j][2], dl);
-                    dh = __dp4a((int)m[j].w, (int)qh[j][3], dh); dl = __dp4a((int)m[j].w, (int)ql[j][3], dl);
+                    const int c = lane + 32 * j;
+                    ma[j] = c < c8 ? pa[c] : make_uint4(0u, 0u, 0u, 0u);
+                    mbv[j] = c < c8 ? pb[c] : make_uint4(0u, 0u, 0u, 0u);
                 }
-                dh = __reduce_add_sync(0xffffffffu, dh);
-                dl = __reduce_add_sync(0xffffffffu, dl);
-                float sc = sr * fmaf(s2, (float)dl, s1 * (float)dh);
-                if (!alive) sc = dead_score();
+                int dha, dla, dhb, dlb;
+                dot8<NC>(ma, qh, ql, dha, dla);
+                dot8<NC>(mbv, qh, ql, dhb, dlb);
+                dha = __reduce_add_sync(0xffffffffu, dha);
+                dla = __reduce_add_sync(0xffffffffu, dla);
+                dhb = __reduce_add_sync(0xffffffffu, dhb);
+                dlb = __reduce_add_sync(0xffffffffu, dlb);
+                float sca = ssc[ra] * fmaf(s2, (float)dla, s1 * (float)dha);
+                float scb = ssc[rb] * fmaf(s2, (float)dlb, s1 * (float)dhb);
+                if (live) {
+                    if (!slive[ra]) sca = dead_score();
+                    if (!slive[rb]) scb = dead_score();
+                }
                 if (lane == 0) {
-                    scores[r0 + r] = sc;
-                    const u64 k0 = make_key(sc, (uint32_t)(r0 + r));
-                    kmax = k0 > kmax ? k0 : kmax;
+                    scores[r0 + ra] = sca;
+                    const u64 ka = make_key(sca, (uint32_t)(r0 + ra));
+                    kmax = ka > kmax ? ka : kmax;
+                    if (rb != ra) {
+                        scores[r0 + rb] = scb;
+                        const u64 kb = make_key(scb, (uint32_t)(r0 + rb));
+                        kmax = kb > kmax ? kb : kmax;
+                    }
                 }
             }
             __syncwarp();
@@ -1063,7 +1126,10 @@ cudaError_t launch_filter8(cudaStream_t st, int device, const void* M8, const fl
     int tile_rows = 64;
     while (tile_rows > 1 && (size_t)tile_rows * row_bytes > 48 * 1024) tile_rows >>= 1;
     const int stages = 3;
-    const size_t smem = (size_t)stages * tile_rows * row_bytes + (size_t)stages * 16 + 64;
+    // the side data's bulk copies need 16-byte aligned sources: scale8 + r0 and live + r0 with r0 a multiple of tile_rows
+    if (tile_rows % 16 || (reinterpret_cast<uintptr_t>(scale8) & 15) || (reinterpret_cast<uintptr_t>(live) & 15))
+        return cudaErrorInvalidValue;
+    const size_t smem = filter8_smem_bytes(tile_rows, stages, ld8);
     const int64_t ntiles = (n + tile_rows - 1) / tile_rows;
     int64_t grid = sm_count(device) - reserve_sms;
     if (grid > ntiles) grid = ntiles;

@@ -114,7 +114,9 @@ extern "C" int svsb_apply_mutations(svsb_t* e, const int64_t* del_ids, int64_t n
         const long long lowest = LLONG_MIN;
         CU(cudaMemcpyAsync(d_max[i], &lowest, 8, cudaMemcpyHostToDevice, st));
         if (need_live && new_n > 0) {
-            CU(cudaMalloc(&s.live, (size_t)new_n));              // owned by ng from here on (freed with it on any error below)
+            // owned by ng from here on (freed with it on any error below); rounded up to 16 bytes because the int8 filter
+            // copies a partial last tile's tombstone bytes in 16-byte units (gemv8_tma_kernel)
+            CU(cudaMalloc(&s.live, ((size_t)new_n + 15) & ~(size_t)15));
             live_init_kernel<<<grid_for(new_n), 256, 0, st>>>(s.live, os.live, os.n, new_n);
             count_launch();
             if (n_del > 0 && os.n > 0) {
