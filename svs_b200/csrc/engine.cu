@@ -668,13 +668,42 @@ static cudaError_t filter_finish(cudaStream_t st, const DevWs& w, const Generati
                                 (1.0f + g->max_dev) * 1.000001f, route == 8 ? s.buf->e8 : nullptr, s.live, w.fstate);
 }
 
+int similarity_phase(cudaStream_t st, DevWs& w, const Generation* g, const Shard& s, const float* q, int route,
+                     int reserve_sms, bool pdl, cudaEvent_t* t) {
+    if (t) CU(cudaEventRecord(t[0], st));
+    w.gmax_dirty = true;
+    {
+        PdlScope scope(pdl);
+        CU(similarity_pass(st, w, g, s, q, group_shift_for(s.n), reserve_sms, route));
+    }
+    if (t) CU(cudaEventRecord(t[1], st));
+    return SVSB_OK;
+}
+
+int select_phase(cudaStream_t st, DevWs& w, const Generation* g, const Shard& s, const float* q, int route, int64_t k,
+                 const SelOut& o, u64* stamps, const PeerPush* push) {
+    const int shift = group_shift_for(s.n);
+    const int64_t kk = std::min(k, s.n_live);
+    if (route) CU(filter_finish(st, w, g, s, q, shift, kk, route));
+    if (k <= K_FAST_MAX)
+        CU(launch_select(st, w.scores, s.n, w.gmax, shift, (int)kk, s.ids, s.row0, w.cand, w.cand_cap, o.keys, o.scores, o.ids,
+                         o.count, stamps, push));
+    else
+        CU(launch_fullsort_topk(st, w.scores, s.n, w.gmax, shift, kk, s.ids, s.row0, w.sortbuf, o.keys, o.scores, o.ids, o.count));
+    w.gmax_dirty = false;
+    return SVSB_OK;
+}
+
 int prepare_ws(DevWs& w, const Generation* g, const Shard& s, int64_t kk) {
     int rc;
-    if ((rc = w.ensure_rows(s.n)) != SVSB_OK) return rc;
-    if ((rc = w.ensure_q(g->ld)) != SVSB_OK) return rc;
-    if ((rc = w.ensure_out(std::max<int64_t>(kk, 128))) != SVSB_OK) return rc;
-    if (kk > K_FAST_MAX && (rc = w.ensure_sort(s.n)) != SVSB_OK) return rc;
-    return SVSB_OK;
+    if ((rc = w.ensure_query(s.n, std::max<int64_t>(kk, 128), kk)) != SVSB_OK) return rc;
+    return w.ensure_q(g->ld);
+}
+
+DevWs& shard_slot(svsb_engine* e, size_t i) {
+    if (e->shard_ws.size() <= i) e->shard_ws.resize(i + 1);
+    if (!e->shard_ws[i]) { e->shard_ws[i].reset(new DevWs()); e->shard_ws[i]->dev = e->devs[0]; }
+    return *e->shard_ws[i];
 }
 
 // Argument checks shared by the synchronous and the submit / wait forms.  Returns 1 when there is nothing to compute
@@ -707,10 +736,8 @@ static int enqueue_single(QueryCtx* c, const Generation* g, const float* q, int3
     int rc;
     if ((rc = ctx_ensure_host(c, g->ld, kk)) != SVSB_OK) return rc;
     if ((rc = prepare_ws(w, g, s, kk)) != SVSB_OK) return rc;
-    memcpy(c->h_q, q, (size_t)d * 4);
-    for (int i = d; i < g->ld; ++i) c->h_q[i] = 0.f;
+    stage_queries(c->h_q, q, 1, d, g->ld);
     CU(cudaSetDevice(w.dev));
-    const int shift = group_shift_for(s.n);
     *c->h_count = -1;
     if (kk <= K_FAST_MAX) {
         cudaStream_t gst = w.st;                                 // stream of the staging + similarity kernels
@@ -722,29 +749,19 @@ static int enqueue_single(QueryCtx* c, const Generation* g, const float* q, int3
             gst = chain->submit_st;
         }
         CU(launch_stage_query(gst, c->h_q, w.d_q, g->ld));
-        w.gmax_dirty = true;
         const int route = filter_route(s, kk);
-        {   // programmatic dependent launch: the similarity kernel streams its first tiles under the staging kernel
-            PdlScope pdl(env_int("SVSB_PDL", 1) != 0);
-            CU(similarity_pass(gst, w, g, s, w.d_q, shift, reserve_sm ? 1 : 0, route));
-        }
+        // programmatic dependent launch: the similarity kernel streams its first tiles under the staging kernel
+        if ((rc = similarity_phase(gst, w, g, s, w.d_q, route, reserve_sm ? 1 : 0, env_int("SVSB_PDL", 1) != 0)) != SVSB_OK) return rc;
         if (chain) {
             CU(cudaEventRecord(c->ev_gemv, gst));
             chain_lk.unlock();
             CU(cudaStreamWaitEvent(w.st, c->ev_gemv, 0));
         }
-        if (route) CU(filter_finish(w.st, w, g, s, w.d_q, shift, kk, route));
-        CU(launch_select(w.st, w.scores, s.n, w.gmax, shift, (int)kk, s.ids, s.row0, w.cand, w.cand_cap,
-                         w.out_keys, c->h_scores, c->h_ids, c->h_count));
-        w.gmax_dirty = false;
-        return SVSB_OK;
+        return select_phase(w.st, w, g, s, w.d_q, route, kk, {w.out_keys, c->h_scores, c->h_ids, c->h_count});
     }
     CU(cudaMemcpyAsync(w.d_q, c->h_q, (size_t)g->ld * 4, cudaMemcpyHostToDevice, w.st));
-    w.gmax_dirty = true;
-    CU(launch_gemv(w.st, w.dev, s.M, s.n, g->d, g->ld, w.d_q, w.scores, w.gmax, shift, 0, 0, 0, 0, s.live));
-    CU(launch_fullsort_topk(w.st, w.scores, s.n, w.gmax, shift, kk, s.ids, s.row0, w.sortbuf,
-                            w.out_keys, w.out_scores, w.out_ids, w.out_count));
-    w.gmax_dirty = false;
+    if ((rc = similarity_phase(w.st, w, g, s, w.d_q, 0)) != SVSB_OK) return rc;
+    if ((rc = select_phase(w.st, w, g, s, w.d_q, 0, kk, w.out())) != SVSB_OK) return rc;
     CU(cudaMemcpyAsync(c->h_scores, w.out_scores, (size_t)kk * 4, cudaMemcpyDeviceToHost, w.st));
     CU(cudaMemcpyAsync(c->h_ids, w.out_ids, (size_t)kk * 8, cudaMemcpyDeviceToHost, w.st));
     CU(cudaMemcpyAsync(c->h_count, w.out_count, 4, cudaMemcpyDeviceToHost, w.st));
@@ -1818,20 +1835,12 @@ extern "C" int svsb_topk_scores(svsb_t* e, const float* scores, int64_t n, int32
     QueryCtx* c = lease.c.get();
     DevWs& w = c->ws[0];
     if ((rc = ctx_ensure_host(c, 4, kk)) != SVSB_OK) return rc;
-    if ((rc = w.ensure_rows(n)) != SVSB_OK) return rc;
-    if ((rc = w.ensure_out(std::max<int64_t>(kk, 128))) != SVSB_OK) return rc;
-    if (kk > K_FAST_MAX && (rc = w.ensure_sort(n)) != SVSB_OK) return rc;
+    if ((rc = w.ensure_query(n, std::max<int64_t>(kk, 128), kk)) != SVSB_OK) return rc;
     CU(cudaSetDevice(w.dev));
-    const int shift = group_shift_for(n);
+    Shard rows; rows.n = rows.n_live = n;                         // no ids: the selection returns rows
     CU(cudaMemcpyAsync(w.scores, scores, (size_t)n * 4, cudaMemcpyHostToDevice, w.st));
-    if (kk <= K_FAST_MAX) {
-        CU(launch_groupmax(w.st, w.dev, w.scores, n, w.gmax, shift));
-        CU(launch_select(w.st, w.scores, n, w.gmax, shift, (int)kk, nullptr, 0, w.cand, w.cand_cap,
-                         w.out_keys, w.out_scores, w.out_ids, w.out_count));
-    } else {
-        CU(launch_fullsort_topk(w.st, w.scores, n, w.gmax, shift, kk, nullptr, 0, w.sortbuf,
-                                w.out_keys, w.out_scores, w.out_ids, w.out_count));
-    }
+    if (kk <= K_FAST_MAX) CU(launch_groupmax(w.st, w.dev, w.scores, n, w.gmax, group_shift_for(n)));
+    if ((rc = select_phase(w.st, w, nullptr, rows, nullptr, 0, kk, w.out())) != SVSB_OK) return rc;
     CU(cudaMemcpyAsync(c->h_scores, w.out_scores, (size_t)kk * 4, cudaMemcpyDeviceToHost, w.st));
     CU(cudaMemcpyAsync(c->h_ids, w.out_ids, (size_t)kk * 8, cudaMemcpyDeviceToHost, w.st));
     CU(cudaMemcpyAsync(c->h_count, w.out_count, 4, cudaMemcpyDeviceToHost, w.st));
@@ -1850,7 +1859,7 @@ extern "C" int svsb_bench_set_queries(svsb_t* e, const float* Q, int32_t nq, int
     if (!Q || nq <= 0 || d <= 0) return fail(SVSB_E_INVALID, "svsb_bench_set_queries: bad arguments");
     const int ld = round_up4(d);
     std::vector<float> padded((size_t)nq * ld, 0.f);
-    for (int i = 0; i < nq; ++i) memcpy(&padded[(size_t)i * ld], Q + (size_t)i * d, (size_t)d * 4);
+    stage_queries(padded.data(), Q, nq, d, ld);
     if (e->bench_q.size() != e->devs.size()) e->bench_q.assign(e->devs.size(), nullptr);
     for (size_t i = 0; i < e->devs.size(); ++i) {
         CU(cudaSetDevice(e->devs[i]));
@@ -1914,50 +1923,25 @@ extern "C" int svsb_bench_run(svsb_t* e, int32_t k, int32_t iters, float* total_
         if ((rc = prepare_ws(*c->alt, g.get(), s, kk)) != SVSB_OK) return rc;
     }
     std::vector<cudaEvent_t>& kev = e->bench_kev;
-    const int shift = group_shift_for(s.n);
     CU(cudaSetDevice(w0.dev));
     CU(cudaStreamSynchronize(w0.st));
     if (pipelined) CU(cudaStreamSynchronize(c->alt->st));
     CU(cudaEventRecord(w0.ev0, w0.st));
+    for (int it = 0; it < iters; ++it) {
+        DevWs& W = (pipelined && (it & 1)) ? *c->alt : w0;
+        cudaStream_t sb = pipelined ? c->alt->st : w0.st;           // the selections' stream
+        const float* q = e->bench_q[0] + (int64_t)(it % e->bench_nq) * e->bench_ld;
+        if (pipelined && it >= 2) CU(cudaStreamWaitEvent(w0.st, W.ev_sel, 0));   // selection of query it-2 is done with W
+        cudaEvent_t* t = timed_it(it) ? &kev[2 * it] : nullptr;
+        if ((rc = similarity_phase(w0.st, W, g.get(), s, q, route, pipelined ? 1 : 0, false, t)) != SVSB_OK) return rc;
+        if (pipelined && (rc = W.hand_off(w0.st, sb)) != SVSB_OK) return rc;
+        if ((rc = select_phase(sb, W, g.get(), s, q, route, kk, W.out())) != SVSB_OK) return rc;
+        if (pipelined) CU(cudaEventRecord(W.ev_sel, sb));
+        c->last = &W;
+    }
     if (pipelined) {
-        DevWs& w1 = *c->alt;
-        cudaStream_t sa = w0.st, sb = w1.st;
-        for (int it = 0; it < iters; ++it) {
-            DevWs& W = (it & 1) ? w1 : w0;
-            const int64_t qoff = (int64_t)(it % e->bench_nq) * e->bench_ld;
-            if (it >= 2) CU(cudaStreamWaitEvent(sa, W.ev_sel, 0));           // selection of query it-2 is done with W
-            if (timed_it(it)) CU(cudaEventRecord(kev[2 * it], sa));
-            W.gmax_dirty = true;
-            CU(similarity_pass(sa, W, g.get(), s, e->bench_q[0] + qoff, shift, /*reserve_sms=*/1, route));
-            if (timed_it(it)) CU(cudaEventRecord(kev[2 * it + 1], sa));
-            CU(cudaEventRecord(W.ev, sa));
-            CU(cudaStreamWaitEvent(sb, W.ev, 0));
-            if (route) CU(filter_finish(sb, W, g.get(), s, e->bench_q[0] + qoff, shift, kk, route));
-            CU(launch_select(sb, W.scores, s.n, W.gmax, shift, (int)kk, s.ids, s.row0, W.cand, W.cand_cap,
-                             W.out_keys, W.out_scores, W.out_ids, W.out_count));
-            W.gmax_dirty = false;
-            CU(cudaEventRecord(W.ev_sel, sb));
-            c->last = &W;
-        }
-        CU(cudaStreamWaitEvent(sa, w0.ev_sel, 0));
-        if (iters > 1) CU(cudaStreamWaitEvent(sa, w1.ev_sel, 0));
-    } else {
-        for (int it = 0; it < iters; ++it) {
-            const int64_t qoff = (int64_t)(it % e->bench_nq) * e->bench_ld;
-            if (timed_it(it)) CU(cudaEventRecord(kev[2 * it], w0.st));
-            w0.gmax_dirty = true;
-            CU(similarity_pass(w0.st, w0, g.get(), s, e->bench_q[0] + qoff, shift, 0, route));
-            if (timed_it(it)) CU(cudaEventRecord(kev[2 * it + 1], w0.st));
-            if (route) CU(filter_finish(w0.st, w0, g.get(), s, e->bench_q[0] + qoff, shift, kk, route));
-            if (kk <= K_FAST_MAX)
-                CU(launch_select(w0.st, w0.scores, s.n, w0.gmax, shift, (int)kk, s.ids, s.row0, w0.cand, w0.cand_cap,
-                                 w0.out_keys, w0.out_scores, w0.out_ids, w0.out_count));
-            else
-                CU(launch_fullsort_topk(w0.st, w0.scores, s.n, w0.gmax, shift, kk, s.ids, s.row0, w0.sortbuf,
-                                        w0.out_keys, w0.out_scores, w0.out_ids, w0.out_count));
-            w0.gmax_dirty = false;
-        }
-        c->last = &w0;
+        CU(cudaStreamWaitEvent(w0.st, w0.ev_sel, 0));
+        if (iters > 1) CU(cudaStreamWaitEvent(w0.st, c->alt->ev_sel, 0));
     }
     CU(cudaEventRecord(w0.ev1, w0.st));
     CU(cudaEventSynchronize(w0.ev1));
@@ -2012,10 +1996,9 @@ extern "C" int svsb_debug_select_phases(svsb_t* e, int32_t qi, int32_t k, uint64
     u64* dbg = nullptr;
     CU(cudaMalloc(&dbg, 16 * 8));
     CU(cudaMemsetAsync(dbg, 0, 16 * 8, w.st));
-    const int shift = group_shift_for(s.n);
-    CU(launch_gemv(w.st, w.dev, s.M, s.n, g->d, g->ld, e->bench_q[0] + (int64_t)qi * e->bench_ld, w.scores, w.gmax, shift, 0, 0, 0, 0, s.live));
-    CU(launch_select(w.st, w.scores, s.n, w.gmax, shift, (int)kk, s.ids, s.row0, w.cand, w.cand_cap,
-                     w.out_keys, w.out_scores, w.out_ids, w.out_count, dbg));
+    const float* q = e->bench_q[0] + (int64_t)qi * e->bench_ld;
+    if ((rc = similarity_phase(w.st, w, g.get(), s, q, 0)) != SVSB_OK) return rc;
+    if ((rc = select_phase(w.st, w, g.get(), s, q, 0, kk, w.out(), dbg)) != SVSB_OK) return rc;
     CU(cudaMemcpyAsync(stamps16, dbg, 16 * 8, cudaMemcpyDeviceToHost, w.st));
     CU(cudaStreamSynchronize(w.st));
     CU(cudaFree(dbg));
@@ -2112,11 +2095,10 @@ static int engine_merge_records(svsb_engine* e, cudaStream_t st, const RecordVie
                                 int k, float* out_scores, int64_t* out_ids, int32_t* out_counts, int verify_k, const int* status = nullptr) {
     u64* sk = nullptr; int64_t* sp = nullptr;
     if ((int64_t)n_lists * recs.cap > K_FAST_MAX) {
-        if (e->shard_ws.empty()) e->shard_ws.resize(1);
-        if (!e->shard_ws[0]) { e->shard_ws[0].reset(new DevWs()); e->shard_ws[0]->dev = e->devs[0]; }
-        int rc = e->shard_ws[0]->ensure_merge_scratch((int64_t)batch * n_lists * recs.cap);
+        DevWs& w = shard_slot(e, 0);
+        int rc = w.ensure_merge_scratch((int64_t)batch * n_lists * recs.cap);
         if (rc != SVSB_OK) return rc;
-        sk = e->shard_ws[0]->mscr_keys; sp = e->shard_ws[0]->mscr_ids;
+        sk = w.mscr_keys; sp = w.mscr_ids;
     }
     return merge_records(st, recs, n_lists, list_words, batch, k, sk, sp, out_scores, out_ids, out_counts, verify_k, status);
 }
@@ -2127,6 +2109,14 @@ extern "C" int svsb_enqueue_local_topk(svsb_t* e, void* stream, int32_t slot, co
                                        int64_t* d_record, int32_t flags) {
     if (!e) return fail(SVSB_E_INVALID, "engine is NULL");
     return enqueue_local_topk_gen(e, pin(e), stream, slot, d_query, k, d_record, flags);
+}
+
+// The next timing bracket of e->kev (svsb_kernel_time_collect), its two events created on first use.  The caller
+// advances e->kev_used once the bracketed pass is enqueued.
+static int kev_next(svsb_engine* e, cudaEvent_t*& t) {
+    while (e->kev.size() < e->kev_used + 2) { cudaEvent_t ev; CU(cudaEventCreate(&ev)); e->kev.push_back(ev); }
+    t = &e->kev[e->kev_used];
+    return SVSB_OK;
 }
 
 static int enqueue_local_topk_gen(svsb_engine* e, const std::shared_ptr<Generation>& g, void* stream, int32_t slot, const float* d_query,
@@ -2143,47 +2133,28 @@ static int enqueue_local_topk_gen(svsb_engine* e, const std::shared_ptr<Generati
     CU(cudaSetDevice(s.dev));
     const RecordView r{d_record, k};
     if (s.n_live == 0) { CU(cudaMemsetAsync(r.count(0), 0, 8, st)); return SVSB_OK; }
-    if ((size_t)slot >= e->shard_ws.size()) e->shard_ws.resize(slot + 1);
-    if (e->sel_pending.size() < e->shard_ws.size()) e->sel_pending.resize(e->shard_ws.size(), 0);
-    if (!e->shard_ws[slot]) { e->shard_ws[slot].reset(new DevWs()); e->shard_ws[slot]->dev = s.dev; }
-    DevWs& w = *e->shard_ws[slot];
+    DevWs& w = shard_slot(e, slot);
     int rc;
-    const int64_t kl = std::min<int64_t>(k, s.n_live);
-    if ((rc = w.ensure_rows(s.n)) != SVSB_OK) return rc;
-    if ((rc = w.ensure_out(std::max<int64_t>(kl, K_FAST_MAX))) != SVSB_OK) return rc;
-    if (big && (rc = w.ensure_sort(s.n)) != SVSB_OK) return rc;
+    if ((rc = w.ensure_query(s.n, std::max<int64_t>(std::min<int64_t>(k, s.n_live), K_FAST_MAX), k)) != SVSB_OK) return rc;
     if (pipelined) {
         if (!e->side_st) CU(cudaStreamCreateWithFlags(&e->side_st, cudaStreamNonBlocking));
         if (!w.ev) CU(cudaEventCreateWithFlags(&w.ev, cudaEventDisableTiming));
         if (!w.ev_sel) CU(cudaEventCreateWithFlags(&w.ev_sel, cudaEventDisableTiming));
-        // the slot's previous selection must have finished reading scores / group maxima before they are overwritten
-        if (e->sel_pending[slot]) CU(cudaStreamWaitEvent(st, w.ev_sel, 0));
-    } else if (e->sel_pending[slot] && w.ev_sel) {
-        CU(cudaStreamWaitEvent(st, w.ev_sel, 0));           // a caller mixing pipelined and plain calls on one slot
-        e->sel_pending[slot] = 0;
     }
-    const int shift = group_shift_for(s.n);
-    if (time_kernel) {
-        while (e->kev.size() < e->kev_used + 2) { cudaEvent_t ev; CU(cudaEventCreate(&ev)); e->kev.push_back(ev); }
-        CU(cudaEventRecord(e->kev[e->kev_used], st));
-    }
-    w.gmax_dirty = true;
-    CU(launch_gemv(st, s.dev, s.M, s.n, g->d, g->ld, d_query, w.scores, w.gmax, shift, 0, 0, 0, pipelined ? 1 : 0, s.live));
-    if (time_kernel) { CU(cudaEventRecord(e->kev[e->kev_used + 1], st)); e->kev_used += 2; }
-    cudaStream_t sel_st = st;
-    if (pipelined) {
-        CU(cudaEventRecord(w.ev, st));
-        CU(cudaStreamWaitEvent(e->side_st, w.ev, 0));
-        sel_st = e->side_st;
-    }
-    if (big)
-        CU(launch_fullsort_topk(st, w.scores, s.n, w.gmax, shift, kl, s.ids, s.row0, w.sortbuf, r.keys(0), w.out_scores, r.ids(0),
-                                r.count(0)));
-    else
-        CU(launch_select(sel_st, w.scores, s.n, w.gmax, shift, (int)kl, s.ids, s.row0, w.cand, w.cand_cap,
-                         r.keys(0), w.out_scores, r.ids(0), r.count(0)));
-    w.gmax_dirty = false;
-    if (pipelined) { CU(cudaEventRecord(w.ev_sel, e->side_st)); e->sel_pending[slot] = 1; }
+    // the slot's previous selection must have finished reading scores / group maxima before they are overwritten
+    // (a plain call after a pipelined one on this slot, too)
+    if ((rc = w.sel_wait(st)) != SVSB_OK) return rc;
+    if (!pipelined) w.sel_pending = false;
+    cudaEvent_t* t = nullptr;
+    if (time_kernel && (rc = kev_next(e, t)) != SVSB_OK) return rc;
+    // route 0 on purpose: filter_attach gives a one-process-per-GPU rank with enough rows the filter's shadows as well,
+    // but only the single-device query paths take the filter (filter_route); the sharded and peer paths run K1
+    if ((rc = similarity_phase(st, w, g.get(), s, d_query, 0, pipelined ? 1 : 0, false, t)) != SVSB_OK) return rc;
+    if (t) e->kev_used += 2;
+    if (pipelined && (rc = w.hand_off(st, e->side_st)) != SVSB_OK) return rc;
+    if ((rc = select_phase(pipelined ? e->side_st : st, w, g.get(), s, d_query, 0, k, {r.keys(0), w.out_scores, r.ids(0), r.count(0)})) != SVSB_OK)
+        return rc;
+    if (pipelined) { CU(cudaEventRecord(w.ev_sel, e->side_st)); w.sel_pending = true; }
     return SVSB_OK;
 }
 
@@ -2585,23 +2556,12 @@ static int xchg_prepare(svsb_engine* e, const Generation* g) {
     Xchg* x = e->xchg.get();
     const Shard& s = g->shards[0];
     CU(cudaSetDevice(s.dev));
-    if (e->shard_ws.size() < 2) e->shard_ws.resize(2);
-    if (e->sel_pending.size() < e->shard_ws.size()) e->sel_pending.resize(e->shard_ws.size(), 0);
     if (!e->side_st) CU(cudaStreamCreateWithFlags(&e->side_st, cudaStreamNonBlocking));
-    DevWs* sets[3] = {&x->ws, nullptr, nullptr};
-    for (int i = 0; i < 2; ++i) {
-        if (!e->shard_ws[i]) { e->shard_ws[i].reset(new DevWs()); e->shard_ws[i]->dev = s.dev; }
-        sets[1 + i] = e->shard_ws[i].get();
-    }
-    for (DevWs* w : sets) {
-        int rc;
-        if (s.n > 0 && (rc = w->ensure_rows(s.n)) != SVSB_OK) return rc;
-        if ((rc = w->ensure_out(K_FAST_MAX)) != SVSB_OK) return rc;
-        if ((int64_t)x->world * x->cap > K_FAST_MAX && (rc = w->ensure_merge_scratch((int64_t)x->world * x->cap)) != SVSB_OK) return rc;
-        if (!w->ev) CU(cudaEventCreateWithFlags(&w->ev, cudaEventDisableTiming));
-        if (!w->ev_sel) CU(cudaEventCreateWithFlags(&w->ev_sel, cudaEventDisableTiming));
-    }
     int rc;
+    for (DevWs* w : {&x->ws, &shard_slot(e, 0), &shard_slot(e, 1)}) {
+        if ((rc = w->ensure_set(s.n)) != SVSB_OK) return rc;
+        if ((int64_t)x->world * x->cap > K_FAST_MAX && (rc = w->ensure_merge_scratch((int64_t)x->world * x->cap)) != SVSB_OK) return rc;
+    }
     if ((rc = x->ws.ensure_q(g->ld)) != SVSB_OK) return rc;
     if (g->ld > x->h_q_cap) {
         if (x->h_q) cudaFreeHost(x->h_q);
@@ -2609,7 +2569,8 @@ static int xchg_prepare(svsb_engine* e, const Generation* g) {
         CU(cudaMallocHost(&x->h_q, (size_t)g->ld * 4));
         x->h_q_cap = g->ld;
     }
-    while (e->kev.size() < e->kev_used + 2) { cudaEvent_t ev; CU(cudaEventCreate(&ev)); e->kev.push_back(ev); }
+    cudaEvent_t* t;                                              // the timing bracket of the call's pass, if it asks
+    if ((rc = kev_next(e, t)) != SVSB_OK) return rc;
     if (!x->ev_join) CU(cudaEventCreateWithFlags(&x->ev_join, cudaEventDisableTiming));
     return SVSB_OK;
 }
@@ -2638,40 +2599,35 @@ static int xchg_flush_merge(svsb_engine* e, cudaStream_t st_sel) {
 }
 
 // similarity on st_main, then (on st_sel) selection with the fused push and the waiting merge into out_*.
-// defer_merge: the merge is enqueued by the NEXT call (or by svsb_enqueue_join), behind that call's selection.
+// pipelined: ev_sel marks the end of the selection (scores reusable by the similarity pass two queries on), and the merge
+// is enqueued by the NEXT call (or by svsb_enqueue_join), behind that call's selection.
 // Window slots stay safe with 4 of them: a rank pushes query j+4 after its merge(j+2), i.e. after every peer pushed
 // j+2, and each peer enqueues merge(j) before its selection j+2.
-static int xchg_enqueue(svsb_engine* e, const Generation* g, DevWs& w, cudaStream_t st_main, cudaStream_t st_sel, cudaEvent_t ev_main_done,
+static int xchg_enqueue(svsb_engine* e, const Generation* g, DevWs& w, cudaStream_t st_main, cudaStream_t st_sel,
                         const float* d_query, int32_t k, float* out_scores, int64_t* out_ids, int32_t* out_count,
-                        bool time_kernel, int reserve_sms, bool defer_merge = false, cudaEvent_t ev_sel_done = nullptr,
-                        bool pdl_gemv = false) {
+                        bool time_kernel, int reserve_sms, bool pipelined, bool pdl_gemv = false) {
     Xchg* x = e->xchg.get();
     const Shard& s = g->shards[0];
     PeerPush push{};
     const int slot = xchg_next(x, push);
+    int rc;
     if (s.n_live == 0) {
         CU(launch_push_empty(st_sel, push));
     } else {
-        const int shift = group_shift_for(s.n);
-        if (time_kernel) CU(cudaEventRecord(e->kev[e->kev_used], st_main));
-        w.gmax_dirty = true;
-        {
-            PdlScope pdl(pdl_gemv);                               // only after the staging kernel of the synchronous path
-            CU(launch_gemv(st_main, s.dev, s.M, s.n, g->d, g->ld, d_query, w.scores, w.gmax, shift, 0, 0, 0, reserve_sms, s.live));
-        }
-        if (time_kernel) { CU(cudaEventRecord(e->kev[e->kev_used + 1], st_main)); e->kev_used += 2; }
-        if (st_sel != st_main) { CU(cudaEventRecord(ev_main_done, st_main)); CU(cudaStreamWaitEvent(st_sel, ev_main_done, 0)); }
-        u64* sel_stamps = (x->stamps && !defer_merge) ? x->stamps + (push.seq % Xchg::STAMP_RING) * Xchg::STAMP_WORDS : nullptr;
-        CU(launch_select(st_sel, w.scores, s.n, w.gmax, shift, (int)std::min<int64_t>(k, s.n_live), s.ids, s.row0, w.cand, w.cand_cap,
-                         w.out_keys, w.out_scores, w.out_ids, w.out_count, sel_stamps, &push));
-        w.gmax_dirty = false;
+        cudaEvent_t* t = nullptr;
+        if (time_kernel && (rc = kev_next(e, t)) != SVSB_OK) return rc;
+        // route 0 on purpose, as in enqueue_local_topk_gen; PDL only after the staging kernel of the host-buffer paths
+        if ((rc = similarity_phase(st_main, w, g, s, d_query, 0, reserve_sms, pdl_gemv, t)) != SVSB_OK) return rc;
+        if (t) e->kev_used += 2;
+        if (st_sel != st_main && (rc = w.hand_off(st_main, st_sel)) != SVSB_OK) return rc;
+        u64* sel_stamps = (x->stamps && !pipelined) ? x->stamps + (push.seq % Xchg::STAMP_RING) * Xchg::STAMP_WORDS : nullptr;
+        if ((rc = select_phase(st_sel, w, g, s, d_query, 0, k, w.out(), sel_stamps, &push)) != SVSB_OK) return rc;
     }
-    if (ev_sel_done) CU(cudaEventRecord(ev_sel_done, st_sel));   // the workspace's scores are free from here on
+    if (pipelined) { CU(cudaEventRecord(w.ev_sel, st_sel)); w.sel_pending = true; }
     u64* sk = nullptr; int64_t* sp = nullptr;
     if ((int64_t)x->world * k > K_FAST_MAX) { sk = w.mscr_keys; sp = w.mscr_ids; }
-    if (defer_merge) {
-        int rc = xchg_flush_merge(e, st_sel);                    // the previous query's merge goes behind this selection
-        if (rc != SVSB_OK) return rc;
+    if (pipelined) {
+        if ((rc = xchg_flush_merge(e, st_sel)) != SVSB_OK) return rc;   // the previous query's merge goes behind this selection
         Xchg::DeferredMerge& m = x->deferred;
         m.pending = true; m.slot = slot; m.k = k; m.seq = push.seq; m.sk = sk; m.sp = sp;
         m.out_scores = out_scores; m.out_ids = out_ids; m.out_count = out_count; m.ev_done = nullptr;
@@ -2698,24 +2654,13 @@ extern "C" int svsb_enqueue_query_peer(svsb_t* e, void* stream, const float* d_q
     int rc = xchg_prepare(e, g.get());
     if (rc != SVSB_OK) return rc;
     const int slot = (int)(e->xchg->seq & 1);              // workspace set: alternates so that query i+1's similarity pass
-    DevWs& w = *e->shard_ws[slot];                         // overlaps query i's selection
-    cudaStream_t sel_st = st;
-    if (pipelined) {
-        if (e->sel_pending[slot]) CU(cudaStreamWaitEvent(st, w.ev_sel, 0));   // the slot's scores are free again
-        sel_st = e->side_st;
-    } else {
-        if (e->xchg->deferred.pending && (rc = xchg_flush_merge(e, e->side_st)) != SVSB_OK) return rc;
-        if (e->sel_pending[slot]) {                               // a pipelined call used this slot before: its selection on
-            CU(cudaStreamWaitEvent(st, w.ev_sel, 0));             // the side stream may still be reading scores / group maxima
-            e->sel_pending[slot] = 0;
-        }
-    }
-    // pipelined: ev_sel marks "selection done" (scores reusable by the similarity pass two queries on); the merge is deferred
-    rc = xchg_enqueue(e, g.get(), w, st, sel_st, w.ev, d_query, k, out_scores, out_ids, out_count, time_kernel, pipelined ? 1 : 0,
-                      /*defer_merge=*/pipelined, pipelined ? w.ev_sel : nullptr);
-    if (rc != SVSB_OK) return rc;
-    if (pipelined) e->sel_pending[slot] = 1;
-    return SVSB_OK;
+    DevWs& w = shard_slot(e, slot);                        // overlaps query i's selection
+    if (!pipelined && e->xchg->deferred.pending && (rc = xchg_flush_merge(e, e->side_st)) != SVSB_OK) return rc;
+    // the set's scores are free again (a plain call after a pipelined one on this set, too)
+    if ((rc = w.sel_wait(st)) != SVSB_OK) return rc;
+    if (!pipelined) w.sel_pending = false;
+    return xchg_enqueue(e, g.get(), w, st, pipelined ? e->side_st : st, d_query, k, out_scores, out_ids, out_count, time_kernel,
+                        pipelined ? 1 : 0, pipelined);
 }
 
 extern "C" int svsb_query_peer(svsb_t* e, const float* q, int32_t d, int32_t k,
@@ -2733,13 +2678,12 @@ extern "C" int svsb_query_peer(svsb_t* e, const float* q, int32_t d, int32_t k,
     int rc = xchg_prepare(e, g.get());
     if (rc != SVSB_OK) return rc;
     if (x->deferred.pending && (rc = xchg_flush_merge(e, e->side_st)) != SVSB_OK) return rc;   // keep merges in sequence order
-    memcpy(x->h_q, q, (size_t)d * 4);
-    for (int i = d; i < g->ld; ++i) x->h_q[i] = 0.f;
+    stage_queries(x->h_q, q, 1, d, g->ld);
     CU(launch_stage_query(x->st, x->h_q, x->ws.d_q, g->ld));     // a kernel reads the pinned query: no copy-engine hop
     *x->h_count = -1;
     // the merge kernel writes the result into pinned (mapped) host memory: no copy back, one synchronize
-    if ((rc = xchg_enqueue(e, g.get(), x->ws, x->st, x->st, nullptr, x->ws.d_q, k, x->h_scores, x->h_ids, x->h_count, false, 0,
-                           false, nullptr, /*pdl_gemv=*/env_int("SVSB_PDL", 1) != 0)) != SVSB_OK) return rc;
+    if ((rc = xchg_enqueue(e, g.get(), x->ws, x->st, x->st, x->ws.d_q, k, x->h_scores, x->h_ids, x->h_count, false, 0,
+                           /*pipelined=*/false, /*pdl_gemv=*/env_int("SVSB_PDL", 1) != 0)) != SVSB_OK) return rc;
     CU(cudaStreamSynchronize(x->st));
     const int32_t cnt = *x->h_count;
     if (cnt == MERGE_WINDOW_TIMED_OUT)
@@ -2795,18 +2739,15 @@ extern "C" int svsb_query_peer_submit(svsb_t* e, const float* q, int32_t d, int3
     const int ti = x->tk_next;
     Xchg::Ticket& t = x->tk[ti];
     if (t.busy) return fail(SVSB_E_STATE, "svsb_query_peer_submit: 3 queries are pending already (wait for the oldest first)");
-    memcpy(t.h_q, q, (size_t)d * 4);
-    for (int i = d; i < g->ld; ++i) t.h_q[i] = 0.f;
+    stage_queries(t.h_q, q, 1, d, g->ld);
     *t.h_count = -1;
-    const int slot = (int)(x->seq & 1);                        // workspace set (xchg_enqueue takes sequence number seq + 1)
-    DevWs& w = *e->shard_ws[slot];
+    DevWs& w = shard_slot(e, x->seq & 1);                      // workspace set (xchg_enqueue takes sequence number seq + 1)
     CU(cudaSetDevice(e->devs[0]));
-    if (e->sel_pending[slot]) CU(cudaStreamWaitEvent(x->st, w.ev_sel, 0));      // the set's previous selection is done with it
+    if ((rc = w.sel_wait(x->st)) != SVSB_OK) return rc;        // the set's previous selection is done with it
     CU(launch_stage_query(x->st, t.h_q, t.d_q, g->ld));
-    rc = xchg_enqueue(e, g.get(), w, x->st, e->side_st, w.ev, t.d_q, k, t.h_scores, t.h_ids, t.h_count, false, /*reserve_sms=*/1,
-                      /*defer_merge=*/true, w.ev_sel, /*pdl_gemv=*/env_int("SVSB_PDL", 1) != 0);
+    rc = xchg_enqueue(e, g.get(), w, x->st, e->side_st, t.d_q, k, t.h_scores, t.h_ids, t.h_count, false, /*reserve_sms=*/1,
+                      /*pipelined=*/true, /*pdl_gemv=*/env_int("SVSB_PDL", 1) != 0);
     if (rc != SVSB_OK) return rc;
-    e->sel_pending[slot] = 1;
     x->deferred.ev_done = t.ev;                                // recorded when this query's merge is enqueued
     t.busy = true; t.k = k; t.seq = x->seq;
     x->tk_next = (ti + 1) % Xchg::N_TICKETS;
@@ -2863,9 +2804,10 @@ extern "C" int svsb_enqueue_join(svsb_t* e, void* stream) {
         CU(cudaEventRecord(e->xchg->ev_join, e->side_st));
         CU(cudaStreamWaitEvent((cudaStream_t)stream, e->xchg->ev_join, 0));
     }
-    for (size_t i = 0; i < e->sel_pending.size(); ++i)
-        if (e->sel_pending[i] && e->shard_ws[i] && e->shard_ws[i]->ev_sel)
-            CU(cudaStreamWaitEvent((cudaStream_t)stream, e->shard_ws[i]->ev_sel, 0));
+    for (auto& w : e->shard_ws) {
+        int rc;
+        if (w && (rc = w->sel_wait((cudaStream_t)stream)) != SVSB_OK) return rc;
+    }
     return SVSB_OK;
 }
 
@@ -2931,10 +2873,8 @@ extern "C" int svsb_ws_create(int device, int64_t n_rows, int32_t k_max, svsb_ws
     std::unique_ptr<svsb_workspace> w(new svsb_workspace());
     w->dev = device;
     int rc;
-    if (n_rows > 0 && (rc = w->ensure_rows(n_rows)) != SVSB_OK) { w->release(); return rc; }
-    const int64_t kcap = std::max<int64_t>(k_max, 128);
-    if ((rc = w->ensure_out(kcap)) != SVSB_OK) { w->release(); return rc; }
-    if (k_max > K_FAST_MAX && n_rows > 0 && (rc = w->ensure_sort(n_rows)) != SVSB_OK) { w->release(); return rc; }
+    // n_rows = 0: outputs only (rows and the sort buffer are sized by the first launch)
+    if ((rc = w->ensure_query(n_rows, std::max<int64_t>(k_max, 128), n_rows > 0 ? k_max : 0)) != SVSB_OK) { w->release(); return rc; }
     *out = w.release();
     return SVSB_OK;
 }
@@ -2954,22 +2894,15 @@ extern "C" int svsb_launch_local_topk(svsb_ws_t* ws, void* stream, const float* 
     if (!d_matrix || !d_query || !d_out_keys || !d_out_ids || !d_out_count) return fail(SVSB_E_INVALID, "svsb_launch_local_topk: NULL pointer");
     const int64_t kk = std::min<int64_t>(k, n);
     int rc;
-    if ((rc = ws->ensure_rows(n)) != SVSB_OK) return rc;
-    if ((rc = ws->ensure_out(std::max<int64_t>(kk, 128))) != SVSB_OK) return rc;
-    if (kk > K_FAST_MAX && (rc = ws->ensure_sort(n)) != SVSB_OK) return rc;
+    if ((rc = ws->ensure_query(n, std::max<int64_t>(kk, 128), kk)) != SVSB_OK) return rc;
     CU(cudaSetDevice(ws->dev));
+    // the caller's rows as a shard of one generation; they are only read
+    Generation g; g.d = d; g.ld = ld;
+    Shard s; s.dev = ws->dev; s.row0 = global_row0; s.n = s.n_live = n;
+    s.M = const_cast<float*>(d_matrix); s.ids = const_cast<int64_t*>(d_emb_ids);
     cudaStream_t st = (cudaStream_t)stream;
-    const int shift = group_shift_for(n);
-    ws->gmax_dirty = true;
-    CU(launch_gemv(st, ws->dev, d_matrix, n, d, ld, d_query, ws->scores, ws->gmax, shift));
-    if (kk <= K_FAST_MAX)
-        CU(launch_select(st, ws->scores, n, ws->gmax, shift, (int)kk, d_emb_ids, global_row0, ws->cand, ws->cand_cap,
-                         (u64*)d_out_keys, ws->out_scores, d_out_ids, d_out_count));
-    else
-        CU(launch_fullsort_topk(st, ws->scores, n, ws->gmax, shift, kk, d_emb_ids, global_row0, ws->sortbuf,
-                                (u64*)d_out_keys, ws->out_scores, d_out_ids, d_out_count));
-    ws->gmax_dirty = false;
-    return SVSB_OK;
+    if ((rc = similarity_phase(st, *ws, &g, s, d_query, 0)) != SVSB_OK) return rc;
+    return select_phase(st, *ws, &g, s, d_query, 0, kk, {(u64*)d_out_keys, ws->out_scores, d_out_ids, d_out_count});
 }
 
 extern "C" int svsb_launch_merge(svsb_ws_t* ws, void* stream, const uint64_t* d_keys, const int64_t* d_ids,

@@ -108,6 +108,9 @@ struct Generation {
     }
 };
 
+// Where a selection writes (select_phase): a workspace's outputs, pinned host memory or a record (RecordView).
+struct SelOut { u64* keys; float* scores; int64_t* ids; int32_t* count; };
+
 // per-device scratch for one in-flight query
 struct svsb_workspace {
     int dev = 0;
@@ -127,6 +130,8 @@ struct svsb_workspace {
     // (select.cu).  Set before the similarity launch, cleared once the selection is enqueued: a call that failed in
     // between leaves it set and the next user of this (pooled) workspace re-zeroes gmax first.
     bool gmax_dirty = false;
+    // pipelined paths: a selection of this set was enqueued on a side stream; ev_sel marks its end
+    bool sel_pending = false;
 
     int ensure_rows(int64_t n) {
         cudaSetDevice(dev);
@@ -192,6 +197,35 @@ struct svsb_workspace {
             CU(cudaMalloc(&mscr_ids, (size_t)entries * 8));
             mscr_cap = entries;
         }
+        return SVSB_OK;
+    }
+    // one query over n rows with outputs of `out` entries; the full sort's buffer too when it asks for k > K_FAST_MAX
+    int ensure_query(int64_t n, int64_t out, int64_t k) {
+        int rc;
+        if ((rc = ensure_rows(n)) != SVSB_OK) return rc;
+        if ((rc = ensure_out(out)) != SVSB_OK) return rc;
+        if (k > K_FAST_MAX && (rc = ensure_sort(n)) != SVSB_OK) return rc;
+        return SVSB_OK;
+    }
+    // a set of the pipelined peer paths (n rows, n = 0: none yet): K_FAST_MAX outputs and the events of its hand-offs
+    int ensure_set(int64_t n) {
+        int rc;
+        if (n > 0 && (rc = ensure_rows(n)) != SVSB_OK) return rc;
+        if ((rc = ensure_out(K_FAST_MAX)) != SVSB_OK) return rc;
+        if (!ev) CU(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
+        if (!ev_sel) CU(cudaEventCreateWithFlags(&ev_sel, cudaEventDisableTiming));
+        return SVSB_OK;
+    }
+    SelOut out() const { return {out_keys, out_scores, out_ids, out_count}; }
+    // the similarity pass on `from` is done before anything enqueued on `to` from now on
+    int hand_off(cudaStream_t from, cudaStream_t to) {
+        CU(cudaEventRecord(ev, from));
+        CU(cudaStreamWaitEvent(to, ev, 0));
+        return SVSB_OK;
+    }
+    // this set's previous selection (side stream) is done reading scores / group maxima before `on` overwrites them
+    int sel_wait(cudaStream_t on) const {
+        if (sel_pending) CU(cudaStreamWaitEvent(on, ev_sel, 0));
         return SVSB_OK;
     }
     void release() {
@@ -512,7 +546,6 @@ struct svsb_engine {
     std::vector<std::unique_ptr<DevWs>> shard_ws;        // workspaces for svsb_enqueue_local_topk (by slot)
     std::vector<cudaEvent_t> kev; size_t kev_used = 0;   // similarity-kernel timing events
     cudaStream_t side_st = nullptr;                      // selection kernels of the pipelined sharded path
-    std::vector<char> sel_pending;                       // per slot: a selection is (or was) in flight on side_st
     std::unique_ptr<Xchg> xchg;
     std::unique_ptr<BXchg> bxchg;
     std::unique_ptr<PairsShard> pairs;
@@ -525,7 +558,7 @@ struct svsb_engine {
 
 static inline int round_up4(int d) { return (d + 3) & ~3; }
 
-// host queries Q[b][d] -> dst[b][ld], zero padded to the rows' leading dimension (staging of the batched paths)
+// host queries Q[b][d] -> dst[b][ld], zero padded to the rows' leading dimension
 static inline void stage_queries(float* dst, const float* Q, int b, int d, int ld) {
     for (int i = 0; i < b; ++i) {
         memcpy(dst + (size_t)i * ld, Q + (size_t)i * d, (size_t)d * 4);
@@ -541,6 +574,17 @@ struct svsb_snapshot { std::shared_ptr<Generation> gen; };
 // ------------------------------------------------------------------------------------------------
 std::shared_ptr<Generation> pin(svsb_engine* e);
 int prepare_ws(DevWs& w, const Generation* g, const Shard& s, int64_t kk);
+// The two phases of one single query over shard s in workspace w.  The caller chooses the route (0 = K1, 16 / 8 = the
+// fp16 / int8 filter) and passes the same to both.  similarity_phase marks w's group maxima dirty and launches the pass
+// on st (pdl: under programmatic dependent launch; t: a pair of timing events around it, or null).  select_phase
+// enqueues the filter's threshold + exact re-score (route != 0), then the top min(k, s.n_live) rows into o: the
+// selection kernel (stamps, push: its options) or, for k > K_FAST_MAX, the full sort; and clears the mark.
+int similarity_phase(cudaStream_t st, DevWs& w, const Generation* g, const Shard& s, const float* q, int route,
+                     int reserve_sms = 0, bool pdl = false, cudaEvent_t* t = nullptr);
+int select_phase(cudaStream_t st, DevWs& w, const Generation* g, const Shard& s, const float* q, int route, int64_t k,
+                 const SelOut& o, u64* stamps = nullptr, const PeerPush* push = nullptr);
+// workspace set i of the sharded / peer paths (svsb_engine::shard_ws), created on the engine's device on first use
+DevWs& shard_slot(svsb_engine* e, size_t i);
 // Convert rows [buf->m16_rows, s.n) of the shard's fp16 shadow (rows from `fresh_from` on were (re)written: they are
 // converted again).  No shadow yet: create = 0 leaves it so (*out = null), 1 allocates it when the device keeps ample
 // room after it (else *out = null, not an error), 2 allocates it or fails.  The int8 shadow (ShardBuf::M8) is kept the

@@ -251,16 +251,10 @@ int multi_publish(svsb_engine* e, const std::shared_ptr<Generation>& g) {
         if (i == 0 && (rc = x->ws.ensure_merge_scratch((int64_t)nd * K_FAST_MAX)) != SVSB_OK) return rc;
         // the fused path is software-pipelined per device: two workspace sets alternate, selection + push run on a side stream
         if (!kid->side_st) CU(cudaStreamCreateWithFlags(&kid->side_st, cudaStreamNonBlocking));
-        if (kid->shard_ws.size() < 2) kid->shard_ws.resize(2);
-        if (kid->sel_pending.size() < 2) kid->sel_pending.resize(2, 0);
         for (int t = 0; t < 2; ++t) {
-            if (!kid->shard_ws[t]) { kid->shard_ws[t].reset(new DevWs()); kid->shard_ws[t]->dev = s.dev; }
-            DevWs& w = *kid->shard_ws[t];
-            if (s.n > 0 && (rc = w.ensure_rows(s.n)) != SVSB_OK) return rc;
+            DevWs& w = shard_slot(kid, t);
+            if ((rc = w.ensure_set(s.n)) != SVSB_OK) return rc;
             if (g->ld > 0 && (rc = w.ensure_q(g->ld)) != SVSB_OK) return rc;
-            if ((rc = w.ensure_out(K_FAST_MAX)) != SVSB_OK) return rc;
-            if (!w.ev) CU(cudaEventCreateWithFlags(&w.ev, cudaEventDisableTiming));
-            if (!w.ev_sel) CU(cudaEventCreateWithFlags(&w.ev_sel, cudaEventDisableTiming));
         }
         return SVSB_OK;
     });
@@ -277,7 +271,7 @@ struct FastJob {
     float* const* d_q = nullptr; int64_t q_off = 0; // ... or device-resident queries (bench): d_q[i] + q_off on device i
     float* out_scores = nullptr; int64_t* out_ids = nullptr; int32_t* out_count = nullptr;
     cudaEvent_t ev_done = nullptr;
-    cudaEvent_t kev0 = nullptr, kev1 = nullptr;    // optional bracket of device 0's similarity kernel
+    cudaEvent_t* kev = nullptr;                    // optional bracket (two events) of device 0's similarity kernel
 };
 
 // Per device, software-pipelined like the one-process-per-GPU loop (engine.cu: svsb_enqueue_query_peer): the similarity
@@ -291,7 +285,7 @@ static int kid_fast(Multi* m, int i, const FastJob& j) {
     const Generation* cg = j.g->child_gen[i].get();
     const Shard& s = cg->shards[0];
     const int set = (int)(j.seq & 1);
-    DevWs& w = *kid->shard_ws[set];
+    DevWs& w = shard_slot(kid, set);
     cudaStream_t st = x->st, side = kid->side_st;
     CU(cudaSetDevice(s.dev));
     const int slot = (int)(j.seq % (unsigned long long)xr->slots);
@@ -303,25 +297,19 @@ static int kid_fast(Multi* m, int i, const FastJob& j) {
         CU(launch_push_empty(side, push));
         return SVSB_OK;
     }
-    const int shift = group_shift_for(s.n);
-    const bool pipelined = sm_count(s.dev) > 8;
-    if (kid->sel_pending[set]) CU(cudaStreamWaitEvent(st, w.ev_sel, 0));   // the set's previous selection is done with it
+    int rc;
+    if ((rc = w.sel_wait(st)) != SVSB_OK) return rc;          // the set's previous selection is done with it
     const float* dq = j.d_q ? j.d_q[i] + j.q_off : w.d_q;
     if (!j.d_q) CU(launch_stage_query(st, j.h_q, w.d_q, cg->ld));
-    if (i == 0 && j.kev0) CU(cudaEventRecord(j.kev0, st));
-    w.gmax_dirty = true;
-    {   // the similarity kernel streams its first tiles under the staging kernel (programmatic dependent launch)
-        PdlScope pdl(!j.d_q && env_int("SVSB_PDL", 1) != 0);
-        CU(launch_gemv(st, s.dev, s.M, s.n, cg->d, cg->ld, dq, w.scores, w.gmax, shift, 0, 0, 0, pipelined ? 1 : 0, s.live));
-    }
-    if (i == 0 && j.kev1) CU(cudaEventRecord(j.kev1, st));
-    CU(cudaEventRecord(w.ev, st));
-    CU(cudaStreamWaitEvent(side, w.ev, 0));
-    CU(launch_select(side, w.scores, s.n, w.gmax, shift, (int)std::min<int64_t>(j.kk, s.n_live), s.ids, s.row0, w.cand, w.cand_cap,
-                     w.out_keys, w.out_scores, w.out_ids, w.out_count, nullptr, &push));
-    w.gmax_dirty = false;
+    // route 0 on purpose: the devices of a multi-device engine have no filter shadows and run K1.  The similarity kernel
+    // streams its first tiles under the staging kernel (programmatic dependent launch).
+    if ((rc = similarity_phase(st, w, cg, s, dq, 0, sm_count(s.dev) > 8 ? 1 : 0, !j.d_q && env_int("SVSB_PDL", 1) != 0,
+                               i == 0 ? j.kev : nullptr)) != SVSB_OK)
+        return rc;
+    if ((rc = w.hand_off(st, side)) != SVSB_OK) return rc;
+    if ((rc = select_phase(side, w, cg, s, dq, 0, j.kk, w.out(), nullptr, &push)) != SVSB_OK) return rc;
     CU(cudaEventRecord(w.ev_sel, side));
-    kid->sel_pending[set] = 1;
+    w.sel_pending = true;
     return SVSB_OK;
 }
 
@@ -394,8 +382,7 @@ int multi_submit(svsb_engine* e, const std::shared_ptr<Generation>& g, const flo
         CU(cudaHostAlloc(&t->h_q, (size_t)g->ld * 4, cudaHostAllocPortable));
         t->q_cap = g->ld;
     }
-    memcpy(t->h_q, q, (size_t)d * 4);
-    for (int i = d; i < g->ld; ++i) t->h_q[i] = 0.f;
+    stage_queries(t->h_q, q, 1, d, g->ld);
     t->gen = g;
     FastJob j; j.g = g.get(); j.kk = kk; j.h_q = t->h_q;
     const int rc = submit_locked(m, t, j, /*host_out=*/true);
@@ -453,8 +440,7 @@ static int multi_query_big(svsb_engine* e, const std::shared_ptr<Generation>& g,
         m->h_Q_cap = g->ld;
     }
     float* hq = m->h_Q;
-    memcpy(hq, q, (size_t)d * 4);
-    for (int i = d; i < g->ld; ++i) hq[i] = 0.f;
+    stage_queries(hq, q, 1, d, g->ld);
     if (kk > m->g_cap) {
         void* ptrs[] = {m->g_keys, m->g_ids, m->m_scores, m->m_ids};
         for (void* p : ptrs) if (p) cudaFree(p);
@@ -484,17 +470,9 @@ static int multi_query_big(svsb_engine* e, const std::shared_ptr<Generation>& g,
             const int64_t kl = std::min(kk, s.n_live);
             int rc2 = prepare_ws(w, cg, s, kl);
             if (rc2 != SVSB_OK) return rc2;
-            const int shift = group_shift_for(s.n);
             CU(cudaMemcpyAsync(w.d_q, hq, (size_t)cg->ld * 4, cudaMemcpyHostToDevice, x->st));
-            w.gmax_dirty = true;
-            CU(launch_gemv(x->st, s.dev, s.M, s.n, cg->d, cg->ld, w.d_q, w.scores, w.gmax, shift, 0, 0, 0, 0, s.live));
-            if (kl <= K_FAST_MAX)
-                CU(launch_select(x->st, w.scores, s.n, w.gmax, shift, (int)kl, s.ids, s.row0, w.cand, w.cand_cap,
-                                 w.out_keys, w.out_scores, w.out_ids, w.out_count));
-            else
-                CU(launch_fullsort_topk(x->st, w.scores, s.n, w.gmax, shift, kl, s.ids, s.row0, w.sortbuf,
-                                        w.out_keys, w.out_scores, w.out_ids, w.out_count));
-            w.gmax_dirty = false;
+            if ((rc2 = similarity_phase(x->st, w, cg, s, w.d_q, 0)) != SVSB_OK) return rc2;   // route 0: as in kid_fast
+            if ((rc2 = select_phase(x->st, w, cg, s, w.d_q, 0, kl, w.out())) != SVSB_OK) return rc2;
         }
         CU(cudaEventRecord(m->scratch[i].ev, x->st));
         return SVSB_OK;
@@ -717,7 +695,7 @@ int multi_bench_run(svsb_engine* e, const std::shared_ptr<Generation>& g, int32_
             if (rc != SVSB_OK) return rc;
         }
         FastJob j; j.g = g.get(); j.kk = kk; j.d_q = e->bench_q.data(); j.q_off = (int64_t)(it % e->bench_nq) * e->bench_ld;
-        if (ktime && it % KTIME_EVERY == 0) { j.kev0 = m->kev[2 * it]; j.kev1 = m->kev[2 * it + 1]; }
+        if (ktime && it % KTIME_EVERY == 0) j.kev = &m->kev[2 * it];
         std::unique_lock<std::mutex> lk(m->mu);
         svsb_ticket* t = free_ticket_locked(m, lk);
         if (!t) return fail(SVSB_E_STATE, "svsb_bench_run: no free ticket (pending svsb_query_submit handles?)");

@@ -603,3 +603,54 @@ def test_peer_windows_over_cuda_ipc_in_two_processes():
         assert len(many) == len(qs)
         for q, got in zip(qs, many):
             oracle.compare_retrieval(got, oracle.superheavy(m, ids, q, k), oracle.scores_of(m, q), ids)
+
+
+def test_stateless_local_topk_matches_the_oracle():
+    """svsb_launch_local_topk on caller-owned memory: one shard's rows at global row `row0`, d not a multiple of 4 (ld
+    padded), from one result through the selection kernel's largest k to the full sort of all n rows.  Keys carry the
+    global row; scores and ids are the single-device engine's, bit for bit."""
+    torch = pytest.importorskip("torch")
+    import ctypes as C
+    import svs_b200
+    from svs_b200 import _lib
+    lib = _lib.load()
+    n, d, ld, row0 = 20_011, 190, 192, 1_000_000
+    m = oracle.synth_matrix_uniform(n, d, 31)
+    m[5] = m[n - 2]                                            # an exact tie
+    ids = np.cumsum(np.random.default_rng(32).integers(1, 4, size=n)).astype(np.int64)
+    q = oracle.synth_queries(1, d, 33)[0]
+    dev = torch.device("cuda", 0)
+    dm = torch.zeros((n, ld), dtype=torch.float32, device=dev)
+    dm[:, :d] = torch.from_numpy(m).to(dev)
+    dq = torch.zeros(ld, dtype=torch.float32, device=dev)
+    dq[:d] = torch.from_numpy(q).to(dev)
+    di = torch.from_numpy(ids).to(dev)
+    ws = C.c_void_p()
+    _lib.check(lib.svsb_ws_create(0, 0, 1, C.byref(ws)))      # grown by the calls below
+    try:
+        with svs_b200.Engine([0]) as one:
+            one.load(m, ids)
+            for k in (1, 100, 2048, 2049, n):
+                keys = torch.zeros(k, dtype=torch.int64, device=dev)
+                out_ids = torch.zeros(k, dtype=torch.int64, device=dev)
+                cnt = torch.zeros(1, dtype=torch.int32, device=dev)
+                st = torch.cuda.current_stream().cuda_stream
+                _lib.check(lib.svsb_launch_local_topk(ws, C.c_void_p(st), C.c_void_p(dm.data_ptr()), n, d, ld,
+                                                      C.c_void_p(di.data_ptr()), row0, C.c_void_p(dq.data_ptr()), k,
+                                                      C.c_void_p(keys.data_ptr()), C.c_void_p(out_ids.data_ptr()),
+                                                      C.c_void_p(cnt.data_ptr())))
+                torch.cuda.synchronize()
+                assert int(cnt.item()) == k
+                kh = keys.cpu().numpy().view(np.uint64)
+                o = (kh >> np.uint64(32)).astype(np.uint32)        # order-preserving score bits (common.cuh make_key)
+                scores = np.where(o & np.uint32(0x80000000), o & np.uint32(0x7fffffff), ~o).astype(np.uint32).view(np.float32)
+                rows = ~(kh & np.uint64(0xffffffff)).astype(np.uint32)
+                got_ids = out_ids.cpu().numpy()
+                assert np.array_equal(ids[rows.astype(np.int64) - row0], got_ids)
+                oracle.compare_retrieval(list(zip(scores.tolist(), got_ids.tolist())), oracle.superheavy(m, ids, q, k),
+                                         oracle.scores_of(m, q), ids)
+                want = one.query(q, k)
+                assert np.array_equal(scores.view(np.uint32), want[0].view(np.uint32))
+                assert np.array_equal(got_ids, want[1])
+    finally:
+        lib.svsb_ws_destroy(ws)
