@@ -179,6 +179,11 @@ int svsb_host_free(void* p);
 /* Diagnostics of the last batch chunk (<= 2048 queries): coarse candidates per query, rows re-scored exactly per
  * query, flag word per query (0 = answered by the coarse path; otherwise it took the single-query kernels). */
 int svsb_batch_stats(svsb_t* e, int32_t b, int32_t* candidates, int32_t* rescored, int32_t* flags);
+/* Diagnostics of the last batch chunk: query q's coarse candidate list -- up to `cap` keys (score bits in the
+ * engine's order << 32 | ~row, the score being the coarse tensor-core value) -- its count (above the list's capacity,
+ * SVSB_BATCH_CAND_CAP, when the list overflowed; only that many keys exist) and its eps, the bound on
+ * |coarse - exact| the thresholds use.  keys and eps may be NULL. */
+int svsb_batch_candidates(svsb_t* e, int32_t q, int64_t cap, uint64_t* keys, int32_t* count, float* eps);
 /* Diagnostics of the last svsb_bench_run: *filter = 1 when its queries took the fp16 filter (a pass over the fp16
  * shadow, then an exact fp32 re-score of the candidate rows), 0 for the fp32 similarity kernel; *rescored = rows the
  * last query re-scored exactly (0 without the filter). */

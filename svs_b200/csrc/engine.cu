@@ -1812,6 +1812,25 @@ extern "C" int svsb_batch_stats(svsb_t* e, int32_t b, int32_t* candidates, int32
     return SVSB_OK;
 }
 
+// Diagnostics: query q's coarse candidate list of the last chunk (keys make_key(coarse score, row), in the order the
+// coarse pass appended them), its full count (above the list's capacity when the list overflowed) and its eps.  The
+// refine kernels only read the lists, so they are intact after the batch has been answered.
+extern "C" int svsb_batch_candidates(svsb_t* e, int32_t q, int64_t cap, uint64_t* keys, int32_t* count, float* eps) {
+    if (!e || !count) return fail(SVSB_E_INVALID, "svsb_batch_candidates: NULL argument");
+    std::lock_guard<std::mutex> lk(e->batch_mu);
+    BatchWs* w = e->batch_ws.get();
+    if (!w || q < 0 || q >= w->cap_b || !w->cand) return fail(SVSB_E_STATE, "svsb_batch_candidates: no batch has run with that query");
+    CU(cudaSetDevice(w->dev));
+    CU(cudaStreamSynchronize(w->st));
+    int32_t cnt = 0;
+    CU(cudaMemcpy(&cnt, w->cand_cnt + q, 4, cudaMemcpyDeviceToHost));
+    *count = cnt;
+    const int64_t m = std::min<int64_t>(std::min<int64_t>(cnt, w->cand_cap), std::max<int64_t>(cap, 0));
+    if (keys && m > 0) CU(cudaMemcpy(keys, w->cand + (size_t)q * w->cand_cap, (size_t)m * 8, cudaMemcpyDeviceToHost));
+    if (eps) CU(cudaMemcpy(eps, w->eps + q, 4, cudaMemcpyDeviceToHost));
+    return SVSB_OK;
+}
+
 extern "C" int svsb_batch_threshold_mode(svsb_t* e) {
     if (!e) return fail(SVSB_E_INVALID, "engine is NULL");
     auto g = pin(e);

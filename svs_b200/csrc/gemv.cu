@@ -47,9 +47,14 @@ gemv_ldg_kernel(const float4* __restrict__ M, int64_t n, int d4, const float4* _
             int64_t rr = r0 + r; if (rr > n - 1) rr = n - 1;     // tail rows alias the last row (discarded)
             rowp[r] = M + rr * (int64_t)d4;
         }
-        float4 acc[R];
+        // K1's summation order, bit for bit the one of gemv_tma_kernel (which every exact path copies): lane l owns
+        // chunks l, l+32, ...; the lane's even chunks accumulate into one float4, its odd ones into another.  a0 always
+        // holds the accumulator of the NEXT chunk's parity: chunk u of an unrolled step goes to a0 when u is even, and
+        // after a step of an odd number of chunks the two trade places.  The combine adds them pairwise, which commutes,
+        // so it does not matter which of the two ends up holding the even chunks.
+        float4 a0[R], a1[R];
 #pragma unroll
-        for (int r = 0; r < R; ++r) acc[r] = make_float4(0.f, 0.f, 0.f, 0.f);
+        for (int r = 0; r < R; ++r) { a0[r] = make_float4(0.f, 0.f, 0.f, 0.f); a1[r] = a0[r]; }
 
         int c = lane;
         for (; c + 32 * (U - 1) < d4; c += 32 * U) {
@@ -62,7 +67,11 @@ gemv_ldg_kernel(const float4* __restrict__ M, int64_t n, int d4, const float4* _
             for (int u = 0; u < U; ++u) {
                 const float4 qv = sq[c + 32 * u];
 #pragma unroll
-                for (int r = 0; r < R; ++r) fma4(acc[r], m[u][r], qv);
+                for (int r = 0; r < R; ++r) fma4((u & 1) ? a1[r] : a0[r], m[u][r], qv);
+            }
+            if (U & 1) {
+#pragma unroll
+                for (int r = 0; r < R; ++r) { const float4 t = a0[r]; a0[r] = a1[r]; a1[r] = t; }
             }
         }
         for (; c < d4; c += 32) {
@@ -71,14 +80,14 @@ gemv_ldg_kernel(const float4* __restrict__ M, int64_t n, int d4, const float4* _
             for (int r = 0; r < R; ++r) m[r] = ldg_stream(rowp[r] + c);
             const float4 qv = sq[c];
 #pragma unroll
-            for (int r = 0; r < R; ++r) fma4(acc[r], m[r], qv);
+            for (int r = 0; r < R; ++r) { fma4(a0[r], m[r], qv); const float4 t = a0[r]; a0[r] = a1[r]; a1[r] = t; }
         }
 
         u64 kmax = 0;
         float mine = 0.f;
 #pragma unroll
         for (int r = 0; r < R; ++r) {
-            float s = warp_sum((acc[r].x + acc[r].y) + (acc[r].z + acc[r].w));
+            float s = warp_sum(((a0[r].x + a1[r].x) + (a0[r].y + a1[r].y)) + ((a0[r].z + a1[r].z) + (a0[r].w + a1[r].w)));
             if (live && r0 + r < n && !live[r0 + r]) s = dead_score();      // tombstoned row: sorts below every real score
             if (r0 + r < n) {
                 u64 key = make_key(s, (uint32_t)(r0 + r));

@@ -305,6 +305,20 @@ class Engine:
         check(self._lib.svsb_batch_stats(self._h, b, cand.ctypes.data, resc.ctypes.data, flags.ctypes.data))
         return cand, resc, flags
 
+    def batch_candidates(self, q: int) -> Tuple[np.ndarray, np.ndarray, int, float]:
+        """Query q's coarse candidates of the last batch chunk: (coarse scores float32[c], rows int64[c], count, eps).
+        count above c means the list overflowed its capacity (SVSB_BATCH_CAND_CAP); rows are the shard's rows."""
+        cnt, eps = C.c_int32(), C.c_float()
+        check(self._lib.svsb_batch_candidates(self._h, int(q), 0, None, C.byref(cnt), C.byref(eps)))
+        keys = np.zeros(max(cnt.value, 0), dtype=np.uint64)
+        check(self._lib.svsb_batch_candidates(self._h, int(q), len(keys), keys.ctypes.data if len(keys) else None,
+                                              C.byref(cnt), None))
+        keys = keys[keys != 0]        # an overflowed list holds only its capacity; a real key is never 0 (its row < 2^32 - 1)
+        hi = (keys >> np.uint64(32)).astype(np.uint32)               # key_score: the ordered transform, undone
+        b = np.where(hi & np.uint32(0x80000000), hi & np.uint32(0x7FFFFFFF), ~hi).astype(np.uint32)
+        rows = (~(keys & np.uint64(0xFFFFFFFF)).astype(np.uint32)).astype(np.int64)    # key_row
+        return b.view(np.float32), rows, cnt.value, eps.value
+
     def bench_filter_stats(self) -> Tuple[bool, int]:
         """(took the fp16 filter, rows the last query re-scored exactly) of the last bench_run."""
         f, r = C.c_int32(), C.c_int64()

@@ -90,12 +90,20 @@ def test_the_plain_c_oracle_accepts_the_engine_too(engine):
 
 @pytest.mark.parametrize("tune_a", ["1", "2", "3", "4", "5", "6", "7", "8", "9"])
 def test_every_ldg_instantiation_is_correct(engine, tune_a, monkeypatch):
+    """Every LDG instantiation returns K1's bits (oracle/k1_exact.py), not just scores within the oracle's tolerance."""
+    import sys
+    sys.path.insert(0, os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "oracle"))
+    import k1_exact
     monkeypatch.setenv("SVSB_GEMV_VARIANT", "1")
     monkeypatch.setenv("SVSB_GEMV_TUNE_A", tune_a)
     m = oracle.synth_matrix_uniform(30_011, 1536, 3)
     ids = np.arange(1, len(m) + 1, dtype=np.int64)
     engine.load(m, ids)
-    _check(engine, m, ids, oracle.synth_queries(1, 1536, 4)[0], 100)
+    q = oracle.synth_queries(1, 1536, 4)[0]
+    _check(engine, m, ids, q, 100)
+    s, i = engine.query(q, 100)
+    want_bits, want_ids = k1_exact.k1_topk_exact(m, ids, q, 100)
+    assert np.array_equal(s.view(np.uint32), want_bits) and np.array_equal(i, want_ids)
 
 
 def test_reference_unit_test_matrix_and_uninormalised_rows(engine):
