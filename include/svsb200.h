@@ -121,6 +121,33 @@ int svsb_apply_mutations(svsb_t* e, const int64_t* del_ids, int64_t n_del, const
 /* Physical rows of the resident generation (tombstoned ones included) and live rows (== svsb_shape's n). */
 int svsb_generation_rows(svsb_t* e, int64_t* physical, int64_t* live);
 
+/* The same update for one rank of the one-process-per-GPU deployment, in two phases, so that no rank publishes unless
+ * every rank can.  Every rank calls both with the same arguments (SPMD); this engine owns one device.
+ *   svsb_shard_mutations_prepare  builds the next generation of this rank's shard off to the side and keeps it pending in
+ *                            the engine; nothing is published.  A delete id that is not a live row of THIS shard is not an
+ *                            error: *found counts the ones that were.  *max_live_id: this shard's largest live id after
+ *                            the deletes (INT64_MIN: none).  Only the rank with append_here != 0 (the last rank) appends
+ *                            the rows, and it does everything that can fail there: buffer growth, row copy, norm kernel,
+ *                            shadows.  Preconditions as svsb_apply_mutations (ids ascending, d, no duplicate delete ids,
+ *                            2^32 rows counted from svsb_set_shard's offset); SVSB_E_STATE also while another update is
+ *                            pending or a load runs.  The caller accepts the update only if every rank succeeded, the
+ *                            found counts add up to n_del and add_ids[0] is above every rank's max_live_id.
+ *   svsb_shard_mutations_commit   publish != 0 publishes the pending generation, 0 drops it (a no-op when nothing is
+ *                            pending).  It allocates nothing and cannot fail after a successful prepare.
+ * A pending generation blocks loads, updates and svsb_compact until it is committed or dropped; svsb_invalidate and
+ * svsb_destroy drop it. */
+int svsb_shard_mutations_prepare(svsb_t* e, const int64_t* del_ids, int64_t n_del, const float* add_rows, const int64_t* add_ids,
+                                 int64_t n_add, int32_t d, int32_t append_here, int64_t* found, int64_t* max_live_id);
+int svsb_shard_mutations_commit(svsb_t* e, int32_t publish, uint64_t* generation);
+/* Compaction on the device (single-device engines; a multi-device engine gets SVSB_E_INVALID): gathers the live rows of
+ * the resident generation, in row order, into a new buffer and publishes them as a tombstone-free generation whose first
+ * row is global row global_row0 (svsb_set_shard's offset is set to it in the same call).  The result equals a fresh load
+ * of the live rows at that offset: rows, ids, shape, svsb_norm_stats in check mode (normalised rows keep their old,
+ * conservative statistics), shadows and every answer.  Queries and snapshots pinned to the old generation keep reading it,
+ * so for a moment the shard is held twice: SVSB_E_NOMEM when that memory is not there, and nothing is published.  A
+ * generation without tombstones keeps its buffers and only moves to the new offset. */
+int svsb_compact(svsb_t* e, int64_t global_row0, uint64_t* generation);
+
 /* _EmbeddingsMatrix.invalidate (src/svs/kb.py:861-864; call sites kb.py:984,1062,1086,1455,1523,1541). */
 int svsb_invalidate(svsb_t* e);
 /* Cache-hit test of get_sync / get (src/svs/kb.py:867, 880).  Returns 1 / 0. */

@@ -52,6 +52,10 @@ SIGNATURES = {
     "svsb_query_wait": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, c_i32_p]),
     "svsb_apply_mutations": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, c_u64_p]),
     "svsb_generation_rows": (C.c_int, [C.c_void_p, c_i64_p, c_i64_p]),
+    "svsb_shard_mutations_prepare": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_int64, C.c_int32,
+                                               C.c_int32, c_i64_p, c_i64_p]),
+    "svsb_shard_mutations_commit": (C.c_int, [C.c_void_p, C.c_int32, c_u64_p]),
+    "svsb_compact": (C.c_int, [C.c_void_p, C.c_int64, c_u64_p]),
     "svsb_snapshot_rows": (C.c_int, [C.c_void_p, c_i64_p, c_i64_p]),
     "svsb_snapshot_acquire": (C.c_int, [C.c_void_p, C.POINTER(C.c_void_p)]),
     "svsb_snapshot_release": (None, [C.c_void_p]),

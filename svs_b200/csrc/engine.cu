@@ -191,6 +191,7 @@ extern "C" void svsb_destroy(svsb_t* e) {
     for (size_t i = 0; i < e->devs.size(); ++i) { cudaSetDevice(e->devs[i]); cudaDeviceSynchronize(); }
     e->loading.reset();
     e->current.reset();
+    e->pending.reset();
     for (auto& c : e->pool_free) ctx_destroy(e, c.get());
     e->pool_free.clear();
     if (e->bench_ctx) ctx_destroy(e, e->bench_ctx.get());
@@ -214,6 +215,7 @@ extern "C" void svsb_destroy(svsb_t* e) {
 // load path
 // ------------------------------------------------------------------------------------------------
 int alloc_generation(svsb_engine* e, int64_t n, int d, std::shared_ptr<Generation>& out) {
+    if (e->has_pending) return fail(SVSB_E_STATE, "a prepared update is pending: svsb_shard_mutations_commit before loading");
     std::shared_ptr<Generation> g(new Generation());
     g->n = n; g->d = d; g->ld = round_up4(d);
     const int64_t nd = (int64_t)e->devs.size();
@@ -234,9 +236,7 @@ int alloc_generation(svsb_engine* e, int64_t n, int d, std::shared_ptr<Generatio
         CU(cudaSetDevice(s.dev));
         s.buf.reset(new ShardBuf());
         s.buf->dev = s.dev;
-        // a little head-room (0.4 %, at least 1024 rows): the first incremental appends (svsb_apply_mutations) then go in
-        // place instead of paying for a re-allocation and a device-to-device copy of the whole shard
-        const int64_t cap = s.n + std::max<int64_t>(1024, s.n / 256);
+        const int64_t cap = shard_capacity(s.n);
         CU(cudaMalloc(&s.buf->M, (size_t)cap * g->ld * 4));
         CU(cudaMalloc(&s.buf->ids, (size_t)cap * 8));
         s.buf->cap_rows = cap;
@@ -460,7 +460,13 @@ extern "C" int svsb_load_synthetic(svsb_t* e, int64_t n, int32_t d, uint64_t see
 extern "C" int svsb_invalidate(svsb_t* e) {
     if (!e) return fail(SVSB_E_INVALID, "engine is NULL");
     std::shared_ptr<Generation> old;
-    { std::lock_guard<std::mutex> lk(e->mu); old.swap(e->current); }
+    std::shared_ptr<Generation> pending;
+    {
+        std::lock_guard<std::mutex> lk(e->mu);
+        old.swap(e->current);
+        pending.swap(e->pending);                    // a prepared update of the dropped generation is dropped with it
+        e->has_pending = false;
+    }
     return SVSB_OK;          // `old` (and its device memory) dies here unless a query still pins it
 }
 
@@ -469,8 +475,6 @@ extern "C" int svsb_is_loaded(svsb_t* e) {
     std::lock_guard<std::mutex> lk(e->mu);
     return e->current ? 1 : 0;
 }
-
-static int filter_attach(svsb_engine* e, Generation* g);
 
 int publish_generation(svsb_engine* e, const std::shared_ptr<Generation>& g, uint64_t* generation) {
     int rc = filter_attach(e, g.get());
@@ -624,7 +628,7 @@ int shadow_sync(const Shard& s, int ld, int64_t fresh_from, int create, cudaStre
 // SVSB_FILTER_MIN_MB, default 512 MB of fp32 rows.  Measured on a B200 (profiles/r05_filter_ab.txt, 1536-d rows): at
 // 246 MB K1's pass is still faster than filter + threshold + re-score, at 492 MB the filter takes 25 % less time.
 // The int8 shadow is built with it when it fits as well (shadow_sync).
-static int filter_attach(svsb_engine* e, Generation* g) {
+int filter_attach(svsb_engine* e, Generation* g) {
     for (auto& s : g->shards) { s.M16 = nullptr; s.M8 = nullptr; }
     if (e->devs.size() != 1 || e->is_kid || g->shards.size() != 1) return SVSB_OK;
     Shard& s = g->shards[0];

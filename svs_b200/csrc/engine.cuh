@@ -554,6 +554,10 @@ struct svsb_engine {
     struct Multi* multi = nullptr;
     bool is_kid = false;                                 // a per-device shard engine owned by a multi-device engine
     std::mutex mutate_mu;                                // one svsb_apply_mutations / load publication at a time
+    // svsb_shard_mutations_prepare's generation until svsb_shard_mutations_commit publishes or drops it (set under mu and
+    // mutate_mu); while it is pending, loads, updates and compactions are refused
+    std::shared_ptr<Generation> pending;
+    std::atomic<bool> has_pending{false};
 };
 
 static inline int round_up4(int d) { return (d + 3) & ~3; }
@@ -592,6 +596,11 @@ DevWs& shard_slot(svsb_engine* e, size_t i);
 int shadow_sync(const Shard& s, int ld, int64_t fresh_from, int create, cudaStream_t st, void** out);
 int engine_create(const int* device_ids, int n_dev, bool as_kid, svsb_engine** out);
 int alloc_generation(svsb_engine* e, int64_t n, int d, std::shared_ptr<Generation>& out);
+// rows a load allocates for a shard of n rows: a little head-room (0.4 %, at least 1024 rows), so the first incremental
+// appends (svsb_apply_mutations) go in place instead of paying for a re-allocation and a device-to-device copy of the shard
+static inline int64_t shard_capacity(int64_t n) { return n + std::max<int64_t>(1024, n / 256); }
+// the filters' shadows of a single-device generation about to be published (engine.cu; part of publish_generation)
+int filter_attach(svsb_engine* e, Generation* g);
 int finish_generation(svsb_engine* e, Generation* g, int norm_mode);
 // publish `g` as the engine's resident generation (assigns the id; builds the per-device views of a multi-device engine)
 int publish_generation(svsb_engine* e, const std::shared_ptr<Generation>& g, uint64_t* generation);

@@ -205,6 +205,14 @@ class Engine:
                                              C.byref(gen)))
         return gen.value
 
+    def compact(self, global_row0: int = 0) -> int:
+        """Gather the live rows of a tombstoned generation into a new buffer on the device and publish them as a
+        tombstone-free generation whose first row is global row `global_row0` (include/svsb200.h: svsb_compact).  The
+        result equals a fresh load of the live rows.  Single-device engines only; returns the new generation."""
+        gen = C.c_uint64()
+        check(self._lib.svsb_compact(self._h, int(global_row0), C.byref(gen)))
+        return gen.value
+
     def generation_rows(self) -> Tuple[int, int]:
         """(physical rows incl. tombstoned ones, live rows) of the resident generation."""
         p, l = C.c_int64(), C.c_int64()

@@ -23,6 +23,7 @@ import numpy as np
 
 from . import _lib
 from .engine import Engine, Snapshot
+from .mutations import compaction_due
 
 _LOG = logging.getLogger(__name__)
 
@@ -208,8 +209,7 @@ class DeviceEmbeddingsMatrix:
             return None
         # past this fraction of dead rows a rebuild (which also compacts) is the better deal
         physical, live = self._engine.generation_rows()
-        dead_after = physical - live + len(dels)
-        if dead_after > 64 and dead_after * 4 > physical + len(add_ids):
+        if compaction_due(physical + len(add_ids), physical - live + len(dels)):
             return None
         rows = np.frombuffer(b"".join(blobs), dtype="<f4").reshape(len(blobs), d) if blobs else None
         try:

@@ -28,6 +28,13 @@ _DELETE = "DELETE FROM EMBEDDINGS WHERE ID = ?;"
 _WRITE_VERBS = ("INSERT", "DELETE", "UPDATE", "REPLACE", "DROP", "ALTER", "CREATE", "VACUUM")
 
 
+
+def compaction_due(physical: int, dead: int) -> bool:
+    """Past this fraction of dead (tombstoned) rows among `physical` rows, compacting is the better deal than further
+    incremental updates: every query still streams the dead rows."""
+    return dead > 64 and dead * 4 > physical
+
+
 class MutationLog:
     """Per-database log.  Thread-safe: AsyncKB runs the querier in executor threads."""
 

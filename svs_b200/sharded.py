@@ -12,8 +12,8 @@ No reduction over scores is needed: rows are independent (splitting D instead wo
 of N floats).
 
 k > 2048 (up to the full ranking n = N) takes its own path under either exchange: every rank fully sorts its shard's
-keys into one record of cap = min(k, ceil(N / world)) entries -- no shard holds more rows, so every record is complete
---, the ranks agree on the outcome of that local phase, all-gather the records and rank-merge the sorted lists on every
+keys into one record of cap = min(k, live rows of the largest shard) entries (ceil(N / world) after a load) -- no shard
+holds more rows, so every record is complete --, the ranks agree on the outcome of that local phase, all-gather the records and rank-merge the sorted lists on every
 rank (include/svsb200.h svsb_enqueue_merge_sorted_records).
 
 Single queries do not call a collective at all by default (`exchange="peer"`): steps 2 and 3 are fused into the
@@ -30,6 +30,13 @@ its peers' rows -- with its own threshold, re-scores its survivors exactly and k
 lists (at most 20 bytes x n per rank) and a rank merge on every rank give every rank the single-device answer, bit for
 bit (include/svsb200.h svsb_pairs_*).
 
+Incremental adds and deletes (`apply_mutations`) are collective: every rank builds its shard's next generation off to
+the side, the ranks all-gather what they found, and every rank then publishes it or every rank drops it
+(include/svsb200.h svsb_shard_mutations_*).  Appends always go to the last rank, which keeps global row order equal to
+id order (the merges' tie-break), so the last shard grows and sets the query time until a load rebalances.  `compact`
+gathers every shard's live rows on its device at the prefix sum of the live counts (svsb_compact); the pair path and
+updates past the drop-in's dead-row fraction run it.
+
 The collective / packing / batching logic is backend-agnostic so that it can be exercised on CPU with
 `gloo` (tests/test_sharded_gloo.py and tests/test_sharded_pairs_gloo.py inject NumPy backends); the product backend is
 `CudaShardBackend`.
@@ -41,7 +48,8 @@ from typing import List, Optional, Tuple
 
 import numpy as np
 
-from ._lib import K_FAST_MAX, SVSB_E_CUDA, SVSB_E_NOMEM, EngineError
+from ._lib import K_FAST_MAX, SVSB_E_CUDA, SVSB_E_NOMEM, SVSB_E_STATE, EngineError
+from .mutations import compaction_due
 
 MICRO_BATCH = 16
 TIME_EVERY = 8        # bracket one similarity launch in 8 with timing events (two records cost ~5 us of stream time)
@@ -84,6 +92,23 @@ class CudaShardBackend:
         self.engine.load_synthetic(n_local, d, seed, id0, id_step)
         self.d = d
         self.ld = (d + 3) & ~3
+
+    def mutations_prepare(self, del_ids: np.ndarray, add_ids: np.ndarray, add_rows: np.ndarray, append_here: bool) -> Tuple[int, int]:
+        """Build this shard's next generation and keep it pending (svsb_shard_mutations_prepare): (delete ids found
+        here, largest live id after the deletes)."""
+        found, max_live = C.c_int64(), C.c_int64()
+        n_del, n_add = len(del_ids), len(add_ids)
+        self._check(self._lib.svsb_shard_mutations_prepare(self.engine._h, del_ids.ctypes.data if n_del else None, n_del,
+                                                           add_rows.ctypes.data if n_add else None, add_ids.ctypes.data if n_add else None,
+                                                           n_add, add_rows.shape[1] if n_add else 0, 1 if append_here else 0,
+                                                           C.byref(found), C.byref(max_live)))
+        return found.value, max_live.value
+
+    def mutations_commit(self, publish: bool) -> None:
+        self._check(self._lib.svsb_shard_mutations_commit(self.engine._h, 1 if publish else 0, None))
+
+    def compact(self, global_row0: int) -> None:
+        self.engine.compact(global_row0)
 
     def device_queries(self, Q: np.ndarray):
         """(nq, d) host float32 -> (nq, ld) device tensor, zero padded, staged through a cached pinned buffer."""
@@ -342,7 +367,9 @@ class ShardedRetriever:
         self.n = 0
         self.d = 0
         self.row0 = 0
-        self.local_rows = 0
+        self.local_rows = 0              # live rows of this rank's shard
+        self._shard_live = [0] * world   # live rows of every rank's shard
+        self._shard_rows = [0] * world   # physical rows (tombstoned ones included) of every rank's shard
         self._queries = None
         self._bufs = {}
         self._big = None                 # (cap, record, gathered records, outputs) of the large-k path: one set at a time
@@ -358,7 +385,7 @@ class ShardedRetriever:
         self.n, self.d = n, d
         self._epoch += 1
         self._big = None
-        self.row0, self.local_rows = partition(n, self.world, self.rank)
+        self._set_partition()
         self.backend.set_shard(self.row0)
         self.backend.load_synthetic(self.local_rows, d, seed, id0, id_step)
 
@@ -367,10 +394,83 @@ class ShardedRetriever:
         self.n, self.d = rows.shape
         self._epoch += 1
         self._big = None
-        self.row0, self.local_rows = partition(self.n, self.world, self.rank)
+        self._set_partition()
         self.backend.set_shard(self.row0)
         sl = slice(self.row0, self.row0 + self.local_rows)
         self.backend.load_rows(np.ascontiguousarray(rows[sl]), np.ascontiguousarray(emb_ids[sl]))
+
+    def _set_partition(self) -> None:
+        self.row0, self.local_rows = partition(self.n, self.world, self.rank)
+        self._shard_live = [partition(self.n, self.world, r)[1] for r in range(self.world)]
+        self._shard_rows = list(self._shard_live)
+
+    # -- incremental updates ---------------------------------------------------------------------
+    def apply_mutations(self, del_ids, add_ids, add_rows: Optional[np.ndarray] = None) -> None:
+        """Delete the rows with embeddings.id in `del_ids` and append `add_rows` (len(add_ids), d) with ids `add_ids`
+        (ascending, above every live id) on every rank, as Engine.apply_mutations does on one device.  Collective: every
+        rank passes the same arguments.  Either every rank publishes the update or none does and every rank raises the
+        same EngineError (SVSB_E_STATE: a delete id that is not a live row, ids not above every live id, ...), with the
+        resident rows unchanged.  Past the drop-in's dead-row fraction the shards are compacted afterwards."""
+        dels = np.ascontiguousarray(np.asarray(del_ids, dtype=np.int64).reshape(-1))
+        aids = np.ascontiguousarray(np.asarray(add_ids, dtype=np.int64).reshape(-1))
+        n_add = len(aids)
+        rows = np.zeros((0, 0), np.float32)
+        if n_add:
+            rows = np.ascontiguousarray(add_rows, dtype=np.float32)
+            if rows.ndim != 2 or rows.shape[0] != n_add:
+                raise ValueError("add_rows must be (len(add_ids), d)")
+        last = self.rank == self.world - 1
+        try:
+            found, max_live = self.backend.mutations_prepare(dels, aids, rows, last)
+            outcome = (0, "", found, max_live, self.local_rows - found + (n_add if last else 0))
+        except EngineError as ex:
+            outcome = (ex.code, ex.message, 0, 0, 0)
+        got = self._all_gather_object(outcome)
+        refusal = next(((g[0], g[1]) for g in got if g[0] != 0), None)
+        missing = len(dels) - sum(g[2] for g in got)
+        if refusal is None and missing:
+            refusal = (SVSB_E_STATE, f"sharded apply_mutations: {missing} of {len(dels)} deleted ids are not live rows of the "
+                                     "resident matrix (rebuild)")
+        if refusal is None and n_add and aids[0] <= max(g[3] for g in got):
+            refusal = (SVSB_E_STATE, "sharded apply_mutations: an inserted id is not above every live id (rebuild)")
+        self.backend.mutations_commit(refusal is None)          # every rank publishes, or every rank drops its build
+        if refusal is not None:
+            raise EngineError(*refusal)
+        self._shard_live = [g[4] for g in got]
+        self._shard_rows[-1] += n_add
+        self._rows_changed()
+        if compaction_due(sum(self._shard_rows), sum(self._shard_rows) - self.n):
+            self.compact()
+
+    def compact(self) -> None:
+        """Collective: every rank gathers its shard's live rows on its device (svsb_compact), at the prefix sum of the
+        ranks' live counts, so rows stay contiguous in rank order.  If a rank cannot (SVSB_E_NOMEM), the ranks that did
+        move back to their old first rows -- without an allocation, their shards have no tombstones left -- so that the
+        shards' global rows stay disjoint and ordered, and every rank raises the same EngineError."""
+        live = self._all_gather_object(self.local_rows)
+        row0 = sum(live[:self.rank])
+        try:
+            self.backend.compact(row0)
+            outcome = (0, "")
+        except EngineError as ex:
+            outcome = (ex.code, ex.message)
+        got = self._all_gather_object(outcome)
+        refusal = next((g for g in got if g[0] != 0), None)
+        if refusal is None:
+            self.row0 = row0
+        elif outcome[0] == 0 and row0 != self.row0:
+            self.backend.compact(self.row0)
+        self._shard_rows = [lv if g[0] == 0 else r for lv, g, r in zip(live, got, self._shard_rows)]
+        self._rows_changed()
+        if refusal is not None:
+            raise EngineError(*refusal)
+
+    def _rows_changed(self) -> None:
+        """The resident rows changed: everything derived from them is rebuilt on next use."""
+        self.local_rows = self._shard_live[self.rank]
+        self.n = sum(self._shard_live)
+        self._epoch += 1
+        self._big = None
 
     def _all_gather_object(self, obj) -> list:
         if self.world == 1:
@@ -661,7 +761,7 @@ class ShardedRetriever:
     def _retrieve_big(self, q: np.ndarray, k: int) -> Tuple[np.ndarray, np.ndarray]:
         """superheavy() for 2048 < k <= N, on every rank, through the collective under either exchange (the peer
         windows are sized for k <= 2048)."""
-        cap = min(k, -(-self.n // self.world))                     # rows of the largest shard (partition) bound every record
+        cap = min(k, max(self._shard_live))                         # live rows of the largest shard bound every record
         try:
             rec, gath, (o_s, o_i, o_c) = self._big_buffers(cap)
             self.backend.enqueue_local(self.backend.device_queries(q[None, :])[0], cap, rec[0])
@@ -725,6 +825,8 @@ class ShardedRetriever:
         n = min(int(n), self.n * (self.n - 1) // 2)
         if n <= 0 or self.d == 0:
             return []
+        if sum(self._shard_rows) != self.n:                         # the pair search runs on tombstone-free shards
+            self.compact()
         self._ensure_pairs()
         be = self.backend
         own = be.new_pair_lists(n)
