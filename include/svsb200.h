@@ -211,12 +211,12 @@ int svsb_batch_stats(svsb_t* e, int32_t b, int32_t* candidates, int32_t* rescore
  * SVSB_BATCH_CAND_CAP, when the list overflowed; only that many keys exist) and its eps, the bound on
  * |coarse - exact| the thresholds use.  keys and eps may be NULL. */
 int svsb_batch_candidates(svsb_t* e, int32_t q, int64_t cap, uint64_t* keys, int32_t* count, float* eps);
-/* Diagnostics of the last svsb_bench_run: *filter = 1 when its queries took the fp16 filter (a pass over the fp16
- * shadow, then an exact fp32 re-score of the candidate rows), 0 for the fp32 similarity kernel; *rescored = rows the
- * last query re-scored exactly (0 without the filter). */
+/* Diagnostics of the last svsb_bench_run: *filter = 1 when its queries took the filter (a pass over the int8 shadow,
+ * then an exact fp32 re-score of the candidate rows), 0 for the fp32 similarity kernel; *rescored = rows the last query
+ * re-scored exactly (0 without the filter). */
 int svsb_bench_filter_stats(svsb_t* e, int32_t* filter, int64_t* rescored);
-/* The route the last svsb_bench_run's queries took: *route = 0 for the fp32 similarity kernel, 16 for the filter over the
- * fp16 shadow, 8 for the filter over the int8 shadow (one scale per row; +25 % of the matrix in device memory). */
+/* The route the last svsb_bench_run's queries took: *route = 0 for the fp32 similarity kernel, 8 for the filter over the
+ * int8 shadow (one scale per row; +25 % of the matrix in device memory). */
 int svsb_bench_filter_route(svsb_t* e, int32_t* route);
 /* How the resident generation picks the coarse pass's filter thresholds: 0 = an order statistic of a row sample that
  * bounds the true cut-off with overwhelming probability and is VERIFIED per query after the pass (default; several

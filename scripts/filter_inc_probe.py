@@ -1,4 +1,4 @@
-"""Incremental update with the single-query fp16 filter on and off: load 1M x 1536, then three times add one row and
+"""Incremental update with the single-query filter on and off: load 1M x 1536, then three times add one row and
 query it twice, timing svsb_apply_mutations and each query on the host (profiles/r05_filter_ab.txt)."""
 import os, sys, time
 import numpy as np

@@ -1,13 +1,13 @@
-"""Single-query filters (DESIGN.md section 4, K1f and K1f8) against K1: real bytes and rates, candidates per query.
+"""The single-query filter (DESIGN.md section 4, K1f8) against K1: real bytes and rates, candidates per query.
 
     python scripts/filter_roofline.py [--iters 256] [--sweep] [--c4]
 
-For each shape the device-resident loop (svsb_bench_run, pipelined, the bench's loop) runs with SVSB_FILTER=0 (K1),
-=16 (fp16 filter) and =8 (int8 filter), in turn, twice each.  Reported per query: the step time, the bracketed
-similarity-kernel time, the REAL bytes the kernel streams (K1: n*ld*4; fp16 filter: n*ld16*2; int8 filter: n*ld8 + 4n
-for the row scales) over that time, the rows re-scored exactly and the bytes they re-read (rows * ld * 4), and whether
-every route returned the same last answer (bit for bit).  bench.py's `roofline` key keeps dividing n*d*4 by the
-bracketed kernel, which for the filters is an effective figure, ~2x (fp16) or ~4x (int8) the real one.
+For each shape the device-resident loop (svsb_bench_run, pipelined, the bench's loop) runs with SVSB_FILTER=0 (K1) and
+=1 (automatic: the int8 filter wherever its shadow exists), in turn, twice each.  Reported per query: the step time, the
+bracketed similarity-kernel time, the REAL bytes the kernel streams (K1: n*ld*4; int8 filter: n*ld8 + 4n for the row
+scales) over that time, the rows re-scored exactly and the bytes they re-read (rows * ld * 4), and whether every route
+returned the same last answer (bit for bit).  bench.py's `roofline` key keeps dividing n*d*4 by the bracketed kernel,
+which for the filter is an effective figure, ~4x the real one.
 --sweep: matrices from 10 548 rows (the bench's C1) up, to place the size cut-off (SVSB_FILTER_MIN_MB).
 --c4: also the bench's C4 (10M x 1536, top-100; ~107 GB of device memory with both shadows)."""
 import argparse
@@ -42,9 +42,9 @@ for n, d, k, name in shapes:
     e.load_synthetic(n, d, seed=0, id0=1, id_step=1)
     e.bench_set_queries(Q)
     ld = (d + 3) & ~3
-    real_bytes = {0: n * ld * 4, 16: n * ((d + 7) & ~7) * 2, 8: n * ((d + 15) & ~15) + 4 * n}
+    real_bytes = {0: n * ld * 4, 8: n * ((d + 15) & ~15) + 4 * n}
     last = {}
-    for f in ("0", "16", "8", "1", "0", "16", "8"):
+    for f in ("0", "1", "0", "1"):
         os.environ["SVSB_FILTER"] = f
         e.bench_run(k, 16, with_gemv=True)                   # warm-up
         r = e.bench_run(k, args.iters, with_gemv=True)

@@ -1,5 +1,5 @@
 #!/bin/bash
-# A/B of the single-query fp16 filter against K1 in one run (profiles/r05_filter_ab.txt): the card, bench.py --only
+# A/B of the single-query filter against K1 in one run (profiles/r05_filter_ab.txt): the card, bench.py --only
 # alternating SVSB_FILTER=0 / 1 three times each, one full bench.py line of each, --dump-outputs of both compared file
 # by file, and scripts/filter_roofline.py (real bytes, candidates, size cut-off).
 set -u

@@ -623,13 +623,14 @@ int shadow_sync(const Shard& s, int ld, int64_t fresh_from, int create, cudaStre
     return SVSB_OK;
 }
 
-// Single queries of a single-device engine take the fp16 filter (DESIGN.md section 4, K1f) when the view has a shadow:
-// rows of norm <= 8 (fp16 range of the scaled operands), d <= FILTER_MAX_LD, and a matrix large enough to gain:
+// Single queries of a single-device engine take the int8 filter (DESIGN.md section 4, K1f8) when the view has its
+// shadow: rows of norm <= 8 (fp16 range of the scaled operands), d <= FILTER_MAX_LD, and a matrix large enough to gain:
 // SVSB_FILTER_MIN_MB, default 512 MB of fp32 rows.  Measured on a B200 (profiles/r05_filter_ab.txt, 1536-d rows): at
 // 246 MB K1's pass is still faster than filter + threshold + re-score, at 492 MB the filter takes 25 % less time.
-// The int8 shadow is built with it when it fits as well (shadow_sync).
+// shadow_sync builds the fp16 shadow here too, first, and the int8 shadow after it when that fits as well: single
+// queries read only the int8 one, but the batched path (ensure_m16) and the pair search expect to find the fp16 one.
 int filter_attach(svsb_engine* e, Generation* g) {
-    for (auto& s : g->shards) { s.M16 = nullptr; s.M8 = nullptr; }
+    for (auto& s : g->shards) s.M8 = nullptr;
     if (e->devs.size() != 1 || e->is_kid || g->shards.size() != 1) return SVSB_OK;
     Shard& s = g->shards[0];
     if (s.n == 0 || g->ld > FILTER_MAX_LD || !(1.0f + g->max_dev <= 8.0f)) return SVSB_OK;
@@ -637,39 +638,33 @@ int filter_attach(svsb_engine* e, Generation* g) {
     void* p = nullptr;
     int rc = shadow_sync(s, g->ld, INT64_MAX, 1, e->copy_st[0], &p);
     if (rc != SVSB_OK) return rc;
-    s.M16 = p;
     if (p) s.M8 = s.buf->M8;
     return SVSB_OK;
 }
 
-// The route of one single query: 0 = K1, 16 = the fp16 filter, 8 = the int8 filter (DESIGN.md section 4, K1f8).
-// SVSB_FILTER (read per call): 0 forces K1, 16 or 8 force that filter where the view has its shadow, 1 or unset choose:
-// int8 wherever its shadow exists.  Measured on a B200 (profiles/r06_filter8_ab.txt), int8 against fp16 per query: C2
-// (1M x 1536, k = 100) 254 against 426 us, C4 (10M x 1536) 2.76 against 4.30 ms, and C5 (1M x 3072, k = 1000: ~99 000 rows
-// re-scored, 1.2 GB) still 741 against 936 us -- no shape the filters serve favours fp16.
+// The route of one single query: 0 = K1, 8 = the int8 filter (DESIGN.md section 4, K1f8).  SVSB_FILTER (read per
+// call): 0 forces K1; unset or any other value takes the filter wherever the view has its shadow.
 // The LDG variant of K1 (SVSB_GEMV_VARIANT=1) sums in another order than the re-score, which reproduces the TMA kernel's
-// bits: it turns the filters off.
+// bits: it turns the filter off.
 static int filter_route(const Shard& s, int64_t kk) {
-    const int f = env_int("SVSB_FILTER", 1);
-    if (!s.M16 || kk > K_FAST_MAX || f == 0) return 0;
+    if (!s.M8 || kk > K_FAST_MAX || env_int("SVSB_FILTER", 1) == 0) return 0;
     const char* v = getenv("SVSB_GEMV_VARIANT");
     if (v && atoi(v) == 1) return 0;
-    return s.M8 && f != 16 ? 8 : 16;
+    return 8;
 }
 
-// The similarity pass of one query: K1, or a filter (then filter_finish before the selection).
+// The similarity pass of one query: K1, or the filter (then filter_finish before the selection).
 static cudaError_t similarity_pass(cudaStream_t st, const DevWs& w, const Generation* g, const Shard& s, const float* q,
                                    int shift, int reserve_sms, int route) {
     if (route == 8)
         return launch_filter8(st, w.dev, s.M8, s.buf->s8, s.n, g->ld, s.buf->ld8, q, w.scores, w.gmax, shift, reserve_sms, s.live);
-    if (route == 16) return launch_filter(st, w.dev, s.M16, s.n, g->ld, (g->ld + 7) & ~7, q, w.scores, w.gmax, shift, reserve_sms, s.live);
     return launch_gemv(st, w.dev, s.M, s.n, g->d, g->ld, q, w.scores, w.gmax, shift, 0, 0, 0, reserve_sms, s.live);
 }
 // Threshold + exact re-score: afterwards scores / gmax give launch_select K1's top-kk.
 static cudaError_t filter_finish(cudaStream_t st, const DevWs& w, const Generation* g, const Shard& s, const float* q,
-                                 int shift, int64_t kk, int route) {
-    return launch_filter_refine(st, w.dev, s.M, s.n, g->ld, q, w.scores, w.gmax, shift, (int)kk, coarse_eps_coef(g->d),
-                                (1.0f + g->max_dev) * 1.000001f, route == 8 ? s.buf->e8 : nullptr, s.live, w.fstate);
+                                 int shift, int64_t kk) {
+    return launch_filter_refine(st, w.dev, s.M, s.n, g->ld, q, w.scores, w.gmax, shift, (int)kk, (1.0f + g->max_dev) * 1.000001f,
+                                s.buf->e8, s.live, w.fstate);
 }
 
 int similarity_phase(cudaStream_t st, DevWs& w, const Generation* g, const Shard& s, const float* q, int route,
@@ -688,7 +683,7 @@ int select_phase(cudaStream_t st, DevWs& w, const Generation* g, const Shard& s,
                  const SelOut& o, u64* stamps, const PeerPush* push) {
     const int shift = group_shift_for(s.n);
     const int64_t kk = std::min(k, s.n_live);
-    if (route) CU(filter_finish(st, w, g, s, q, shift, kk, route));
+    if (route) CU(filter_finish(st, w, g, s, q, shift, kk));
     if (k <= K_FAST_MAX)
         CU(launch_select(st, w.scores, s.n, w.gmax, shift, (int)kk, s.ids, s.row0, w.cand, w.cand_cap, o.keys, o.scores, o.ids,
                          o.count, stamps, push));

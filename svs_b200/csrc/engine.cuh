@@ -48,13 +48,13 @@ struct ShardBuf {
     int64_t* ids = nullptr;      // cap_rows
     int64_t cap_rows = 0;
     // fp16 shadow M16 = fp16(M * 2^12), cap_rows x ld16 halfs (DESIGN.md section 6): rows [0, m16_rows) are converted.
-    // Built at load for the single-query filter when it fits, else lazily by the first batch; appended rows are
+    // Built at load with the int8 shadow when it fits (filter_attach), else lazily by the first batch; appended rows are
     // converted by the update that writes them (shadow_sync).
     std::mutex m16_mu;
     void* M16 = nullptr; int ld16 = 0; int64_t m16_rows = 0;
     // int8 shadow for the single-query int8 filter (DESIGN.md section 4, K1f8), one allocation: M8 = cap_rows x ld8 bytes,
-    // then s8 = cap_rows scales, then e8 = the error word E (only raised).  Built next to M16 by filter_attach when it fits,
-    // rows [0, m8_rows) converted; guarded by m16_mu.
+    // then s8 = cap_rows scales, then e8 = the error word E (only raised).  Built after M16 by filter_attach when it fits
+    // as well, rows [0, m8_rows) converted; guarded by m16_mu.
     void* M8 = nullptr; float* s8 = nullptr; float* e8 = nullptr; int ld8 = 0; int64_t m8_rows = 0;
     ~ShardBuf() {
         if (M || ids || M16 || M8) cudaSetDevice(dev);
@@ -75,10 +75,8 @@ struct Shard {
     // generation (a delete must not disturb queries still running on the previous generation).
     uint8_t* live = nullptr;
     int64_t n_live = 0;
-    // == buf->M16 when this view's single queries take the fp16 filter (set before the generation is published, never
-    // changed after; null: K1 -- see filter_shadow in engine.cu)
-    const void* M16 = nullptr;
-    // == buf->M8 when the int8 filter is available to this view as well (set with M16)
+    // == buf->M8 when this view's single queries take the int8 filter (set before the generation is published, never
+    // changed after; null: K1 -- see filter_attach in engine.cu)
     const void* M8 = nullptr;
 };
 
@@ -123,7 +121,7 @@ struct svsb_workspace {
     u64* sortbuf = nullptr;  int64_t sort_cap = 0;
     u64* out_keys = nullptr; float* out_scores = nullptr; int64_t* out_ids = nullptr; int64_t out_cap = 0;
     int32_t* out_count = nullptr;
-    uint32_t* fstate = nullptr;      // fp16 filter: candidate threshold + rows re-scored (launch_filter_refine)
+    uint32_t* fstate = nullptr;      // int8 filter: candidate threshold + rows re-scored (launch_filter_refine)
     u64* mscr_keys = nullptr; int64_t* mscr_ids = nullptr; int64_t mscr_cap = 0;   // merge scratch
     cudaEvent_t ev = nullptr, ev0 = nullptr, ev1 = nullptr, ev_sel = nullptr;
     // The similarity kernel leaves group maxima in gmax and only a SUCCESSFUL selection kernel re-zeroes them
@@ -540,7 +538,7 @@ struct svsb_engine {
     std::vector<float*> bench_q; int bench_nq = 0, bench_d = 0, bench_ld = 0;
     std::unique_ptr<QueryCtx> bench_ctx;
     std::vector<cudaEvent_t> bench_kev;                  // similarity-kernel timing events of svsb_bench_run (device 0)
-    int bench_route = 0;                                 // the last svsb_bench_run's route: 0 K1, 16 / 8 the fp16 / int8 filter
+    int bench_route = 0;                                 // the last svsb_bench_run's route: 0 K1, 8 the int8 filter
     // sharded deployment (one process per GPU)
     int64_t shard_row0 = 0;                              // global row of this engine's first row
     std::vector<std::unique_ptr<DevWs>> shard_ws;        // workspaces for svsb_enqueue_local_topk (by slot)
@@ -578,8 +576,8 @@ struct svsb_snapshot { std::shared_ptr<Generation> gen; };
 // ------------------------------------------------------------------------------------------------
 std::shared_ptr<Generation> pin(svsb_engine* e);
 int prepare_ws(DevWs& w, const Generation* g, const Shard& s, int64_t kk);
-// The two phases of one single query over shard s in workspace w.  The caller chooses the route (0 = K1, 16 / 8 = the
-// fp16 / int8 filter) and passes the same to both.  similarity_phase marks w's group maxima dirty and launches the pass
+// The two phases of one single query over shard s in workspace w.  The caller chooses the route (0 = K1, 8 = the int8
+// filter) and passes the same to both.  similarity_phase marks w's group maxima dirty and launches the pass
 // on st (pdl: under programmatic dependent launch; t: a pair of timing events around it, or null).  select_phase
 // enqueues the filter's threshold + exact re-score (route != 0), then the top min(k, s.n_live) rows into o: the
 // selection kernel (stamps, push: its options) or, for k > K_FAST_MAX, the full sort; and clears the mark.
@@ -599,7 +597,7 @@ int alloc_generation(svsb_engine* e, int64_t n, int d, std::shared_ptr<Generatio
 // rows a load allocates for a shard of n rows: a little head-room (0.4 %, at least 1024 rows), so the first incremental
 // appends (svsb_apply_mutations) go in place instead of paying for a re-allocation and a device-to-device copy of the shard
 static inline int64_t shard_capacity(int64_t n) { return n + std::max<int64_t>(1024, n / 256); }
-// the filters' shadows of a single-device generation about to be published (engine.cu; part of publish_generation)
+// the filter's shadows of a single-device generation about to be published (engine.cu; part of publish_generation)
 int filter_attach(svsb_engine* e, Generation* g);
 int finish_generation(svsb_engine* e, Generation* g, int norm_mode);
 // publish `g` as the engine's resident generation (assigns the id; builds the per-device views of a multi-device engine)

@@ -388,111 +388,16 @@ gemv_tma_mq_kernel(const float* __restrict__ M, int64_t n, int d4, int tile_rows
 }
 
 // =============================================================================================
-// variant 3: the fp16 filter -- the same ring over the fp16 shadow, then an exact re-score of the few candidates
+// variant 3: the int8 filter -- the same ring over the int8 shadow, then an exact re-score of the few candidates
 // =============================================================================================
-// A single query reads n*d*4 bytes with K1 at the HBM rate; the filter reads the shadow M16 = fp16(M * 2^12) instead
-// (n*d*2 bytes) and writes K1's outputs -- scores[n], group maxima -- as COARSE values.  filter_threshold_kernel turns
-// them into a threshold T <= tau~ - 2 eps (tau~ = the kk-th largest coarse score), filter_rescore_kernel gives every
-// row with coarse >= T its exact score (K1's arithmetic, bit for bit) and every other row of the groups it rescans the
-// tombstone score, and rewrites the group maxima so that the unchanged selection kernel sees only exact scores.
-// Exactness (DESIGN.md section 4, "K1f"): |coarse - exact| <= eps, kk rows have coarse >= tau~, so every row of the exact
-// top-kk has coarse >= tau~ - 2 eps >= T.
-
-// NC: 16-byte chunks (8 halfs) of the shadow row per lane, c16 = ld16 / 8 <= 32 * NC.  The query stays fp32 (its
-// 8 floats per chunk in registers); the row is widened exactly to fp32 and accumulated with fp32 FMAs.
-template <int CW, int NC>
-__global__ void __launch_bounds__((CW + 1) * 32, 1)
-gemv16_tma_kernel(const __half* __restrict__ M16, int64_t n, int c16, int tile_rows, int stages,
-                  const float* __restrict__ q, int ld, float* __restrict__ scores, u64* __restrict__ gmax, int group_shift,
-                  const uint8_t* __restrict__ live)
-{
-    extern __shared__ __align__(128) unsigned char smem_raw[];
-    const uint32_t row_bytes = (uint32_t)c16 * 16u;
-    const uint32_t stage_bytes = (uint32_t)tile_rows * row_bytes;
-    uint64_t* full = reinterpret_cast<uint64_t*>(smem_raw + (size_t)stages * stage_bytes);
-    uint64_t* empty = full + stages;
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    if (threadIdx.x == 0) {
-        pdl_trigger();
-        for (int s = 0; s < stages; ++s) { mbar_init(&full[s], 1); mbar_init(&empty[s], CW); }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncthreads();
-
-    const int64_t ntiles = (n + tile_rows - 1) / tile_rows;
-    if (warp == CW) {
-        if (lane == 0) {
-            u64 policy;
-            asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(policy));
-            int s = 0; uint32_t phase = 0;
-            for (int64_t t = blockIdx.x; t < ntiles; t += gridDim.x) {
-                mbar_wait(&empty[s], phase ^ 1u);
-                const int64_t r0 = t * tile_rows;
-                const int64_t left = n - r0;
-                const uint32_t rows = left < tile_rows ? (uint32_t)left : (uint32_t)tile_rows;
-                const uint32_t bytes = rows * row_bytes;
-                mbar_arrive_expect_tx(&full[s], bytes);
-                bulk_g2s(smem_raw + (size_t)s * stage_bytes, reinterpret_cast<const unsigned char*>(M16) + (size_t)r0 * row_bytes,
-                         bytes, &full[s], policy);
-                if (++s == stages) { s = 0; phase ^= 1u; }
-            }
-        }
-    } else {
-        pdl_wait();                                   // the query is written by the previous kernel (see gemv_tma_kernel)
-        float4 qr[NC][2];
-        const int ld4 = ld >> 2;
-#pragma unroll
-        for (int j = 0; j < NC; ++j) {
-            const int c = lane + 32 * j;
-            qr[j][0] = 2 * c < ld4 ? __ldcg(reinterpret_cast<const float4*>(q) + 2 * c) : make_float4(0.f, 0.f, 0.f, 0.f);
-            qr[j][1] = 2 * c + 1 < ld4 ? __ldcg(reinterpret_cast<const float4*>(q) + 2 * c + 1) : make_float4(0.f, 0.f, 0.f, 0.f);
-        }
-        int s = 0; uint32_t phase = 0;
-        for (int64_t t = blockIdx.x; t < ntiles; t += gridDim.x) {
-            const int64_t r0 = t * tile_rows;
-            const int64_t left = n - r0;
-            const int rows = left < tile_rows ? (int)left : tile_rows;
-            mbar_wait(&full[s], phase);
-            const uint4* tile = reinterpret_cast<const uint4*>(smem_raw + (size_t)s * stage_bytes);
-            u64 kmax = 0;
-            for (int r = warp; r < rows; r += CW) {
-                const uint4* p = tile + (size_t)r * c16;
-                const uint8_t alive = live ? __ldg(live + r0 + r) : (uint8_t)1;
-                uint4 m[NC];
-#pragma unroll
-                for (int j = 0; j < NC; ++j) { const int c = lane + 32 * j; m[j] = c < c16 ? p[c] : make_uint4(0u, 0u, 0u, 0u); }
-                float4 a0 = make_float4(0.f, 0.f, 0.f, 0.f), a1 = a0;
-#pragma unroll
-                for (int j = 0; j < NC; ++j) {
-                    const float2 h0 = __half22float2(*reinterpret_cast<const __half2*>(&m[j].x));
-                    const float2 h1 = __half22float2(*reinterpret_cast<const __half2*>(&m[j].y));
-                    const float2 h2 = __half22float2(*reinterpret_cast<const __half2*>(&m[j].z));
-                    const float2 h3 = __half22float2(*reinterpret_cast<const __half2*>(&m[j].w));
-                    fma4(a0, make_float4(h0.x, h0.y, h1.x, h1.y), qr[j][0]);
-                    fma4(a1, make_float4(h2.x, h2.y, h3.x, h3.y), qr[j][1]);
-                }
-                // x 2^-12 undoes the operand scale exactly
-                float sc = warp_sum(((a0.x + a1.x) + (a0.y + a1.y)) + ((a0.z + a1.z) + (a0.w + a1.w))) * (1.0f / COARSE_OPERAND_SCALE);
-                if (!alive) sc = dead_score();
-                if (lane == 0) {
-                    scores[r0 + r] = sc;
-                    const u64 k0 = make_key(sc, (uint32_t)(r0 + r));
-                    kmax = k0 > kmax ? k0 : kmax;
-                }
-            }
-            __syncwarp();
-            if (lane == 0) {
-                mbar_arrive(&empty[s]);
-                if (kmax) atomicMax(&gmax[r0 >> group_shift], kmax);
-            }
-            if (++s == stages) { s = 0; phase ^= 1u; }
-        }
-    }
-}
-
-// =============================================================================================
-// variant 4: the int8 filter -- the same ring over the int8 shadow (DESIGN.md section 4, "K1f8")
-// =============================================================================================
+// A single query reads n*d*4 bytes with K1 at the HBM rate; the filter reads the int8 shadow instead (n*ld8 bytes plus
+// 4n for the row scales) and writes K1's outputs -- scores[n], group maxima -- as COARSE values.  filter_threshold_kernel
+// turns them into a threshold T <= tau~ - 2 eps (tau~ = the kk-th largest coarse score), filter_rescore_kernel gives
+// every row with coarse >= T its exact score (K1's arithmetic, bit for bit) and every other row of the groups it rescans
+// the tombstone score, and rewrites the group maxima so that the unchanged selection kernel sees only exact scores.
+// Exactness (DESIGN.md section 4, "K1f8"): |coarse - exact| <= eps, kk rows have coarse >= tau~, so every row of the
+// exact top-kk has coarse >= tau~ - 2 eps >= T.
+//
 // Row r of the shadow is Q_r[ld8] (int8, zero padded) with one fp32 scale s_r = max|r_j| / 127: r^ = s_r * Q_r.  The
 // device word E >= max_r ||r - r^|| bounds the quantisation error of every row converted so far (it only grows).  The
 // query is split into two int8 terms q^ = s1 * q_hi + s2 * q_lo (s1 = max|q_j| / 127, s2 = s1 / 254) by q8_split, the
@@ -737,15 +642,14 @@ gemv8_tma_kernel(const int8_t* __restrict__ M8, const float* __restrict__ scale8
 // candidates; T = 0 takes every row (no usable threshold: at most kk groups, a non-finite query, bound or group maximum).
 // state[1] = 0 (the re-score kernel counts its rows there).
 // T = (kk-th largest group maximum) - 2 eps, rounded down: that maximum comes from kk distinct rows, so it is <= tau~.
-// e8 == null: the fp16 filter's bound, eps = eps_coef * ||q|| * max_row_norm + 1e-8.  e8 = the int8 shadow's E: the int8
-// filter's bound (DESIGN.md section 4, "K1f8"), with R = max_row_norm, R^ = R + E >= max ||r^||, q^ from q8_split,
-// eps = ||q|| E + ||q - q^|| R^ + ld 2^-23 ||q|| R (K1's fp32 sum) + 2^-21 (||s1 q_hi|| + ||s2 q_lo||) R^ (the combine's
-// five roundings) + 1e-8, times 1 + 2^-10 for the fp32 norms.
+// eps bounds |coarse - exact| (DESIGN.md section 4, "K1f8"): with e8 = the int8 shadow's E, R = max_row_norm,
+// R^ = R + E >= max ||r^||, q^ from q8_split, eps = ||q|| E + ||q - q^|| R^ + ld 2^-23 ||q|| R (K1's fp32 sum)
+// + 2^-21 (||s1 q_hi|| + ||s2 q_lo||) R^ (the combine's five roundings), times 1 + 2^-10 for the fp32 norms, + 1e-8.
 constexpr int FT_THREADS = 1024;
 constexpr int FT_PER_THREAD = (int)(GROUPS_TARGET / FT_THREADS);
 __global__ void __launch_bounds__(FT_THREADS, 1)
 filter_threshold_kernel(const u64* __restrict__ gmax, int G, int kk, const float* __restrict__ q, int ld,
-                        float eps_coef, float max_row_norm, const float* __restrict__ e8, uint32_t* __restrict__ state)
+                        float max_row_norm, const float* __restrict__ e8, uint32_t* __restrict__ state)
 {
     __shared__ uint32_t hist[256];
     __shared__ float red[FT_THREADS / 32];
@@ -765,7 +669,7 @@ filter_threshold_kernel(const u64* __restrict__ gmax, int G, int kk, const float
     for (int j = 0; j < FT_PER_THREAD; ++j) { const int i = tid + j * FT_THREADS; v[j] = i < G ? (uint32_t)(__ldcg(gmax + i) >> 32) : 0u; }
     if (tid == 0) { sh_prefix = 0u; sh_want = (uint32_t)kk; }
     __syncthreads();
-    if (e8) {                                          // ||q - q^||^2, ||s1 q_hi||^2, ||s2 q_lo||^2 (double: exact enough)
+    {                                                  // ||q - q^||^2, ||s1 q_hi||^2, ||s2 q_lo||^2 (double: exact enough)
         for (int w = 0; w < FT_THREADS / 32; ++w) mb = max(mb, amx[w]);
         float s1, s2;
         q8_scales(mb, s1, s2);
@@ -823,14 +727,12 @@ filter_threshold_kernel(const u64* __restrict__ gmax, int G, int kk, const float
         const float qn = sqrtf(qq);
         const float tau = ordered_to_f32(sh_prefix);
         uint32_t T = 0u;
-        double eps = (double)eps_coef * (double)qn * (double)max_row_norm + 1e-8;
-        if (e8) {
-            double a[3] = {0.0, 0.0, 0.0};
-            for (int w = 0; w < FT_THREADS / 32; ++w) for (int c = 0; c < 3; ++c) a[c] += red8[c][w];
-            const double E = (double)__ldcg(e8), R = (double)max_row_norm, Rh = R + E;
-            eps = ((double)qn * E + sqrt(a[0]) * Rh + (double)ld * 0x1p-23 * (double)qn * R + 0x1p-21 * (sqrt(a[1]) + sqrt(a[2])) * Rh)
-                  * (1.0 + 0x1p-10) + 1e-8;
-        }
+        double a[3] = {0.0, 0.0, 0.0};
+        for (int w = 0; w < FT_THREADS / 32; ++w) for (int c = 0; c < 3; ++c) a[c] += red8[c][w];
+        const double E = (double)__ldcg(e8), R = (double)max_row_norm, Rh = R + E;
+        const double sum = (double)qn * E + sqrt(a[0]) * Rh + (double)ld * 0x1p-23 * (double)qn * R
+                           + 0x1p-21 * (sqrt(a[1]) + sqrt(a[2])) * Rh;
+        const double eps = __dadd_rn(__dmul_rn(sum, 1.0 + 0x1p-10), 1e-8);   // two roundings, not one fused multiply-add
         if (G > kk && isfinite(tau) && isfinite(qn) && isfinite(eps)) {
             float t = __double2float_rd((double)tau - 2.0 * eps);
             if (t == 0.f) t = -0.f;                         // f32_to_ordered(-0) < f32_to_ordered(+0): keep both zeros
@@ -1008,8 +910,6 @@ cudaError_t preload_gemv_kernels()
     SVSB_PRE((gemv_tma_kernel<16, 2>)); SVSB_PRE((gemv_tma_kernel<16, 6>)); SVSB_PRE((gemv_tma_kernel<16, 12>));
     SVSB_PRE((gemv_tma_kernel<16, 24>)); SVSB_PRE((gemv_tma_kernel<16, 0>));
     SVSB_PRE((gemv_ldg_kernel<4, 3, 256>));
-    SVSB_PRE((gemv16_tma_kernel<8, 1>)); SVSB_PRE((gemv16_tma_kernel<8, 2>)); SVSB_PRE((gemv16_tma_kernel<8, 4>));
-    SVSB_PRE((gemv16_tma_kernel<8, 6>)); SVSB_PRE((gemv16_tma_kernel<8, 8>)); SVSB_PRE((gemv16_tma_kernel<8, 12>));
     SVSB_PRE((gemv8_tma_kernel<8, 1>)); SVSB_PRE((gemv8_tma_kernel<8, 2>)); SVSB_PRE((gemv8_tma_kernel<8, 3>));
     SVSB_PRE((gemv8_tma_kernel<8, 4>)); SVSB_PRE((gemv8_tma_kernel<8, 6>));
     SVSB_PRE(filter_threshold_kernel);
@@ -1054,47 +954,6 @@ cudaError_t launch_gemv(cudaStream_t st, int device, const float* M, int64_t n, 
         case 9:  return run_ldg<8, 3, 128>(st, device, M, n, d4, q, scores, gmax, group_shift, live, tune_b);
         default: return run_ldg<4, 3, 256>(st, device, M, n, d4, q, scores, gmax, group_shift, live, tune_b);
     }
-}
-
-// ---- fp16 filter launchers --------------------------------------------------------------------
-template <int CW, int NC>
-static cudaError_t run_filter_inst(cudaStream_t st, int64_t grid, size_t smem, const void* M16, int64_t n, int c16, int tile_rows,
-                                   int stages, const float* q, int ld, float* scores, u64* gmax, int group_shift, const uint8_t* live)
-{
-    auto kern = gemv16_tma_kernel<CW, NC>;
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return e;
-    e = launch_kernel(kern, dim3((unsigned)grid), dim3((CW + 1) * 32), smem, st, reinterpret_cast<const __half*>(M16), n, c16,
-                      tile_rows, stages, q, ld, scores, gmax, group_shift, live);
-    count_launch();
-    return e != cudaSuccess ? e : cudaGetLastError();
-}
-
-cudaError_t launch_filter(cudaStream_t st, int device, const void* M16, int64_t n, int ld, int ld16, const float* q,
-                          float* scores, u64* gmax, int group_shift, int reserve_sms, const uint8_t* live)
-{
-    if (n <= 0) return cudaSuccess;
-    if (ld > FILTER_MAX_LD || ld16 < ld || (ld16 & 7)) return cudaErrorInvalidValue;
-    const int c16 = ld16 / 8;
-    const size_t row_bytes = (size_t)ld16 * 2;
-    // K1's ring: ~48 KB tiles x 3 stages (profiles/r01_tune_gemv.md)
-    int tile_rows = 64;
-    while (tile_rows > 1 && (size_t)tile_rows * row_bytes > 48 * 1024) tile_rows >>= 1;
-    const int stages = 3;
-    const size_t smem = (size_t)stages * tile_rows * row_bytes + (size_t)stages * 16 + 64;
-    const int64_t ntiles = (n + tile_rows - 1) / tile_rows;
-    int64_t grid = sm_count(device) - reserve_sms;
-    if (grid > ntiles) grid = ntiles;
-    if (grid < 1) grid = 1;
-#define SVSB_F16_CASE(NCV) \
-    return run_filter_inst<8, NCV>(st, grid, smem, M16, n, c16, tile_rows, stages, q, ld, scores, gmax, group_shift, live)
-    if (c16 <= 32) SVSB_F16_CASE(1);
-    if (c16 <= 64) SVSB_F16_CASE(2);
-    if (c16 <= 128) SVSB_F16_CASE(4);
-    if (c16 <= 192) SVSB_F16_CASE(6);
-    if (c16 <= 256) SVSB_F16_CASE(8);
-    SVSB_F16_CASE(12);
-#undef SVSB_F16_CASE
 }
 
 cudaError_t launch_rows_to_i8(cudaStream_t st, int device, const float* M, int64_t n, int ld, void* M8, int ld8, float* scale8,
@@ -1167,14 +1026,14 @@ static cudaError_t run_rescore_inst(cudaStream_t st, int device, const float* M,
 }
 
 cudaError_t launch_filter_refine(cudaStream_t st, int device, const float* M, int64_t n, int ld, const float* q, float* scores,
-                                 u64* gmax, int group_shift, int kk, float eps_coef, float max_row_norm, const float* e8,
-                                 const uint8_t* live, uint32_t* state)
+                                 u64* gmax, int group_shift, int kk, float max_row_norm, const float* e8, const uint8_t* live,
+                                 uint32_t* state)
 {
     if (n <= 0) return cudaSuccess;
     if (ld > FILTER_MAX_LD) return cudaErrorInvalidValue;
     const int64_t G = (n + ((int64_t)1 << group_shift) - 1) >> group_shift;
     if (G > GROUPS_TARGET) return cudaErrorInvalidValue;
-    filter_threshold_kernel<<<1, FT_THREADS, 0, st>>>(gmax, (int)G, kk, q, ld, eps_coef, max_row_norm, e8, state);
+    filter_threshold_kernel<<<1, FT_THREADS, 0, st>>>(gmax, (int)G, kk, q, ld, max_row_norm, e8, state);
     count_launch();
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return e;

@@ -48,33 +48,23 @@ cudaError_t launch_gemv(cudaStream_t st, int device, const float* M, int64_t n, 
                         int variant = 0, int tune_a = 0, int tune_b = 0, int reserve_sms = 0,
                         const uint8_t* live = nullptr);
 
-// K1f, the fp16 filter (gemv.cu, DESIGN.md section 4): launch_filter writes launch_gemv's outputs as COARSE values from
-// the shadow M16[n][ld16] = fp16(M * 2^12) (launch_rows_to_f16) and the fp32 query q[ld]; launch_filter_refine then
-// (1 CTA) sets the candidate threshold state[0] from the group maxima and the bound
-// eps = eps_coef * ||q|| * max_row_norm + 1e-8 on |coarse - exact|, and (many CTAs) re-scores every candidate exactly --
-// the bits launch_gemv writes -- leaving scores / gmax such that launch_select returns launch_gemv's top-kk.
-// state: 2 device words, state[1] = rows re-scored.  ld <= FILTER_MAX_LD.
+// K1f8, the single-query int8 filter (gemv.cu, DESIGN.md section 4): launch_filter8 writes launch_gemv's outputs as
+// COARSE values from the int8 shadow M8[n][ld8] with one scale per row (launch_rows_to_i8) and the fp32 query q[ld];
+// launch_filter_refine then (1 CTA) sets the candidate threshold state[0] from the group maxima and the bound eps on
+// |coarse - exact| (from the shadow's error word e8 and max_row_norm), and (many CTAs) re-scores every candidate exactly
+// -- the bits launch_gemv writes -- leaving scores / gmax such that launch_select returns launch_gemv's top-kk.
+// state: 2 device words, state[1] = rows re-scored.  ld8 % 16 == 0, ld <= FILTER_MAX_LD.
 constexpr int FILTER_MAX_LD = 3072;
-cudaError_t launch_filter(cudaStream_t st, int device, const void* M16, int64_t n, int ld, int ld16, const float* q,
-                          float* scores, u64* gmax, int group_shift, int reserve_sms = 0, const uint8_t* live = nullptr);
-// e8: null for the fp16 filter; the int8 shadow's error word E for launch_filter8's coarse scores (then the threshold
-// uses the int8 bound, gemv.cu filter_threshold_kernel).
-cudaError_t launch_filter_refine(cudaStream_t st, int device, const float* M, int64_t n, int ld, const float* q, float* scores,
-                                 u64* gmax, int group_shift, int kk, float eps_coef, float max_row_norm, const float* e8,
-                                 const uint8_t* live, uint32_t* state);
-// K1f8, the int8 filter (gemv.cu, DESIGN.md section 4): launch_filter's contract over the int8 shadow M8[n][ld8] with
-// one scale per row (launch_rows_to_i8).  ld8 % 16 == 0, ld <= FILTER_MAX_LD.
 cudaError_t launch_filter8(cudaStream_t st, int device, const void* M8, const float* scale8, int64_t n, int ld, int ld8,
                            const float* q, float* scores, u64* gmax, int group_shift, int reserve_sms = 0,
                            const uint8_t* live = nullptr);
+cudaError_t launch_filter_refine(cudaStream_t st, int device, const float* M, int64_t n, int ld, const float* q, float* scores,
+                                 u64* gmax, int group_shift, int kk, float max_row_norm, const float* e8, const uint8_t* live,
+                                 uint32_t* state);
 // M8[r] = round(M[r] / scale8[r]) with scale8[r] = max|M[r][.]| / 127, zero padded; *emax (a float, only raised) >= every
 // converted row's ||M[r] - scale8[r] * M8[r]||.  ld % 4 == 0, ld8 % 16 == 0, ld8 >= ld.
 cudaError_t launch_rows_to_i8(cudaStream_t st, int device, const float* M, int64_t n, int ld, void* M8, int ld8, float* scale8,
                               float* emax);
-// the bound's coefficient for d components (fp16 operands, fp32 accumulation; DESIGN.md section 6, step 4)
-inline float coarse_eps_coef(int d) {
-    return 9.765625e-4f + 2.384185791015625e-7f + (float)d * (2.384185791015625e-7f + 1.1920928955078125e-7f);
-}
 
 // b queries Q[b][ld] in ONE pass over the matrix: scores[q * n_stride + r], gmax[q * g_stride + (r >> shift)] (zero on
 // entry), bit-identical to b launch_gemv calls.  cudaErrorInvalidConfiguration: rows too long (ld > 3072) or b larger
@@ -188,6 +178,10 @@ constexpr int REFINE_SURVIVOR_CAP = 4096;           // exact re-scores per query
 
 // M16[r][0..ld16) = fp16(M[r][.] * 2^12), zero padded.  ld % 4 == 0, ld16 % 8 == 0, ld16 >= ld.
 cudaError_t launch_rows_to_f16(cudaStream_t st, int device, const float* M, int64_t n, int ld, void* M16, int ld16);
+// the coarse bound's coefficient for d components (fp16 operands, fp32 accumulation; DESIGN.md section 6, step 4)
+inline float coarse_eps_coef(int d) {
+    return 9.765625e-4f + 2.384185791015625e-7f + (float)d * (2.384185791015625e-7f + 1.1920928955078125e-7f);
+}
 // Q16 (b_pad rows, rows >= b zero) from fp32 queries Q[b][ldq]; eps[q] = eps_coef * ||q|| * max_row_norm + 1e-8,
 // thr[q] = +inf, flags[q] = 1 for queries the coarse path must not handle (non-finite / huge norm).
 cudaError_t launch_queries_to_f16(cudaStream_t st, const float* Q, int b, int b_pad, int d, int ldq, void* Q16, int ld16,

@@ -328,13 +328,13 @@ class Engine:
         return b.view(np.float32), rows, cnt.value, eps.value
 
     def bench_filter_stats(self) -> Tuple[bool, int]:
-        """(took the fp16 filter, rows the last query re-scored exactly) of the last bench_run."""
+        """(took the int8 filter, rows the last query re-scored exactly) of the last bench_run."""
         f, r = C.c_int32(), C.c_int64()
         check(self._lib.svsb_bench_filter_stats(self._h, C.byref(f), C.byref(r)))
         return bool(f.value), int(r.value)
 
     def bench_filter_route(self) -> int:
-        """Route of the last bench_run: 0 = fp32 similarity kernel, 16 = fp16 filter, 8 = int8 filter."""
+        """Route of the last bench_run: 0 = fp32 similarity kernel, 8 = int8 filter."""
         r = C.c_int32()
         check(self._lib.svsb_bench_filter_route(self._h, C.byref(r)))
         return int(r.value)

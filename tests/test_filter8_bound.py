@@ -4,14 +4,70 @@ The shadow is what rows_to_i8_kernel writes: per row s_r = fp32(max|r_j| / 127),
 E = max_r ||r - s_r Q_r|| (float64, rounded up).  The query split is q8_split: s1 = fp32(max|q_j| / 127),
 s2 = fp32(s1 / 254), q_hi = clip(rint(q / s1)), q_lo = clip(rint(fma(-s1, q_hi, q) / s2)).  The coarse score is
 gemv8_tma_kernel's: two exact integer dot products, then s_r * fma(s2, D_lo, s1 * D_hi) in fp32.  The exact score is K1's
-fp32 arithmetic (test_filter_bound.k1_scores).  On adversarial data this checks |coarse - exact| <= eps (the bound of
-filter_threshold_kernel) for every row and that the rows with coarse >= T contain the exact top-k."""
+fp32 arithmetic (k1_scores: FMAs emulated as one float64 product-sum rounded to fp32).  On adversarial data this checks
+|coarse - exact| <= eps (the bound of filter_threshold_kernel) for every row and that the rows with coarse >= T (the
+threshold filter_threshold_kernel derives from the group maxima) contain the exact top-k."""
 import numpy as np
 import pytest
 
-from test_filter_bound import exact_topk_rows, k1_scores, threshold
-
 f32 = np.float32
+
+
+def _fma(acc, a, b):
+    return (acc.astype(np.float64) + a.astype(np.float64) * b.astype(np.float64)).astype(np.float32)
+
+
+def _combine_and_tree(a0, a1):
+    f = np.float32
+    v = ((a0[..., 0] + a1[..., 0]).astype(f) + (a0[..., 1] + a1[..., 1]).astype(f)).astype(f) + \
+        ((a0[..., 2] + a1[..., 2]).astype(f) + (a0[..., 3] + a1[..., 3]).astype(f)).astype(f)
+    v = v.astype(f)                                                  # [n, 32]
+    lanes = np.arange(32)
+    for o in (16, 8, 4, 2, 1):
+        v = (v + v[:, lanes ^ o]).astype(f)
+    return v[:, 0]
+
+
+def k1_scores(M, q):
+    """gemv_tma_kernel: lane l owns float4 chunks l, l+32, ...; even chunks into a0, odd into a1."""
+    n, ld = M.shape
+    d4 = ld // 4
+    nq = -(-d4 // 32)
+    Mp = np.zeros((n, nq * 32 * 4), np.float32); Mp[:, :ld] = M
+    qp = np.zeros(nq * 32 * 4, np.float32); qp[:ld] = q
+    Mc = Mp.reshape(n, nq, 32, 4); qc = qp.reshape(nq, 32, 4)
+    a = [np.zeros((n, 32, 4), np.float32), np.zeros((n, 32, 4), np.float32)]
+    for j in range(nq):
+        a[j & 1] = _fma(a[j & 1], Mc[:, j], qc[j][None])
+    return _combine_and_tree(a[0], a[1])
+
+
+def group_shift_for(n):
+    s = 6
+    while ((n + (1 << s) - 1) >> s) > 16384:
+        s += 1
+    return s
+
+
+def threshold(coarse, kk, eps):
+    """filter_threshold_kernel: (kk-th largest group maximum) - 2 eps, rounded down; None = every row."""
+    n = len(coarse)
+    m = 1 << group_shift_for(n)
+    G = -(-n // m)
+    pad = np.full(G * m, -np.inf, np.float32); pad[:n] = coarse
+    gmax = pad.reshape(G, m).max(axis=1)
+    if G <= kk or not np.isfinite(eps):
+        return None
+    tau = np.sort(gmax)[::-1][kk - 1]
+    t = np.float32(np.float64(tau) - 2.0 * np.float64(eps))
+    if np.float64(t) > np.float64(tau) - 2.0 * np.float64(eps):
+        t = np.nextafter(t, np.float32(-np.inf))
+    return t
+
+
+def exact_topk_rows(exact, k):
+    order = np.lexsort((np.arange(len(exact)), -exact.astype(np.float64)))
+    return order[:k]
 
 
 def _round_q(x):
@@ -175,3 +231,4 @@ def test_rows_sorted_by_similarity_and_near_ties():
     M = M[np.argsort(M @ q)]
     for k in (1, 100, 1000):
         check(M, q, k)
+

@@ -3,7 +3,7 @@
 Each path promises svsb_query's bits, and svsb_query's bits are K1's summation order (gemv_tma_kernel).  Here they are
 compared with that order computed on the CPU, as uint32 score bits plus ids, nothing else allowed: the single-query
 kernels (TMA and LDG variants, every instantiation), the batched paths (tensor-core coarse pass + exact refine, the
-multi-query passes), the fp16 and int8 filters, the in-process multi-device merge, the bench loop, a generation with
+multi-query passes), the int8 filter, the in-process multi-device merge, the bench loop, a generation with
 tombstones and appended rows, and the pair search.  d covers one chunk per lane and less (d <= 128), ragged ld, the
 multi-query limits, and both sides of the TMA kernel's row limit (d = 12 800) where K1 hands over to the LDG kernel."""
 import os
@@ -117,8 +117,8 @@ def test_query_batch_multi_query_path(engine, d, monkeypatch):
 @pytest.mark.parametrize("route", ["1", "8"])
 @pytest.mark.parametrize("d", D_ALL)
 def test_filters(d, route, monkeypatch):
-    """The fp16 (=1, automatic: fp16 or int8) and int8 (=8) filters on a matrix of any size: the re-scored candidates
-    must carry K1's bits.  d above the filters' row limit takes K1 itself."""
+    """The int8 filter, switched on by SVSB_FILTER=1 and by =8 (any value but 0), on a matrix of any size: the
+    re-scored candidates must carry K1's bits.  d above the filter's row limit takes K1 itself."""
     import svs_b200
     monkeypatch.setenv("SVSB_FILTER", route)
     monkeypatch.setenv("SVSB_FILTER_MIN_MB", "0")

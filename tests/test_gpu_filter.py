@@ -1,8 +1,9 @@
-"""GPU: the single-query fp16 filter (DESIGN.md section 4, K1f) returns exactly what the fp32 similarity kernel K1 returns.
+"""GPU: the single-query int8 filter (DESIGN.md section 4, K1f8) returns exactly what the fp32 similarity kernel K1 returns.
 
-Every case answers the same query with SVSB_FILTER=0 (K1) and SVSB_FILTER=1 (filter pass over the fp16 shadow, exact
-re-score of the candidates) and compares scores as uint32, ids and order.  SVSB_FILTER_MIN_MB=0 lets small matrices
-take the filter; `bench_filter_stats` confirms that they did."""
+Every case answers the same query with SVSB_FILTER=0 (K1) and SVSB_FILTER=1 (pass over the int8 shadow, exact re-score of
+the candidates) and compares scores as uint32, ids and order.  SVSB_FILTER_MIN_MB=0 lets small matrices take the filter;
+`bench_filter_route` and `bench_filter_stats` confirm which route the device-resident loop took.  The helpers serve
+test_gpu_filter8.py and test_gpu_filter8_edges.py as well."""
 import numpy as np
 import pytest
 
@@ -38,6 +39,10 @@ def _check_query(monkeypatch, e, q, k):
     return got
 
 
+def _bits(res):
+    return [np.float32(s).view(np.uint32) for s, _ in res]
+
+
 def _check_bench(monkeypatch, e, qs, k, expect_filter=True):
     """The device-resident loop (pipelined and serial): last answer and the route it took."""
     e.bench_set_queries(qs)
@@ -48,12 +53,13 @@ def _check_bench(monkeypatch, e, qs, k, expect_filter=True):
             monkeypatch.setenv("SVSB_FILTER", f)
             e.bench_run(k, len(qs) + 1)
             res.append(e.bench_last_result(k))
+            filtered = f == "1" and expect_filter
+            assert e.bench_filter_route() == (8 if filtered else 0)
             took, rescored = e.bench_filter_stats()
-            assert took == (f == "1" and expect_filter)
+            assert took == filtered
             if took:
                 assert rescored >= min(k, e.generation_rows()[1])
-        assert res[0] == res[1] and [np.float32(s).view(np.uint32) for s, _ in res[0]] == \
-            [np.float32(s).view(np.uint32) for s, _ in res[1]]
+        assert res[0] == res[1] and _bits(res[0]) == _bits(res[1])
     monkeypatch.delenv("SVSB_PIPELINE")
     monkeypatch.delenv("SVSB_FILTER")
 
@@ -93,7 +99,7 @@ def test_filter_matches_k1_over_k(monkeypatch, k):
 
 @pytest.mark.parametrize("n", [1, 5, 63, 64, 65, 700])
 def test_filter_small_n(monkeypatch, n):
-    d = 1536                                   # 16 rows per TMA tile of the fp16 ring
+    d = 1536                                   # 32 rows per TMA tile of the int8 ring
     m = oracle.synth_matrix_uniform(n, d, 7)
     ids = np.arange(n, dtype=np.int64) + 100
     q = oracle.synth_queries(1, d, 8)[0]

@@ -1,62 +1,17 @@
-"""GPU: the single-query int8 filter (DESIGN.md section 4, K1f8) returns exactly what the fp32 similarity kernel K1 returns.
+"""GPU: more cases of the single-query int8 filter (DESIGN.md section 4, K1f8) against K1, next to test_gpu_filter.py's.
 
-Every case answers the same query with SVSB_FILTER=0 (K1) and SVSB_FILTER=8 (pass over the int8 shadow, exact re-score of
-the candidates) and compares scores as uint32, ids and order.  SVSB_FILTER_MIN_MB=0 lets small matrices take the filter;
-`bench_filter_route` confirms which route the device-resident loop took."""
+d = 2000, small n around the int8 ring's 32-row tiles, signed and adversarial rows, tiny-scale queries, an append that
+raises the shadow's error word E, and the automatic route on a C2-like shape, besides the kinds of case both modules
+run.  Every case compares SVSB_FILTER=0 (K1) with the filter as uint32 scores, ids and order, through
+test_gpu_filter.py's helpers."""
 import numpy as np
 import pytest
 
 import svs_b200
 from _util import oracle
+from test_gpu_filter import _bits, _both, _check_bench, _check_query, _filter_on_small_matrices, _same  # noqa: F401
 
 pytestmark = pytest.mark.gpu
-
-
-@pytest.fixture(autouse=True)
-def _filter_on_small_matrices(monkeypatch):
-    monkeypatch.setenv("SVSB_FILTER_MIN_MB", "0")
-    monkeypatch.delenv("SVSB_FILTER", raising=False)
-
-
-def _same(a, b):
-    return (len(a[0]) == len(b[0]) and np.array_equal(a[0].view(np.uint32), b[0].view(np.uint32))
-            and np.array_equal(a[1], b[1]))
-
-
-def _both(monkeypatch, fn):
-    monkeypatch.setenv("SVSB_FILTER", "0")
-    ref = fn()
-    monkeypatch.setenv("SVSB_FILTER", "8")
-    got = fn()
-    monkeypatch.delenv("SVSB_FILTER")
-    return ref, got
-
-
-def _check_query(monkeypatch, e, q, k):
-    ref, got = _both(monkeypatch, lambda: e.query(q, k))
-    assert _same(ref, got), (k, ref[0][:5], got[0][:5])
-    return got
-
-
-def _check_bench(monkeypatch, e, qs, k):
-    """The device-resident loop (pipelined and serial): last answer and the route it took."""
-    e.bench_set_queries(qs)
-    for pipe in ("1", "0"):
-        monkeypatch.setenv("SVSB_PIPELINE", pipe)
-        res = []
-        for f in ("0", "8"):
-            monkeypatch.setenv("SVSB_FILTER", f)
-            e.bench_run(k, len(qs) + 1)
-            res.append(e.bench_last_result(k))
-            assert e.bench_filter_route() == int(f)
-            took, rescored = e.bench_filter_stats()
-            assert took == (f == "8")
-            if took:
-                assert rescored >= min(k, e.generation_rows()[1])
-        assert res[0] == res[1] and [np.float32(s).view(np.uint32) for s, _ in res[0]] == \
-            [np.float32(s).view(np.uint32) for s, _ in res[1]]
-    monkeypatch.delenv("SVSB_PIPELINE")
-    monkeypatch.delenv("SVSB_FILTER")
 
 
 @pytest.mark.parametrize("d", [64, 100, 762, 1536, 2000, 3072])
@@ -193,7 +148,7 @@ def test_filter8_submit_wait_three_in_flight(monkeypatch):
         assert all(_same(a, b) for a, b in zip(ref, got))
 
 
-def test_automatic_route_takes_int8_on_c2_like_shape(monkeypatch):
+def test_automatic_route_takes_int8_and_matches_k1_on_c2_like_shape(monkeypatch):
     n, d, k = 200_000, 1536, 100
     qs = oracle.synth_queries(4, d, 24)
     with svs_b200.Engine([0]) as e:
@@ -204,7 +159,8 @@ def test_automatic_route_takes_int8_on_c2_like_shape(monkeypatch):
         took, rescored = e.bench_filter_stats()
         assert took and k <= rescored < n // 10
         auto = e.bench_last_result(k)
-        monkeypatch.setenv("SVSB_FILTER", "16")
+        monkeypatch.setenv("SVSB_FILTER", "0")
         e.bench_run(k, 8)
-        assert e.bench_filter_route() == 16
-        assert e.bench_last_result(k) == auto
+        assert e.bench_filter_route() == 0
+        k1 = e.bench_last_result(k)
+        assert k1 == auto and _bits(k1) == _bits(auto)

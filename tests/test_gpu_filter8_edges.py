@@ -4,13 +4,13 @@ The pass copies each tile's row scales (and tombstone bytes) into shared memory 
 consumer warp scores two rows of a tile at once.  These cases put the last tile's row count off every multiple of 2, 4
 and 16, place tombstones in the partial last tile and on tile boundaries (32-row tiles at d = 1536, 16-row tiles at
 d = 3072), and append rows in place after the shadow exists, so their scales come in through the staged copy.  Each
-case compares SVSB_FILTER=0 (K1) with =8 as uint32 scores, ids and order, through `query` and the bench loop."""
+case compares SVSB_FILTER=0 (K1) with =1 as uint32 scores, ids and order, through `query` and the bench loop."""
 import numpy as np
 import pytest
 
 import svs_b200
 from _util import oracle
-from test_gpu_filter8 import _check_bench, _check_query, _filter_on_small_matrices  # noqa: F401  (autouse fixture)
+from test_gpu_filter import _check_bench, _check_query, _filter_on_small_matrices  # noqa: F401  (autouse fixture)
 
 pytestmark = pytest.mark.gpu
 

@@ -2,7 +2,7 @@
 
 The GPU suites compare every exact path with this reference bit for bit, so it must itself be right: its FMA against
 fractions.Fraction (random operands and constructed cases where a float64 product-sum rounded to fp32 rounds twice),
-its summation order against test_filter_bound.k1_scores on data where no double rounding can occur, and its
+its summation order against test_filter8_bound.k1_scores on data where no double rounding can occur, and its
 prefiltered top-k and top-pairs against emulating every row or pair."""
 import os
 import sys
@@ -12,7 +12,7 @@ import pytest
 
 sys.path.insert(0, os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "oracle"))
 import k1_exact as kx  # noqa: E402
-from test_filter_bound import k1_scores  # noqa: E402
+from test_filter8_bound import k1_scores  # noqa: E402
 
 F32 = np.float32
 
